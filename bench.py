@@ -2,6 +2,7 @@
 """bench.py - ViT images/sec (fwd + CE + bwd + AdamW) on the B200 attention hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 One process per GPU (torchrun sets RANK / LOCAL_RANK / WORLD_SIZE for N > 1).  Prints ONE JSON
 line on rank 0.  A "step" is the reference's training step (train.py:108-116: zero_grad -> forward
@@ -29,6 +30,7 @@ import torch.nn.functional as F
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # a benchmark run leaves the (possibly read-only) tree as it found it
 
 WORKLOADS = {
     # BASELINE.json configs[2]: the configuration the metric's "fused-attn % of tensor-core peak" and
@@ -77,7 +79,14 @@ def parse_args():
                     help="skip timing the reference's eager PyTorch path (oracle port) on the same GPU")
     ap.add_argument("--attn-impl", default="auto", choices=["auto", "simt", "tcgen05"])
     ap.add_argument("--no-graph", action="store_true", help="issue the training step eagerly instead of replaying a CUDA graph")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float32), for comparing builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the timed GPU path: it needs --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------ helpers
@@ -136,6 +145,34 @@ class ClockSampler:
         reasons = sorted({n for _, _, fl in self.samples for n, v in zip(self.NAMES, fl) if v.lower().startswith("active")})
         return {"sm_mhz": statistics.median(s[0] for s in self.samples), "sm_max_mhz": self.samples[0][1],
                 "reasons": reasons, "samples": len(self.samples)}
+
+
+DUMP_ELEMENTS = 8 << 20  # float32 elements in one --dump-outputs directory (32 MB)
+
+
+def dump_outputs(out_dir, train, model, runner, inf_runner):
+    """What a caller of the timed step holds after its last step, as ``out_dir/<name>.npy`` in float32.
+    Training: ``loss`` and every updated parameter as ``param.<name>``, a tensor larger than its even share
+    of DUMP_ELEMENTS as a fixed seeded sample of its elements (same positions in every run of a workload).
+    Inference: ``logits``.  The inputs are the same in every run; the training values are not bit-stable,
+    because some backward reductions sum in no fixed order (include/vrr.h) and every step builds on the last,
+    so compare two builds with a tolerance."""
+    import numpy as np
+    if train:
+        arrays = {"loss": runner.static_loss}
+        params = list(model.named_parameters())
+        share = DUMP_ELEMENTS // len(params)
+        g = torch.Generator().manual_seed(0)
+        for name, p in params:
+            flat = p.detach().reshape(-1)
+            if flat.numel() > share:
+                flat = flat[torch.randperm(flat.numel(), generator=g)[:share].sort().values.to(flat.device)]
+            arrays["param." + name] = flat
+    else:
+        arrays = {"logits": inf_runner.static_out}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def attn_algorithmic(model_cfg, tokens):
@@ -360,6 +397,8 @@ def main():
     else:
         gpu_launches = _lib.launch_count() - launches0
     ms_total = max_over_ranks(e0.elapsed_time(e1))
+    if args.dump_outputs and rank == 0:  # before the passes below step the model further
+        dump_outputs(args.dump_outputs, train, model, runner, inf_runner)
 
     # ---- per-launch kernel timing (CUDA events on the launching stream) -> `roofline`.  A graph replay has
     # no host-side launch sites, so the same K steps are issued eagerly once more with events around

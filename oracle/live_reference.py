@@ -1,9 +1,8 @@
 """Import the UNMODIFIED reference from ``/root/reference`` (build container only).
 
-TEST INFRASTRUCTURE ONLY (see ``oracle/__init__.py``).  ``/root/reference`` does
-not exist on the GPU box, so nothing marked ``gpu``, ``smoke()`` or ``bench.py``
-may call this; it is used by ``oracle/make_golden.py`` (fixture generation)
-and by the ``not gpu`` pinning tests, which skip when the directory is absent.
+TEST INFRASTRUCTURE ONLY (see ``oracle/__init__.py``).  Only ``oracle/make_golden.py``
+(fixture generation) calls this: the tests, ``smoke()`` and ``bench.py`` compare with
+the reference through the fixtures it wrote under ``tests/golden/``.
 """
 import importlib
 import os

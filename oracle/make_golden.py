@@ -118,12 +118,12 @@ def make_attention(vit, pe, mode, tag, shared=True):
     np.savez_compressed(os.path.join(GOLDEN, f"attn_{tag}.npz"), **out)
 
 
-def make_model(vit, mode, tag, shared=True):
-    kw = dict(img_size=16, patch_size=4, in_chans=3, num_classes=5, embed_dim=32, depth=2,
-              num_heads=2, pos_encoding=mode, rope_theta=100.0, poly_degree=3,
-              poly_shared_heads=shared)
+def seeded_model(ctor, kw, tag):
+    """``ctor(**kw)`` under the seed of ``model_<tag>.npz``, then perturbed in place.  Run with the
+    reference's ``VisionTransformer`` it makes the fixture's state_dict; run with the product's, the
+    same RNG order must give the same tensors (tests/test_host_api.py)."""
     torch.manual_seed(200 + len(tag))
-    model = vit.VisionTransformer(**kw)
+    model = ctor(**kw)
     with torch.no_grad():  # cls_token / biases are zero-initialised: perturb so their paths are live
         for name, p_ in model.named_parameters():
             if name == "cls_token" or name.endswith(".bias"):
@@ -132,6 +132,14 @@ def make_model(vit, mode, tag, shared=True):
                 p_.mul_(0.25)
             if name.endswith("relative_position_bias_table"):
                 p_.mul_(4.0)
+    return model
+
+
+def make_model(vit, mode, tag, shared=True):
+    kw = dict(img_size=16, patch_size=4, in_chans=3, num_classes=5, embed_dim=32, depth=2,
+              num_heads=2, pos_encoding=mode, rope_theta=100.0, poly_degree=3,
+              poly_shared_heads=shared)
+    model = seeded_model(vit.VisionTransformer, kw, tag)
     images = torch.randn(3, 3, 16, 16)
     labels = torch.tensor([1, 4, 0])
     logits = model(images)

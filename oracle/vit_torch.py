@@ -5,9 +5,8 @@ to ``/root/reference``.  The model is written functionally over a plain dict of
 tensors that uses the reference's ``state_dict`` key names (SURVEY.md row B3),
 so weights move between the reference, this oracle and the product model with
 ``state_dict()`` / ``load_state_dict()`` alone.  It issues the same torch ops in
-the same order as the reference's eager path, so on one machine and torch build
-it reproduces the reference bit for bit (checked in
-``tests/test_oracle_golden.py`` whenever ``/root/reference`` is mounted), and it
+the same order as the reference's eager path, so it reproduces the reference's
+stored outputs bit for bit (checked in ``tests/test_oracle_golden.py``), and it
 is what ``bench.py --impl reference`` and the ``cpu_baseline`` leg time.
 """
 import math

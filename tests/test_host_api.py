@@ -1,11 +1,12 @@
 """Host-side mirror of the reference module API (CPU: construction, tables, state_dict, errors)."""
+import ast
 import os
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import live_reference, tables_np as T
+from oracle import make_golden, tables_np as T
 from vit_rpe_rope_b200 import models
 from vit_rpe_rope_b200.models import positional_encoding as PE
 from vit_rpe_rope_b200.models.rope_utils import reshape_for_broadcast
@@ -143,21 +144,18 @@ def test_state_dict_contract_vs_golden(mode):
     assert n_pe == 0
 
 
-needs_ref = pytest.mark.skipif(not live_reference.available(), reason="/root/reference not mounted")
-
-
-@needs_ref
 @pytest.mark.parametrize("mode", MODES)
 def test_seeded_construction_matches_reference_bit_for_bit(mode):
-    """Same RNG consumption order as the reference constructor -> identical initial weights."""
-    vit, _, _ = live_reference.load()
-    torch.manual_seed(123)
-    ref = vit.VisionTransformer(pos_encoding=mode, embed_dim=96, depth=2, num_heads=3)
-    torch.manual_seed(123)
-    mine = VisionTransformer(pos_encoding=mode, embed_dim=96, depth=2, num_heads=3)
-    a, b = ref.state_dict(), mine.state_dict()
-    assert list(a.keys()) == list(b.keys())
-    for k in a:
-        assert torch.equal(a[k], b[k]), k
-    mine.load_state_dict(a, strict=True)
-    ref.load_state_dict(b, strict=True)
+    """Same RNG consumption order as the reference constructor -> identical initial weights.  The fixture's
+    state_dict is the reference's model built and perturbed by the same seeded recipe; the perturbation draws
+    in named_parameters() order, so that order must match the reference's too."""
+    tag = mode.replace("-", "_")
+    z = np.load(os.path.join(GOLDEN, f"model_{tag}.npz"))
+    kw = ast.literal_eval(str(z["kwargs"]))
+    mine = make_golden.seeded_model(VisionTransformer, kw, tag)
+    want = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd.")}
+    got = mine.state_dict()
+    assert list(got.keys()) == list(want.keys())
+    for k in want:
+        assert got[k].dtype == want[k].dtype and torch.equal(got[k], want[k]), k
+    mine.load_state_dict(want, strict=True)
