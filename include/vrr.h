@@ -199,7 +199,9 @@ int vrr_gemm(const void* a, const void* b, void* c, int M, int N, int K, int tra
  * bf16 operands with N % 8 == 0, K % 8 == 0 (and M % 8 == 0 when trans_a) and 16-byte aligned pointers run
  * the tcgen05 CTA-pair kernel (cta_group::2, TMA in, TMA store / reduce-add out; fp32 C is split over K and
  * combined by TMA reduce-add, so its summation order is not deterministic); everything else (fp32 operands,
- * odd shapes) runs the FFMA kernel.  vrr_set_impl() forces a family; vrr_family_count() reports it. */
+ * odd shapes, a pointer that is not 16-byte aligned, e.g. a view at an offset into a larger buffer) runs the
+ * FFMA kernel.  vrr_set_impl() forces a family (VRR_IMPL_TCGEN05 with a case the tcgen05 kernel cannot take:
+ * VRR_ERR_UNSUPPORTED); vrr_family_count() reports it.  The same dispatch applies to vrr_gemm_mul_colsum. */
 int vrr_gemm_ex(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K,
                 int trans_a, int trans_b, int dtype, int c_dtype, int epilogue, int accumulate, void* stream);
 

@@ -722,7 +722,7 @@ def test_attention_kernel_variants_agree(n):
 
 
 @pytest.mark.parametrize("rope", ["axial", "mixed"])
-@pytest.mark.parametrize("b,n,e,h", [(3, 197, 768, 12), (2, 50, 128, 2), (5, 65, 192, 3)])
+@pytest.mark.parametrize("b,n,e,h", [(3, 197, 768, 12), (2, 50, 128, 2), (5, 65, 192, 3), (32, 197, 768, 12)])
 def test_qkv_rope_packed_tables_bit_identical(rope, b, n, e, h):
     """vrr_rope_pack_tables + vrr_qkv_rope_fwd_packed (coalesced table reads in the tcgen05 epilogue) against
     vrr_qkv_rope_fwd on the same inputs: bit-identical planes; and the Python-side cache notices a table that changed
@@ -789,7 +789,7 @@ def test_long_sequence_forward_variants_vs_oracle(b, h, n):
         _set_option("attn_fwd_poly_exp", 2)
 
 
-@pytest.mark.parametrize("m,n,k", [(394, 3072, 768), (130, 104, 72), (1000, 256, 520)])
+@pytest.mark.parametrize("m,n,k", [(394, 3072, 768), (130, 104, 72), (1000, 256, 520), (6304, 3072, 768)])
 def test_gemm_epilogues_gelu_grad_and_mul(m, n, k):
     """VRR_EPI_BIAS_GELU_GRAD (c = gelu(h), c2 = gelu'(h), h = bf16(a.b^T + bias)) and VRR_EPI_MUL (c = (a.b) * c2),
     the pair that replaces the stand-alone GELU backward: against torch in fp32 on the bf16-rounded h."""

@@ -21,6 +21,10 @@
 //   warp 1        TMEM allocator (both CTAs) + MMA issuer (leader only); accumulators double-buffered
 //   warps 2..9    epilogue: tcgen05.ld -> registers -> (bias / GELU / RoPE) -> swizzled shared staging
 //                 -> TMA store / TMA reduce-add (fp32 split-K), or a direct mapped store (planes, tokens)
+//
+// The bias of the BIAS epilogue is rounded to bf16 before it is added for an fp32 C too (vrr.h: "cast to `dtype`
+// first"); the fp32-C path once added the unrounded fp32 value.  tests/test_kernels_at_scale.py pins both C types
+// bit for bit with biases off the bf16 grid.
 #include <string.h>
 
 #include "common.cuh"
@@ -136,7 +140,7 @@ struct PatchEmbedEpi2 {
 struct StoreEpi {
   static constexpr bool kTma = true;
   static constexpr bool kPlaneStore = false;
-  const float* bias;  // fp32 [N] or null; rounded to bf16 first when C is bf16 (autocast casts the bias)
+  const float* bias;  // fp32 [N] or null; rounded to bf16 first for either C type (autocast casts the bias)
   int out_f32;        // C element type: 0 bf16, 1 fp32
   int reduce;         // fp32 only: C += tile via TMA reduce-add (split-K partial sums / gradient accumulation)
   int gelu;           // bf16 only.  1: C = h = bf16(acc + bias), C2 = bf16(gelu(h)) (exact erf GELU);
@@ -152,6 +156,7 @@ struct StoreEpi {
 //   Phi(h) = 1 - erfc(|h| / sqrt 2) / 2 (h >= 0), erfc / 2 otherwise; erfc(z) = (a1 t + .. + a5 t^5) exp(-z^2),
 //   t = 1 / (1 + p z) (Abramowitz-Stegun 7.1.26, |error| <= 1.5e-7); gelu = h Phi, gelu' = Phi + h phi(h) with
 //   phi(h) = exp(-h^2 / 2) / sqrt(2 pi) - the same exponential.
+__device__ __forceinline__ float bf16_round(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
 __device__ __forceinline__ float rcp_approx(float x) {
   float y;
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -571,7 +576,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                 if (epi.bias != nullptr && first_split) {
                   const int nb = min(n0 + hb * 32 + c4 * 4, g.N - 4);
                   const float4 b0 = __ldg(reinterpret_cast<const float4*>(epi.bias + nb));
-                  x[0] += b0.x; x[1] += b0.y; x[2] += b0.z; x[3] += b0.w;
+                  x[0] += bf16_round(b0.x); x[1] += bf16_round(b0.y); x[2] += bf16_round(b0.z); x[3] += bf16_round(b0.w);
                 }
                 st_shared_v4(row_base + hb * 4096u + (((uint32_t)c4 ^ sw) << 4), __float_as_uint(x[0]), __float_as_uint(x[1]),
                              __float_as_uint(x[2]), __float_as_uint(x[3]));

@@ -99,6 +99,9 @@ bool first_use_on_device(std::atomic<unsigned char>* flags) {
 }
 
 static bool dtype_ok(int d) { return d == VRR_F32 || d == VRR_BF16; }
+static bool gemm_ptrs_aligned16(const void* a, const void* b, const void* c, const void* c2, const void* bias) {
+  return (((uintptr_t)a | (uintptr_t)b | (uintptr_t)c | (uintptr_t)c2 | (uintptr_t)bias) & 15) == 0;
+}
 static bool dh_ok(int dh) { return dh == 16 || dh == 32 || dh == 64; }
 
 static int check_bias(const vrr_bias_desc* b, int H, int N) {
@@ -318,13 +321,18 @@ int vrr_gemm_ex(const void* a, const void* b, void* c, void* c2, const float* bi
               "gemm_ex: the two-output GELU epilogues and MUL need `c2`");
   if (int rc = require_device()) return rc;
   const int impl = g_impl.load();
-  if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && gemm_bf16_tc_supported(M, N, K, trans_a, trans_b, c_dtype, epilogue)) {
+  // TMA needs 16-byte aligned base addresses: a view at an odd offset into a larger buffer runs the SIMT kernel
+  const bool uses_c2 = epilogue == VRR_EPI_BIAS_GELU || epilogue == VRR_EPI_BIAS_GELU_GRAD || epilogue == VRR_EPI_MUL;
+  const bool uses_bias = epilogue != VRR_EPI_NONE && epilogue != VRR_EPI_MUL;
+  const bool aligned = gemm_ptrs_aligned16(a, b, c, uses_c2 ? c2 : nullptr, uses_bias ? bias : nullptr);
+  if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && aligned &&
+      gemm_bf16_tc_supported(M, N, K, trans_a, trans_b, c_dtype, epilogue)) {
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
     return gemm_bf16_tc(a, b, c, c2, bias, M, N, K, trans_a, trans_b, c_dtype, epilogue, accumulate, (cudaStream_t)stream);
   }
   VRR_REQUIRE(impl != VRR_IMPL_TCGEN05 || dtype != VRR_BF16, VRR_ERR_UNSUPPORTED,
               "gemm_ex: tcgen05 kernel forced but M=%d N=%d K=%d (trans %d/%d) needs N %% 8 == 0, K %% 8 == 0 "
-              "(M %% 8 == 0 when trans_a)", M, N, K, trans_a, trans_b);
+              "(M %% 8 == 0 when trans_a) and 16-byte aligned pointers", M, N, K, trans_a, trans_b);
   VRR_REQUIRE(!accumulate, VRR_ERR_UNSUPPORTED, "gemm_ex: accumulate is implemented by the tcgen05 kernel only");
   VRR_COUNT_FAMILY(VRR_IMPL_SIMT);
   if (epilogue == VRR_EPI_MUL) {
@@ -351,7 +359,8 @@ int vrr_gemm_mul_colsum(const void* a, const void* b, void* c, const void* mul, 
   VRR_REQUIRE(dtype_ok(dtype), VRR_ERR_INVALID_ARG, "gemm_mul_colsum: bad dtype %d", dtype);
   if (int rc = require_device()) return rc;
   const int impl = g_impl.load();
-  if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && gemm_bf16_tc_supported(M, N, K, trans_a, trans_b, VRR_BF16, VRR_EPI_MUL)) {
+  if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && gemm_ptrs_aligned16(a, b, c, mul, nullptr) &&
+      gemm_bf16_tc_supported(M, N, K, trans_a, trans_b, VRR_BF16, VRR_EPI_MUL)) {
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
     VRR_CUDA(cudaMemsetAsync(col_sums, 0, (size_t)N * sizeof(float), (cudaStream_t)stream));
     return gemm_bf16_tc(a, b, c, const_cast<void*>(mul), nullptr, M, N, K, trans_a, trans_b, VRR_BF16, VRR_EPI_MUL, 0,
