@@ -255,7 +255,8 @@ int vrr_gemm_mul_colsum(const void* a, const void* b, void* c, const void* mul, 
                         int K, int trans_a, int trans_b, int dtype, void* stream);
 
 /* Bias gradient of a Linear layer (out-proj vit.py:91, Mlp fc1/fc2 vit.py:118, head vit.py:285):
- * out[c] = sum_m x[m][c], fp32 [C] (written); x [M][C] `dtype`, C % 4 == 0. */
+ * out[c] = sum_m x[m][c], fp32 [C] (written); x [M][C] `dtype`, C % 4 == 0, any element-aligned address (a view
+ * at an offset into a larger buffer takes an element-wise kernel). */
 int vrr_colsum(const void* x, float* out, int M, int C, int dtype, void* stream);
 /* Backward of the exact (erf) GELU between fc1 and fc2 of the Mlp (vit.py:118, act_layer=nn.GELU):
  * dh = dy * gelu'(h), written in `dtype`, and db[c] = sum_m dh[m][c] (fp32, written) - the fc1 bias

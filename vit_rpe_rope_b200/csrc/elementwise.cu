@@ -104,6 +104,27 @@ __global__ void __launch_bounds__(kCsThreads) colsum_kernel(const T* __restrict_
   }
 }
 
+// Any alignment (a view at an odd offset into a larger buffer): grid (ceil(C / 32), ceil(M / kCsRows)); thread = one
+// column x rows rl, rl + 8, ...; element loads, a warp reads 32 consecutive columns of a row.
+template <typename T>
+__global__ void __launch_bounds__(kCsThreads) colsum_scalar_kernel(const T* __restrict__ x, float* __restrict__ out, int M,
+                                                                   int C) {
+  __shared__ float part[8][32];
+  const int cl = threadIdx.x & 31, rl = threadIdx.x >> 5;
+  const int c = blockIdx.x * 32 + cl;
+  const int r0 = blockIdx.y * kCsRows, r1 = min(M, r0 + kCsRows);
+  float acc = 0.f;
+  if (c < C)
+    for (int r = r0 + rl; r < r1; r += 8) acc += Elem<T>::ld(x + (size_t)r * C + c);
+  part[rl][cl] = acc;
+  __syncthreads();
+  if (rl == 0 && c < C) {
+#pragma unroll
+    for (int k = 1; k < 8; ++k) acc += part[k][cl];
+    atomicAdd(out + c, acc);
+  }
+}
+
 __device__ __forceinline__ float gelu_grad(float h) {
   // d/dh [ 0.5 h (1 + erf(h / sqrt 2)) ] = Phi(h) + h * phi(h),  phi(h) = exp(-h^2/2) / sqrt(2 pi).
   // erf by Abramowitz-Stegun 7.1.26 (|error| <= 1.5e-7): erf(z) = 1 - (a1 t + .. + a5 t^5) exp(-z^2),
@@ -200,6 +221,15 @@ int colsum(const void* x, float* out, int M, int C, int dtype, cudaStream_t st) 
     dim3 grid(ceil_div(C, 16 * vec), ceil_div(M, kCsRows));
     if (dtype == VRR_F32) colsum_vec_kernel<float><<<grid, kCsThreads, 0, st>>>((const float*)x, out, M, C);
     else colsum_vec_kernel<__nv_bfloat16><<<grid, kCsThreads, 0, st>>>((const __nv_bfloat16*)x, out, M, C);
+    VRR_LAUNCHED();
+    return VRR_OK;
+  }
+  // colsum_kernel reads 4 elements at a time (16 bytes fp32, 8 bytes bf16): a base address off that grid takes the
+  // element-wise kernel
+  if (((uintptr_t)x & (dtype == VRR_F32 ? 15 : 7)) != 0) {
+    dim3 grid(ceil_div(C, 32), ceil_div(M, kCsRows));
+    if (dtype == VRR_F32) colsum_scalar_kernel<float><<<grid, kCsThreads, 0, st>>>((const float*)x, out, M, C);
+    else colsum_scalar_kernel<__nv_bfloat16><<<grid, kCsThreads, 0, st>>>((const __nv_bfloat16*)x, out, M, C);
     VRR_LAUNCHED();
     return VRR_OK;
   }

@@ -487,7 +487,6 @@ int vrr_add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new,
 int vrr_colsum(const void* x, float* out, int M, int C, int dtype, void* stream) {
   VRR_REQUIRE(x && out, VRR_ERR_INVALID_ARG, "colsum: NULL pointer");
   VRR_REQUIRE(dtype_ok(dtype) && M > 0 && C > 0, VRR_ERR_INVALID_ARG, "colsum: bad arguments");
-  VRR_REQUIRE(((uintptr_t)x & 15) == 0, VRR_ERR_INVALID_ARG, "colsum: x must be 16-byte aligned");
   if (int rc = require_device()) return rc;
   return colsum(x, out, M, C, dtype, (cudaStream_t)stream);
 }
