@@ -99,13 +99,10 @@ uint64_t vrr_launch_count(void);
  * took that family since load.  Lets a caller (and the parity tests) assert which family ran under
  * VRR_IMPL_AUTO instead of trusting the selection silently. */
 uint64_t vrr_family_count(int family);
-/* Tuning / experiment switches (process-wide): "attn_fwd_table_bulk" (0/1),
- * "attn_fwd_rescale_threshold_x100", "gemm_variant" (2 = CTA-pair kernels, default; 1 = 1-CTA kernels for the
- * QKV / patch-embed GEMMs, kept for A/B measurements), "attn_fwd_variant" (4, default: without bias the four-CTA-per-SM
- * kernel at every sequence length, with bias as 3; 3 = whole-sequence persistent kernel for N <= 256; 2 = one CTA per
- * 128-row tile always), "attn_bwd_variant" (3 = persistent kernel, default; 2 = two kernels), "attn_fwd_streams" (4 / 2
- * CTAs per SM in the tiled forward), "attn_fwd_poly_exp" (0..4 of every 8 exponential pairs by polynomial),
- * "ln_reg", "ln_bwd_minb", "simt_gemm_tile" - all kept for A/B measurements. */
+/* Tuning switches (process-wide), kept for A/B measurements: "ln_reg" (0 = generic multi-pass LayerNorm kernels only;
+ * the tests use them as the bit-exact reference for the register-resident ones), "ln_bwd_minb" (1 / 2 / 3: launch
+ * shape of the register-resident add+LayerNorm backward), "simt_gemm_tile" (128 / 64: tile of the fp32 FFMA GEMM).
+ * Any other name returns VRR_ERR_INVALID_ARG. */
 int vrr_set_option(const char* name, int value);
 /* Debug: CTA 0 of the next attention launches records clock64() phase stamps of its producer, issuer and
  * softmax roles into `device_buf` (1024 x int64, zero it first); NULL switches it off. */

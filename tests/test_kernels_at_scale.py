@@ -22,7 +22,7 @@ import torch
 import torch.nn.functional as F
 
 from oracle import tables_np as T
-from test_parity_gpu import _set_option, report, tcgen05_must_run
+from test_parity_gpu import report, tcgen05_must_run
 from vit_rpe_rope_b200 import _lib, ops
 
 pytestmark = pytest.mark.gpu
@@ -644,63 +644,52 @@ def test_attention_dispatch_boundaries(n, kind):
     _check_attention(kind, 2, 4, n, seed=n)
 
 
-def _batch_invariance(kind, b, h, n, variant=None):
+def _batch_invariance(kind, b, h, n):
     desc, param, _ = _bias_case(kind, h, n, seed=n)
     planes = _planes(b, h, n, seed=61)
     g = torch.Generator(device=DEV).manual_seed(62)
     d_out = (torch.randn(b, n, h * 64, generator=g, device=DEV) * 0.5).to(BF)
-    if variant is not None:
-        _set_option("attn_fwd_variant", variant)
-    try:
-        with tcgen05_must_run():
-            out, lse = _fwd(planes, desc)
-            d_planes, _ = _bwd(planes, desc, param, out, d_out, lse)
-            for img in (0, 1, b // 2, b - 1):
-                one = planes[:, img:img + 1].contiguous()
-                o1, l1 = _fwd(one, desc)
-                assert torch.equal(o1[0], out[img]) and torch.equal(l1[0], lse[img]), ("forward", img)
-                dp1, _ = _bwd(one, desc, param, out[img:img + 1].contiguous(), d_out[img:img + 1].contiguous(),
-                              lse[img:img + 1].contiguous())
-                assert torch.equal(dp1[:, 0], d_planes[:, img]), ("backward", img)
-    finally:
-        _set_option("attn_fwd_variant", 4)
+    with tcgen05_must_run():
+        out, lse = _fwd(planes, desc)
+        d_planes, _ = _bwd(planes, desc, param, out, d_out, lse)
+        for img in (0, 1, b // 2, b - 1):
+            one = planes[:, img:img + 1].contiguous()
+            o1, l1 = _fwd(one, desc)
+            assert torch.equal(o1[0], out[img]) and torch.equal(l1[0], lse[img]), ("forward", img)
+            dp1, _ = _bwd(one, desc, param, out[img:img + 1].contiguous(), d_out[img:img + 1].contiguous(),
+                          lse[img:img + 1].contiguous())
+            assert torch.equal(dp1[:, 0], d_planes[:, img]), ("backward", img)
 
 
-@pytest.mark.parametrize("kind,n,variant", [
-    ("table", 197, None),   # whole-sequence forward with a bias (attn_fwd_ws), two-kernel backward (attn_bwd_tc2)
-    ("poly", 197, None),
-    ("none", 197, None),    # four-CTA forward (attn_fwd_tc4), whole-sequence backward (attn_bwd_ws)
-    ("none", 197, 3),       # whole-sequence forward without bias
-    ("table", 257, None),   # tiled forward with a bias (attn_fwd_tc2), attn_bwd_tc2
+@pytest.mark.parametrize("kind,n", [
+    ("table", 197),   # whole-sequence forward with a bias (attn_fwd_ws), two-kernel backward (attn_bwd_tc2)
+    ("poly", 197),
+    ("none", 197),    # four-CTA forward (attn_fwd_tc4), whole-sequence backward (attn_bwd_ws)
+    ("table", 257),   # tiled forward with a bias (attn_fwd_tc2), attn_bwd_tc2
 ])
-def test_attention_batch_invariance_bitwise(kind, n, variant):
+def test_attention_batch_invariance_bitwise(kind, n):
     """Image b's out, lse and d_planes computed inside a batch of B*H >= 3 x SM items equal, bit for bit, the same
     image computed alone: the forward kernels and dQ / dK / dV have no atomics, so any difference is cross-item
     contamination (a stale buffer, a wrong item index) that no tolerance would catch."""
     h = 12
-    _batch_invariance(kind, -(-3 * _sms() // h), h, n, variant)
+    _batch_invariance(kind, -(-3 * _sms() // h), h, n)
 
 
-LSE_CASES = [  # (attn_fwd_variant, attn_fwd_streams, bias kind, N)
-    (4, 4, "none", 197), (4, 2, "none", 197), (4, 4, "none", 257), (4, 2, "none", 257),
-    (3, 4, "none", 197), (3, 4, "table", 197), (2, 4, "none", 197), (2, 4, "table", 197), (2, 4, "table", 257)]
+LSE_CASES = [  # (bias kind, N): each tcgen05 forward kernel through the default dispatch
+    ("none", 197), ("none", 257),     # attn_fwd_tc4_kernel
+    ("table", 197),                   # attn_fwd_ws_kernel
+    ("table", 257)]                   # attn_fwd_tc2_kernel
 
 
-@pytest.mark.parametrize("variant,streams,kind,n", LSE_CASES)
-def test_lse_every_tcgen05_forward(variant, streams, kind, n):
+@pytest.mark.parametrize("kind,n", LSE_CASES)
+def test_lse_every_tcgen05_forward(kind, n):
     """lse (natural log of sum exp of the scaled, biased logits, vrr.h) of every tcgen05 forward kernel, every row
     including those of the ragged last tile, against float64 logsumexp."""
     b, h = 3, 4
     desc, _, bias64 = _bias_case(kind, h, n, seed=5)
     planes = _planes(b, h, n, seed=71)
-    try:
-        _set_option("attn_fwd_variant", variant)
-        _set_option("attn_fwd_streams", streams)
-        with tcgen05_must_run():
-            out, lse = _fwd(planes, desc)
-    finally:
-        _set_option("attn_fwd_variant", 4)
-        _set_option("attn_fwd_streams", 4)
+    with tcgen05_must_run():
+        out, lse = _fwd(planes, desc)
     o, lse_ref = _ref(planes, bias64)
     e = ((lse.double() - lse_ref).abs() / lse_ref.abs().clamp_min(1.0)).max().item()
     assert e <= 1e-3, e

@@ -663,25 +663,22 @@ def _set_option(name, value):
 
 
 @pytest.mark.parametrize("b,h,n", [(30, 12, 197), (40, 8, 65), (2, 3, 130), (171, 2, 197)])
-def test_persistent_attention_many_items_per_cta(b, h, n):
-    """The whole-sequence kernels (attn_fwd_ws.cu / attn_bwd_ws.cu) are persistent: with more (image, head) items
-    than SMs every CTA walks several items through its double-buffered shared memory, TMEM and barrier phases.
-    fwd + bwd of ALL items against float64 numpy (rotating-buffer bugs only show from the second item on), and
-    bit-for-bit run-to-run reproducibility of the forward (no atomics on this path)."""
+def test_persistent_backward_many_items_per_cta(b, h, n):
+    """Without bias at N <= 208 the forward is attn_fwd_tc4_kernel (one CTA per 128-row tile, four per SM) and the
+    backward the persistent whole-sequence kernel (attn_bwd_ws.cu): with more (image, head) items than SMs every
+    backward CTA walks several items through its double-buffered shared memory, TMEM and barrier phases.
+    fwd + bwd of ALL items against float64 numpy, error checked per item (rotating-buffer bugs only show from the
+    second item on), and bit-for-bit run-to-run reproducibility of the forward (no atomics on this path)."""
     d = 64
     planes = _planes(b, h, n, d, torch.bfloat16, seed=21).to(DEV).requires_grad_(True)
     g = torch.Generator().manual_seed(22)
     d_out = (torch.randn(b, n, h * d, generator=g) * 0.5).to(torch.bfloat16)
     scale = d ** -0.5
-    _set_option("attn_fwd_variant", 3)  # the whole-sequence forward (the default without bias is the four-CTA kernel)
-    try:
-        with tcgen05_must_run():
-            out = ops.fused_attention(planes, scale)
-            out.backward(d_out.to(DEV))
-        out2 = ops.fused_attention(planes.detach(), scale)
-    finally:
-        _set_option("attn_fwd_variant", 4)
-    assert torch.equal(out, out2), "persistent forward is not reproducible run to run"
+    with tcgen05_must_run():
+        out = ops.fused_attention(planes, scale)
+        out.backward(d_out.to(DEV))
+    out2 = ops.fused_attention(planes.detach(), scale)
+    assert torch.equal(out, out2), "forward is not reproducible run to run"
     pl = planes.detach().double().cpu().numpy()
     o_np, _, _, _ = A.attention_forward(pl[0], pl[1], pl[2], scale, None)
     gr = A.attention_backward(d_out.double().numpy(), pl[0], pl[1], pl[2], scale, None, out=out.detach().double().cpu().numpy())
@@ -693,32 +690,6 @@ def test_persistent_attention_many_items_per_cta(b, h, n):
     per_item = np.abs(got - want).max(axis=(2, 3)) / np.maximum(np.abs(want).max(axis=(2, 3)), 1e-6)
     report(f"persistent attention b={b} h={h} n={n}: worst per-item grad err {per_item.max():.2e}")
     assert per_item.max() <= 2 * BF16_TOL, (np.unravel_index(per_item.argmax(), per_item.shape), per_item.max())
-
-
-@pytest.mark.parametrize("n", [65, 197])
-def test_attention_kernel_variants_agree(n):
-    """A/B switches (vrr_set_option): the whole-sequence kernels against variant 2 (one CTA per 128-row tile; two
-    backward kernels) on the same inputs - two independent schedules of the same math."""
-    b, h, d = 6, 12, 64
-    planes = _planes(b, h, n, d, torch.bfloat16, seed=31).to(DEV)
-    g = torch.Generator().manual_seed(32)
-    d_out = (torch.randn(b, n, h * d, generator=g) * 0.5).to(torch.bfloat16).to(DEV)
-    res = {}
-    try:
-        for variant in (4, 3, 2):
-            _set_option("attn_fwd_variant", variant)
-            _set_option("attn_bwd_variant", min(variant, 3))
-            pl = planes.clone().requires_grad_(True)
-            out = ops.fused_attention(pl, d ** -0.5)
-            out.backward(d_out)
-            res[variant] = (out.detach().float(), pl.grad.float())
-    finally:
-        _set_option("attn_fwd_variant", 4)
-        _set_option("attn_bwd_variant", 3)
-    assert err_rel(res[3][0], res[2][0].cpu().numpy()) <= 1e-2
-    assert err_rel(res[4][0], res[2][0].cpu().numpy()) <= 1e-2
-    assert err_rel(res[3][1], res[2][1].cpu().numpy()) <= BF16_TOL
-    assert err_rel(res[4][1], res[2][1].cpu().numpy()) <= BF16_TOL
 
 
 @pytest.mark.parametrize("rope", ["axial", "mixed"])
@@ -767,26 +738,19 @@ def test_qkv_rope_packed_tables_bit_identical(rope, b, n, e, h):
 
 
 @pytest.mark.parametrize("b,h,n", [(2, 3, 257), (1, 2, 577), (3, 2, 641), (1, 2, 1025)])
-def test_long_sequence_forward_variants_vs_oracle(b, h, n):
-    """N > 256 without bias: the four-CTAs-per-SM forward (single S buffer, chunked TMEM re-reads, a share of the
-    exponentials by polynomial on the FMA pipe) at polynomial shares 0, 2 (default) and 4 of 8, and the two-CTA
-    kernel, each against the float64 numpy oracle; ragged last key tile (n % 64 = 1) and ragged last row tile."""
+def test_long_sequence_forward_vs_oracle(b, h, n):
+    """N > 256 without bias: the four-CTAs-per-SM forward (single S buffer, chunked TMEM re-reads, 2 of every 8
+    exponential pairs by polynomial on the FMA pipe) against the float64 numpy oracle; ragged last key tile
+    (n % 64 = 1) and ragged last row tile."""
     d = 64
     planes = _planes(b, h, n, d, torch.bfloat16, seed=41).to(DEV)
     pl = planes.double().cpu().numpy()
     want, _, _, _ = A.attention_forward(pl[0], pl[1], pl[2], d ** -0.5, None)  # [B, N, H*D]
-    try:
-        for streams, poly in ((4, 0), (4, 2), (4, 4), (2, 2)):
-            _set_option("attn_fwd_streams", streams)
-            _set_option("attn_fwd_poly_exp", poly)
-            with tcgen05_must_run():
-                out = ops.fused_attention(planes, d ** -0.5)
-            e = err_rel(out.float(), want)
-            report(f"long forward b={b} h={h} n={n} streams={streams} poly={poly}: err {e:.2e}")
-            assert e <= 1e-2, (streams, poly, e)
-    finally:
-        _set_option("attn_fwd_streams", 4)
-        _set_option("attn_fwd_poly_exp", 2)
+    with tcgen05_must_run():
+        out = ops.fused_attention(planes, d ** -0.5)
+    e = err_rel(out.float(), want)
+    report(f"long forward b={b} h={h} n={n}: err {e:.2e}")
+    assert e <= 1e-2, e
 
 
 @pytest.mark.parametrize("m,n,k", [(394, 3072, 768), (130, 104, 72), (1000, 256, 520), (6304, 3072, 768)])

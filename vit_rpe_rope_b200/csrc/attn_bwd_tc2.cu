@@ -1,8 +1,8 @@
-// Fused attention backward, variant 2 (default): the forward kernel's pipeline applied to both
-// backward kernels - a dedicated issuer warp (TMA + every tcgen05.mma), 32-row streamed tiles,
-// double-buffered S / dP accumulators in TMEM so the issuer computes tile t+1 while the four
+// Fused attention backward for every case the whole-sequence kernel (attn_bwd_ws.cu) does not take: the bias modes
+// and N > 208.  Two kernels with the tiled forward's pipeline - a dedicated issuer warp (TMA + every tcgen05.mma),
+// 32-row streamed tiles, double-buffered S / dP accumulators in TMEM so the issuer computes tile t+1 while the four
 // row-owner warps work on tile t, dS / P written back in place (bf16) and consumed from TMEM by the
-// accumulating MMAs.  Math and operand forms are those of attn_bwd_tc.cu (variant 1, kept for A/B).
+// accumulating MMAs.
 //
 //  dQ kernel  (CTA = 128 query rows):  TMEM cols  S[2] 0..63 | dP[2] 64..127 | dQ 128..191
 //       S = Q K_t^T, dP = dO V_t^T  ->  thread: P = exp2(S*c + bias - lse), dS = P (dP - delta)
@@ -584,8 +584,8 @@ int attn_bwd_tc2(const void* planes, const vrr_bias_desc* bias, const void* out,
               VRR_ERR_INVALID_ARG, "attn_bwd (tcgen05): planes / out / d_out / d_planes must be 16-byte aligned");
   const int E = H * kDh;
   CUtensorMap tm_pl, tm_do;
-  if (int rc = make_tmap_bf16(&tm_pl, planes, (uint64_t)3 * B * H * N, kDh, kDh * 2, kT)) return rc;
-  if (int rc = make_tmap_bf16(&tm_do, d_out, (uint64_t)B * N, (uint64_t)E, (uint64_t)E * 2, kT)) return rc;
+  if (int rc = make_tmap_2d(&tm_pl, planes, 2, (uint64_t)3 * B * H * N, kDh, kDh * 2, kT, 64)) return rc;
+  if (int rc = make_tmap_2d(&tm_do, d_out, 2, (uint64_t)B * N, (uint64_t)E, (uint64_t)E * 2, kT, 64)) return rc;
   Bwd2Params p;
   p.out = (const __nv_bfloat16*)out;
   p.d_out = (const __nv_bfloat16*)d_out;

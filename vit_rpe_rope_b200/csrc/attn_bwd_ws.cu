@@ -2,7 +2,7 @@
 // persistent kernel: the whole-sequence variant.  Autograd of models/vit.py:71-88 of the reference (SURVEY row A18):
 //   P = softmax(S), dV = P^T dO, dP = dO V^T, dS = P o (dP - delta), dQ = scale dS K, dK = scale dS^T Q.
 //
-// Variant 2 (attn_bwd_tc2.cu) is two kernels (dQ; dK/dV) that each read Q, K, V, dO from HBM (1.44x the algorithmic
+// attn_bwd_tc2.cu is two kernels (dQ; dK/dV) that each read Q, K, V, dO from HBM (1.44x the algorithmic
 // traffic, measured) and walk the sequence in 32-row tiles: ten small tcgen05.mma, four mbarrier round trips and a
 // CTA prologue per tile.  Here
 //   * one CTA per SM loops over work items (image, head); Q, K, V, dO of the NEXT item are prefetched by TMA into the
@@ -23,12 +23,12 @@
 //     behind the accumulating MMAs that read the columns they overwrite;
 //   * delta = rowsum(dO o O) and lse*log2(e) of the NEXT item are computed by a helper warp into shared memory
 //     while the current item runs (rows past N get lse = +inf -> P = 0).
-// Bias modes (relative table / polynomial) stay on variant 2: a version of this kernel with the bias in the exponent
+// Bias modes (relative table / polynomial) stay on attn_bwd_tc2.cu: a version of this kernel with the bias in the exponent
 // of both orientations and the gradients taken in the dQ tiles (systolic diagonal sums into a shared histogram;
-// per-thread power sums) was built and was correct, but its per-element extras made it slower than variant 2
+// per-thread power sums) was built and was correct, but its per-element extras made it slower than attn_bwd_tc2.cu
 // (relative table 1 104 us against 856 us, polynomial 716 us against 627 us at ViT-B) - not kept.
 //
-// Measured alternatives (ViT-B/16-224, B = 256; this kernel: 303 us, variant 2: 399 us):
+// Measured alternatives (ViT-B/16-224, B = 256; this kernel: 303 us, attn_bwd_tc2.cu: 399 us):
 //   * one stream of all eight warps walking double-buffered 96-column groups with a TMA-store epilogue: 315 us - the
 //     S / dP waits disappear but twelve small groups per item cost as much in per-group overhead;
 //   * staging the outputs through 1 KB of shared memory per warp for coalesced stores: no gain (the 8-row rounds

@@ -1,5 +1,5 @@
-// Fused attention forward for SHORT sequences (N <= 256: the 65..197-token ViT configurations): the
-// whole-sequence variant.  Replaces models/vit.py:71-88 of the reference
+// Fused attention forward with a relative-table or polynomial bias for SHORT sequences (N <= 256: the 65..197-token
+// ViT configurations), the whole sequence resident per item.  Replaces models/vit.py:71-88 of the reference
 // (S = q k^T * scale (+ bias) -> softmax -> . v -> merge heads) without materialising S or P in HBM.
 //
 // Why a separate kernel.  clock64 timelines of the streaming kernel (attn_tc.cu, and of a persistent two-group
@@ -81,7 +81,7 @@ __device__ __forceinline__ void for_chunks(uint32_t t_s, int nch32, bool tail16,
   }
 }
 
-// pass 1: mask, scale + bias (bias modes; written back to TMEM for pass 2), row max
+// pass 1: mask, scale + bias (written back to TMEM for pass 2), row max
 template <int BIAS>
 struct Pass1 {
   const WsParams& p;
@@ -93,17 +93,6 @@ struct Pass1 {
   template <int W>
   __device__ __forceinline__ void run(uint32_t (&s)[W], int j0) {
     const bool full = j0 + W <= p.N;  // warp-uniform: only the last chunk has keys past the sequence
-    if (BIAS == VRR_BIAS_NONE) {
-      if (full) {
-#pragma unroll
-        for (int jl = 0; jl < W; ++jl) tm[jl & 3] = fmaxf(tm[jl & 3], __uint_as_float(s[jl]));
-      } else {
-#pragma unroll
-        for (int jl = 0; jl < W; ++jl)
-          tm[jl & 3] = fmaxf(tm[jl & 3], j0 + jl < p.N ? __uint_as_float(s[jl]) : -INFINITY);
-      }
-      return;
-    }
 #pragma unroll
     for (int jl = 0; jl < W; ++jl) {
       const int j = j0 + jl;
@@ -124,35 +113,21 @@ struct Pass1 {
   }
 };
 
-// pass 2: exponentials against the row max, row sum, P (bf16 pairs) written in place over S
-template <int BIAS>
+// pass 2: exponentials against the row max, row sum, P (bf16 pairs) written in place over S; masked keys hold -inf
+// from pass 1
 struct Pass2 {
-  const WsParams& p;
   uint32_t t_s;
   float neg_m;
   float ls[2];
   template <int W>
   __device__ __forceinline__ void run(const uint32_t (&s)[W], int j0) {
-    const bool full = BIAS != VRR_BIAS_NONE || j0 + W <= p.N;  // bias modes: masked keys hold -inf from pass 1
 #pragma unroll
     for (int q = 0; q < W / 16; ++q) {
       uint32_t packed[8];
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
         const int jl = q * 16 + 2 * e;
-        const float a0 = __uint_as_float(s[jl]), a1 = __uint_as_float(s[jl + 1]);
-        float p0, p1;
-        if (BIAS == VRR_BIAS_NONE) {
-          p0 = ex2(fmaf(a0, p.scale_log2, neg_m));
-          p1 = ex2(fmaf(a1, p.scale_log2, neg_m));
-          if (!full) {
-            p0 = j0 + jl < p.N ? p0 : 0.f;
-            p1 = j0 + jl + 1 < p.N ? p1 : 0.f;
-          }
-        } else {
-          p0 = ex2(a0 + neg_m);
-          p1 = ex2(a1 + neg_m);
-        }
+        const float p0 = ex2(__uint_as_float(s[jl]) + neg_m), p1 = ex2(__uint_as_float(s[jl + 1]) + neg_m);
         ls[0] += p0;
         ls[1] += p1;
         packed[e] = pack_bf16(p0, p1);
@@ -367,9 +342,8 @@ attn_fwd_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
         Pass1<BIAS> p1{p, tmem_row, i, yi, xi, lut, key_yx, {-INFINITY, -INFINITY, -INFINITY, -INFINITY}};
         for_chunks(tmem_row, nch32, tail16, p1);
         m_row = fmaxf(fmaxf(p1.tm[0], p1.tm[1]), fmaxf(p1.tm[2], p1.tm[3]));
-        if (BIAS == VRR_BIAS_NONE) m_row *= p.scale_log2;
-        else tmem_wait_st();
-        Pass2<BIAS> p2{p, tmem_row, -m_row, {0.f, 0.f}};
+        tmem_wait_st();
+        Pass2 p2{tmem_row, -m_row, {0.f, 0.f}};
         for_chunks(tmem_row, nch32, tail16, p2);
         l_row = p2.ls[0] + p2.ls[1];
         tmem_wait_st();
@@ -426,11 +400,11 @@ attn_fwd_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
 
 size_t ws_smem_bytes(int N, const vrr_bias_desc* bias, int* lut_floats, int* raw_floats) {
   int lf = 0, rf = 0;
-  const int mode = bias ? bias->mode : VRR_BIAS_NONE;
+  const int mode = bias->mode;
   if (mode == VRR_BIAS_TABLE) {
     lf = (2 * N - 1 + 3) & ~3;
     rf = (2 * N - 1 + 8 + 3) & ~3;  // + slack for the aligned span
-  } else if (mode == VRR_BIAS_POLY) {
+  } else {
     lf = (2 * bias->grid - 1 + 3) & ~3;
   }
   if (lut_floats) *lut_floats = lf;
@@ -451,9 +425,10 @@ int ws_launch(const CUtensorMap& tmap, const CUtensorMap& tmap_out, const WsPara
 }  // namespace
 
 bool attn_fwd_ws_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bias) {
+  if (!bias || bias->mode == VRR_BIAS_NONE) return false;  // attn_fwd_tc4_kernel is faster without bias
   if (Dh != kDh || N < 1 || N > 256) return false;
   if ((long long)3 * B * H * N >= (1ll << 31)) return false;
-  if (bias && bias->mode == VRR_BIAS_POLY && bias->grid > 255) return false;
+  if (bias->mode == VRR_BIAS_POLY && bias->grid > 255) return false;
   return ws_smem_bytes(N, bias, nullptr, nullptr) <= (size_t)kSmemMax;
 }
 
@@ -463,26 +438,25 @@ int attn_fwd_ws(const void* planes, const vrr_bias_desc* bias, void* out, float*
   VRR_REQUIRE(((uintptr_t)planes & 15) == 0 && ((uintptr_t)out & 15) == 0, VRR_ERR_INVALID_ARG,
               "attn_fwd (tcgen05): planes/out must be 16-byte aligned");
   CUtensorMap tmap, tmap_out;
-  if (int rc = make_tmap_bf16(&tmap, planes, (uint64_t)3 * B * H * N, kDh, kDh * 2, 64)) return rc;
+  if (int rc = make_tmap_2d(&tmap, planes, 2, (uint64_t)3 * B * H * N, kDh, kDh * 2, 64, 64)) return rc;
   const uint64_t E = (uint64_t)H * kDh;
   if (int rc = make_tmap_3d_bf16(&tmap_out, out, E, (uint64_t)N, (uint64_t)B, E * 2, (uint64_t)N * E * 2, kDh, 32)) return rc;
   WsParams p;
   p.lse = lse;
   p.B = B; p.H = H; p.N = N;
   p.scale_log2 = scale * kLog2e;
-  const int mode = bias ? bias->mode : VRR_BIAS_NONE;
-  p.bias_param = mode != VRR_BIAS_NONE ? bias->param : nullptr;
-  p.bias_heads = mode != VRR_BIAS_NONE ? bias->heads : 0;
-  p.bias_len = mode != VRR_BIAS_NONE ? bias->len : 0;
-  p.bias_grid = mode != VRR_BIAS_NONE ? bias->grid : 0;
+  const int mode = bias->mode;  // a bias: attn_fwd_ws_supported
+  p.bias_param = bias->param;
+  p.bias_heads = bias->heads;
+  p.bias_len = bias->len;
+  p.bias_grid = bias->grid;
   if (mode == VRR_BIAS_TABLE)
     VRR_REQUIRE(((uintptr_t)bias->param & 15) == 0, VRR_ERR_INVALID_ARG, "attn_fwd (tcgen05): bias table must be 16-byte aligned");
   p.total_items = B * H;
   const size_t smem = ws_smem_bytes(N, bias, &p.lut_floats, &p.raw_floats);
   const int grid = p.total_items < sm_count() ? p.total_items : sm_count();
   if (mode == VRR_BIAS_TABLE) return ws_launch<VRR_BIAS_TABLE>(tmap, tmap_out, p, grid, smem, st);
-  if (mode == VRR_BIAS_POLY) return ws_launch<VRR_BIAS_POLY>(tmap, tmap_out, p, grid, smem, st);
-  return ws_launch<VRR_BIAS_NONE>(tmap, tmap_out, p, grid, smem, st);
+  return ws_launch<VRR_BIAS_POLY>(tmap, tmap_out, p, grid, smem, st);
 }
 
 }  // namespace vrr

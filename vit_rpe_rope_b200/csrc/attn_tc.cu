@@ -1,24 +1,18 @@
-// Fused attention forward on the 5th-generation tensor cores (tcgen05 + TMEM), bf16, head dim 64.
+// Fused attention forward on the 5th-generation tensor cores (tcgen05 + TMEM), bf16, head dim 64, tiled over the
+// keys: every N without bias, and N > 256 with a bias (attn_fwd_ws.cu takes the shorter biased sequences).
 //
 // Replaces models/vit.py:71-88 of the reference: S = q k^T * scale (+ relative-position table /
 // polynomial bias) -> softmax -> . v -> merge heads, without materialising S or P in HBM.
 //
-// One CTA = 128 query rows of one (image, head); 128 threads, thread t owns query row t = TMEM lane t.
-//   * Q tile and 128-key K / V tiles arrive by TMA (cp.async.bulk.tensor, 128-byte swizzle) into a
-//     2-stage ring; for the 65..197-token ViT sequences the whole sequence is resident in shared
-//     memory after the prologue, longer sequences (577, 1025 tokens) stream through the ring.
-//   * S = Q K^T : tcgen05.mma kind::f16, both operands from shared memory, fp32 accumulator in
-//     TMEM columns [0,128).
-//   * softmax  : each thread pulls its row with tcgen05.ld, applies scale*log2e and the bias
-//     (table row staged into shared memory by a TMA bulk copy / polynomial evaluated into a
-//     distance LUT), keeps running max / sum (online softmax across key tiles), packs P to bf16
-//     and writes it back over S with tcgen05.st (columns [0,64)).
-//   * O_tile = P V : tcgen05.mma with A = P from TMEM and B = V from shared memory (MN-major),
-//     accumulator in TMEM columns [128,192); the thread folds it into its fp32 register accumulator
-//     with the online-softmax correction.
-//   * epilogue: O / l -> bf16 -> out[b][i][h*64 ..], lse.
-// 256 TMEM columns and ~85 KB shared memory per CTA -> two CTAs per SM, so one CTA's softmax
-// overlaps the other's TMA / MMA.
+// Both kernels: one CTA = 128 query rows of one (image, head), 160 threads - warps 0-3 softmax (thread t = query
+// row t = TMEM lane t), warp 4 the issuer of every TMA load and tcgen05.mma.  Q and 64-key K / V tiles arrive by
+// TMA (128-byte swizzle); S = Q K^T and O += P V (P from TMEM) accumulate in TMEM, O across all key tiles, with a
+// lazy online-softmax rescale; epilogue O / l -> bf16 -> out[b][i][h*64 ..], lse.
+//   * attn_fwd_tc4_kernel (no bias): one S buffer, 2-stage ring, 128 TMEM columns, ~50 KB of shared memory, four
+//     CTAs per SM;
+//   * attn_fwd_tc2_kernel (relative table / polynomial bias): double-buffered S, 4-stage ring, 256 TMEM columns,
+//     the bias row staged in shared memory (table row by a TMA bulk copy, polynomial as a distance LUT), two CTAs
+//     per SM.
 #include "common.cuh"
 #include "kernels.h"
 #include "tc_common.cuh"
@@ -43,13 +37,11 @@ struct FwdParams {
   float scale_log2;  // scale * log2(e)
   int bias_heads, bias_len, bias_grid;
   int lut_floats;    // shared-memory floats reserved for the LUT (incl. alignment slack)
-  int table_bulk;           // stage the relative table with a TMA bulk copy (1) or plain loads (0)
-  float rescale_threshold;  // lazy reference-max update threshold (log2 units)
   long long* dbg;    // optional phase timestamps (clock64) of one CTA, 8 per key tile; NULL in production
 };
 
 // =====================================================================================================
-// Variant 2 (default): a dedicated issuer warp, double-buffered S, O accumulated in TMEM.
+// attn_fwd_tc2_kernel (bias modes): a dedicated issuer warp, double-buffered S, O accumulated in TMEM.
 //   warps 0-3 : softmax, thread t = query row t = TMEM lane t
 //   warp 4    : issuer - TMA loads and every tcgen05.mma, descriptors kept warp-uniform
 // 64-key tiles.  TMEM: S/P buffer 0 = cols [0,64), buffer 1 = [64,128), O = [128,192).
@@ -133,7 +125,7 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
         mbar_expect_tx(&bar_vfull[s], kTileBytes);
         tma_load_2d(sV + s * kTileBytes, &tmap, &bar_vfull[s], 0, 2 * BHN + bh * N + s * kKT);
       }
-      if (BIAS == VRR_BIAS_TABLE && p.table_bulk) {
+      if (BIAS == VRR_BIAS_TABLE) {
         // TMA bulk copy of the head's table row (rows of 2N-1 floats are not 16-byte aligned in general:
         // copy the enclosing aligned span that stays inside the table; the softmax warps patch the tail)
         const size_t row_b = (size_t)h * p.bias_len * 4, row_e = row_b + (size_t)p.bias_len * 4;
@@ -240,11 +232,11 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
       const size_t a0 = row_b & ~size_t(15);
       size_t a1 = (row_e + 15) & ~size_t(15);
       if (a1 > (tot & ~size_t(15))) a1 = tot & ~size_t(15);
-      const int have = (p.table_bulk && a1 > row_b) ? (int)((a1 - row_b) / 4) : 0;  // elements the bulk copy delivered
+      const int have = a1 > row_b ? (int)((a1 - row_b) / 4) : 0;  // elements the bulk copy delivered
       float* lw = lut_raw + (row_b - a0) / 4;
       lut = lw;
       const float* grow = p.bias_param + (size_t)h * p.bias_len;
-      if (p.table_bulk) mbar_wait(bar_lut, 0);
+      mbar_wait(bar_lut, 0);
       for (int t = tid; t < p.bias_len; t += 128) lw[t] = (t < have ? lw[t] : grow[t]) * kLog2e;
       asm volatile("bar.sync 1, 128;" ::: "memory");
     } else if (BIAS == VRR_BIAS_POLY) {
@@ -292,26 +284,21 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
 #pragma unroll
         for (int jl = 0; jl < kKT; ++jl) {
           const int j = t * kKT + jl;
-          if (BIAS == VRR_BIAS_NONE) {
-            tmax = fmaxf(tmax, __uint_as_float(sraw[jl]));
+          float bsv;
+          if (BIAS == VRR_BIAS_TABLE) {
+            bsv = lut[min(max(i - j + N - 1, 0), 2 * N - 2)];
           } else {
-            float bsv;
-            if (BIAS == VRR_BIAS_TABLE) {
-              bsv = lut[min(max(i - j + N - 1, 0), 2 * N - 2)];
-            } else {
-              const int yx = key_yx[min(j, N - 1)];
-              const int dist = abs(yi - (yx >> 8)) + abs(xi - (yx & 255));
-              bsv = (i == 0 || j == 0) ? 0.f : lut[dist];
-            }
-            const float v = fmaf(__uint_as_float(sraw[jl]), p.scale_log2, bsv);
-            sraw[jl] = __float_as_uint(v);
-            tmax = fmaxf(tmax, v);
+            const int yx = key_yx[min(j, N - 1)];
+            const int dist = abs(yi - (yx >> 8)) + abs(xi - (yx & 255));
+            bsv = (i == 0 || j == 0) ? 0.f : lut[dist];
           }
+          const float v = fmaf(__uint_as_float(sraw[jl]), p.scale_log2, bsv);
+          sraw[jl] = __float_as_uint(v);
+          tmax = fmaxf(tmax, v);
         }
-        if (BIAS == VRR_BIAS_NONE) tmax *= p.scale_log2;
         if (dbg_on) dbg[3] = clock64();
         // reference-max update: warp-uniform decision (tcgen05.ld/st are warp-collective)
-        const bool jump = tmax > m_ref + p.rescale_threshold;
+        const bool jump = tmax > m_ref + kRescaleThreshold;
         if (__any_sync(0xffffffffu, jump)) {
           const float m_new = fmaxf(m_ref, tmax);
           if (t > 0) {
@@ -340,8 +327,8 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
 #pragma unroll
           for (int e = 0; e < 16; ++e) {
             const float a0 = __uint_as_float(sraw[c * 32 + 2 * e]), a1 = __uint_as_float(sraw[c * 32 + 2 * e + 1]);
-            const float p0 = BIAS == VRR_BIAS_NONE ? ex2(fmaf(a0, p.scale_log2, neg_m)) : ex2(a0 + neg_m);
-            const float p1 = BIAS == VRR_BIAS_NONE ? ex2(fmaf(a1, p.scale_log2, neg_m)) : ex2(a1 + neg_m);
+            const float p0 = ex2(a0 + neg_m);
+            const float p1 = ex2(a1 + neg_m);
             l_run += p0 + p1;
             packed[e] = pack_bf16(p0, p1);
           }
@@ -386,9 +373,9 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
 }
 
 // =====================================================================================================
-// Variant 4 (default for N > 256 without bias): the same tile loop with HALF the on-chip footprint per CTA and four
-// CTAs per SM.  Variant 2 at 1025 tokens runs at ~45 % of the exponential (MUFU) roof: with two CTAs per SM a
-// scheduler holds two softmax warps, and each of them spends about half of a tile waiting (S barrier, tcgen05.ld,
+// attn_fwd_tc4_kernel (no bias, every N): the same tile loop with HALF the on-chip footprint per CTA and four CTAs
+// per SM.  attn_fwd_tc2_kernel's layout at 1025 tokens runs at ~45 % of the exponential (MUFU) roof: with two CTAs
+// per SM a scheduler holds two softmax warps, and each of them spends about half of a tile waiting (S barrier, tcgen05.ld,
 // tcgen05.st, P barrier).  Here a CTA keeps ONE S buffer (P written in place, the next S issued right behind the PV
 // MMA that reads it - the tensor pipe executes in issue order), a 2-stage K / V ring and 128 TMEM columns (S/P
 // [0,64), O [64,128)), so four CTAs = four independent streams share an SM: a stream's barrier and tensor-pipe
@@ -398,6 +385,9 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
 constexpr int kV4Stages = 2, kV4Threads = 160;
 constexpr uint32_t kV4TmemCols = 128, kV4ColO = 64;
 constexpr int kV4NumBars = 4 * kV4Stages + 4;
+// pairs out of every 8 whose exponential takes the FMA-pipe polynomial (tc::ex2_poly2) instead of MUFU.EX2; of the
+// shares 0..4, 2 was the fastest at 577 and 1025 tokens (profiles/r2_attn_long_probe.txt)
+constexpr int kPolyPairs = 2;
 
 __device__ __forceinline__ float v4_max16(const uint32_t (&r)[16], float mx) {
 #pragma unroll
@@ -415,16 +405,16 @@ __device__ __forceinline__ float v4_max16m(const uint32_t (&r)[16], float mx, in
     return mx;
   }
 }
-// P = 2^(s * scale - m) for 16 scores -> 8 packed bf16x2; the row sum accumulates in l2.  POLY of the 8 pairs take
-// the polynomial, the others MUFU.EX2.
-template <bool FULL, int POLY>
+// P = 2^(s * scale - m) for 16 scores -> 8 packed bf16x2; the row sum accumulates in l2.  kPolyPairs of the 8 pairs
+// take the polynomial, the others MUFU.EX2.
+template <bool FULL>
 __device__ __forceinline__ void v4_exp16(const uint32_t (&r)[16], uint32_t (&pk)[8], float2 sc2, float2 nm2, float2& l2,
                                          int first, int nvalid) {
 #pragma unroll
   for (int e = 0; e < 8; ++e) {
     const float2 x = __ffma2_rn(make_float2(__uint_as_float(r[2 * e]), __uint_as_float(r[2 * e + 1])), sc2, nm2);
-    // spread the polynomial pairs between the MUFU ones: e * POLY / 8 steps at the chosen pairs
-    const bool poly = ((e + 1) * POLY) / 8 != (e * POLY) / 8;
+    // spread the polynomial pairs between the MUFU ones: e * kPolyPairs / 8 steps at the chosen pairs
+    const bool poly = ((e + 1) * kPolyPairs) / 8 != (e * kPolyPairs) / 8;
     float2 pv = poly ? ex2_poly2(x) : make_float2(ex2(x.x), ex2(x.y));
     if (!FULL) {
       if (first + 2 * e >= nvalid) pv.x = 0.f;
@@ -436,9 +426,8 @@ __device__ __forceinline__ void v4_exp16(const uint32_t (&r)[16], uint32_t (&pk)
 }
 
 // one key tile of one query row: lazy reference-max update, then P over the first 32 of the 64 columns S occupied
-template <bool FULL, int POLY>
-__device__ __forceinline__ void v4_tile(uint32_t trow, int nvalid, int t, float scale_log2, float thr, float& m_ref,
-                                        float& l_run) {
+template <bool FULL>
+__device__ __forceinline__ void v4_tile(uint32_t trow, int nvalid, int t, float scale_log2, float& m_ref, float& l_run) {
   uint32_t ab[32];
   uint32_t(&a)[16] = *reinterpret_cast<uint32_t(*)[16]>(&ab[0]);
   uint32_t(&b)[16] = *reinterpret_cast<uint32_t(*)[16]>(&ab[16]);
@@ -465,7 +454,7 @@ __device__ __forceinline__ void v4_tile(uint32_t trow, int nvalid, int t, float 
   }
   tmax *= scale_log2;
   tmem_ld16(trow, a);  // first chunk of pass 2
-  const bool jump = tmax > m_ref + thr;
+  const bool jump = tmax > m_ref + kRescaleThreshold;
   if (__any_sync(0xffffffffu, jump)) {
     const float m_new = fmaxf(m_ref, tmax);
     if (t > 0) {
@@ -491,24 +480,24 @@ __device__ __forceinline__ void v4_tile(uint32_t trow, int nvalid, int t, float 
   if (FULL) {
     tmem_wait_ld();
     tmem_ld16(trow + 16, b);
-    v4_exp16<true, POLY>(a, pk, sc2, nm2, l2, 0, nvalid);
+    v4_exp16<true>(a, pk, sc2, nm2, l2, 0, nvalid);
     tmem_st8(trow, pk);  // columns [0,8): scores already consumed
     tmem_wait_ld();
     tmem_ld16(trow + 32, a);
-    v4_exp16<true, POLY>(b, pk, sc2, nm2, l2, 16, nvalid);
+    v4_exp16<true>(b, pk, sc2, nm2, l2, 16, nvalid);
     tmem_st8(trow + 8, pk);
     tmem_wait_ld();
     tmem_ld16(trow + 48, b);
-    v4_exp16<true, POLY>(a, pk, sc2, nm2, l2, 32, nvalid);
+    v4_exp16<true>(a, pk, sc2, nm2, l2, 32, nvalid);
     tmem_st8(trow + 16, pk);
     tmem_wait_ld();
-    v4_exp16<true, POLY>(b, pk, sc2, nm2, l2, 48, nvalid);
+    v4_exp16<true>(b, pk, sc2, nm2, l2, 48, nvalid);
     tmem_st8(trow + 24, pk);
   } else {
     for (int c = 0; c < nchunks; ++c) {
       if (c > 0) tmem_ld16(trow + c * 16, a);
       tmem_wait_ld();
-      v4_exp16<false, POLY>(a, pk, sc2, nm2, l2, c * 16, nvalid);
+      v4_exp16<false>(a, pk, sc2, nm2, l2, c * 16, nvalid);
       tmem_st8(trow + c * 8, pk);  // columns [8c, 8c+8) lie below every chunk still to be read
     }
   }
@@ -516,7 +505,6 @@ __device__ __forceinline__ void v4_tile(uint32_t trow, int nvalid, int t, float 
   tmem_wait_st();
 }
 
-template <int POLY>
 __global__ void __launch_bounds__(kV4Threads, 4)
 attn_fwd_tc4_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p) {
   constexpr int kKT = kV2KT, kStages = kV4Stages;
@@ -658,8 +646,8 @@ attn_fwd_tc4_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
       mbar_wait(bar_s, (uint32_t)(t & 1));
       tc_fence_after();
       if (warp_active) {
-        if (nvalid == kKT) v4_tile<true, POLY>(tmem_row, nvalid, t, p.scale_log2, p.rescale_threshold, m_ref, l_run);
-        else v4_tile<false, POLY>(tmem_row, nvalid, t, p.scale_log2, p.rescale_threshold, m_ref, l_run);
+        if (nvalid == kKT) v4_tile<true>(tmem_row, nvalid, t, p.scale_log2, m_ref, l_run);
+        else v4_tile<false>(tmem_row, nvalid, t, p.scale_log2, m_ref, l_run);
       }
       tc_fence_before();
       __syncwarp();
@@ -709,10 +697,6 @@ size_t fwd2_smem_bytes(int N, const vrr_bias_desc* bias, int* lut_floats) {
   return 1024 + (size_t)kQBytes + (size_t)2 * kV2Stages * kV2KT * kDh * 2 + (size_t)lf * 4 + yx + (size_t)kV2NumBars * 8 + 16;
 }
 
-std::atomic<int> g_fwd_table_bulk{1};
-std::atomic<int> g_fwd_poly{2};     // pairs out of 8 whose exponential the 4-CTA kernel computes by polynomial (0..4)
-std::atomic<int> g_fwd_streams{4};  // 4: attn_fwd_tc4_kernel (four CTAs per SM); 2: attn_fwd_tc2_kernel
-std::atomic<int> g_fwd_thresh_x100{(int)(kRescaleThreshold * 100)};
 std::atomic<long long*> g_fwd_dbg{nullptr};
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -720,10 +704,8 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 EncodeTiledFn g_encode = nullptr;
 
-}  // namespace
-
-int make_tmap_bf16(CUtensorMap* map, const void* base, uint64_t rows, uint64_t cols, uint64_t row_stride_bytes,
-                   uint32_t box_rows) {
+// cuTensorMapEncodeTiled through the runtime's driver entry point (no link against libcuda), looked up once
+int encode_tiled(EncodeTiledFn* fn_out) {
   if (!g_encode) {
     void* fn = nullptr;
     cudaDriverEntryPointQueryResult qres;
@@ -731,33 +713,23 @@ int make_tmap_bf16(CUtensorMap* map, const void* base, uint64_t rows, uint64_t c
     VRR_REQUIRE(fn && qres == cudaDriverEntryPointSuccess, VRR_ERR_CUDA, "cuTensorMapEncodeTiled not available");
     g_encode = reinterpret_cast<EncodeTiledFn>(fn);
   }
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {row_stride_bytes};
-  cuuint32_t box[2] = {64, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = g_encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  VRR_REQUIRE(r == CUDA_SUCCESS, VRR_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
+  *fn_out = g_encode;
   return VRR_OK;
 }
 
+}  // namespace
+
 int make_tmap_2d(CUtensorMap* map, const void* base, int elem_bytes, uint64_t rows, uint64_t cols,
                  uint64_t row_stride_bytes, uint32_t box_rows, uint32_t box_cols) {
-  if (!g_encode) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    VRR_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-    VRR_REQUIRE(fn && qres == cudaDriverEntryPointSuccess, VRR_ERR_CUDA, "cuTensorMapEncodeTiled not available");
-    g_encode = reinterpret_cast<EncodeTiledFn>(fn);
-  }
+  EncodeTiledFn encode;
+  if (int rc = encode_tiled(&encode)) return rc;
   cuuint64_t dims[2] = {cols, rows};
   cuuint64_t strides[1] = {row_stride_bytes};
   cuuint32_t box[2] = {box_cols, box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = g_encode(map, elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2,
-                        const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  CUresult r = encode(map, elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2,
+                      const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   VRR_REQUIRE(r == CUDA_SUCCESS, VRR_ERR_CUDA,
               "cuTensorMapEncodeTiled failed with CUresult %d (rows %llu cols %llu stride %llu box %ux%u)", (int)r,
               (unsigned long long)rows, (unsigned long long)cols, (unsigned long long)row_stride_bytes, box_rows, box_cols);
@@ -766,20 +738,15 @@ int make_tmap_2d(CUtensorMap* map, const void* base, int elem_bytes, uint64_t ro
 
 int make_tmap_3d_bf16(CUtensorMap* map, const void* base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t stride1_bytes,
                       uint64_t stride2_bytes, uint32_t box0, uint32_t box1, int swizzle128) {
-  if (!g_encode) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    VRR_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-    VRR_REQUIRE(fn && qres == cudaDriverEntryPointSuccess, VRR_ERR_CUDA, "cuTensorMapEncodeTiled not available");
-    g_encode = reinterpret_cast<EncodeTiledFn>(fn);
-  }
+  EncodeTiledFn encode;
+  if (int rc = encode_tiled(&encode)) return rc;
   cuuint64_t dims[3] = {d0, d1, d2};
   cuuint64_t strides[2] = {stride1_bytes, stride2_bytes};
   cuuint32_t box[3] = {box0, box1, 1};
   cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = g_encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE,
-                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
+                      CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE,
+                      CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   VRR_REQUIRE(r == CUDA_SUCCESS, VRR_ERR_CUDA, "cuTensorMapEncodeTiled (3-D) failed with CUresult %d", (int)r);
   return VRR_OK;
 }
@@ -792,10 +759,6 @@ bool attn_fwd_tc_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bia
 }
 
 void attn_fwd_tc_set_debug(long long* buf) { g_fwd_dbg.store(buf); }
-void attn_fwd_tc_set_threshold_x100(int v) { g_fwd_thresh_x100.store(v); }
-void attn_fwd_tc_set_table_bulk(int v) { g_fwd_table_bulk.store(v); }
-void attn_fwd_tc_set_streams(int v) { g_fwd_streams.store(v == 2 ? 2 : 4); }
-void attn_fwd_tc_set_poly(int v) { g_fwd_poly.store(v < 0 ? 0 : (v > 4 ? 4 : v)); }
 
 template <int MODE>
 static int fwd2_launch_tc(const CUtensorMap& tmap, const FwdParams& p, dim3 grid, size_t smem, cudaStream_t st) {
@@ -811,15 +774,13 @@ int attn_fwd_tc(const void* planes, const vrr_bias_desc* bias, void* out, float*
   VRR_REQUIRE(((uintptr_t)planes & 15) == 0 && ((uintptr_t)out & 15) == 0, VRR_ERR_INVALID_ARG,
               "attn_fwd (tcgen05): planes/out must be 16-byte aligned");
   CUtensorMap tmap;
-  if (int rc = make_tmap_bf16(&tmap, planes, (uint64_t)3 * B * H * N, kDh, kDh * 2, kV2KT)) return rc;
+  if (int rc = make_tmap_2d(&tmap, planes, 2, (uint64_t)3 * B * H * N, kDh, kDh * 2, kV2KT, 64)) return rc;
   FwdParams p;
   p.out = (__nv_bfloat16*)out;
   p.lse = lse;
   p.B = B; p.H = H; p.N = N;
   p.scale_log2 = scale * kLog2e;
   p.dbg = g_fwd_dbg.load();
-  p.rescale_threshold = g_fwd_thresh_x100.load() * 0.01f;
-  p.table_bulk = g_fwd_table_bulk.load();
   const int mode = bias ? bias->mode : VRR_BIAS_NONE;
   p.bias_param = mode != VRR_BIAS_NONE ? bias->param : nullptr;
   p.bias_heads = mode != VRR_BIAS_NONE ? bias->heads : 0;
@@ -828,29 +789,18 @@ int attn_fwd_tc(const void* planes, const vrr_bias_desc* bias, void* out, float*
   if (mode == VRR_BIAS_TABLE)
     VRR_REQUIRE(((uintptr_t)bias->param & 15) == 0, VRR_ERR_INVALID_ARG, "attn_fwd (tcgen05): bias table must be 16-byte aligned");
   dim3 grid(ceil_div(N, kM), B * H);
-  if (g_fwd_streams.load() == 4 && mode == VRR_BIAS_NONE) {
-    // the bias modes stay on variant 2: evaluating the bias in both passes made the 4-CTA kernel slower there
-    // (577 tokens: table 118 vs 82 us, polynomial 175 vs 108 us)
+  if (mode == VRR_BIAS_NONE) {
+    // the bias modes stay on attn_fwd_tc2_kernel: evaluating the bias in both passes made the four-CTA kernel slower
+    // there (577 tokens: table 118 vs 82 us, polynomial 175 vs 108 us)
     p.lut_floats = 0;
-    switch (g_fwd_poly.load()) {
-#define VRR_FWD4(P)                                                              \
-  case P:                                                                        \
-    VRR_SMEM_ATTR_ONCE(attn_fwd_tc4_kernel<P>, 64 * 1024);                       \
-    attn_fwd_tc4_kernel<P><<<grid, kV4Threads, kFwd4SmemBytes, st>>>(tmap, p);   \
-    break;
-      VRR_FWD4(0) VRR_FWD4(1) VRR_FWD4(2) VRR_FWD4(3) VRR_FWD4(4)
-#undef VRR_FWD4
-      default:
-        VRR_SMEM_ATTR_ONCE(attn_fwd_tc4_kernel<2>, 64 * 1024);
-        attn_fwd_tc4_kernel<2><<<grid, kV4Threads, kFwd4SmemBytes, st>>>(tmap, p);
-    }
+    VRR_SMEM_ATTR_ONCE(attn_fwd_tc4_kernel, 64 * 1024);
+    attn_fwd_tc4_kernel<<<grid, kV4Threads, kFwd4SmemBytes, st>>>(tmap, p);
     VRR_LAUNCHED();
     return VRR_OK;
   }
   const size_t smem2 = fwd2_smem_bytes(N, bias, &p.lut_floats);
   if (mode == VRR_BIAS_TABLE) return fwd2_launch_tc<VRR_BIAS_TABLE>(tmap, p, grid, smem2, st);
-  if (mode == VRR_BIAS_POLY) return fwd2_launch_tc<VRR_BIAS_POLY>(tmap, p, grid, smem2, st);
-  return fwd2_launch_tc<VRR_BIAS_NONE>(tmap, p, grid, smem2, st);
+  return fwd2_launch_tc<VRR_BIAS_POLY>(tmap, p, grid, smem2, st);
 }
 
 }  // namespace vrr

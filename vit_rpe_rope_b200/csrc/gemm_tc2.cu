@@ -701,12 +701,25 @@ int launch_store(const void* a, const void* b, void* c, void* c2, const float* b
   return launch_pair<128, A_MN, B_MN, StoreEpi>(a, b, M, N, K, splits, tc_, tc2_, epi, st);
 }
 
-std::atomic<int> g_gemm_variant{2};
+// unfold(images)[m][k], m = b*Np + py*gw + px, k = c*P*P + i*P + j  ->  bf16; 8 consecutive j per thread
+template <typename TI>
+__global__ void patch_unfold_kernel(const TI* __restrict__ img, __nv_bfloat16* __restrict__ out, int B, int C, int Hi,
+                                    int Wi, int P, int gw, int Np) {
+  const int K8 = C * P * P / 8;
+  const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (size_t)B * Np * K8) return;
+  const int k8 = (int)(idx % K8);
+  const size_t m = idx / K8;
+  const int b = (int)(m / Np), p = (int)(m - (size_t)b * Np), py = p / gw, px = p - py * gw;
+  const int k = k8 * 8, c = k / (P * P), r = k - c * P * P, i = r / P, j = r - i * P;
+  const TI* src = img + (((size_t)b * C + c) * Hi + (py * P + i)) * Wi + (px * P + j);
+  float4 lo = ld4(src), hi = ld4(src + 4);
+  __nv_bfloat16* dst = out + m * (size_t)(K8 * 8) + k;
+  st4(dst, lo);
+  st4(dst + 4, hi);
+}
 
 }  // namespace
-
-void gemm_tc_set_variant(int v) { g_gemm_variant.store(v == 1 ? 1 : 2); }
-int gemm_tc_variant() { return g_gemm_variant.load(); }
 
 // bf16 operands; TMA needs 16-byte row strides: the CONTIGUOUS dimension of every operand and of C must be a
 // multiple of 8 elements (4 for an fp32 C); the other dimensions are free (ragged tiles are zero-filled / clipped).
@@ -743,6 +756,12 @@ int gemm_bf16_tc(const void* a, const void* b, void* c, void* c2, const float* b
 }
 
 // ---- QKV projection + RoPE epilogue on the CTA-pair kernel -----------------------------------------------
+bool qkv_rope_fwd_tc_supported(int B, int N, int E, int H) {
+  if (H <= 0 || E % H != 0 || E / H != 64) return false;
+  if ((long long)B * N >= (1ll << 31) / 4) return false;
+  return true;
+}
+
 int qkv_rope_fwd_tc2(const void* x, const void* w, const float* cos_tab, const float* sin_tab, const float* packed,
                      void* planes, int B, int N, int E, int H, int rope_mode, cudaStream_t st) {
   VRR_REQUIRE(((uintptr_t)x & 15) == 0 && ((uintptr_t)w & 15) == 0 && ((uintptr_t)planes & 15) == 0,
@@ -759,19 +778,47 @@ int qkv_rope_fwd_tc2(const void* x, const void* w, const float* cos_tab, const f
   return launch_pair<128, false, false, QkvRopeEpi2>(x, w, B * N, 3 * E, E, 1, tplanes, tplanes, epi, st);
 }
 
-int patch_embed_gemm_tc2(const void* unfolded, const void* weight, const void* bias, const void* pos, void* tokens, int M,
-                         int Np, int K, int E, int tok_dtype, cudaStream_t st) {
-  CUtensorMap dummy;
+// ---- patch embedding: unfold pre-pass (fused fp32->bf16 cast) + the CTA-pair kernel ----------------------
+bool patch_embed_tc_supported(int B, int C, int Hi, int Wi, int P, int E) {
+  const int K = C * P * P;
+  if (P % 8 != 0 || Wi % 4 != 0 || K % 64 != 0 || E % 64 != 0) return false;
+  if ((long long)B * (Hi / P) * (Wi / P) >= (1ll << 31) / 4) return false;
+  return true;
+}
+size_t patch_embed_tc_workspace_bytes(int B, int C, int Hi, int Wi, int P) {
+  return (size_t)B * (Hi / P) * (Wi / P) * C * P * P * 2;
+}
+int patch_unfold(const void* images, void* out, int B, int C, int Hi, int Wi, int P, int img_dtype, cudaStream_t st) {
+  const int gw = Wi / P, Np = (Hi / P) * gw;
+  VRR_REQUIRE(P % 8 == 0 && Wi % 4 == 0, VRR_ERR_UNSUPPORTED, "patch_unfold: needs P %% 8 == 0 and Wi %% 4 == 0");
+  VRR_REQUIRE(((uintptr_t)images & 15) == 0 && ((uintptr_t)out & 15) == 0, VRR_ERR_INVALID_ARG,
+              "patch_unfold: pointers must be 16-byte aligned");
+  const size_t total = (size_t)B * Np * (C * P * P / 8);
+  const unsigned blocks = (unsigned)((total + 255) / 256);
+  if (img_dtype == VRR_F32)
+    patch_unfold_kernel<float><<<blocks, 256, 0, st>>>((const float*)images, (__nv_bfloat16*)out, B, C, Hi, Wi, P, gw, Np);
+  else
+    patch_unfold_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>((const __nv_bfloat16*)images, (__nv_bfloat16*)out, B, C,
+                                                              Hi, Wi, P, gw, Np);
+  VRR_LAUNCHED();
+  return VRR_OK;
+}
+int patch_embed_fwd_tc(const void* images, const void* weight, const void* bias, const void* pos, void* tokens,
+                       void* workspace, int B, int C, int Hi, int Wi, int P, int E, int img_dtype, int tok_dtype,
+                       cudaStream_t st) {
+  const int Np = (Hi / P) * (Wi / P), K = C * P * P, M = B * Np;
+  if (int rc = patch_unfold(images, workspace, B, C, Hi, Wi, P, img_dtype, st)) return rc;
+  CUtensorMap dummy;  // PatchEmbedEpi2 stores its rows directly: no C map
   memset(&dummy, 0, sizeof(dummy));
   if (tok_dtype == VRR_F32) {
     PatchEmbedEpi2<float> epi{(float*)tokens, (const __nv_bfloat16*)bias, (const float*)pos, Np, E};
-    if (E > 128) return launch_pair<256, false, false, PatchEmbedEpi2<float>>(unfolded, weight, M, E, K, 1, dummy, dummy, epi, st);
-    return launch_pair<128, false, false, PatchEmbedEpi2<float>>(unfolded, weight, M, E, K, 1, dummy, dummy, epi, st);
+    if (E > 128) return launch_pair<256, false, false, PatchEmbedEpi2<float>>(workspace, weight, M, E, K, 1, dummy, dummy, epi, st);
+    return launch_pair<128, false, false, PatchEmbedEpi2<float>>(workspace, weight, M, E, K, 1, dummy, dummy, epi, st);
   }
   PatchEmbedEpi2<__nv_bfloat16> epi{(__nv_bfloat16*)tokens, (const __nv_bfloat16*)bias, (const __nv_bfloat16*)pos, Np, E};
   if (E > 128)
-    return launch_pair<256, false, false, PatchEmbedEpi2<__nv_bfloat16>>(unfolded, weight, M, E, K, 1, dummy, dummy, epi, st);
-  return launch_pair<128, false, false, PatchEmbedEpi2<__nv_bfloat16>>(unfolded, weight, M, E, K, 1, dummy, dummy, epi, st);
+    return launch_pair<256, false, false, PatchEmbedEpi2<__nv_bfloat16>>(workspace, weight, M, E, K, 1, dummy, dummy, epi, st);
+  return launch_pair<128, false, false, PatchEmbedEpi2<__nv_bfloat16>>(workspace, weight, M, E, K, 1, dummy, dummy, epi, st);
 }
 
 }  // namespace vrr

@@ -13,22 +13,20 @@ int attn_bwd_simt(const void* planes, const vrr_bias_desc* bias, const void* out
                   const float* lse, void* d_planes, float* d_bias_param, float* delta, float* d_lut_ws, int B,
                   int H, int N, int Dh, float scale, int dtype, cudaStream_t st);
 
-// attn_tc.cu (tcgen05 / TMEM, bf16, Dh == 64)
+// attn_tc.cu (tcgen05 / TMEM, bf16, Dh == 64; tiled over 64-key tiles): without bias attn_fwd_tc4_kernel (four CTAs
+// per SM), with a bias attn_fwd_tc2_kernel (two CTAs per SM)
 bool attn_fwd_tc_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bias);
-void attn_fwd_tc_set_threshold_x100(int v);
-void attn_fwd_tc_set_table_bulk(int v);
-void attn_fwd_tc_set_poly(int v);     // 0..4 of every 8 exponential pairs by polynomial in attn_fwd_tc4_kernel
-void attn_fwd_tc_set_streams(int v);  // 4 (default): attn_fwd_tc4_kernel, four CTAs per SM; 2: attn_fwd_tc2_kernel
 void attn_fwd_tc_set_debug(long long* buf);
 int attn_fwd_tc(const void* planes, const vrr_bias_desc* bias, void* out, float* lse, int B, int H, int N,
                 int Dh, float scale, cudaStream_t st);
 
-// attn_fwd_ws.cu (whole-sequence forward for N <= 256: persistent, one round trip per (image, head))
+// attn_fwd_ws.cu (whole-sequence forward with a bias for N <= 256: persistent, one round trip per (image, head))
 bool attn_fwd_ws_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bias);
 int attn_fwd_ws(const void* planes, const vrr_bias_desc* bias, void* out, float* lse, int B, int H, int N, int Dh,
                 float scale, cudaStream_t st);
 
-// attn_bwd_tc2.cu (variant 2: issuer warp, double-buffered 32-row tiles)
+// attn_bwd_tc2.cu (dQ and dK/dV kernels: issuer warp, double-buffered 32-row tiles; every case attn_bwd_ws.cu does
+// not take)
 bool attn_bwd_tc2_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bias);
 int attn_bwd_tc2(const void* planes, const vrr_bias_desc* bias, const void* out, const void* d_out, const float* lse,
                  void* d_planes, float* d_bias_param, float* delta, int B, int H, int N, int Dh, float scale,
@@ -57,10 +55,16 @@ int patch_embed_bwd_simt(const void* images, const void* d_tokens, float* d_weig
                          int tok_dtype, cudaStream_t st);
 int patch_cls_rows(void* tokens, const void* cls, int B, int Np, int E, int tok_dtype, cudaStream_t st);
 
-// gemm_tc.cu (tcgen05 / TMEM / TMA, bf16)
+// gemm_tc2.cu (tcgen05 CTA pairs, cta_group::2: every operand layout, TMA-store epilogues)
+bool gemm_bf16_tc_supported(int M, int N, int K, int trans_a, int trans_b, int c_dtype, int epilogue);
+int gemm_bf16_tc(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int trans_a,
+                 int trans_b, int c_dtype, int epilogue, int accumulate, cudaStream_t st, float* colsum = nullptr);
+// colsum (bf16 C, plain / bias / multiply epilogues): colsum[n] += sum_m C[m][n] of the values as stored; zeroed by the caller
+int rope_pack_tables(const float* cos_tab, const float* sin_tab, float* packed, int heads, int rows, int hd, cudaStream_t st);
 bool qkv_rope_fwd_tc_supported(int B, int N, int E, int H);
-int qkv_rope_fwd_tc(const void* x, const void* w, const float* cos_tab, const float* sin_tab, void* planes,
-                    int B, int N, int E, int H, int rope_mode, cudaStream_t st);
+// `packed`: optional output of rope_pack_tables for the same tables (NULL: the epilogue reads cos_tab / sin_tab)
+int qkv_rope_fwd_tc2(const void* x, const void* w, const float* cos_tab, const float* sin_tab, const float* packed, void* planes, int B, int N,
+                     int E, int H, int rope_mode, cudaStream_t st);
 
 bool patch_embed_tc_supported(int B, int C, int Hi, int Wi, int P, int E);
 size_t patch_embed_tc_workspace_bytes(int B, int C, int Hi, int Wi, int P);
@@ -68,20 +72,6 @@ int patch_unfold(const void* images, void* out, int B, int C, int Hi, int Wi, in
 int patch_embed_fwd_tc(const void* images, const void* weight, const void* bias, const void* pos, void* tokens,
                        void* workspace, int B, int C, int Hi, int Wi, int P, int E, int img_dtype, int tok_dtype,
                        cudaStream_t st);
-
-// gemm_tc2.cu (tcgen05 CTA pairs, cta_group::2: every operand layout, TMA-store epilogues)
-void gemm_tc_set_variant(int v);  // 2 (default): CTA-pair kernels; 1: the 1-CTA kernels of gemm_tc.cu (QKV / patch embed only)
-int gemm_tc_variant();
-bool gemm_bf16_tc_supported(int M, int N, int K, int trans_a, int trans_b, int c_dtype, int epilogue);
-int gemm_bf16_tc(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int trans_a,
-                 int trans_b, int c_dtype, int epilogue, int accumulate, cudaStream_t st, float* colsum = nullptr);
-// colsum (bf16 C, plain / bias / multiply epilogues): colsum[n] += sum_m C[m][n] of the values as stored; zeroed by the caller
-int rope_pack_tables(const float* cos_tab, const float* sin_tab, float* packed, int heads, int rows, int hd, cudaStream_t st);
-// `packed`: optional output of rope_pack_tables for the same tables (NULL: the epilogue reads cos_tab / sin_tab)
-int qkv_rope_fwd_tc2(const void* x, const void* w, const float* cos_tab, const float* sin_tab, const float* packed, void* planes, int B, int N,
-                     int E, int H, int rope_mode, cudaStream_t st);
-int patch_embed_gemm_tc2(const void* unfolded, const void* weight, const void* bias, const void* pos, void* tokens, int M,
-                         int Np, int K, int E, int tok_dtype, cudaStream_t st);
 
 // layernorm.cu
 int layernorm_fwd(const void* x, const float* gamma, const float* beta, void* y, float* mean, float* rstd, int M, int E,

@@ -349,12 +349,8 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
 
 }  // namespace tc
 
-// Host: build a 2-D bf16 tensor map over a row-major [rows][cols] buffer with a box of
-// [box_rows][64 columns] (= 128 bytes wide) and 128-byte swizzle.
-int make_tmap_bf16(CUtensorMap* map, const void* base, uint64_t rows, uint64_t cols, uint64_t row_stride_bytes,
-                   uint32_t box_rows);
-// General 2-D map: `elem_bytes` 2 (bf16) or 4 (fp32); box = [box_rows][box_cols], box_cols * elem_bytes <= 128;
-// 128-byte swizzle.
+// Host: 2-D tensor map over a row-major [rows][cols] buffer: `elem_bytes` 2 (bf16) or 4 (fp32);
+// box = [box_rows][box_cols], box_cols * elem_bytes <= 128; 128-byte swizzle.
 int make_tmap_2d(CUtensorMap* map, const void* base, int elem_bytes, uint64_t rows, uint64_t cols,
                  uint64_t row_stride_bytes, uint32_t box_rows, uint32_t box_cols);
 

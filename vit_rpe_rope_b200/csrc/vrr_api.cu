@@ -25,10 +25,6 @@ constexpr int kMaxDevices = 64;
 static std::atomic<int> g_dev_state[kMaxDevices];
 static std::atomic<int> g_dev_sms[kMaxDevices];
 std::atomic<uint64_t> g_family_launches[3];  // [VRR_IMPL_SIMT], [VRR_IMPL_TCGEN05] dispatch counters
-// 4: without bias the four-CTA kernel of attn_tc.cu at every N, with bias as 3;  3: whole-sequence kernel for N <= 256
-// (attn_fwd_ws.cu), else attn_tc.cu;  2: attn_tc.cu always
-static std::atomic<int> g_attn_fwd_variant{4};
-static std::atomic<int> g_attn_bwd_variant{3};  // 3: attn_bwd_ws.cu for N <= 208 without bias, else attn_bwd_tc2.cu; 2: attn_bwd_tc2.cu always
 
 int current_device() {
   int dev = 0;
@@ -148,19 +144,9 @@ int vrr_debug_timestamps(void* device_buf) {  /* 64 x int64 device buffer, or NU
 }
 int vrr_set_option(const char* name, int value) {
   if (!name) return VRR_ERR_INVALID_ARG;
-  if (!strcmp(name, "gemm_variant")) { gemm_tc_set_variant(value); return VRR_OK; }
   if (!strcmp(name, "simt_gemm_tile")) { gemm_simt_set_tile(value); return VRR_OK; }
   if (!strcmp(name, "ln_reg")) { layernorm_set_option(0, value); return VRR_OK; }
   if (!strcmp(name, "ln_bwd_minb")) { layernorm_set_option(1, value); return VRR_OK; }
-  if (!strcmp(name, "attn_fwd_variant")) { g_attn_fwd_variant.store(value); return VRR_OK; }
-  if (!strcmp(name, "attn_bwd_variant")) { g_attn_bwd_variant.store(value); return VRR_OK; }
-  if (!strcmp(name, "attn_fwd_poly_exp")) { attn_fwd_tc_set_poly(value); return VRR_OK; }
-  if (!strcmp(name, "attn_fwd_streams")) { attn_fwd_tc_set_streams(value); return VRR_OK; }
-  if (!strcmp(name, "attn_fwd_table_bulk")) { attn_fwd_tc_set_table_bulk(value); return VRR_OK; }
-  if (!strcmp(name, "attn_fwd_rescale_threshold_x100")) {
-    attn_fwd_tc_set_threshold_x100(value);
-    return VRR_OK;
-  }
   set_error("vrr_set_option: unknown option '%s'", name);
   return VRR_ERR_INVALID_ARG;
 }
@@ -247,9 +233,7 @@ int vrr_qkv_rope_fwd_packed(const void* x, const void* w_qkv, const float* cos_t
   const int impl = g_impl.load();
   if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && qkv_rope_fwd_tc_supported(B, N, E, H)) {
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
-    if (gemm_tc_variant() == 2)
-      return qkv_rope_fwd_tc2(x, w_qkv, cos_tab, sin_tab, packed, planes, B, N, E, H, rope_mode, (cudaStream_t)stream);
-    return qkv_rope_fwd_tc(x, w_qkv, cos_tab, sin_tab, planes, B, N, E, H, rope_mode, (cudaStream_t)stream);
+    return qkv_rope_fwd_tc2(x, w_qkv, cos_tab, sin_tab, packed, planes, B, N, E, H, rope_mode, (cudaStream_t)stream);
   }
   VRR_REQUIRE(impl != VRR_IMPL_TCGEN05, VRR_ERR_UNSUPPORTED,
               "qkv_rope_fwd: tcgen05 kernel forced but shape/dtype unsupported (bf16, Dh=64, E%%64==0)");
@@ -382,9 +366,8 @@ int vrr_attn_fwd(const void* planes, const vrr_bias_desc* bias, void* out, float
   const int impl = g_impl.load();
   if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && attn_fwd_tc_supported(B, H, N, Dh, bias)) {
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
-    const int variant = g_attn_fwd_variant.load();
-    const bool no_bias = bias == nullptr || bias->mode == VRR_BIAS_NONE;
-    if (variant >= 3 && !(variant >= 4 && no_bias) && attn_fwd_ws_supported(B, H, N, Dh, bias))  // short sequences with bias
+    // with a bias, N <= 256: the whole-sequence kernel; otherwise the tiled kernels (four CTAs per SM without bias)
+    if (attn_fwd_ws_supported(B, H, N, Dh, bias))
       return attn_fwd_ws(planes, bias, out, lse, B, H, N, Dh, scale, (cudaStream_t)stream);
     return attn_fwd_tc(planes, bias, out, lse, B, H, N, Dh, scale, (cudaStream_t)stream);
   }
@@ -421,7 +404,7 @@ int vrr_attn_bwd(const void* planes, const vrr_bias_desc* bias, const void* out,
   const int impl = g_impl.load();
   if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && attn_bwd_tc2_supported(B, H, N, Dh, bias)) {
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
-    if (g_attn_bwd_variant.load() >= 3 && attn_bwd_ws_supported(B, H, N, Dh, bias))  // short sequences, no bias
+    if (attn_bwd_ws_supported(B, H, N, Dh, bias))  // short sequences, no bias: the whole-sequence kernel
       return attn_bwd_ws(planes, out, d_out, lse, d_planes, B, H, N, Dh, scale, (cudaStream_t)stream);
     return attn_bwd_tc2(planes, bias, out, d_out, lse, d_planes, d_bias_param, delta, B, H, N, Dh, scale,
                         (cudaStream_t)stream);
