@@ -15,7 +15,9 @@
  *     (a cudaStream_t passed as void*; NULL = legacy default stream);
  *   - return value: VRR_OK (0) or a negative vrr_status; vrr_last_error() gives the reason;
  *   - tensors are dense row-major with the shapes documented per argument; `dtype` selects the
- *     element type of activations/weights (VRR_F32 or VRR_BF16).  Position tables (cos/sin, bias
+ *     element type of activations/weights (VRR_F32, VRR_BF16 or VRR_F16).  Where an entry point takes several
+ *     dtypes, bf16 and fp16 never meet in one call (VRR_ERR_INVALID_ARG); each pairs with fp32 in exactly the
+ *     combinations documented for bf16, and fp16 runs the same kernels as bf16.  Position tables (cos/sin, bias
  *     table, polynomial coefficients), softmax statistics and all parameter-gradient outputs that
  *     are reductions (d_table, d_coef, d_cos, d_sin) are ALWAYS fp32;
  *   - there is no CPU path: on a machine without an sm_100 device every compute entry point
@@ -23,7 +25,7 @@
  *
  * Token / head geometry: B images, N tokens per image (token 0 is the cls token, tokens 1..N-1 are
  * the g*g patches in raster order), E = H * Dh channels, H heads of Dh channels.  Dh must be one of
- * 16, 32, 64 (the tcgen05 bf16 kernels need Dh == 64).
+ * 16, 32, 64 (the tcgen05 bf16 / fp16 kernels need Dh == 64).
  *
  * "qkv planes": one buffer [3][B][H][N][Dh] holding q (rotated when RoPE is on), k (likewise), v.
  */
@@ -48,7 +50,9 @@ typedef enum {
   VRR_ERR_WORKSPACE = -5      /* workspace too small (see vrr_*_workspace_bytes)        */
 } vrr_status;
 
-typedef enum { VRR_F32 = 0, VRR_BF16 = 1 } vrr_dtype;
+/* fp16 (IEEE binary16) results that overflow are +-inf, never a clamped finite value (mixed-precision training
+ * with a loss scaler detects the overflow from them). */
+typedef enum { VRR_F32 = 0, VRR_BF16 = 1, VRR_F16 = 2 } vrr_dtype;
 
 /* RoPE variants of models/vit.py:51-68.  AXIAL: cos/sin are [N-1][Dh/2] shared by all heads
  * (positional_encoding.py:216-245).  MIXED: cos/sin are [H][N-1][Dh/2]
@@ -63,8 +67,9 @@ typedef enum { VRR_ROPE_NONE = 0, VRR_ROPE_AXIAL = 1, VRR_ROPE_MIXED = 2 } vrr_r
  *        d = |(i-1)%g - (j-1)%g| + |(i-1)/g - (j-1)/g| (positional_encoding.py:127-171). */
 typedef enum { VRR_BIAS_NONE = 0, VRR_BIAS_TABLE = 1, VRR_BIAS_POLY = 2 } vrr_bias_mode;
 
-/* Kernel family selection for the bf16 attention / QKV kernels.  AUTO picks the tcgen05 (tensor
- * core, TMEM) kernels whenever the shape allows and the SIMT kernels otherwise; the other two
+/* Kernel family selection for the bf16 / fp16 attention, QKV, GEMM and patch-embedding kernels.
+ * AUTO picks the tcgen05 (tensor core, TMEM) kernels whenever the shape allows and the SIMT kernels
+ * otherwise (fp16 exactly where bf16 would); the other two
  * force one family (tests use them to cross-check).  fp32 always runs the SIMT FFMA kernels:
  * tcgen05 has no fp32 MMA and the fp32 parity bar is 1e-5. */
 typedef enum { VRR_IMPL_AUTO = 0, VRR_IMPL_SIMT = 1, VRR_IMPL_TCGEN05 = 2 } vrr_impl;
@@ -117,7 +122,8 @@ int vrr_debug_timestamps(void* device_buf);
  * pos_embed: NULL, or the absolute table [>= Np][E] (positional_encoding.py:37-40: added to patch
  * rows only).  (img fp32, dtype bf16, tok fp32) is the reference's autocast semantics: the image is
  * rounded to bf16 on load, the conv result is bf16, and the concatenation with the fp32 cls token
- * promotes the stream to fp32.  The bf16 tensor-core path (P % 8 == 0, C*P*P % 64 == 0, E % 64 == 0)
+ * promotes the stream to fp32; fp16 in place of every bf16 gives the float16-autocast semantics.  The 16-bit
+ * tensor-core path (P % 8 == 0, C*P*P % 64 == 0, E % 64 == 0)
  * unfolds the patches into `workspace` (vrr_patch_embed_workspace_bytes, 256-byte aligned) and runs
  * a tcgen05 GEMM; otherwise workspace may be NULL. */
 size_t vrr_patch_embed_workspace_bytes(int B, int C, int Hi, int Wi, int P, int E, int dtype);
@@ -130,6 +136,10 @@ int vrr_patch_embed_fwd(const void* images, const void* weight, const void* bias
  * weight gradient with a plain library GEMM. */
 int vrr_patch_unfold(const void* images, void* out, int B, int C, int Hi, int Wi, int P,
                      int img_dtype, void* stream);
+/* The same with an explicit output element type `out_dtype` (VRR_BF16 or VRR_F16); images are fp32 or
+ * `out_dtype`. */
+int vrr_patch_unfold_ex(const void* images, void* out, int B, int C, int Hi, int Wi, int P,
+                        int img_dtype, int out_dtype, void* stream);
 /* d_tokens [B][Np+1][E] (`tok_dtype`).  Parameter gradients are reductions and ALWAYS fp32:
  * d_weight [E][C*P*P] (or NULL: skip it), d_bias [E], d_cls [E], d_pos [Np][E] or NULL; written (not
  * accumulated).  Images need no gradient (train.py:109-115). */
@@ -178,7 +188,7 @@ int vrr_rope_table_grad(const void* q_in, const void* k_in, const void* dq, cons
 
 /* Plain GEMM used by the backward of the projection: C = op(A) . op(B), row-major operands,
  * op(A) is [M][K] (trans_a: A is stored [K][M]), op(B) is [K][N] (trans_b: B is stored [N][K]).
- * `dtype` is the element type of A and B, `c_dtype` that of C (fp32 C is allowed for bf16 inputs:
+ * `dtype` is the element type of A and B, `c_dtype` that of C (fp32 C is allowed for bf16 / fp16 inputs:
  * weight gradients).  fp32 accumulation always. */
 int vrr_gemm(const void* a, const void* b, void* c, int M, int N, int K, int trans_a, int trans_b,
              int dtype, int c_dtype, void* stream);
@@ -193,7 +203,7 @@ int vrr_gemm(const void* a, const void* b, void* c, int M, int N, int K, int tra
  * (timm Mlp, act_layer=nn.GELU); BIAS_GELU_GRAD writes C = gelu(h) and C2 = gelu'(h) for h = round(acc + bias)
  * (h itself is not stored: the Mlp backward only needs gelu'); MUL multiplies by the INPUT matrix C2[M][N]
  * before rounding (fc2's dX fused with the GELU backward: dh = (dy . W2) * gelu'(h)).  accumulate != 0 (fp32 C, tcgen05 kernel only): C += result.
- * bf16 operands with N % 8 == 0, K % 8 == 0 (and M % 8 == 0 when trans_a) and 16-byte aligned pointers run
+ * bf16 or fp16 operands with N % 8 == 0, K % 8 == 0 (and M % 8 == 0 when trans_a) and 16-byte aligned pointers run
  * the tcgen05 CTA-pair kernel (cta_group::2, TMA in, TMA store / reduce-add out; fp32 C is split over K and
  * combined by TMA reduce-add, so its summation order is not deterministic); everything else (fp32 operands,
  * odd shapes, a pointer that is not 16-byte aligned, e.g. a view at an offset into a larger buffer) runs the
@@ -245,8 +255,8 @@ int vrr_add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new,
 /* fc2's input gradient with the GELU backward and fc1's bias gradient fused (autograd of timm Mlp, vit.py:118):
  *   c[m][n] = (op(a) . op(b))[m][n] * mul[m][n]   (`dtype`, as VRR_EPI_MUL)
  *   col_sums[n] = sum_m c[m][n]                   (fp32 [N], written; sums the values AS STORED, like autograd's
- *                                                  sum over the bf16 tensor)
- * bf16 on the tcgen05 kernel: the epilogue adds the column sums of each staged tile (fp32 atomics - summation
+ *                                                  sum over the bf16 / fp16 tensor)
+ * bf16 / fp16 on the tcgen05 kernel: the epilogue adds the column sums of each staged tile (fp32 atomics - summation
  * order not deterministic); otherwise vrr_gemm_ex(VRR_EPI_MUL) followed by vrr_colsum. */
 int vrr_gemm_mul_colsum(const void* a, const void* b, void* c, const void* mul, float* col_sums, int M, int N,
                         int K, int trans_a, int trans_b, int dtype, void* stream);

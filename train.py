@@ -9,6 +9,8 @@ tests/test_host_api.py).  Same loop: AdamW(lr, weight_decay), CosineAnnealingLR(
 
 Additions (all off by default, so a reference command line behaves like the reference):
   --amp bf16         run the step under torch.autocast(bfloat16) - the tcgen05 kernels (head dim 64)
+  --amp fp16         run the step under torch.autocast(float16) with torch.amp.GradScaler (loss scaling; a step whose
+                     gradients overflow is skipped and the scale lowered) - the same kernels in fp16
   --synthetic        class-conditional synthetic images instead of MNIST / CIFAR-10.  Chosen automatically when the
                      dataset is not on disk: this repository never downloads anything.
   --max_steps N      stop every epoch after N batches (smoke runs)
@@ -53,7 +55,7 @@ def get_args(argv=None):
     p.add_argument("--depth", type=int, default=6)
     p.add_argument("--num_heads", type=int, default=6)
     # additions
-    p.add_argument("--amp", type=str, default="none", choices=["none", "bf16"])
+    p.add_argument("--amp", type=str, default="none", choices=["none", "bf16", "fp16"])
     p.add_argument("--synthetic", action="store_true")
     p.add_argument("--synthetic_size", type=int, default=4096, help="training images of the synthetic set")
     p.add_argument("--max_steps", type=int, default=0)
@@ -101,9 +103,10 @@ def get_dataset(args):
     return mk(train_set, True), mk(test_set, False), 10, in_chans
 
 
-def run_epoch(model, loader, criterion, optimizer, device, amp, max_steps):
+def run_epoch(model, loader, criterion, optimizer, device, amp, max_steps, amp_dtype=torch.bfloat16, scaler=None):
     """One pass; trains when ``optimizer`` is given.  Returns (mean batch loss, accuracy %) like the reference's
-    train() / test() (train.py:97-155); the loss / accuracy counters stay on the device until the end of the pass."""
+    train() / test() (train.py:97-155); the loss / accuracy counters stay on the device until the end of the pass.
+    ``amp``: autocast to ``amp_dtype``; ``scaler``: a torch.amp.GradScaler for the backward and the optimizer step."""
     training = optimizer is not None
     model.train(training)
     loss_sum = torch.zeros((), device=device)
@@ -114,10 +117,14 @@ def run_epoch(model, loader, criterion, optimizer, device, amp, max_steps):
             images, labels = images.to(device, non_blocking=True), labels.to(device, non_blocking=True)
             if training:
                 optimizer.zero_grad()
-            with torch.autocast("cuda", dtype=torch.bfloat16, enabled=amp):
+            with torch.autocast("cuda", dtype=amp_dtype, enabled=amp):
                 outputs = model(images)
                 loss = criterion(outputs.float(), labels)
-            if training:
+            if training and scaler is not None:
+                scaler.scale(loss).backward()
+                scaler.step(optimizer)
+                scaler.update()
+            elif training:
                 loss.backward()
                 optimizer.step()
             loss_sum += loss.detach()
@@ -149,12 +156,15 @@ def main(argv=None):
     criterion = nn.CrossEntropyLoss()
     optimizer = torch.optim.AdamW(model.parameters(), lr=args.lr, weight_decay=args.weight_decay)
     scheduler = torch.optim.lr_scheduler.CosineAnnealingLR(optimizer, T_max=args.epochs)
-    amp = args.amp == "bf16"
+    amp = args.amp != "none"
+    amp_dtype = torch.float16 if args.amp == "fp16" else torch.bfloat16
+    scaler = torch.amp.GradScaler("cuda") if args.amp == "fp16" else None
     best_acc, ckpt = 0.0, os.path.join(args.ckpt_dir, f"{args.dataset}_{args.pos_encoding}_best.pth")
     for epoch in range(args.epochs):
         t0 = time.time()
-        train_loss, train_acc = run_epoch(model, train_loader, criterion, optimizer, device, amp, args.max_steps)
-        test_loss, test_acc = run_epoch(model, test_loader, criterion, None, device, amp, args.max_steps)
+        train_loss, train_acc = run_epoch(model, train_loader, criterion, optimizer, device, amp, args.max_steps, amp_dtype,
+                                          scaler)
+        test_loss, test_acc = run_epoch(model, test_loader, criterion, None, device, amp, args.max_steps, amp_dtype)
         scheduler.step()
         if test_acc > best_acc:
             best_acc = test_acc

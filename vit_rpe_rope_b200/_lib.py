@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libvrr_b200.so")
 HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "vrr.h")
 
-VRR_F32, VRR_BF16 = 0, 1
+VRR_F32, VRR_BF16, VRR_F16 = 0, 1, 2
 ROPE_NONE, ROPE_AXIAL, ROPE_MIXED = 0, 1, 2
 BIAS_NONE, BIAS_TABLE, BIAS_POLY = 0, 1, 2
 IMPL_AUTO, IMPL_SIMT, IMPL_TCGEN05 = 0, 1, 2
@@ -43,6 +43,7 @@ SIGNATURES = {
     "vrr_patch_embed_workspace_bytes": (c_size_t, [c_int] * 7),
     "vrr_patch_embed_fwd": (c_int, [c_void_p] * 7 + [c_size_t] + [c_int] * 9 + [c_void_p]),
     "vrr_patch_unfold": (c_int, [c_void_p] * 2 + [c_int] * 6 + [c_void_p]),
+    "vrr_patch_unfold_ex": (c_int, [c_void_p] * 2 + [c_int] * 7 + [c_void_p]),
     "vrr_patch_embed_bwd": (c_int, [c_void_p] * 6 + [c_int] * 9 + [c_void_p]),
     "vrr_qkv_rope_fwd": (c_int, [c_void_p] * 5 + [c_int] * 6 + [c_void_p]),
     "vrr_qkv_rope_fwd_packed": (c_int, [c_void_p] * 6 + [c_int] * 6 + [c_void_p]),
@@ -85,7 +86,7 @@ def load():
     if lib.vrr_abi_version() != 1:
         raise ImportError(f"libvrr_b200.so ABI {lib.vrr_abi_version()} != 1: rebuild")
     _lib = lib
-    # Debug switch (never set by the product): force one kernel family for the bf16 kernels.
+    # Debug switch (never set by the product): force one kernel family for the bf16 / fp16 kernels.
     forced = os.environ.get("VRR_IMPL", "").lower()
     if forced in ("simt", "tcgen05"):
         lib.vrr_set_impl(IMPL_SIMT if forced == "simt" else IMPL_TCGEN05)

@@ -1,17 +1,17 @@
 // Fused attention backward for every case the whole-sequence kernel (attn_bwd_ws.cu) does not take: the bias modes
 // and N > 208.  Two kernels with the tiled forward's pipeline - a dedicated issuer warp (TMA + every tcgen05.mma),
 // 32-row streamed tiles, double-buffered S / dP accumulators in TMEM so the issuer computes tile t+1 while the four
-// row-owner warps work on tile t, dS / P written back in place (bf16) and consumed from TMEM by the
+// row-owner warps work on tile t, dS / P written back in place (bf16 / fp16) and consumed from TMEM by the
 // accumulating MMAs.
 //
 //  dQ kernel  (CTA = 128 query rows):  TMEM cols  S[2] 0..63 | dP[2] 64..127 | dQ 128..191
 //       S = Q K_t^T, dP = dO V_t^T  ->  thread: P = exp2(S*c + bias - lse), dS = P (dP - delta)
-//       -> dS (bf16) over S buffer  ->  dQ += dS K_t.   Also delta, and the bias gradients:
+//       -> dS (T) over S buffer  ->  dQ += dS K_t.   Also delta, and the bias gradients:
 //       relative table: each warp transposes its 32x32 dS block through shared memory and every lane
 //       sums two diagonals (conflict-free, 33-float pitch) -> 2 shared atomics per lane per tile;
 //       polynomial: per-thread power sums.
 //  dK/dV kernel (CTA = 128 key rows):  TMEM cols  S^T[2] 0..63 | dP^T[2] 64..127 | dV 128..191 | dK 192..255
-//       S^T = K Q_t^T, dP^T = V dO_t^T -> thread: P^T, dS^T -> bf16 in place -> dV += P^T dO_t, dK += dS^T Q_t.
+//       S^T = K Q_t^T, dP^T = V dO_t^T -> thread: P^T, dS^T -> T in place -> dV += P^T dO_t, dK += dS^T Q_t.
 #include "common.cuh"
 #include "kernels.h"
 #include "tc_common.cuh"
@@ -33,10 +33,10 @@ constexpr uint32_t kTmemCols = 256;
 constexpr float kLog2e = 1.4426950408889634f;
 
 struct Bwd2Params {
-  const __nv_bfloat16 *out, *d_out;
+  const void *out, *d_out;  // element type T of the kernels
   const float* lse;
   float* delta;
-  __nv_bfloat16* d_planes;
+  void* d_planes;           // T
   const float* bias_param;
   float* d_bias_param;
   int B, H, N;
@@ -67,21 +67,22 @@ __device__ __forceinline__ void fill_lut2(float* lut, uint16_t* key_yx, const Bw
   }
 }
 
-__device__ __forceinline__ void store_row64(__nv_bfloat16* dst, const uint32_t (&lo)[32], const uint32_t (&hi)[32], float mul) {
+template <typename T>
+__device__ __forceinline__ void store_row64(T* dst, const uint32_t (&lo)[32], const uint32_t (&hi)[32], float mul) {
 #pragma unroll
   for (int v8 = 0; v8 < 8; ++v8) {
     const uint32_t* src = v8 < 4 ? &lo[v8 * 8] : &hi[(v8 - 4) * 8];
     uint4 w;
-    w.x = pack_bf16(__uint_as_float(src[0]) * mul, __uint_as_float(src[1]) * mul);
-    w.y = pack_bf16(__uint_as_float(src[2]) * mul, __uint_as_float(src[3]) * mul);
-    w.z = pack_bf16(__uint_as_float(src[4]) * mul, __uint_as_float(src[5]) * mul);
-    w.w = pack_bf16(__uint_as_float(src[6]) * mul, __uint_as_float(src[7]) * mul);
+    w.x = Elem16<T>::pack2(__uint_as_float(src[0]) * mul, __uint_as_float(src[1]) * mul);
+    w.y = Elem16<T>::pack2(__uint_as_float(src[2]) * mul, __uint_as_float(src[3]) * mul);
+    w.z = Elem16<T>::pack2(__uint_as_float(src[4]) * mul, __uint_as_float(src[5]) * mul);
+    w.w = Elem16<T>::pack2(__uint_as_float(src[6]) * mul, __uint_as_float(src[7]) * mul);
     *reinterpret_cast<uint4*>(dst + v8 * 8) = w;
   }
 }
 
 // ============================================================================================ dQ
-template <int BIAS>
+template <typename T, int BIAS>
 __global__ void __launch_bounds__(kThreads, 2)
 attn_bwd_dq_tc2_kernel(const __grid_constant__ CUtensorMap tmap_pl, const __grid_constant__ CUtensorMap tmap_do,
                        const Bwd2Params p) {
@@ -161,8 +162,8 @@ attn_bwd_dq_tc2_kernel(const __grid_constant__ CUtensorMap tmap_pl, const __grid
     // =========================================== issuer ===========================================
     const uint64_t desc_q = smem_desc_sw128(smem_u32(sQ));
     const uint64_t desc_g = smem_desc_sw128(smem_u32(sG));
-    constexpr uint32_t idesc_s = idesc_bf16(kRows, kT, 0, 0);
-    constexpr uint32_t idesc_q = idesc_bf16(kRows, kDh, 0, 1);
+    constexpr uint32_t idesc_s = idesc_16<T>(kRows, kT, 0, 0);
+    constexpr uint32_t idesc_q = idesc_16<T>(kRows, kDh, 0, 1);
     auto issue_s_dp = [&](int t) {  // S(t), dP(t) into buffer t & 1
       const int st = t % kSt;
       mbar_wait(&bar_kfull[st], (uint32_t)((t / kSt) & 1));
@@ -228,16 +229,16 @@ attn_bwd_dq_tc2_kernel(const __grid_constant__ CUtensorMap tmap_pl, const __grid
     float lse2 = 0.f, delta = 0.f;
     {
       const size_t off = ((size_t)b * N + ic) * E + h * kDh;
-      const uint4* o4 = reinterpret_cast<const uint4*>(p.out + off);
-      const uint4* g4 = reinterpret_cast<const uint4*>(p.d_out + off);
+      const uint4* o4 = reinterpret_cast<const uint4*>(static_cast<const T*>(p.out) + off);
+      const uint4* g4 = reinterpret_cast<const uint4*>(static_cast<const T*>(p.d_out) + off);
 #pragma unroll
       for (int v8 = 0; v8 < 8; ++v8) {
         const uint4 ov = __ldg(o4 + v8), gv = __ldg(g4 + v8);
         const uint32_t ow[4] = {ov.x, ov.y, ov.z, ov.w}, gw[4] = {gv.x, gv.y, gv.z, gv.w};
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
-          const float2 of = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&ow[e]));
-          const float2 gf = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&gw[e]));
+          const float2 of = Elem16<T>::unpack2(ow[e]);
+          const float2 gf = Elem16<T>::unpack2(gw[e]);
           delta = fmaf(of.x, gf.x, delta);
           delta = fmaf(of.y, gf.y, delta);
         }
@@ -291,10 +292,10 @@ attn_bwd_dq_tc2_kernel(const __grid_constant__ CUtensorMap tmap_pl, const __grid
             pw2 += w2;
             pw3 = fmaf(w2, dist_f, pw3);
           }
-          if (e & 1) packed[e >> 1] = pack_bf16(__uint_as_float(sr[e - 1]), ds);
+          if (e & 1) packed[e >> 1] = Elem16<T>::pack2(__uint_as_float(sr[e - 1]), ds);
           else sr[e] = __float_as_uint(ds);
         }
-        tmem_st16(tmem_row + sb * kT, packed);  // dS (bf16 pairs) over this S buffer
+        tmem_st16(tmem_row + sb * kT, packed);  // dS (pairs of T) over this S buffer
         if (BIAS == VRR_BIAS_TABLE) {
           // diagonal sums of the warp's 32x32 dS block: element (r, c) lies on diagonal r - c; lane l
           // owns diagonal l (rows l.., cols 0..) and diagonal l-32 (rows 0.., cols 32-l..): 32 elements.
@@ -321,7 +322,7 @@ attn_bwd_dq_tc2_kernel(const __grid_constant__ CUtensorMap tmap_pl, const __grid
       tmem_ld32(tmem_row + 128, lo);
       tmem_ld32(tmem_row + 160, hi);
       tmem_wait_ld();
-      if (live) store_row64(p.d_planes + ((size_t)bh * N + i) * kDh, lo, hi, p.scale);
+      if (live) store_row64(static_cast<T*>(p.d_planes) + ((size_t)bh * N + i) * kDh, lo, hi, p.scale);
     }
     if (BIAS == VRR_BIAS_TABLE) {
       asm volatile("bar.sync 1, 128;" ::: "memory");
@@ -349,7 +350,7 @@ attn_bwd_dq_tc2_kernel(const __grid_constant__ CUtensorMap tmap_pl, const __grid
 }
 
 // ============================================================================================ dK, dV
-template <int BIAS>
+template <typename T, int BIAS>
 __global__ void __launch_bounds__(kThreads, 2)
 attn_bwd_dkv_tc2_kernel(const __grid_constant__ CUtensorMap tmap_pl, const __grid_constant__ CUtensorMap tmap_do,
                         const Bwd2Params p) {
@@ -421,8 +422,8 @@ attn_bwd_dkv_tc2_kernel(const __grid_constant__ CUtensorMap tmap_pl, const __gri
   if (warp == 4) {
     const uint64_t desc_k = smem_desc_sw128(smem_u32(sK));
     const uint64_t desc_v = smem_desc_sw128(smem_u32(sV));
-    constexpr uint32_t idesc_s = idesc_bf16(kRows, kT, 0, 0);
-    constexpr uint32_t idesc_acc = idesc_bf16(kRows, kDh, 0, 1);
+    constexpr uint32_t idesc_s = idesc_16<T>(kRows, kT, 0, 0);
+    constexpr uint32_t idesc_acc = idesc_16<T>(kRows, kDh, 0, 1);
     auto issue_st = [&](int t) {  // S^T(t), dP^T(t) into buffer t & 1
       const int st = t % kSt;
       mbar_wait(&bar_full[st], (uint32_t)((t / kSt) & 1));
@@ -514,8 +515,8 @@ attn_bwd_dkv_tc2_kernel(const __grid_constant__ CUtensorMap tmap_pl, const __gri
           const float pr = ex2(x);
           const float ds = pr * (__uint_as_float(dr[e]) - stt.y);
           if (e & 1) {
-            pp[e >> 1] = pack_bf16(__uint_as_float(sr[e - 1]), pr);
-            pd[e >> 1] = pack_bf16(__uint_as_float(dr[e - 1]), ds);
+            pp[e >> 1] = Elem16<T>::pack2(__uint_as_float(sr[e - 1]), pr);
+            pd[e >> 1] = Elem16<T>::pack2(__uint_as_float(dr[e - 1]), ds);
           } else {
             sr[e] = __float_as_uint(pr);
             dr[e] = __float_as_uint(ds);
@@ -537,12 +538,12 @@ attn_bwd_dkv_tc2_kernel(const __grid_constant__ CUtensorMap tmap_pl, const __gri
       tmem_ld32(tmem_row + 128, lo);
       tmem_ld32(tmem_row + 160, hi);
       tmem_wait_ld();
-      if (live) store_row64(p.d_planes + 2 * plane + ((size_t)bh * N + j) * kDh, lo, hi, 1.f);
+      if (live) store_row64(static_cast<T*>(p.d_planes) + 2 * plane + ((size_t)bh * N + j) * kDh, lo, hi, 1.f);
       __syncwarp();
       tmem_ld32(tmem_row + 192, lo);
       tmem_ld32(tmem_row + 224, hi);
       tmem_wait_ld();
-      if (live) store_row64(p.d_planes + plane + ((size_t)bh * N + j) * kDh, lo, hi, p.scale);
+      if (live) store_row64(static_cast<T*>(p.d_planes) + plane + ((size_t)bh * N + j) * kDh, lo, hi, p.scale);
     }
   }
   tc_fence_before();
@@ -575,23 +576,23 @@ bool attn_bwd_tc2_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bi
   return bwd2_smem_bytes(N, bias, nullptr, false) <= 200 * 1024 && bwd2_smem_bytes(N, bias, nullptr, true) <= 200 * 1024;
 }
 
-int attn_bwd_tc2(const void* planes, const vrr_bias_desc* bias, const void* out, const void* d_out, const float* lse,
-                 void* d_planes, float* d_bias_param, float* delta, int B, int H, int N, int Dh, float scale,
-                 cudaStream_t st) {
-  (void)Dh;
+template <typename T>
+static int attn_bwd_tc2_t(const void* planes, const vrr_bias_desc* bias, const void* out, const void* d_out, const float* lse,
+                          void* d_planes, float* d_bias_param, float* delta, int B, int H, int N, float scale,
+                          cudaStream_t st) {
   VRR_REQUIRE(((uintptr_t)planes & 15) == 0 && ((uintptr_t)out & 15) == 0 && ((uintptr_t)d_out & 15) == 0 &&
                   ((uintptr_t)d_planes & 15) == 0,
               VRR_ERR_INVALID_ARG, "attn_bwd (tcgen05): planes / out / d_out / d_planes must be 16-byte aligned");
   const int E = H * kDh;
   CUtensorMap tm_pl, tm_do;
-  if (int rc = make_tmap_2d(&tm_pl, planes, 2, (uint64_t)3 * B * H * N, kDh, kDh * 2, kT, 64)) return rc;
-  if (int rc = make_tmap_2d(&tm_do, d_out, 2, (uint64_t)B * N, (uint64_t)E, (uint64_t)E * 2, kT, 64)) return rc;
+  if (int rc = make_tmap_2d(&tm_pl, planes, Elem16<T>::kTmap, (uint64_t)3 * B * H * N, kDh, kDh * 2, kT, 64)) return rc;
+  if (int rc = make_tmap_2d(&tm_do, d_out, Elem16<T>::kTmap, (uint64_t)B * N, (uint64_t)E, (uint64_t)E * 2, kT, 64)) return rc;
   Bwd2Params p;
-  p.out = (const __nv_bfloat16*)out;
-  p.d_out = (const __nv_bfloat16*)d_out;
+  p.out = out;
+  p.d_out = d_out;
   p.lse = lse;
   p.delta = delta;
-  p.d_planes = (__nv_bfloat16*)d_planes;
+  p.d_planes = d_planes;
   p.B = B; p.H = H; p.N = N;
   p.scale = scale;
   p.scale_log2 = scale * kLog2e;
@@ -608,11 +609,11 @@ int attn_bwd_tc2(const void* planes, const vrr_bias_desc* bias, const void* out,
   const size_t smem_kv = bwd2_smem_bytes(N, bias, &p.lut_floats, true);
 #define LAUNCH(MODE)                                                                                             \
   do {                                                                                                           \
-    VRR_SMEM_ATTR_ONCE(attn_bwd_dq_tc2_kernel<MODE>, 200 * 1024);                                                \
-    VRR_SMEM_ATTR_ONCE(attn_bwd_dkv_tc2_kernel<MODE>, 200 * 1024);                                               \
-    attn_bwd_dq_tc2_kernel<MODE><<<grid, kThreads, smem_q, st>>>(tm_pl, tm_do, p);                               \
+    VRR_SMEM_ATTR_ONCE((attn_bwd_dq_tc2_kernel<T, MODE>), 200 * 1024);                                           \
+    VRR_SMEM_ATTR_ONCE((attn_bwd_dkv_tc2_kernel<T, MODE>), 200 * 1024);                                          \
+    attn_bwd_dq_tc2_kernel<T, MODE><<<grid, kThreads, smem_q, st>>>(tm_pl, tm_do, p);                            \
     VRR_LAUNCHED();                                                                                              \
-    attn_bwd_dkv_tc2_kernel<MODE><<<grid, kThreads, smem_kv, st>>>(tm_pl, tm_do, p);                             \
+    attn_bwd_dkv_tc2_kernel<T, MODE><<<grid, kThreads, smem_kv, st>>>(tm_pl, tm_do, p);                          \
     VRR_LAUNCHED();                                                                                              \
   } while (0)
   if (mode == VRR_BIAS_TABLE) LAUNCH(VRR_BIAS_TABLE);
@@ -620,6 +621,15 @@ int attn_bwd_tc2(const void* planes, const vrr_bias_desc* bias, const void* out,
   else LAUNCH(VRR_BIAS_NONE);
 #undef LAUNCH
   return VRR_OK;
+}
+
+int attn_bwd_tc2(const void* planes, const vrr_bias_desc* bias, const void* out, const void* d_out, const float* lse,
+                 void* d_planes, float* d_bias_param, float* delta, int B, int H, int N, int Dh, float scale, int dtype,
+                 cudaStream_t st) {
+  (void)Dh;
+  if (dtype == VRR_F16)
+    return attn_bwd_tc2_t<__half>(planes, bias, out, d_out, lse, d_planes, d_bias_param, delta, B, H, N, scale, st);
+  return attn_bwd_tc2_t<__nv_bfloat16>(planes, bias, out, d_out, lse, d_planes, d_bias_param, delta, B, H, N, scale, st);
 }
 
 }  // namespace vrr

@@ -17,7 +17,7 @@
 //     and its own lane tiles (group w: the dQ tiles of parity w and the dKV tiles of parity 1 - w), so one group's
 //     exponentials overlap the other's MMAs and epilogue;
 //   * per stream TMEM: S at [0,128), dP at [128,256) for the first column group; P / dS are written back in place
-//     (bf16) and consumed from TMEM by the accumulating MMAs; the accumulators live in columns the group has already
+//     (bf16 / fp16) and consumed from TMEM by the accumulating MMAs; the accumulators live in columns the group has already
 //     consumed (dQ or dV at [192,256), dK at [64,128)); later column groups reuse [0,96) / [96,192) (dQ) or
 //     [0,64) / [128,192) (dKV) - the tensor pipe executes in issue order, so a group's S MMAs may be issued right
 //     behind the accumulating MMAs that read the columns they overwrite;
@@ -58,9 +58,9 @@ constexpr int kNumBars = 14;
 constexpr int kSmemMax = 232448;
 
 struct BwsParams {
-  const __nv_bfloat16* out;
+  const void* out;  // element type T of the kernel
   const float* lse;
-  __nv_bfloat16* d_planes;
+  void* d_planes;   // T
   int B, H, N;
   float scale, scale_log2;
   int total_items;
@@ -71,24 +71,25 @@ __device__ __forceinline__ void dbg_stamp(const BwsParams& p, int region, int id
   if (p.dbg != nullptr && blockIdx.x == 0 && idx < 256) p.dbg[region * 256 + idx] = clock64();
 }
 
-// Store this thread's row (64 fp32 channels in two 32-register halves) as 128 bytes of bf16.
-__device__ __forceinline__ void store_row(__nv_bfloat16* dst, const uint32_t (&lo)[32], const uint32_t (&hi)[32], float mul) {
+// Store this thread's row (64 fp32 channels in two 32-register halves) as 128 bytes of T.
+template <typename T>
+__device__ __forceinline__ void store_row(T* dst, const uint32_t (&lo)[32], const uint32_t (&hi)[32], float mul) {
 #pragma unroll
   for (int v8 = 0; v8 < 4; ++v8) {
     uint4 w;
-    w.x = pack_bf16(__uint_as_float(lo[v8 * 8 + 0]) * mul, __uint_as_float(lo[v8 * 8 + 1]) * mul);
-    w.y = pack_bf16(__uint_as_float(lo[v8 * 8 + 2]) * mul, __uint_as_float(lo[v8 * 8 + 3]) * mul);
-    w.z = pack_bf16(__uint_as_float(lo[v8 * 8 + 4]) * mul, __uint_as_float(lo[v8 * 8 + 5]) * mul);
-    w.w = pack_bf16(__uint_as_float(lo[v8 * 8 + 6]) * mul, __uint_as_float(lo[v8 * 8 + 7]) * mul);
+    w.x = Elem16<T>::pack2(__uint_as_float(lo[v8 * 8 + 0]) * mul, __uint_as_float(lo[v8 * 8 + 1]) * mul);
+    w.y = Elem16<T>::pack2(__uint_as_float(lo[v8 * 8 + 2]) * mul, __uint_as_float(lo[v8 * 8 + 3]) * mul);
+    w.z = Elem16<T>::pack2(__uint_as_float(lo[v8 * 8 + 4]) * mul, __uint_as_float(lo[v8 * 8 + 5]) * mul);
+    w.w = Elem16<T>::pack2(__uint_as_float(lo[v8 * 8 + 6]) * mul, __uint_as_float(lo[v8 * 8 + 7]) * mul);
     *reinterpret_cast<uint4*>(dst + v8 * 8) = w;
   }
 #pragma unroll
   for (int v8 = 0; v8 < 4; ++v8) {
     uint4 w;
-    w.x = pack_bf16(__uint_as_float(hi[v8 * 8 + 0]) * mul, __uint_as_float(hi[v8 * 8 + 1]) * mul);
-    w.y = pack_bf16(__uint_as_float(hi[v8 * 8 + 2]) * mul, __uint_as_float(hi[v8 * 8 + 3]) * mul);
-    w.z = pack_bf16(__uint_as_float(hi[v8 * 8 + 4]) * mul, __uint_as_float(hi[v8 * 8 + 5]) * mul);
-    w.w = pack_bf16(__uint_as_float(hi[v8 * 8 + 6]) * mul, __uint_as_float(hi[v8 * 8 + 7]) * mul);
+    w.x = Elem16<T>::pack2(__uint_as_float(hi[v8 * 8 + 0]) * mul, __uint_as_float(hi[v8 * 8 + 1]) * mul);
+    w.y = Elem16<T>::pack2(__uint_as_float(hi[v8 * 8 + 2]) * mul, __uint_as_float(hi[v8 * 8 + 3]) * mul);
+    w.z = Elem16<T>::pack2(__uint_as_float(hi[v8 * 8 + 4]) * mul, __uint_as_float(hi[v8 * 8 + 5]) * mul);
+    w.w = Elem16<T>::pack2(__uint_as_float(hi[v8 * 8 + 6]) * mul, __uint_as_float(hi[v8 * 8 + 7]) * mul);
     *reinterpret_cast<uint4*>(dst + 32 + v8 * 8) = w;
   }
 }
@@ -96,10 +97,10 @@ __device__ __forceinline__ void store_row(__nv_bfloat16* dst, const uint32_t (&l
 // One column group of a lane tile for one thread (= one TMEM lane), 16 accumulator columns at a time with the NEXT
 // 16 columns' tcgen05.ld in flight while the current ones are processed (two register buffers, A / B).
 //   DQ  (lane = query row i, column = key j):  dS = exp2(S c - lse2_i) (dP - delta_i), keys past N masked;
-//        dS (bf16 pairs) written over the S columns.
+//        dS (pairs of T) written over the S columns.
 //   !DQ (lane = key j, column = query row i):  per-column (lse2_i, delta_i) from shared memory (lse2 = +inf past N
-//        -> P = 0);  P^T (bf16) over the S^T columns, dS^T (bf16) over the dP^T columns.
-template <bool DQ>
+//        -> P = 0);  P^T (T) over the S^T columns, dS^T (T) over the dP^T columns.
+template <typename T, bool DQ>
 __device__ __forceinline__ void process16(const BwsParams& p, const uint32_t (&s)[16], const uint32_t (&d)[16], uint32_t t_dst_p,
                                           uint32_t t_dst_ds, int col0, float neg_lse2, float delta, const float4* stats2) {
   uint32_t pp[8], pd[8];
@@ -113,7 +114,7 @@ __device__ __forceinline__ void process16(const BwsParams& p, const uint32_t (&s
         p0 = col0 + e < p.N ? p0 : 0.f;
         p1 = col0 + e + 1 < p.N ? p1 : 0.f;
       }
-      pd[e >> 1] = pack_bf16(p0 * (__uint_as_float(d[e]) - delta), p1 * (__uint_as_float(d[e + 1]) - delta));
+      pd[e >> 1] = Elem16<T>::pack2(p0 * (__uint_as_float(d[e]) - delta), p1 * (__uint_as_float(d[e + 1]) - delta));
     }
     tmem_st8(t_dst_p, pd);
   } else {
@@ -122,15 +123,15 @@ __device__ __forceinline__ void process16(const BwsParams& p, const uint32_t (&s
       const float4 st = stats2[e >> 1];  // (lse2, delta) of rows col0+e and col0+e+1
       const float p0 = ex2(fmaf(__uint_as_float(s[e]), p.scale_log2, -st.x));
       const float p1 = ex2(fmaf(__uint_as_float(s[e + 1]), p.scale_log2, -st.z));
-      pp[e >> 1] = pack_bf16(p0, p1);
-      pd[e >> 1] = pack_bf16(p0 * (__uint_as_float(d[e]) - st.y), p1 * (__uint_as_float(d[e + 1]) - st.w));
+      pp[e >> 1] = Elem16<T>::pack2(p0, p1);
+      pd[e >> 1] = Elem16<T>::pack2(p0 * (__uint_as_float(d[e]) - st.y), p1 * (__uint_as_float(d[e + 1]) - st.w));
     }
     tmem_st8(t_dst_p, pp);
     tmem_st8(t_dst_ds, pd);
   }
 }
 
-template <bool DQ>
+template <typename T, bool DQ>
 __device__ __forceinline__ void process_group(const BwsParams& p, uint32_t t_s, uint32_t t_dp, int n16, int col0, float neg_lse2,
                                               float delta, const float4* stats2) {
   // (a version with the next chunk's tcgen05.ld in flight behind a second register buffer measured SLOWER: 3 400 vs
@@ -141,7 +142,7 @@ __device__ __forceinline__ void process_group(const BwsParams& p, uint32_t t_s, 
     tmem_ld16(t_s + c * 16, s);
     tmem_ld16(t_dp + c * 16, d);
     tmem_wait_ld();
-    process16<DQ>(p, s, d, t_s + c * 8, t_dp + c * 8, col0 + c * 16, neg_lse2, delta, stats2 + c * 8);
+    process16<T, DQ>(p, s, d, t_s + c * 8, t_dp + c * 8, col0 + c * 16, neg_lse2, delta, stats2 + c * 8);
   }
 }
 
@@ -170,6 +171,7 @@ __device__ __forceinline__ ColGroup group_at(bool is_dq, int npad, int gi) {
   return g;
 }
 
+template <typename T>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_bwd_ws_kernel(const __grid_constant__ CUtensorMap tm_pl64, const __grid_constant__ CUtensorMap tm_pl16,
                    const __grid_constant__ CUtensorMap tm_do64, const __grid_constant__ CUtensorMap tm_do16,
@@ -253,9 +255,9 @@ attn_bwd_ws_kernel(const __grid_constant__ CUtensorMap tm_pl64, const __grid_con
   } else if (warp == 9 || warp == 10) {
     // ============================================ MMA issuer of stream w ==================================
     const int w = warp - 9;
-    const uint32_t T = tmem_base + (uint32_t)(w * 256);
+    const uint32_t tw = tmem_base + (uint32_t)(w * 256);
     const uint32_t smem_b = smem_u32(smem);
-    constexpr uint32_t idesc_acc = idesc_bf16(128, kDh, 0, 1);
+    constexpr uint32_t idesc_acc = idesc_16<T>(128, kDh, 0, 1);
     uint32_t ng = 0, nt = 0;  // column groups / lane tiles issued so far by this stream (barrier phases)
     int k = 0;
     for (int bh = blockIdx.x; bh < total; bh += gridDim.x, ++k) {
@@ -277,13 +279,13 @@ attn_bwd_ws_kernel(const __grid_constant__ CUtensorMap tm_pl64, const __grid_con
           const bool first = gi == 0;
           const bool last = gi == ngr - 1;
           if (elect_one()) {
-            const uint32_t idesc = idesc_bf16(128, g.cw, 0, 0);
+            const uint32_t idesc = idesc_16<T>(128, g.cw, 0, 0);
             const uint64_t das = smem_desc_sw128(a_s), dap = smem_desc_sw128(a_p);
             const uint64_t dbs = smem_desc_sw128(b_s + g.c0 * 128), dbp = smem_desc_sw128(b_p + g.c0 * 128);
 #pragma unroll
-            for (int kk = 0; kk < 4; ++kk) mma_ss(T, das + 2 * kk, dbs + 2 * kk, idesc, kk > 0);
+            for (int kk = 0; kk < 4; ++kk) mma_ss(tw, das + 2 * kk, dbs + 2 * kk, idesc, kk > 0);
 #pragma unroll
-            for (int kk = 0; kk < 4; ++kk) mma_ss(T + g.dp_off, dap + 2 * kk, dbp + 2 * kk, idesc, kk > 0);
+            for (int kk = 0; kk < 4; ++kk) mma_ss(tw + g.dp_off, dap + 2 * kk, dbp + 2 * kk, idesc, kk > 0);
             mma_commit(&bar_sfull[w]);
           }
           __syncwarp();
@@ -295,13 +297,13 @@ attn_bwd_ws_kernel(const __grid_constant__ CUtensorMap tm_pl64, const __grid_con
             if (is_dq) {
               const uint64_t dk = smem_desc_sw128(k_b) + adv;
               for (int kk = 0; kk < ksteps; ++kk)  // dQ += dS K
-                mma_ts(T + 192, T + kk * 8, dk + 128 * kk, idesc_acc, (!first || kk > 0) ? 1u : 0u);
+                mma_ts(tw + 192, tw + kk * 8, dk + 128 * kk, idesc_acc, (!first || kk > 0) ? 1u : 0u);
             } else {
               const uint64_t dg = smem_desc_sw128(g_b) + adv, dq = smem_desc_sw128(q_b) + adv;
               for (int kk = 0; kk < ksteps; ++kk)  // dV += P^T dO
-                mma_ts(T + 192, T + kk * 8, dg + 128 * kk, idesc_acc, (!first || kk > 0) ? 1u : 0u);
+                mma_ts(tw + 192, tw + kk * 8, dg + 128 * kk, idesc_acc, (!first || kk > 0) ? 1u : 0u);
               for (int kk = 0; kk < ksteps; ++kk)  // dK += dS^T Q
-                mma_ts(T + 64, T + g.dp_off + kk * 8, dq + 128 * kk, idesc_acc, (!first || kk > 0) ? 1u : 0u);
+                mma_ts(tw + 64, tw + g.dp_off + kk * 8, dq + 128 * kk, idesc_acc, (!first || kk > 0) ? 1u : 0u);
             }
             if (last) mma_commit(&bar_accfull[w]);
           }
@@ -329,7 +331,7 @@ attn_bwd_ws_kernel(const __grid_constant__ CUtensorMap tm_pl64, const __grid_con
         const int i = r0 + lane;
         float2 v = make_float2(INFINITY, 0.f);
         if (i < N) {
-          const uint4* o4 = reinterpret_cast<const uint4*>(p.out + ((size_t)b * N + i) * E + h * kDh);
+          const uint4* o4 = reinterpret_cast<const uint4*>(static_cast<const T*>(p.out) + ((size_t)b * N + i) * E + h * kDh);
           const uint8_t* grow = sG + i * 128;
           float acc = 0.f;
 #pragma unroll
@@ -339,8 +341,8 @@ attn_bwd_ws_kernel(const __grid_constant__ CUtensorMap tm_pl64, const __grid_con
             const uint32_t ow[4] = {ov.x, ov.y, ov.z, ov.w}, gw[4] = {gv.x, gv.y, gv.z, gv.w};
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
-              const float2 of = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&ow[e]));
-              const float2 gf = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&gw[e]));
+              const float2 of = Elem16<T>::unpack2(ow[e]);
+              const float2 gf = Elem16<T>::unpack2(gw[e]);
               acc = fmaf(of.x, gf.x, acc);
               acc = fmaf(of.y, gf.y, acc);
             }
@@ -382,8 +384,8 @@ attn_bwd_ws_kernel(const __grid_constant__ CUtensorMap tm_pl64, const __grid_con
           if (dbg_on) dbg_stamp(p, w, (int)ng * 4 + 1);
           if (warp_live) {
             const float4* st2 = reinterpret_cast<const float4*>(st + g.c0);
-            if (is_dq) process_group<true>(p, trow, trow + g.dp_off, g.cw >> 4, g.c0, neg_lse2, delta, st2);
-            else process_group<false>(p, trow, trow + g.dp_off, g.cw >> 4, g.c0, neg_lse2, delta, st2);
+            if (is_dq) process_group<T, true>(p, trow, trow + g.dp_off, g.cw >> 4, g.c0, neg_lse2, delta, st2);
+            else process_group<T, false>(p, trow, trow + g.dp_off, g.cw >> 4, g.c0, neg_lse2, delta, st2);
             tmem_wait_st();
           }
           tc_fence_before();
@@ -409,7 +411,7 @@ attn_bwd_ws_kernel(const __grid_constant__ CUtensorMap tm_pl64, const __grid_con
               tc_fence_before();
               mbar_arrive(&bar_accempty[w]);
             }
-            if (idx < N) store_row(p.d_planes + (is_dq ? 0 : 2) * plane + ((size_t)bh * N + idx) * kDh, a0, a1, is_dq ? p.scale : 1.f);
+            if (idx < N) store_row(static_cast<T*>(p.d_planes) + (is_dq ? 0 : 2) * plane + ((size_t)bh * N + idx) * kDh, a0, a1, is_dq ? p.scale : 1.f);
             if (dbg_on && w == 0) dbg_stamp(p, 3, (int)nt * 4 + 2);
           }
           if (!is_dq) {
@@ -419,7 +421,7 @@ attn_bwd_ws_kernel(const __grid_constant__ CUtensorMap tm_pl64, const __grid_con
             tmem_wait_ld();
             tc_fence_before();
             mbar_arrive(&bar_accempty[w]);
-            if (idx < N) store_row(p.d_planes + plane + ((size_t)bh * N + idx) * kDh, b0, b1, p.scale);
+            if (idx < N) store_row(static_cast<T*>(p.d_planes) + plane + ((size_t)bh * N + idx) * kDh, b0, b1, p.scale);
             if (dbg_on && w == 0) dbg_stamp(p, 3, (int)nt * 4 + 3);
           }
         } else {
@@ -457,22 +459,22 @@ bool attn_bwd_ws_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bia
   return bws_smem_bytes(N) <= (size_t)kSmemMax;
 }
 
-int attn_bwd_ws(const void* planes, const void* out, const void* d_out, const float* lse, void* d_planes, int B, int H,
-                int N, int Dh, float scale, cudaStream_t st) {
-  (void)Dh;
+template <typename T>
+static int attn_bwd_ws_t(const void* planes, const void* out, const void* d_out, const float* lse, void* d_planes, int B,
+                         int H, int N, float scale, cudaStream_t st) {
   VRR_REQUIRE(((uintptr_t)planes & 15) == 0 && ((uintptr_t)out & 15) == 0 && ((uintptr_t)d_out & 15) == 0 &&
                   ((uintptr_t)d_planes & 15) == 0,
               VRR_ERR_INVALID_ARG, "attn_bwd (tcgen05): planes / out / d_out / d_planes must be 16-byte aligned");
   const int E = H * kDh;
   CUtensorMap tm_pl64, tm_pl16, tm_do64, tm_do16;
-  if (int rc = make_tmap_2d(&tm_pl64, planes, 2, (uint64_t)3 * B * H * N, kDh, kDh * 2, 64, 64)) return rc;
-  if (int rc = make_tmap_2d(&tm_pl16, planes, 2, (uint64_t)3 * B * H * N, kDh, kDh * 2, 16, 64)) return rc;
-  if (int rc = make_tmap_2d(&tm_do64, d_out, 2, (uint64_t)B * N, (uint64_t)E, (uint64_t)E * 2, 64, 64)) return rc;
-  if (int rc = make_tmap_2d(&tm_do16, d_out, 2, (uint64_t)B * N, (uint64_t)E, (uint64_t)E * 2, 16, 64)) return rc;
+  if (int rc = make_tmap_2d(&tm_pl64, planes, Elem16<T>::kTmap, (uint64_t)3 * B * H * N, kDh, kDh * 2, 64, 64)) return rc;
+  if (int rc = make_tmap_2d(&tm_pl16, planes, Elem16<T>::kTmap, (uint64_t)3 * B * H * N, kDh, kDh * 2, 16, 64)) return rc;
+  if (int rc = make_tmap_2d(&tm_do64, d_out, Elem16<T>::kTmap, (uint64_t)B * N, (uint64_t)E, (uint64_t)E * 2, 64, 64)) return rc;
+  if (int rc = make_tmap_2d(&tm_do16, d_out, Elem16<T>::kTmap, (uint64_t)B * N, (uint64_t)E, (uint64_t)E * 2, 16, 64)) return rc;
   BwsParams p;
-  p.out = (const __nv_bfloat16*)out;
+  p.out = out;
   p.lse = lse;
-  p.d_planes = (__nv_bfloat16*)d_planes;
+  p.d_planes = d_planes;
   p.B = B; p.H = H; p.N = N;
   p.scale = scale;
   p.scale_log2 = scale * kLog2e;
@@ -480,10 +482,17 @@ int attn_bwd_ws(const void* planes, const void* out, const void* d_out, const fl
   p.dbg = g_bws_dbg.load();
   const size_t smem = bws_smem_bytes(N);
   const int grid = p.total_items < sm_count() ? p.total_items : sm_count();
-  VRR_SMEM_ATTR_ONCE(attn_bwd_ws_kernel, kSmemMax);
-  attn_bwd_ws_kernel<<<grid, kThreads, smem, st>>>(tm_pl64, tm_pl16, tm_do64, tm_do16, p);
+  VRR_SMEM_ATTR_ONCE(attn_bwd_ws_kernel<T>, kSmemMax);
+  attn_bwd_ws_kernel<T><<<grid, kThreads, smem, st>>>(tm_pl64, tm_pl16, tm_do64, tm_do16, p);
   VRR_LAUNCHED();
   return VRR_OK;
+}
+
+int attn_bwd_ws(const void* planes, const void* out, const void* d_out, const float* lse, void* d_planes, int B, int H,
+                int N, int Dh, float scale, int dtype, cudaStream_t st) {
+  (void)Dh;
+  if (dtype == VRR_F16) return attn_bwd_ws_t<__half>(planes, out, d_out, lse, d_planes, B, H, N, scale, st);
+  return attn_bwd_ws_t<__nv_bfloat16>(planes, out, d_out, lse, d_planes, B, H, N, scale, st);
 }
 
 }  // namespace vrr

@@ -14,9 +14,9 @@
 //     warp, so the groups drift out of phase and one group's exponentials overlap the other's MMAs and epilogue;
 //   * S = Q K^T for a 128-row tile against ALL keys is 4 tcgen05.mma (M 128, N = round16(N) <= 256, K 16) into
 //     TMEM columns [0, N); the softmax is exact two-pass (row max, then exponentials) straight out of TMEM - no
-//     online rescaling; P (bf16) is written in place over S; O = P V is N/16 tcgen05.mma with A = P from TMEM into
+//     online rescaling; P (bf16 / fp16) is written in place over S; O = P V is N/16 tcgen05.mma with A = P from TMEM into
 //     columns [192, 256), which S no longer needs by then;
-//   * epilogue: O / l -> bf16 -> 128-byte-swizzled staging -> one TMA store per warp through a 3-D map of
+//   * epilogue: O / l -> bf16 / fp16 -> 128-byte-swizzled staging -> one TMA store per warp through a 3-D map of
 //     out[B][N][E] (rows past N are clipped by the hardware), so every global write is a full line.
 // Bias: the head's relative-position table row is staged by a TMA bulk copy issued by the producer warp one item
 // ahead (positional_encoding.py:58-75,93); the polynomial bias is a per-head distance LUT (:127-171).
@@ -113,8 +113,9 @@ struct Pass1 {
   }
 };
 
-// pass 2: exponentials against the row max, row sum, P (bf16 pairs) written in place over S; masked keys hold -inf
+// pass 2: exponentials against the row max, row sum, P (pairs of T) written in place over S; masked keys hold -inf
 // from pass 1
+template <typename T>
 struct Pass2 {
   uint32_t t_s;
   float neg_m;
@@ -130,14 +131,14 @@ struct Pass2 {
         const float p0 = ex2(__uint_as_float(s[jl]) + neg_m), p1 = ex2(__uint_as_float(s[jl + 1]) + neg_m);
         ls[0] += p0;
         ls[1] += p1;
-        packed[e] = pack_bf16(p0, p1);
+        packed[e] = Elem16<T>::pack2(p0, p1);
       }
       tmem_st8(t_s + (j0 >> 1) + q * 8, packed);
     }
   }
 };
 
-template <int BIAS>
+template <typename T, int BIAS>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_fwd_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_out,
                    const __grid_constant__ WsParams p) {
@@ -248,8 +249,8 @@ attn_fwd_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
     const int w = warp - 9;
     if (w < nwg) {
       const uint32_t tmem_w = tmem_base + (uint32_t)(w * 256);
-      const uint32_t idesc_s = idesc_bf16(128, npad, 0, 0);
-      constexpr uint32_t idesc_o = idesc_bf16(128, kDh, 0, 1);
+      const uint32_t idesc_s = idesc_16<T>(128, npad, 0, 0);
+      constexpr uint32_t idesc_o = idesc_16<T>(128, kDh, 0, 1);
       const uint64_t dq = smem_desc_sw128(smem_u32(sQ + w * (128 * kDh * 2)));
       const int ksteps = npad >> 4;
       int k = 0;
@@ -343,7 +344,7 @@ attn_fwd_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
         for_chunks(tmem_row, nch32, tail16, p1);
         m_row = fmaxf(fmaxf(p1.tm[0], p1.tm[1]), fmaxf(p1.tm[2], p1.tm[3]));
         tmem_wait_st();
-        Pass2 p2{tmem_row, -m_row, {0.f, 0.f}};
+        Pass2<T> p2{tmem_row, -m_row, {0.f, 0.f}};
         for_chunks(tmem_row, nch32, tail16, p2);
         l_row = p2.ls[0] + p2.ls[1];
         tmem_wait_st();
@@ -351,7 +352,7 @@ attn_fwd_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
       tc_fence_before();
       mbar_arrive(&bar_pfull[w]);
 
-      // ---- epilogue: O / l -> bf16 -> swizzled staging -> TMA store; lse ---------------------------
+      // ---- epilogue: O / l -> T -> swizzled staging -> TMA store; lse ---------------------------
       mbar_wait(&bar_ofull[w], par);
       tc_fence_after();
       uint32_t olo[32], ohi[32];
@@ -371,17 +372,17 @@ attn_fwd_ws_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
 #pragma unroll
         for (int c8 = 0; c8 < 4; ++c8)
           st_shared_v4(row_base + (((uint32_t)c8 ^ sw) << 4),
-                       pack_bf16(__uint_as_float(olo[c8 * 8 + 0]) * inv, __uint_as_float(olo[c8 * 8 + 1]) * inv),
-                       pack_bf16(__uint_as_float(olo[c8 * 8 + 2]) * inv, __uint_as_float(olo[c8 * 8 + 3]) * inv),
-                       pack_bf16(__uint_as_float(olo[c8 * 8 + 4]) * inv, __uint_as_float(olo[c8 * 8 + 5]) * inv),
-                       pack_bf16(__uint_as_float(olo[c8 * 8 + 6]) * inv, __uint_as_float(olo[c8 * 8 + 7]) * inv));
+                       Elem16<T>::pack2(__uint_as_float(olo[c8 * 8 + 0]) * inv, __uint_as_float(olo[c8 * 8 + 1]) * inv),
+                       Elem16<T>::pack2(__uint_as_float(olo[c8 * 8 + 2]) * inv, __uint_as_float(olo[c8 * 8 + 3]) * inv),
+                       Elem16<T>::pack2(__uint_as_float(olo[c8 * 8 + 4]) * inv, __uint_as_float(olo[c8 * 8 + 5]) * inv),
+                       Elem16<T>::pack2(__uint_as_float(olo[c8 * 8 + 6]) * inv, __uint_as_float(olo[c8 * 8 + 7]) * inv));
 #pragma unroll
         for (int c8 = 0; c8 < 4; ++c8)
           st_shared_v4(row_base + (((uint32_t)(c8 + 4) ^ sw) << 4),
-                       pack_bf16(__uint_as_float(ohi[c8 * 8 + 0]) * inv, __uint_as_float(ohi[c8 * 8 + 1]) * inv),
-                       pack_bf16(__uint_as_float(ohi[c8 * 8 + 2]) * inv, __uint_as_float(ohi[c8 * 8 + 3]) * inv),
-                       pack_bf16(__uint_as_float(ohi[c8 * 8 + 4]) * inv, __uint_as_float(ohi[c8 * 8 + 5]) * inv),
-                       pack_bf16(__uint_as_float(ohi[c8 * 8 + 6]) * inv, __uint_as_float(ohi[c8 * 8 + 7]) * inv));
+                       Elem16<T>::pack2(__uint_as_float(ohi[c8 * 8 + 0]) * inv, __uint_as_float(ohi[c8 * 8 + 1]) * inv),
+                       Elem16<T>::pack2(__uint_as_float(ohi[c8 * 8 + 2]) * inv, __uint_as_float(ohi[c8 * 8 + 3]) * inv),
+                       Elem16<T>::pack2(__uint_as_float(ohi[c8 * 8 + 4]) * inv, __uint_as_float(ohi[c8 * 8 + 5]) * inv),
+                       Elem16<T>::pack2(__uint_as_float(ohi[c8 * 8 + 6]) * inv, __uint_as_float(ohi[c8 * 8 + 7]) * inv));
         fence_proxy_async_smem();
         __syncwarp();
         if (store_leader) {
@@ -413,11 +414,11 @@ size_t ws_smem_bytes(int N, const vrr_bias_desc* bias, int* lut_floats, int* raw
   return 1024 + (size_t)5 * kSeqBytes + 8 * 4096 + (size_t)(rf + 2 * lf) * 4 + yx + (size_t)kNumBars * 8 + 16;
 }
 
-template <int MODE>
+template <typename T, int MODE>
 int ws_launch(const CUtensorMap& tmap, const CUtensorMap& tmap_out, const WsParams& p, int grid, size_t smem,
               cudaStream_t st) {
-  VRR_SMEM_ATTR_ONCE(attn_fwd_ws_kernel<MODE>, kSmemMax);
-  attn_fwd_ws_kernel<MODE><<<grid, kThreads, smem, st>>>(tmap, tmap_out, p);
+  VRR_SMEM_ATTR_ONCE((attn_fwd_ws_kernel<T, MODE>), kSmemMax);
+  attn_fwd_ws_kernel<T, MODE><<<grid, kThreads, smem, st>>>(tmap, tmap_out, p);
   VRR_LAUNCHED();
   return VRR_OK;
 }
@@ -432,15 +433,16 @@ bool attn_fwd_ws_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bia
   return ws_smem_bytes(N, bias, nullptr, nullptr) <= (size_t)kSmemMax;
 }
 
-int attn_fwd_ws(const void* planes, const vrr_bias_desc* bias, void* out, float* lse, int B, int H, int N, int Dh,
-                float scale, cudaStream_t st) {
-  (void)Dh;
+template <typename T>
+static int attn_fwd_ws_t(const void* planes, const vrr_bias_desc* bias, void* out, float* lse, int B, int H, int N,
+                         float scale, cudaStream_t st) {
   VRR_REQUIRE(((uintptr_t)planes & 15) == 0 && ((uintptr_t)out & 15) == 0, VRR_ERR_INVALID_ARG,
               "attn_fwd (tcgen05): planes/out must be 16-byte aligned");
   CUtensorMap tmap, tmap_out;
-  if (int rc = make_tmap_2d(&tmap, planes, 2, (uint64_t)3 * B * H * N, kDh, kDh * 2, 64, 64)) return rc;
+  if (int rc = make_tmap_2d(&tmap, planes, Elem16<T>::kTmap, (uint64_t)3 * B * H * N, kDh, kDh * 2, 64, 64)) return rc;
   const uint64_t E = (uint64_t)H * kDh;
-  if (int rc = make_tmap_3d_bf16(&tmap_out, out, E, (uint64_t)N, (uint64_t)B, E * 2, (uint64_t)N * E * 2, kDh, 32)) return rc;
+  if (int rc = make_tmap_3d(&tmap_out, out, Elem16<T>::kTmap, E, (uint64_t)N, (uint64_t)B, E * 2, (uint64_t)N * E * 2, kDh, 32))
+    return rc;
   WsParams p;
   p.lse = lse;
   p.B = B; p.H = H; p.N = N;
@@ -455,8 +457,15 @@ int attn_fwd_ws(const void* planes, const vrr_bias_desc* bias, void* out, float*
   p.total_items = B * H;
   const size_t smem = ws_smem_bytes(N, bias, &p.lut_floats, &p.raw_floats);
   const int grid = p.total_items < sm_count() ? p.total_items : sm_count();
-  if (mode == VRR_BIAS_TABLE) return ws_launch<VRR_BIAS_TABLE>(tmap, tmap_out, p, grid, smem, st);
-  return ws_launch<VRR_BIAS_POLY>(tmap, tmap_out, p, grid, smem, st);
+  if (mode == VRR_BIAS_TABLE) return ws_launch<T, VRR_BIAS_TABLE>(tmap, tmap_out, p, grid, smem, st);
+  return ws_launch<T, VRR_BIAS_POLY>(tmap, tmap_out, p, grid, smem, st);
+}
+
+int attn_fwd_ws(const void* planes, const vrr_bias_desc* bias, void* out, float* lse, int B, int H, int N, int Dh,
+                float scale, int dtype, cudaStream_t st) {
+  (void)Dh;
+  if (dtype == VRR_F16) return attn_fwd_ws_t<__half>(planes, bias, out, lse, B, H, N, scale, st);
+  return attn_fwd_ws_t<__nv_bfloat16>(planes, bias, out, lse, B, H, N, scale, st);
 }
 
 }  // namespace vrr

@@ -452,10 +452,14 @@ static int bwd_launch(const void* planes, const vrr_bias_desc* bias, const void*
       if ((DHv) == 16) return CALL(float, 16);                                   \
       if ((DHv) == 32) return CALL(float, 32);                                   \
       if ((DHv) == 64) return CALL(float, 64);                                   \
-    } else {                                                                     \
+    } else if ((dtype) == VRR_BF16) {                                            \
       if ((DHv) == 16) return CALL(__nv_bfloat16, 16);                           \
       if ((DHv) == 32) return CALL(__nv_bfloat16, 32);                           \
       if ((DHv) == 64) return CALL(__nv_bfloat16, 64);                           \
+    } else {                                                                     \
+      if ((DHv) == 16) return CALL(__half, 16);                                  \
+      if ((DHv) == 32) return CALL(__half, 32);                                  \
+      if ((DHv) == 64) return CALL(__half, 64);                                  \
     }                                                                            \
   } while (0)
 

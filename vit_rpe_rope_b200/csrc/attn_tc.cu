@@ -1,5 +1,5 @@
-// Fused attention forward on the 5th-generation tensor cores (tcgen05 + TMEM), bf16, head dim 64, tiled over the
-// keys: every N without bias, and N > 256 with a bias (attn_fwd_ws.cu takes the shorter biased sequences).
+// Fused attention forward on the 5th-generation tensor cores (tcgen05 + TMEM), bf16 or fp16, head dim 64, tiled over
+// the keys: every N without bias, and N > 256 with a bias (attn_fwd_ws.cu takes the shorter biased sequences).
 //
 // Replaces models/vit.py:71-88 of the reference: S = q k^T * scale (+ relative-position table /
 // polynomial bias) -> softmax -> . v -> merge heads, without materialising S or P in HBM.
@@ -7,7 +7,7 @@
 // Both kernels: one CTA = 128 query rows of one (image, head), 160 threads - warps 0-3 softmax (thread t = query
 // row t = TMEM lane t), warp 4 the issuer of every TMA load and tcgen05.mma.  Q and 64-key K / V tiles arrive by
 // TMA (128-byte swizzle); S = Q K^T and O += P V (P from TMEM) accumulate in TMEM, O across all key tiles, with a
-// lazy online-softmax rescale; epilogue O / l -> bf16 -> out[b][i][h*64 ..], lse.
+// lazy online-softmax rescale; epilogue O / l -> bf16 / fp16 -> out[b][i][h*64 ..], lse.
 //   * attn_fwd_tc4_kernel (no bias): one S buffer, 2-stage ring, 128 TMEM columns, ~50 KB of shared memory, four
 //     CTAs per SM;
 //   * attn_fwd_tc2_kernel (relative table / polynomial bias): double-buffered S, 4-stage ring, 256 TMEM columns,
@@ -30,7 +30,7 @@ constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kLn2 = 0.6931471805599453f;
 
 struct FwdParams {
-  __nv_bfloat16* out;
+  void* out;  // element type T of the kernel
   float* lse;
   const float* bias_param;
   int B, H, N;
@@ -49,13 +49,13 @@ struct FwdParams {
 // tile t, and O += P(t) V(t) accumulates in TMEM across ALL key tiles, so the softmax warps never
 // read O until the epilogue.  The running max only has to be a *reference* for exp2: it is updated
 // (and O, l rescaled through tcgen05.ld/st) only when a row's tile max exceeds it by more than 2^8
-// - P <= 256 is harmless in bf16/fp32 - which after the first tile is rare.
+// - P <= 256 is harmless in bf16, fp16 and fp32 - which after the first tile is rare.
 constexpr int kV2KT = 64, kV2Stages = 4, kV2Threads = 160;
 constexpr uint32_t kV2TmemCols = 256, kV2ColO = 128;
 constexpr float kRescaleThreshold = 8.0f;  // log2 units
 constexpr int kV2NumBars = 4 * kV2Stages + 9;
 
-template <int BIAS>
+template <typename T, int BIAS>
 __global__ void __launch_bounds__(kV2Threads, 2)
 attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p) {
   constexpr int kKT = kV2KT, kStages = kV2Stages;
@@ -152,8 +152,8 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
   if (warp == 4) {
     // =========================================== issuer ===========================================
     const uint64_t desc_q = smem_desc_sw128(smem_u32(sQ));
-    constexpr uint32_t idesc_s = idesc_bf16(kM, kKT, 0, 0);
-    constexpr uint32_t idesc_o = idesc_bf16(kM, kDh, 0, 1);
+    constexpr uint32_t idesc_s = idesc_16<T>(kM, kKT, 0, 0);
+    constexpr uint32_t idesc_o = idesc_16<T>(kM, kDh, 0, 1);
     // S(0)
     mbar_wait(bar_q, 0);
     mbar_wait(&bar_kfull[0], 0);
@@ -330,7 +330,7 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
             const float p0 = ex2(a0 + neg_m);
             const float p1 = ex2(a1 + neg_m);
             l_run += p0 + p1;
-            packed[e] = pack_bf16(p0, p1);
+            packed[e] = Elem16<T>::pack2(p0, p1);
           }
           tmem_st16(tmem_row + sb * kKT + c * 16, packed);  // P over the first half of this S buffer
         }
@@ -352,15 +352,15 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
       tmem_wait_ld();
       if (i < N) {
         const float inv = 1.f / l_run;
-        __nv_bfloat16* dst = p.out + ((size_t)b * N + i) * (size_t)(H * kDh) + h * kDh;
+        T* dst = static_cast<T*>(p.out) + ((size_t)b * N + i) * (size_t)(H * kDh) + h * kDh;
 #pragma unroll
         for (int v8 = 0; v8 < 8; ++v8) {
           const uint32_t* src = v8 < 4 ? &lo[v8 * 8] : &hi[(v8 - 4) * 8];
           uint4 w;
-          w.x = pack_bf16(__uint_as_float(src[0]) * inv, __uint_as_float(src[1]) * inv);
-          w.y = pack_bf16(__uint_as_float(src[2]) * inv, __uint_as_float(src[3]) * inv);
-          w.z = pack_bf16(__uint_as_float(src[4]) * inv, __uint_as_float(src[5]) * inv);
-          w.w = pack_bf16(__uint_as_float(src[6]) * inv, __uint_as_float(src[7]) * inv);
+          w.x = Elem16<T>::pack2(__uint_as_float(src[0]) * inv, __uint_as_float(src[1]) * inv);
+          w.y = Elem16<T>::pack2(__uint_as_float(src[2]) * inv, __uint_as_float(src[3]) * inv);
+          w.z = Elem16<T>::pack2(__uint_as_float(src[4]) * inv, __uint_as_float(src[5]) * inv);
+          w.w = Elem16<T>::pack2(__uint_as_float(src[6]) * inv, __uint_as_float(src[7]) * inv);
           *reinterpret_cast<uint4*>(dst + v8 * 8) = w;
         }
         p.lse[(size_t)bh * N + i] = (m_ref + log2f(l_run)) * kLn2;
@@ -405,9 +405,9 @@ __device__ __forceinline__ float v4_max16m(const uint32_t (&r)[16], float mx, in
     return mx;
   }
 }
-// P = 2^(s * scale - m) for 16 scores -> 8 packed bf16x2; the row sum accumulates in l2.  kPolyPairs of the 8 pairs
+// P = 2^(s * scale - m) for 16 scores -> 8 packed pairs of T; the row sum accumulates in l2.  kPolyPairs of the 8 pairs
 // take the polynomial, the others MUFU.EX2.
-template <bool FULL>
+template <typename T, bool FULL>
 __device__ __forceinline__ void v4_exp16(const uint32_t (&r)[16], uint32_t (&pk)[8], float2 sc2, float2 nm2, float2& l2,
                                          int first, int nvalid) {
 #pragma unroll
@@ -421,12 +421,12 @@ __device__ __forceinline__ void v4_exp16(const uint32_t (&r)[16], uint32_t (&pk)
       if (first + 2 * e + 1 >= nvalid) pv.y = 0.f;
     }
     l2 = __fadd2_rn(l2, pv);
-    pk[e] = pack_bf16(pv.x, pv.y);
+    pk[e] = Elem16<T>::pack2(pv.x, pv.y);
   }
 }
 
 // one key tile of one query row: lazy reference-max update, then P over the first 32 of the 64 columns S occupied
-template <bool FULL>
+template <typename T, bool FULL>
 __device__ __forceinline__ void v4_tile(uint32_t trow, int nvalid, int t, float scale_log2, float& m_ref, float& l_run) {
   uint32_t ab[32];
   uint32_t(&a)[16] = *reinterpret_cast<uint32_t(*)[16]>(&ab[0]);
@@ -480,24 +480,24 @@ __device__ __forceinline__ void v4_tile(uint32_t trow, int nvalid, int t, float 
   if (FULL) {
     tmem_wait_ld();
     tmem_ld16(trow + 16, b);
-    v4_exp16<true>(a, pk, sc2, nm2, l2, 0, nvalid);
+    v4_exp16<T, true>(a, pk, sc2, nm2, l2, 0, nvalid);
     tmem_st8(trow, pk);  // columns [0,8): scores already consumed
     tmem_wait_ld();
     tmem_ld16(trow + 32, a);
-    v4_exp16<true>(b, pk, sc2, nm2, l2, 16, nvalid);
+    v4_exp16<T, true>(b, pk, sc2, nm2, l2, 16, nvalid);
     tmem_st8(trow + 8, pk);
     tmem_wait_ld();
     tmem_ld16(trow + 48, b);
-    v4_exp16<true>(a, pk, sc2, nm2, l2, 32, nvalid);
+    v4_exp16<T, true>(a, pk, sc2, nm2, l2, 32, nvalid);
     tmem_st8(trow + 16, pk);
     tmem_wait_ld();
-    v4_exp16<true>(b, pk, sc2, nm2, l2, 48, nvalid);
+    v4_exp16<T, true>(b, pk, sc2, nm2, l2, 48, nvalid);
     tmem_st8(trow + 24, pk);
   } else {
     for (int c = 0; c < nchunks; ++c) {
       if (c > 0) tmem_ld16(trow + c * 16, a);
       tmem_wait_ld();
-      v4_exp16<false>(a, pk, sc2, nm2, l2, c * 16, nvalid);
+      v4_exp16<T, false>(a, pk, sc2, nm2, l2, c * 16, nvalid);
       tmem_st8(trow + c * 8, pk);  // columns [8c, 8c+8) lie below every chunk still to be read
     }
   }
@@ -505,6 +505,7 @@ __device__ __forceinline__ void v4_tile(uint32_t trow, int nvalid, int t, float 
   tmem_wait_st();
 }
 
+template <typename T>
 __global__ void __launch_bounds__(kV4Threads, 4)
 attn_fwd_tc4_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p) {
   constexpr int kKT = kV2KT, kStages = kV4Stages;
@@ -572,14 +573,14 @@ attn_fwd_tc4_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
   if (warp == 4) {
     // =========================================== issuer ===========================================
     const uint64_t desc_q = smem_desc_sw128(smem_u32(sQ));
-    constexpr uint32_t idesc_s = idesc_bf16(kM, kKT, 0, 0);
-    constexpr uint32_t idesc_o = idesc_bf16(kM, kDh, 0, 1);
+    constexpr uint32_t idesc_s = idesc_16<T>(kM, kKT, 0, 0);
+    constexpr uint32_t idesc_o = idesc_16<T>(kM, kDh, 0, 1);
     mbar_wait(bar_q, 0);
     mbar_wait(&bar_kfull[0], 0);
     tc_fence_after();
     // the ragged last tile is a narrow MMA: N = round16(valid keys) instead of 64
     const int last_cols = (N - (ntiles - 1) * kKT + 15) & ~15;
-    const uint32_t idesc_s_last = idesc_bf16(kM, last_cols, 0, 0);
+    const uint32_t idesc_s_last = idesc_16<T>(kM, last_cols, 0, 0);
     if (elect_one()) {
       const uint64_t desc_k = smem_desc_sw128(smem_u32(sK));
       const uint32_t id0 = ntiles == 1 ? idesc_s_last : idesc_s;
@@ -646,8 +647,8 @@ attn_fwd_tc4_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
       mbar_wait(bar_s, (uint32_t)(t & 1));
       tc_fence_after();
       if (warp_active) {
-        if (nvalid == kKT) v4_tile<true>(tmem_row, nvalid, t, p.scale_log2, m_ref, l_run);
-        else v4_tile<false>(tmem_row, nvalid, t, p.scale_log2, m_ref, l_run);
+        if (nvalid == kKT) v4_tile<T, true>(tmem_row, nvalid, t, p.scale_log2, m_ref, l_run);
+        else v4_tile<T, false>(tmem_row, nvalid, t, p.scale_log2, m_ref, l_run);
       }
       tc_fence_before();
       __syncwarp();
@@ -659,7 +660,7 @@ attn_fwd_tc4_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
     tc_fence_after();
     if (warp_active) {
       const float inv = 1.f / l_run;
-      __nv_bfloat16* dst = p.out + ((size_t)b * N + min(i, N - 1)) * (size_t)(H * kDh) + h * kDh;
+      T* dst = static_cast<T*>(p.out) + ((size_t)b * N + min(i, N - 1)) * (size_t)(H * kDh) + h * kDh;
 #pragma unroll
       for (int half = 0; half < 2; ++half) {
         uint32_t o[32];
@@ -669,10 +670,10 @@ attn_fwd_tc4_kernel(const __grid_constant__ CUtensorMap tmap, const FwdParams p)
 #pragma unroll
           for (int v8 = 0; v8 < 4; ++v8) {
             uint4 w;
-            w.x = pack_bf16(__uint_as_float(o[v8 * 8 + 0]) * inv, __uint_as_float(o[v8 * 8 + 1]) * inv);
-            w.y = pack_bf16(__uint_as_float(o[v8 * 8 + 2]) * inv, __uint_as_float(o[v8 * 8 + 3]) * inv);
-            w.z = pack_bf16(__uint_as_float(o[v8 * 8 + 4]) * inv, __uint_as_float(o[v8 * 8 + 5]) * inv);
-            w.w = pack_bf16(__uint_as_float(o[v8 * 8 + 6]) * inv, __uint_as_float(o[v8 * 8 + 7]) * inv);
+            w.x = Elem16<T>::pack2(__uint_as_float(o[v8 * 8 + 0]) * inv, __uint_as_float(o[v8 * 8 + 1]) * inv);
+            w.y = Elem16<T>::pack2(__uint_as_float(o[v8 * 8 + 2]) * inv, __uint_as_float(o[v8 * 8 + 3]) * inv);
+            w.z = Elem16<T>::pack2(__uint_as_float(o[v8 * 8 + 4]) * inv, __uint_as_float(o[v8 * 8 + 5]) * inv);
+            w.w = Elem16<T>::pack2(__uint_as_float(o[v8 * 8 + 6]) * inv, __uint_as_float(o[v8 * 8 + 7]) * inv);
             *reinterpret_cast<uint4*>(dst + half * 32 + v8 * 8) = w;
           }
         }
@@ -719,7 +720,7 @@ int encode_tiled(EncodeTiledFn* fn_out) {
 
 }  // namespace
 
-int make_tmap_2d(CUtensorMap* map, const void* base, int elem_bytes, uint64_t rows, uint64_t cols,
+int make_tmap_2d(CUtensorMap* map, const void* base, CUtensorMapDataType dtype, uint64_t rows, uint64_t cols,
                  uint64_t row_stride_bytes, uint32_t box_rows, uint32_t box_cols) {
   EncodeTiledFn encode;
   if (int rc = encode_tiled(&encode)) return rc;
@@ -727,8 +728,7 @@ int make_tmap_2d(CUtensorMap* map, const void* base, int elem_bytes, uint64_t ro
   cuuint64_t strides[1] = {row_stride_bytes};
   cuuint32_t box[2] = {box_cols, box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = encode(map, elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2,
-                      const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+  CUresult r = encode(map, dtype, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                       CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   VRR_REQUIRE(r == CUDA_SUCCESS, VRR_ERR_CUDA,
               "cuTensorMapEncodeTiled failed with CUresult %d (rows %llu cols %llu stride %llu box %ux%u)", (int)r,
@@ -736,15 +736,15 @@ int make_tmap_2d(CUtensorMap* map, const void* base, int elem_bytes, uint64_t ro
   return VRR_OK;
 }
 
-int make_tmap_3d_bf16(CUtensorMap* map, const void* base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t stride1_bytes,
-                      uint64_t stride2_bytes, uint32_t box0, uint32_t box1, int swizzle128) {
+int make_tmap_3d(CUtensorMap* map, const void* base, CUtensorMapDataType dtype, uint64_t d0, uint64_t d1, uint64_t d2,
+                 uint64_t stride1_bytes, uint64_t stride2_bytes, uint32_t box0, uint32_t box1, int swizzle128) {
   EncodeTiledFn encode;
   if (int rc = encode_tiled(&encode)) return rc;
   cuuint64_t dims[3] = {d0, d1, d2};
   cuuint64_t strides[2] = {stride1_bytes, stride2_bytes};
   cuuint32_t box[3] = {box0, box1, 1};
   cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
+  CUresult r = encode(map, dtype, 3, const_cast<void*>(base), dims, strides, box, estr,
                       CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE,
                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   VRR_REQUIRE(r == CUDA_SUCCESS, VRR_ERR_CUDA, "cuTensorMapEncodeTiled (3-D) failed with CUresult %d", (int)r);
@@ -760,23 +760,23 @@ bool attn_fwd_tc_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bia
 
 void attn_fwd_tc_set_debug(long long* buf) { g_fwd_dbg.store(buf); }
 
-template <int MODE>
+template <typename T, int MODE>
 static int fwd2_launch_tc(const CUtensorMap& tmap, const FwdParams& p, dim3 grid, size_t smem, cudaStream_t st) {
-  VRR_SMEM_ATTR_ONCE(attn_fwd_tc2_kernel<MODE>, 110 * 1024);
-  attn_fwd_tc2_kernel<MODE><<<grid, kV2Threads, smem, st>>>(tmap, p);
+  VRR_SMEM_ATTR_ONCE((attn_fwd_tc2_kernel<T, MODE>), 110 * 1024);
+  attn_fwd_tc2_kernel<T, MODE><<<grid, kV2Threads, smem, st>>>(tmap, p);
   VRR_LAUNCHED();
   return VRR_OK;
 }
 
-int attn_fwd_tc(const void* planes, const vrr_bias_desc* bias, void* out, float* lse, int B, int H, int N, int Dh,
-                float scale, cudaStream_t st) {
-  (void)Dh;
+template <typename T>
+static int attn_fwd_tc_t(const void* planes, const vrr_bias_desc* bias, void* out, float* lse, int B, int H, int N,
+                         float scale, cudaStream_t st) {
   VRR_REQUIRE(((uintptr_t)planes & 15) == 0 && ((uintptr_t)out & 15) == 0, VRR_ERR_INVALID_ARG,
               "attn_fwd (tcgen05): planes/out must be 16-byte aligned");
   CUtensorMap tmap;
-  if (int rc = make_tmap_2d(&tmap, planes, 2, (uint64_t)3 * B * H * N, kDh, kDh * 2, kV2KT, 64)) return rc;
+  if (int rc = make_tmap_2d(&tmap, planes, Elem16<T>::kTmap, (uint64_t)3 * B * H * N, kDh, kDh * 2, kV2KT, 64)) return rc;
   FwdParams p;
-  p.out = (__nv_bfloat16*)out;
+  p.out = out;
   p.lse = lse;
   p.B = B; p.H = H; p.N = N;
   p.scale_log2 = scale * kLog2e;
@@ -793,14 +793,21 @@ int attn_fwd_tc(const void* planes, const vrr_bias_desc* bias, void* out, float*
     // the bias modes stay on attn_fwd_tc2_kernel: evaluating the bias in both passes made the four-CTA kernel slower
     // there (577 tokens: table 118 vs 82 us, polynomial 175 vs 108 us)
     p.lut_floats = 0;
-    VRR_SMEM_ATTR_ONCE(attn_fwd_tc4_kernel, 64 * 1024);
-    attn_fwd_tc4_kernel<<<grid, kV4Threads, kFwd4SmemBytes, st>>>(tmap, p);
+    VRR_SMEM_ATTR_ONCE(attn_fwd_tc4_kernel<T>, 64 * 1024);
+    attn_fwd_tc4_kernel<T><<<grid, kV4Threads, kFwd4SmemBytes, st>>>(tmap, p);
     VRR_LAUNCHED();
     return VRR_OK;
   }
   const size_t smem2 = fwd2_smem_bytes(N, bias, &p.lut_floats);
-  if (mode == VRR_BIAS_TABLE) return fwd2_launch_tc<VRR_BIAS_TABLE>(tmap, p, grid, smem2, st);
-  return fwd2_launch_tc<VRR_BIAS_POLY>(tmap, p, grid, smem2, st);
+  if (mode == VRR_BIAS_TABLE) return fwd2_launch_tc<T, VRR_BIAS_TABLE>(tmap, p, grid, smem2, st);
+  return fwd2_launch_tc<T, VRR_BIAS_POLY>(tmap, p, grid, smem2, st);
+}
+
+int attn_fwd_tc(const void* planes, const vrr_bias_desc* bias, void* out, float* lse, int B, int H, int N, int Dh,
+                float scale, int dtype, cudaStream_t st) {
+  (void)Dh;
+  if (dtype == VRR_F16) return attn_fwd_tc_t<__half>(planes, bias, out, lse, B, H, N, scale, st);
+  return attn_fwd_tc_t<__nv_bfloat16>(planes, bias, out, lse, B, H, N, scale, st);
 }
 
 }  // namespace vrr

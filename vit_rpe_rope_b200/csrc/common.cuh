@@ -1,6 +1,7 @@
 // Shared host/device helpers for libvrr_b200.so (sm_100a only).
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -56,6 +57,8 @@ bool first_use_on_device(std::atomic<unsigned char>* flags);  // flags: static a
 #define VRR_COUNT_FAMILY(f) ::vrr::g_family_launches[(f)].fetch_add(1, std::memory_order_relaxed)
 
 static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
+// bf16 and fp16 run the same kernels (the tcgen05 family where the shape allows): "a 16-bit dtype"
+static inline bool is16(int dtype) { return dtype == VRR_BF16 || dtype == VRR_F16; }
 
 // ---- element type traits -----------------------------------------------------------------------
 template <typename T>
@@ -64,14 +67,22 @@ template <>
 struct Elem<float> {
   static __device__ __forceinline__ float ld(const float* p) { return *p; }
   static __device__ __forceinline__ void st(float* p, float v) { *p = v; }
+  static __device__ __forceinline__ float round(float v) { return v; }
 };
 template <>
 struct Elem<__nv_bfloat16> {
   static __device__ __forceinline__ float ld(const __nv_bfloat16* p) { return __bfloat162float(*p); }
   static __device__ __forceinline__ void st(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
+  static __device__ __forceinline__ float round(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
+};
+template <>
+struct Elem<__half> {
+  static __device__ __forceinline__ float ld(const __half* p) { return __half2float(*p); }
+  static __device__ __forceinline__ void st(__half* p, float v) { *p = __float2half_rn(v); }
+  static __device__ __forceinline__ float round(float v) { return __half2float(__float2half_rn(v)); }
 };
 
-// Load 4 consecutive elements (16B-aligned for float, 8B for bf16) as floats.
+// Load 4 consecutive elements (16B-aligned for float, 8B for bf16 / fp16) as floats.
 __device__ __forceinline__ float4 ld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
 __device__ __forceinline__ float4 ld4(const __nv_bfloat16* p) {
   uint2 raw = *reinterpret_cast<const uint2*>(p);
@@ -83,6 +94,18 @@ __device__ __forceinline__ float4 ld4(const __nv_bfloat16* p) {
 __device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
 __device__ __forceinline__ void st4(__nv_bfloat16* p, float4 v) {
   __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
+  uint2 raw;
+  raw.x = *reinterpret_cast<uint32_t*>(&a);
+  raw.y = *reinterpret_cast<uint32_t*>(&b);
+  *reinterpret_cast<uint2*>(p) = raw;
+}
+__device__ __forceinline__ float4 ld4(const __half* p) {
+  uint2 raw = *reinterpret_cast<const uint2*>(p);
+  float2 fa = __half22float2(*reinterpret_cast<__half2*>(&raw.x)), fb = __half22float2(*reinterpret_cast<__half2*>(&raw.y));
+  return make_float4(fa.x, fa.y, fb.x, fb.y);
+}
+__device__ __forceinline__ void st4(__half* p, float4 v) {
+  __half2 a = __floats2half2_rn(v.x, v.y), b = __floats2half2_rn(v.z, v.w);
   uint2 raw;
   raw.x = *reinterpret_cast<uint32_t*>(&a);
   raw.y = *reinterpret_cast<uint32_t*>(&b);

@@ -39,6 +39,19 @@ struct CsVec<__nv_bfloat16> {
     }
   }
 };
+template <>
+struct CsVec<__half> {
+  static constexpr int kVec = 8;
+  using Raw = uint4;
+  static __device__ __forceinline__ void add(float (&acc)[8], const uint4& v) {
+    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&w[e]));
+      acc[2 * e] += f.x; acc[2 * e + 1] += f.y;
+    }
+  }
+};
 
 template <typename T>
 __global__ void __launch_bounds__(kCsThreads) colsum_vec_kernel(const T* __restrict__ x, float* __restrict__ out, int M, int C) {
@@ -200,7 +213,8 @@ __global__ void mul_inplace_kernel(T* __restrict__ c, const T* __restrict__ m, s
 int gelu_grad_inplace(void* h, size_t n, int dtype, cudaStream_t st) {
   const int grid = (int)((n + 255) / 256 < 148 * 8 ? (n + 255) / 256 : 148 * 8);
   if (dtype == VRR_F32) gelu_grad_inplace_kernel<float><<<grid, 256, 0, st>>>((float*)h, n);
-  else gelu_grad_inplace_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>((__nv_bfloat16*)h, n);
+  else if (dtype == VRR_BF16) gelu_grad_inplace_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>((__nv_bfloat16*)h, n);
+  else gelu_grad_inplace_kernel<__half><<<grid, 256, 0, st>>>((__half*)h, n);
   VRR_LAUNCHED();
   return VRR_OK;
 }
@@ -208,7 +222,8 @@ int gelu_grad_inplace(void* h, size_t n, int dtype, cudaStream_t st) {
 int mul_inplace(void* c, const void* m, size_t n, int dtype, cudaStream_t st) {
   const int grid = (int)((n + 255) / 256 < 148 * 8 ? (n + 255) / 256 : 148 * 8);
   if (dtype == VRR_F32) mul_inplace_kernel<float><<<grid, 256, 0, st>>>((float*)c, (const float*)m, n);
-  else mul_inplace_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>((__nv_bfloat16*)c, (const __nv_bfloat16*)m, n);
+  else if (dtype == VRR_BF16) mul_inplace_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>((__nv_bfloat16*)c, (const __nv_bfloat16*)m, n);
+  else mul_inplace_kernel<__half><<<grid, 256, 0, st>>>((__half*)c, (const __half*)m, n);
   VRR_LAUNCHED();
   return VRR_OK;
 }
@@ -220,22 +235,25 @@ int colsum(const void* x, float* out, int M, int C, int dtype, cudaStream_t st) 
   if (C % vec == 0 && ((uintptr_t)x & 15) == 0) {
     dim3 grid(ceil_div(C, 16 * vec), ceil_div(M, kCsRows));
     if (dtype == VRR_F32) colsum_vec_kernel<float><<<grid, kCsThreads, 0, st>>>((const float*)x, out, M, C);
-    else colsum_vec_kernel<__nv_bfloat16><<<grid, kCsThreads, 0, st>>>((const __nv_bfloat16*)x, out, M, C);
+    else if (dtype == VRR_BF16) colsum_vec_kernel<__nv_bfloat16><<<grid, kCsThreads, 0, st>>>((const __nv_bfloat16*)x, out, M, C);
+    else colsum_vec_kernel<__half><<<grid, kCsThreads, 0, st>>>((const __half*)x, out, M, C);
     VRR_LAUNCHED();
     return VRR_OK;
   }
-  // colsum_kernel reads 4 elements at a time (16 bytes fp32, 8 bytes bf16): a base address off that grid takes the
+  // colsum_kernel reads 4 elements at a time (16 bytes fp32, 8 bytes bf16 / fp16): a base address off that grid takes the
   // element-wise kernel
   if (((uintptr_t)x & (dtype == VRR_F32 ? 15 : 7)) != 0) {
     dim3 grid(ceil_div(C, 32), ceil_div(M, kCsRows));
     if (dtype == VRR_F32) colsum_scalar_kernel<float><<<grid, kCsThreads, 0, st>>>((const float*)x, out, M, C);
-    else colsum_scalar_kernel<__nv_bfloat16><<<grid, kCsThreads, 0, st>>>((const __nv_bfloat16*)x, out, M, C);
+    else if (dtype == VRR_BF16) colsum_scalar_kernel<__nv_bfloat16><<<grid, kCsThreads, 0, st>>>((const __nv_bfloat16*)x, out, M, C);
+    else colsum_scalar_kernel<__half><<<grid, kCsThreads, 0, st>>>((const __half*)x, out, M, C);
     VRR_LAUNCHED();
     return VRR_OK;
   }
   dim3 grid(ceil_div(C, 128), ceil_div(M, kCsRows));
   if (dtype == VRR_F32) colsum_kernel<float><<<grid, kCsThreads, 0, st>>>((const float*)x, out, M, C);
-  else colsum_kernel<__nv_bfloat16><<<grid, kCsThreads, 0, st>>>((const __nv_bfloat16*)x, out, M, C);
+  else if (dtype == VRR_BF16) colsum_kernel<__nv_bfloat16><<<grid, kCsThreads, 0, st>>>((const __nv_bfloat16*)x, out, M, C);
+  else colsum_kernel<__half><<<grid, kCsThreads, 0, st>>>((const __half*)x, out, M, C);
   VRR_LAUNCHED();
   return VRR_OK;
 }
@@ -246,9 +264,11 @@ int gelu_bwd_colsum(const void* dy, const void* h, void* dh, float* db, int M, i
   dim3 grid(ceil_div(C, 128), ceil_div(M, kCsRows));
   if (dtype == VRR_F32)
     gelu_bwd_colsum_kernel<float><<<grid, kCsThreads, 0, st>>>((const float*)dy, (const float*)h, (float*)dh, db, M, C);
-  else
+  else if (dtype == VRR_BF16)
     gelu_bwd_colsum_kernel<__nv_bfloat16><<<grid, kCsThreads, 0, st>>>((const __nv_bfloat16*)dy, (const __nv_bfloat16*)h,
                                                                       (__nv_bfloat16*)dh, db, M, C);
+  else
+    gelu_bwd_colsum_kernel<__half><<<grid, kCsThreads, 0, st>>>((const __half*)dy, (const __half*)h, (__half*)dh, db, M, C);
   VRR_LAUNCHED();
   return VRR_OK;
 }

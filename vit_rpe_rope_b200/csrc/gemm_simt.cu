@@ -9,6 +9,8 @@
 //   * the plain GEMMs of the projection backward (dX, dW) and the patch-embed weight gradient.
 //
 // 64x64 output tile, BK = 16, 256 threads, 4x4 register micro-tile, fp32 accumulation.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace vrr {
@@ -37,7 +39,8 @@ struct StridedOperand {
 // A[m][k] of unfold(images): m = b*Np + p (p = py*gw + px), k = c*P*P + i*P + j
 // TI = storage type of the images; ROUND = round each pixel to bf16 first (bf16 arithmetic on fp32
 // images, i.e. the reference's autocast cast of the conv input fused into the load).
-template <typename TI, bool ROUND>
+// ROUND: the image is rounded to the conv dtype TR on load (fp32 images under autocast)
+template <typename TI, bool ROUND, typename TR>
 struct Im2colOperand {
   static constexpr bool kVec = false;
   const TI* img;
@@ -46,7 +49,7 @@ struct Im2colOperand {
     int b = m / Np, p = m - b * Np, py = p / gw, px = p - py * gw;
     int c = k / (P * P), r = k - c * P * P, i = r / P, j = r - i * P;
     float v = Elem<TI>::ld(img + (((long long)b * C + c) * Hi + (py * P + i)) * Wi + (px * P + j));
-    return ROUND ? __bfloat162float(__float2bfloat16_rn(v)) : v;
+    return ROUND ? Elem<TR>::round(v) : v;
   }
 };
 
@@ -89,7 +92,7 @@ struct BiasEpilogue {
   int gelu;
   __device__ __forceinline__ void operator()(int m, int n, float v, const float*, int) const {
     float b = bias[n];
-    if (sizeof(T) == 2) b = __bfloat162float(__float2bfloat16_rn(b));
+    if (sizeof(T) == 2) b = Elem<T>::round(b);
     T r;
     Elem<T>::st(&r, v + b);
     if (gelu != 2) c[(long long)m * ldc + n] = r;
@@ -387,9 +390,9 @@ static int qkv_rope_fwd_t(const void* x, const void* w, const float* cos_tab, co
 int qkv_rope_fwd_simt(const void* x, const void* w, const float* cos_tab, const float* sin_tab,
                       void* planes, int B, int N, int E, int H, int rope_mode, int dtype,
                       cudaStream_t st) {
-  return dtype == VRR_F32
-             ? qkv_rope_fwd_t<float>(x, w, cos_tab, sin_tab, planes, B, N, E, H, rope_mode, st)
-             : qkv_rope_fwd_t<__nv_bfloat16>(x, w, cos_tab, sin_tab, planes, B, N, E, H, rope_mode, st);
+  if (dtype == VRR_F32) return qkv_rope_fwd_t<float>(x, w, cos_tab, sin_tab, planes, B, N, E, H, rope_mode, st);
+  if (dtype == VRR_BF16) return qkv_rope_fwd_t<__nv_bfloat16>(x, w, cos_tab, sin_tab, planes, B, N, E, H, rope_mode, st);
+  return qkv_rope_fwd_t<__half>(x, w, cos_tab, sin_tab, planes, B, N, E, H, rope_mode, st);
 }
 
 // ---- plain GEMM -------------------------------------------------------------------------------
@@ -441,7 +444,8 @@ static int gemm_bias_t(const void* a, const void* b, void* c, void* c2, const fl
 int gemm_simt_bias(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int ta, int tb,
                    int dtype, int gelu, cudaStream_t st) {
   if (dtype == VRR_F32) return gemm_bias_t<float>(a, b, c, c2, bias, M, N, K, ta, tb, gelu, st);
-  return gemm_bias_t<__nv_bfloat16>(a, b, c, c2, bias, M, N, K, ta, tb, gelu, st);
+  if (dtype == VRR_BF16) return gemm_bias_t<__nv_bfloat16>(a, b, c, c2, bias, M, N, K, ta, tb, gelu, st);
+  return gemm_bias_t<__half>(a, b, c, c2, bias, M, N, K, ta, tb, gelu, st);
 }
 
 void gemm_simt_set_tile(int v) { g_simt_tile.store(v == 64 ? 64 : 128); }
@@ -452,6 +456,8 @@ int gemm_simt(const void* a, const void* b, void* c, int M, int N, int K, int ta
   if (dtype == VRR_BF16 && c_dtype == VRR_F32) return gemm_t<__nv_bfloat16, float>(a, b, c, M, N, K, ta, tb, st);
   if (dtype == VRR_BF16 && c_dtype == VRR_BF16)
     return gemm_t<__nv_bfloat16, __nv_bfloat16>(a, b, c, M, N, K, ta, tb, st);
+  if (dtype == VRR_F16 && c_dtype == VRR_F32) return gemm_t<__half, float>(a, b, c, M, N, K, ta, tb, st);
+  if (dtype == VRR_F16 && c_dtype == VRR_F16) return gemm_t<__half, __half>(a, b, c, M, N, K, ta, tb, st);
   set_error("vrr_gemm: unsupported dtype combination (%d -> %d)", dtype, c_dtype);
   return VRR_ERR_UNSUPPORTED;
 }
@@ -471,7 +477,7 @@ static int patch_fwd_t(const void* images, const void* weight, const void* bias,
                        const void* pos, void* tokens, int B, int C, int Hi, int Wi, int P, int E,
                        cudaStream_t st) {
   constexpr bool kRound = sizeof(TI) == 4 && sizeof(T) == 2;
-  using AOp = Im2colOperand<TI, kRound>;
+  using AOp = Im2colOperand<TI, kRound, T>;
   const int gh = Hi / P, gw = Wi / P, Np = gh * gw, Kd = C * P * P;
   AOp A{(const TI*)images, C, Hi, Wi, P, gw, Np};
   StridedOperand<T> W{(const T*)weight, Kd, 1};
@@ -479,13 +485,16 @@ static int patch_fwd_t(const void* images, const void* weight, const void* bias,
   int rc = launch_gemm<AOp, StridedOperand<T>, PatchEmbedEpilogue<T, TT>, true, true>(
       A, W, epi, B * Np, E, Kd, 1, st);
   if (rc) return rc;
-  return patch_cls_rows(tokens, cls, B, Np, E, sizeof(TT) == 4 ? VRR_F32 : VRR_BF16, st);
+  return patch_cls_rows(tokens, cls, B, Np, E, sizeof(TT) == 4 ? VRR_F32 : (std::is_same<TT, __half>::value ? VRR_F16 : VRR_BF16),
+                        st);
 }
 int patch_cls_rows(void* tokens, const void* cls, int B, int Np, int E, int tok_dtype, cudaStream_t st) {
   if (tok_dtype == VRR_F32)
     cls_rows_kernel<float><<<ceil_div(B * E, 256), 256, 0, st>>>((float*)tokens, (const float*)cls, B, Np, E);
-  else
+  else if (tok_dtype == VRR_BF16)
     cls_rows_kernel<__nv_bfloat16><<<ceil_div(B * E, 256), 256, 0, st>>>((__nv_bfloat16*)tokens, (const __nv_bfloat16*)cls, B, Np, E);
+  else
+    cls_rows_kernel<__half><<<ceil_div(B * E, 256), 256, 0, st>>>((__half*)tokens, (const __half*)cls, B, Np, E);
   VRR_LAUNCHED();
   return VRR_OK;
 }
@@ -498,6 +507,9 @@ int patch_embed_fwd_simt(const void* images, const void* weight, const void* bia
   if (img_dtype == VRR_BF16 && dtype == VRR_BF16 && tok_dtype == VRR_F32) return patch_fwd_t<__nv_bfloat16, __nv_bfloat16, float>(ARGS);
   if (img_dtype == VRR_BF16 && dtype == VRR_BF16 && tok_dtype == VRR_BF16)
     return patch_fwd_t<__nv_bfloat16, __nv_bfloat16, __nv_bfloat16>(ARGS);
+  if (img_dtype == VRR_F32 && dtype == VRR_F16 && tok_dtype == VRR_F32) return patch_fwd_t<float, __half, float>(ARGS);
+  if (img_dtype == VRR_F16 && dtype == VRR_F16 && tok_dtype == VRR_F32) return patch_fwd_t<__half, __half, float>(ARGS);
+  if (img_dtype == VRR_F16 && dtype == VRR_F16 && tok_dtype == VRR_F16) return patch_fwd_t<__half, __half, __half>(ARGS);
 #undef ARGS
   set_error("patch_embed_fwd: unsupported dtype combination (images %d, weights %d, tokens %d)", img_dtype, dtype, tok_dtype);
   return VRR_ERR_UNSUPPORTED;
@@ -520,7 +532,7 @@ __global__ void token_batch_sum_kernel(const T* __restrict__ dtok, float* d_bias
   }
 }
 
-template <typename TI, bool ROUND, typename TT>
+template <typename TI, bool ROUND, typename TT, typename TR>
 static int patch_bwd_t(const void* images, const void* d_tokens, float* d_weight, float* d_bias,
                        float* d_cls, float* d_pos, int B, int C, int Hi, int Wi, int P, int E,
                        cudaStream_t st) {
@@ -530,9 +542,9 @@ static int patch_bwd_t(const void* images, const void* d_tokens, float* d_weight
   VRR_LAUNCHED();
   if (!d_weight) return VRR_OK;  // caller computes the weight gradient itself (plain library GEMM)
   // d_weight[e][k] = sum_m d_tokens[m][e] * unfold(images)[m][k]   (reduction over m = tokens)
-  using BOp = SwapArgs<Im2colOperand<TI, ROUND>>;
+  using BOp = SwapArgs<Im2colOperand<TI, ROUND, TR>>;
   PatchGradOperand<TT> A{(const TT*)d_tokens, Np, E};
-  BOp Bo{Im2colOperand<TI, ROUND>{(const TI*)images, C, Hi, Wi, P, gw, Np}};
+  BOp Bo{Im2colOperand<TI, ROUND, TR>{(const TI*)images, C, Hi, Wi, P, gw, Np}};
   const int tiles = ceil_div(E, BM) * ceil_div(Kd, BN);
   int splits = max(1, min(ceil_div(2 * sm_count(), tiles), Mtok / (4 * BK)));
   VRR_CUDA(cudaMemsetAsync(d_weight, 0, (size_t)E * Kd * sizeof(float), st));
@@ -543,11 +555,14 @@ int patch_embed_bwd_simt(const void* images, const void* d_tokens, float* d_weig
                          float* d_cls, float* d_pos, int B, int C, int Hi, int Wi, int P, int E,
                          int img_dtype, int dtype, int tok_dtype, cudaStream_t st) {
 #define ARGS images, d_tokens, d_weight, d_bias, d_cls, d_pos, B, C, Hi, Wi, P, E, st
-  if (img_dtype == VRR_F32 && dtype == VRR_F32 && tok_dtype == VRR_F32) return patch_bwd_t<float, false, float>(ARGS);
-  if (img_dtype == VRR_F32 && dtype == VRR_BF16 && tok_dtype == VRR_F32) return patch_bwd_t<float, true, float>(ARGS);
-  if (img_dtype == VRR_BF16 && dtype == VRR_BF16 && tok_dtype == VRR_F32) return patch_bwd_t<__nv_bfloat16, false, float>(ARGS);
-  if (img_dtype == VRR_BF16 && dtype == VRR_BF16 && tok_dtype == VRR_BF16)
-    return patch_bwd_t<__nv_bfloat16, false, __nv_bfloat16>(ARGS);
+  using bf16 = __nv_bfloat16;
+  if (img_dtype == VRR_F32 && dtype == VRR_F32 && tok_dtype == VRR_F32) return patch_bwd_t<float, false, float, float>(ARGS);
+  if (img_dtype == VRR_F32 && dtype == VRR_BF16 && tok_dtype == VRR_F32) return patch_bwd_t<float, true, float, bf16>(ARGS);
+  if (img_dtype == VRR_BF16 && dtype == VRR_BF16 && tok_dtype == VRR_F32) return patch_bwd_t<bf16, false, float, bf16>(ARGS);
+  if (img_dtype == VRR_BF16 && dtype == VRR_BF16 && tok_dtype == VRR_BF16) return patch_bwd_t<bf16, false, bf16, bf16>(ARGS);
+  if (img_dtype == VRR_F32 && dtype == VRR_F16 && tok_dtype == VRR_F32) return patch_bwd_t<float, true, float, __half>(ARGS);
+  if (img_dtype == VRR_F16 && dtype == VRR_F16 && tok_dtype == VRR_F32) return patch_bwd_t<__half, false, float, __half>(ARGS);
+  if (img_dtype == VRR_F16 && dtype == VRR_F16 && tok_dtype == VRR_F16) return patch_bwd_t<__half, false, __half, __half>(ARGS);
 #undef ARGS
   set_error("patch_embed_bwd: unsupported dtype combination (images %d, weights %d, tokens %d)", img_dtype, dtype, tok_dtype);
   return VRR_ERR_UNSUPPORTED;

@@ -1,5 +1,5 @@
-// bf16 GEMMs of the ViT hot path on tcgen05 tensor cores with CTA PAIRS (cta_group::2), all operand
-// layouts, fused epilogues.  One kernel template serves
+// bf16 / fp16 GEMMs of the ViT hot path on tcgen05 tensor cores with CTA PAIRS (cta_group::2), all operand
+// layouts, fused epilogues.  T (Elem16) is the element type of the operands and of every 16-bit output.  One kernel template serves
 //   * the QKV projection with the RoPE rotate-half epilogue         (models/vit.py:47-68)
 //   * the patch-embedding GEMM                                      (models/vit.py:164,248-254)
 //   * out-proj / fc1(+bias+GELU) / fc2 / head forward               (models/vit.py:91,118,285)
@@ -22,7 +22,7 @@
 //   warps 2..9    epilogue: tcgen05.ld -> registers -> (bias / GELU / RoPE) -> swizzled shared staging
 //                 -> TMA store / TMA reduce-add (fp32 split-K), or a direct mapped store (planes, tokens)
 //
-// The bias of the BIAS epilogue is rounded to bf16 before it is added for an fp32 C too (vrr.h: "cast to `dtype`
+// The bias of the BIAS epilogue is rounded to T before it is added for an fp32 C too (vrr.h: "cast to `dtype`
 // first"); the fp32-C path once added the unrounded fp32 value.  tests/test_kernels_at_scale.py pins both C types
 // bit for bit with biases off the bf16 grid.
 #include <string.h>
@@ -53,14 +53,15 @@ struct PairShape {
 // Epilogues.  kTma = false: functor called per (row, 64-column chunk) with the fp32 accumulators.
 // ---------------------------------------------------------------------------------------------------
 // kPlaneStore: the functor only transforms the 64 accumulators of (row m, head chunk n0) in registers; the kernel
-// rounds them to bf16, stages 32 rows x 128 B per warp in swizzled shared memory and writes them with TMA through a
+// rounds them to T, stages 32 rows x 128 B per warp in swizzled shared memory and writes them with TMA through a
 // 3-D map of planes[3 B H][N][64]; the one warp tile in N / 32 that runs into the next image falls back to per-thread
 // row stores.  A thread writing its own 128-byte row touched 32 lines per store instruction and made
 // this GEMM 1.7x slower than the plain one.
+template <typename T>
 struct QkvRopeEpi2 {
   static constexpr bool kTma = false;
   static constexpr bool kPlaneStore = true;
-  __nv_bfloat16* planes;
+  T* planes;
   const float *cos_tab, *sin_tab;
   const float4* packed;  // rope_pack_tables layout [heads][16][N-1], or null
   int B, N, E, H, rope_mode;
@@ -105,13 +106,13 @@ struct QkvRopeEpi2 {
   }
 };
 
-// tokens[b][1+p][n] = round_bf16(acc + bias[n]) (+ pos[p][n]); TT = token-stream type
-template <typename TT>
+// tokens[b][1+p][n] = round_T(acc + bias[n]) (+ pos[p][n]); TT = token-stream type
+template <typename T, typename TT>
 struct PatchEmbedEpi2 {
   static constexpr bool kTma = false;
   static constexpr bool kPlaneStore = false;
   TT* tokens;
-  const __nv_bfloat16* bias;
+  const T* bias;
   const TT* pos;  // may be null
   int Np, E;
   __device__ __forceinline__ void operator()(int m, int n0, float (&f)[64]) const {
@@ -122,10 +123,10 @@ struct PatchEmbedEpi2 {
     for (int v4 = 0; v4 < 16; ++v4) {
       const float4 bv = ld4(bias + n0 + v4 * 4);
       float4 o;
-      o.x = __bfloat162float(__float2bfloat16_rn(f[v4 * 4 + 0] + bv.x));
-      o.y = __bfloat162float(__float2bfloat16_rn(f[v4 * 4 + 1] + bv.y));
-      o.z = __bfloat162float(__float2bfloat16_rn(f[v4 * 4 + 2] + bv.z));
-      o.w = __bfloat162float(__float2bfloat16_rn(f[v4 * 4 + 3] + bv.w));
+      o.x = Elem16<T>::round(f[v4 * 4 + 0] + bv.x);
+      o.y = Elem16<T>::round(f[v4 * 4 + 1] + bv.y);
+      o.z = Elem16<T>::round(f[v4 * 4 + 2] + bv.z);
+      o.w = Elem16<T>::round(f[v4 * 4 + 3] + bv.w);
       if (prow) {
         const float4 pv = ld4(prow + v4 * 4);
         o.x += pv.x; o.y += pv.y; o.z += pv.z; o.w += pv.w;
@@ -137,17 +138,18 @@ struct PatchEmbedEpi2 {
 
 // Row-major C through shared staging + TMA store.  Runtime (warp-uniform) switches keep the number of
 // template instances small.
+template <typename T>
 struct StoreEpi {
   static constexpr bool kTma = true;
   static constexpr bool kPlaneStore = false;
-  const float* bias;  // fp32 [N] or null; rounded to bf16 first for either C type (autocast casts the bias)
-  int out_f32;        // C element type: 0 bf16, 1 fp32
+  const float* bias;  // fp32 [N] or null; rounded to T first for either C type (autocast casts the bias)
+  int out_f32;        // C element type: 0 T, 1 fp32
   int reduce;         // fp32 only: C += tile via TMA reduce-add (split-K partial sums / gradient accumulation)
-  int gelu;           // bf16 only.  1: C = h = bf16(acc + bias), C2 = bf16(gelu(h)) (exact erf GELU);
-                      //            2: C = bf16(gelu(h)), C2 = bf16(gelu'(h)) - what an Mlp backward needs instead of h
-                      //            3: C = bf16(gelu(h)) only (inference): its own code path, one TMA store per chunk
-  const __nv_bfloat16* mul;  // bf16 only, or null: C = bf16(acc * mul[m][n]) (mul is [M][N] like C): d_act * gelu'(h)
-  float* colsum;      // bf16 plain / bias / mul paths, or null: colsum[n] += sum_m C[m][n] (values as stored; atomics)
+  int gelu;           // T only.  1: C = h = T(acc + bias), C2 = T(gelu(h)) (exact erf GELU);
+                      //         2: C = T(gelu(h)), C2 = T(gelu'(h)) - what an Mlp backward needs instead of h
+                      //         3: C = T(gelu(h)) only (inference): its own code path, one TMA store per chunk
+  const T* mul;       // T C only, or null: C = T(acc * mul[m][n]) (mul is [M][N] like C): d_act * gelu'(h)
+  float* colsum;      // T plain / bias / mul paths, or null: colsum[n] += sum_m C[m][n] (values as stored; atomics)
 };
 
 // gelu(h) and d gelu / dh for TWO values at a time on the packed fp32x2 pipe (fma.rn.f32x2, sm_100): the epilogue of
@@ -156,7 +158,6 @@ struct StoreEpi {
 //   Phi(h) = 1 - erfc(|h| / sqrt 2) / 2 (h >= 0), erfc / 2 otherwise; erfc(z) = (a1 t + .. + a5 t^5) exp(-z^2),
 //   t = 1 / (1 + p z) (Abramowitz-Stegun 7.1.26, |error| <= 1.5e-7); gelu = h Phi, gelu' = Phi + h phi(h) with
 //   phi(h) = exp(-h^2 / 2) / sqrt(2 pi) - the same exponential.
-__device__ __forceinline__ float bf16_round(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
 __device__ __forceinline__ float rcp_approx(float x) {
   float y;
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -181,7 +182,8 @@ __device__ __forceinline__ void gelu_and_grad2(float2 h, float2& g, float2& dg) 
   dg = __ffma2_rn(__fmul2_rn(h, e), make_float2(0.3989422804014327f, 0.3989422804014327f), cdf);
 }
 
-// gelu(h) alone, packed to bf16x2 (same Phi(h) as above)
+// gelu(h) alone, packed to a pair of T (same Phi(h) as above)
+template <typename T>
 __device__ __forceinline__ uint32_t gelu_only2(float2 h) {
   const float2 hh = __fmul2_rn(h, h);
   const float2 ea = __fmul2_rn(hh, make_float2(-0.72134752044448170f, -0.72134752044448170f));
@@ -196,11 +198,11 @@ __device__ __forceinline__ uint32_t gelu_only2(float2 h) {
   const float2 q = __fmul2_rn(__fmul2_rn(poly, t), e);
   const float2 om = __ffma2_rn(q, make_float2(-1.f, -1.f), make_float2(1.f, 1.f));
   const float2 g = __fmul2_rn(h, make_float2(h.x >= 0.f ? om.x : q.x, h.y >= 0.f ? om.y : q.y));
-  return pack_bf16(g.x, g.y);
+  return Elem16<T>::pack2(g.x, g.y);
 }
 
 // ---------------------------------------------------------------------------------------------------
-template <int BN, bool A_MN, bool B_MN, class Epi>
+template <typename T, int BN, bool A_MN, bool B_MN, class Epi>
 __global__ void __launch_bounds__(kPairThreads, 1)
 gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                  const __grid_constant__ CUtensorMap tmap_c, const __grid_constant__ CUtensorMap tmap_c2,
@@ -283,7 +285,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
   } else if (warp == 1) {
     // ====================================== MMA issuer (leader CTA only) ==================================
     if (rank == 0 && lane == 0) {
-      constexpr uint32_t idesc = idesc_bf16(2 * kPM, BN, A_MN ? 1 : 0, B_MN ? 1 : 0);
+      constexpr uint32_t idesc = idesc_16<T>(2 * kPM, BN, A_MN ? 1 : 0, B_MN ? 1 : 0);
       constexpr uint32_t adv_a = A_MN ? 128 : 2, adv_b = B_MN ? 128 : 2;  // descriptor units (16 B) per K = 16
       int stage = 0, acc = 0;
       uint32_t phase = 0, acc_phase = 0;
@@ -390,9 +392,9 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
             const uint32_t row_base = stage_u32 + buf + (uint32_t)lane * 128u;
 #pragma unroll
             for (int c8 = 0; c8 < 8; ++c8)
-              st_shared_v4(row_base + (((uint32_t)c8 ^ sw) << 4), pack_bf16(f[c8 * 8 + 0], f[c8 * 8 + 1]),
-                           pack_bf16(f[c8 * 8 + 2], f[c8 * 8 + 3]), pack_bf16(f[c8 * 8 + 4], f[c8 * 8 + 5]),
-                           pack_bf16(f[c8 * 8 + 6], f[c8 * 8 + 7]));
+              st_shared_v4(row_base + (((uint32_t)c8 ^ sw) << 4), Elem16<T>::pack2(f[c8 * 8 + 0], f[c8 * 8 + 1]),
+                           Elem16<T>::pack2(f[c8 * 8 + 2], f[c8 * 8 + 3]), Elem16<T>::pack2(f[c8 * 8 + 4], f[c8 * 8 + 5]),
+                           Elem16<T>::pack2(f[c8 * 8 + 6], f[c8 * 8 + 7]));
             fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) {
@@ -404,14 +406,14 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
             // the rows run into the next image (one warp tile in N / 32; TMA stores take no negative coordinates -
             // "illegal instruction" - and a box cannot be shortened): each thread stores its own row
             const int b = m / epi.N, t = m - b * epi.N;
-            __nv_bfloat16* dst = epi.planes + ((size_t)epi.plane_of(b, n0) * epi.N + t) * 64;
+            T* dst = epi.planes + ((size_t)epi.plane_of(b, n0) * epi.N + t) * 64;
 #pragma unroll
             for (int v8 = 0; v8 < 8; ++v8) {
               uint4 wv;
-              wv.x = pack_bf16(f[v8 * 8 + 0], f[v8 * 8 + 1]);
-              wv.y = pack_bf16(f[v8 * 8 + 2], f[v8 * 8 + 3]);
-              wv.z = pack_bf16(f[v8 * 8 + 4], f[v8 * 8 + 5]);
-              wv.w = pack_bf16(f[v8 * 8 + 6], f[v8 * 8 + 7]);
+              wv.x = Elem16<T>::pack2(f[v8 * 8 + 0], f[v8 * 8 + 1]);
+              wv.y = Elem16<T>::pack2(f[v8 * 8 + 2], f[v8 * 8 + 3]);
+              wv.z = Elem16<T>::pack2(f[v8 * 8 + 4], f[v8 * 8 + 5]);
+              wv.w = Elem16<T>::pack2(f[v8 * 8 + 6], f[v8 * 8 + 7]);
               *reinterpret_cast<uint4*>(dst + v8 * 8) = wv;
             }
           }
@@ -422,7 +424,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           const uint32_t sw = (uint32_t)(lane & 7);
           const uint32_t row_base = stage_u32 + (uint32_t)lane * 128u;
           if (!epi.out_f32) {
-            // ---- bf16 C ----
+            // ---- 16-bit C (T) ----
             if (epi.gelu == 3) {
               // inference: gelu(h) alone.  Its own branch - folding it into the two-output code below cost that path
               // 50 us per launch (register allocation of the o0 / o1 arrays).
@@ -432,13 +434,13 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                 const int nb = min(n0 + c8 * 8, g.N - 8);
                 const float4 b0 = __ldg(reinterpret_cast<const float4*>(epi.bias + nb));
                 const float4 b1 = __ldg(reinterpret_cast<const float4*>(epi.bias + nb + 4));
-                const uint32_t br[4] = {pack_bf16(b0.x, b0.y), pack_bf16(b0.z, b0.w), pack_bf16(b1.x, b1.y), pack_bf16(b1.z, b1.w)};
+                const uint32_t br[4] = {Elem16<T>::pack2(b0.x, b0.y), Elem16<T>::pack2(b0.z, b0.w), Elem16<T>::pack2(b1.x, b1.y), Elem16<T>::pack2(b1.z, b1.w)};
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
-                  const float2 bb = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&br[j]));
+                  const float2 bb = Elem16<T>::unpack2(br[j]);
                   const float2 hs = __fadd2_rn(make_float2(f[c8 * 8 + 2 * j], f[c8 * 8 + 2 * j + 1]), bb);
-                  const uint32_t hw = pack_bf16(hs.x, hs.y);
-                  o0[c8 * 4 + j] = gelu_only2(__bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&hw)));
+                  const uint32_t hw = Elem16<T>::pack2(hs.x, hs.y);
+                  o0[c8 * 4 + j] = gelu_only2<T>(Elem16<T>::unpack2(hw));
                 }
               }
               const uint32_t buf = (chunk_counter & 1u) * 4096u;
@@ -469,21 +471,21 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                   const int nb = min(n0 + c8 * 8, g.N - 8);  // N % 8 == 0; clamp keeps the tail read in bounds
                   const float4 b0 = __ldg(reinterpret_cast<const float4*>(epi.bias + nb));
                   const float4 b1 = __ldg(reinterpret_cast<const float4*>(epi.bias + nb + 4));
-                  const uint32_t br[4] = {pack_bf16(b0.x, b0.y), pack_bf16(b0.z, b0.w), pack_bf16(b1.x, b1.y), pack_bf16(b1.z, b1.w)};
+                  const uint32_t br[4] = {Elem16<T>::pack2(b0.x, b0.y), Elem16<T>::pack2(b0.z, b0.w), Elem16<T>::pack2(b1.x, b1.y), Elem16<T>::pack2(b1.z, b1.w)};
 #pragma unroll
                   for (int j = 0; j < 4; ++j) {
-                    const float2 bb = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&br[j]));  // bias as bf16
+                    const float2 bb = Elem16<T>::unpack2(br[j]);  // bias as T
                     const float2 hs = __fadd2_rn(make_float2(f[c8 * 8 + 2 * j], f[c8 * 8 + 2 * j + 1]), bb);
-                    const uint32_t hw = pack_bf16(hs.x, hs.y);
-                    const float2 hr = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&hw));  // h as stored
+                    const uint32_t hw = Elem16<T>::pack2(hs.x, hs.y);
+                    const float2 hr = Elem16<T>::unpack2(hw);  // h as stored
                     float2 gl, dg;
                     gelu_and_grad2(hr, gl, dg);
                     if (epi.gelu == 1) {
                       o0[q * 4 + j] = hw;
-                      o1[q * 4 + j] = pack_bf16(gl.x, gl.y);
+                      o1[q * 4 + j] = Elem16<T>::pack2(gl.x, gl.y);
                     } else {
-                      o0[q * 4 + j] = pack_bf16(gl.x, gl.y);
-                      o1[q * 4 + j] = pack_bf16(dg.x, dg.y);
+                      o0[q * 4 + j] = Elem16<T>::pack2(gl.x, gl.y);
+                      o1[q * 4 + j] = Elem16<T>::pack2(dg.x, dg.y);
                     }
                   }
                 }
@@ -522,19 +524,19 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                   const float4 b1 = __ldg(reinterpret_cast<const float4*>(epi.bias + nb + 4));
                   const float bb[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
 #pragma unroll
-                  for (int j = 0; j < 8; ++j) x[j] += __bfloat162float(__float2bfloat16_rn(bb[j]));
+                  for (int j = 0; j < 8; ++j) x[j] += Elem16<T>::round(bb[j]);
                 }
                 if (epi.mul != nullptr) {
                   const uint32_t mw[4] = {mv[c8].x, mv[c8].y, mv[c8].z, mv[c8].w};
 #pragma unroll
                   for (int j = 0; j < 4; ++j) {
-                    const float2 m2 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&mw[j]));
+                    const float2 m2 = Elem16<T>::unpack2(mw[j]);
                     x[2 * j] *= m2.x;
                     x[2 * j + 1] *= m2.y;
                   }
                 }
-                st_shared_v4(row_base + buf + (((uint32_t)c8 ^ sw) << 4), pack_bf16(x[0], x[1]), pack_bf16(x[2], x[3]),
-                             pack_bf16(x[4], x[5]), pack_bf16(x[6], x[7]));
+                st_shared_v4(row_base + buf + (((uint32_t)c8 ^ sw) << 4), Elem16<T>::pack2(x[0], x[1]), Elem16<T>::pack2(x[2], x[3]),
+                             Elem16<T>::pack2(x[4], x[5]), Elem16<T>::pack2(x[6], x[7]));
               }
               fence_proxy_async_smem();
               __syncwarp();
@@ -543,7 +545,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                 bulk_commit();
               }
               if (epi.colsum != nullptr && store_ok) {
-                // bias gradient of the layer that produced A: column sums of the tile AS STORED (bf16), read back from
+                // bias gradient of the layer that produced A: column sums of the tile AS STORED (T), read back from
                 // the staging buffer while the TMA store drains it; lane = column pair, conflict-free under the swizzle
                 // (rows past M hold zeros: their A rows were zero-filled)
                 float s0 = 0.f, s1 = 0.f;
@@ -551,7 +553,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
 #pragma unroll 8
                 for (uint32_t r = 0; r < 32; ++r) {
                   const uint32_t wv = ld_shared_u32(cbase + r * 128u + ((((uint32_t)lane >> 2) ^ (r & 7u)) << 4));
-                  const float2 v2 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&wv));
+                  const float2 v2 = Elem16<T>::unpack2(wv);
                   s0 += v2.x;
                   s1 += v2.y;
                 }
@@ -576,7 +578,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                 if (epi.bias != nullptr && first_split) {
                   const int nb = min(n0 + hb * 32 + c4 * 4, g.N - 4);
                   const float4 b0 = __ldg(reinterpret_cast<const float4*>(epi.bias + nb));
-                  x[0] += bf16_round(b0.x); x[1] += bf16_round(b0.y); x[2] += bf16_round(b0.z); x[3] += bf16_round(b0.w);
+                  x[0] += Elem16<T>::round(b0.x); x[1] += Elem16<T>::round(b0.y); x[2] += Elem16<T>::round(b0.z); x[3] += Elem16<T>::round(b0.w);
                 }
                 st_shared_v4(row_base + hb * 4096u + (((uint32_t)c4 ^ sw) << 4), __float_as_uint(x[0]), __float_as_uint(x[1]),
                              __float_as_uint(x[2]), __float_as_uint(x[3]));
@@ -635,14 +637,14 @@ int pick_splits(int tiles, int num_k, int clusters) {
   return best;
 }
 
-template <int BN, bool A_MN, bool B_MN, class Epi>
+template <typename T, int BN, bool A_MN, bool B_MN, class Epi>
 int launch_pair(const void* a, const void* b, int M, int N, int K, int splits, const CUtensorMap& tc_, const CUtensorMap& tc2_,
                 const Epi& epi, cudaStream_t st) {
   CUtensorMap ta, tb;
-  if (!A_MN) { if (int rc = make_tmap_2d(&ta, a, 2, (uint64_t)M, (uint64_t)K, (uint64_t)K * 2, kPM, 64)) return rc; }
-  else       { if (int rc = make_tmap_2d(&ta, a, 2, (uint64_t)K, (uint64_t)M, (uint64_t)M * 2, 64, 64)) return rc; }
-  if (!B_MN) { if (int rc = make_tmap_2d(&tb, b, 2, (uint64_t)N, (uint64_t)K, (uint64_t)K * 2, BN / 2, 64)) return rc; }
-  else       { if (int rc = make_tmap_2d(&tb, b, 2, (uint64_t)K, (uint64_t)N, (uint64_t)N * 2, 64, 64)) return rc; }
+  if (!A_MN) { if (int rc = make_tmap_2d(&ta, a, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)K, (uint64_t)K * 2, kPM, 64)) return rc; }
+  else       { if (int rc = make_tmap_2d(&ta, a, Elem16<T>::kTmap, (uint64_t)K, (uint64_t)M, (uint64_t)M * 2, 64, 64)) return rc; }
+  if (!B_MN) { if (int rc = make_tmap_2d(&tb, b, Elem16<T>::kTmap, (uint64_t)N, (uint64_t)K, (uint64_t)K * 2, BN / 2, 64)) return rc; }
+  else       { if (int rc = make_tmap_2d(&tb, b, Elem16<T>::kTmap, (uint64_t)K, (uint64_t)N, (uint64_t)N * 2, 64, 64)) return rc; }
   PairShape g;
   g.M = M; g.N = N; g.K = K;
   g.tiles_m = ceil_div(M, 2 * kPM);
@@ -650,7 +652,7 @@ int launch_pair(const void* a, const void* b, int M, int N, int K, int splits, c
   g.num_k = ceil_div(K, kPK);
   g.splits = splits < 1 ? 1 : (splits > g.num_k ? g.num_k : splits);
   constexpr size_t smem = pair_smem_bytes<BN>();
-  auto kern = gemm_pair_kernel<BN, A_MN, B_MN, Epi>;
+  auto kern = gemm_pair_kernel<T, BN, A_MN, B_MN, Epi>;
   VRR_SMEM_ATTR_ONCE(kern, smem);
   const int clusters_max = sm_count() / 2;
   const long long units = (long long)g.tiles_m * g.tiles_n * g.splits;
@@ -672,15 +674,15 @@ int launch_pair(const void* a, const void* b, int M, int N, int K, int splits, c
   return VRR_OK;
 }
 
-template <bool A_MN, bool B_MN>
+template <typename T, bool A_MN, bool B_MN>
 int launch_store(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int c_f32,
                  int epilogue, int accumulate, float* colsum, cudaStream_t st) {
-  StoreEpi epi;
+  StoreEpi<T> epi;
   epi.colsum = colsum;
   epi.bias = (epilogue != VRR_EPI_NONE && epilogue != VRR_EPI_MUL) ? bias : nullptr;
   epi.out_f32 = c_f32;
   epi.gelu = epilogue == VRR_EPI_BIAS_GELU ? 1 : (epilogue == VRR_EPI_BIAS_GELU_GRAD ? 2 : (epilogue == VRR_EPI_BIAS_GELU_ACT ? 3 : 0));
-  epi.mul = epilogue == VRR_EPI_MUL ? (const __nv_bfloat16*)c2 : nullptr;
+  epi.mul = epilogue == VRR_EPI_MUL ? (const T*)c2 : nullptr;
   if (epilogue == VRR_EPI_MUL) epi.bias = nullptr;
   const int tiles = ceil_div(M, 2 * kPM) * ceil_div(N, N > 128 ? 256 : 128);
   int splits = 1;
@@ -689,21 +691,21 @@ int launch_store(const void* a, const void* b, void* c, void* c2, const float* b
   if (c_f32 && !accumulate && splits > 1) VRR_CUDA(cudaMemsetAsync(c, 0, (size_t)M * N * sizeof(float), st));
   CUtensorMap tc_, tc2_;
   if (c_f32) {
-    if (int rc = make_tmap_2d(&tc_, c, 4, (uint64_t)M, (uint64_t)N, (uint64_t)N * 4, 32, 32)) return rc;
+    if (int rc = make_tmap_2d(&tc_, c, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, (uint64_t)M, (uint64_t)N, (uint64_t)N * 4, 32, 32)) return rc;
     tc2_ = tc_;
   } else {
-    if (int rc = make_tmap_2d(&tc_, c, 2, (uint64_t)M, (uint64_t)N, (uint64_t)N * 2, 32, 64)) return rc;
+    if (int rc = make_tmap_2d(&tc_, c, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)N, (uint64_t)N * 2, 32, 64)) return rc;
     tc2_ = tc_;
     if (epi.gelu == 1 || epi.gelu == 2)
-      if (int rc = make_tmap_2d(&tc2_, c2, 2, (uint64_t)M, (uint64_t)N, (uint64_t)N * 2, 32, 64)) return rc;
+      if (int rc = make_tmap_2d(&tc2_, c2, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)N, (uint64_t)N * 2, 32, 64)) return rc;
   }
-  if (N > 128) return launch_pair<256, A_MN, B_MN, StoreEpi>(a, b, M, N, K, splits, tc_, tc2_, epi, st);
-  return launch_pair<128, A_MN, B_MN, StoreEpi>(a, b, M, N, K, splits, tc_, tc2_, epi, st);
+  if (N > 128) return launch_pair<T, 256, A_MN, B_MN, StoreEpi<T>>(a, b, M, N, K, splits, tc_, tc2_, epi, st);
+  return launch_pair<T, 128, A_MN, B_MN, StoreEpi<T>>(a, b, M, N, K, splits, tc_, tc2_, epi, st);
 }
 
-// unfold(images)[m][k], m = b*Np + py*gw + px, k = c*P*P + i*P + j  ->  bf16; 8 consecutive j per thread
-template <typename TI>
-__global__ void patch_unfold_kernel(const TI* __restrict__ img, __nv_bfloat16* __restrict__ out, int B, int C, int Hi,
+// unfold(images)[m][k], m = b*Np + py*gw + px, k = c*P*P + i*P + j  ->  TO (bf16 / fp16); 8 consecutive j per thread
+template <typename TI, typename TO>
+__global__ void patch_unfold_kernel(const TI* __restrict__ img, TO* __restrict__ out, int B, int C, int Hi,
                                     int Wi, int P, int gw, int Np) {
   const int K8 = C * P * P / 8;
   const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -714,32 +716,46 @@ __global__ void patch_unfold_kernel(const TI* __restrict__ img, __nv_bfloat16* _
   const int k = k8 * 8, c = k / (P * P), r = k - c * P * P, i = r / P, j = r - i * P;
   const TI* src = img + (((size_t)b * C + c) * Hi + (py * P + i)) * Wi + (px * P + j);
   float4 lo = ld4(src), hi = ld4(src + 4);
-  __nv_bfloat16* dst = out + m * (size_t)(K8 * 8) + k;
+  TO* dst = out + m * (size_t)(K8 * 8) + k;
   st4(dst, lo);
   st4(dst + 4, hi);
 }
 
 }  // namespace
 
-// bf16 operands; TMA needs 16-byte row strides: the CONTIGUOUS dimension of every operand and of C must be a
+// 16-bit operands; TMA needs 16-byte row strides: the CONTIGUOUS dimension of every operand and of C must be a
 // multiple of 8 elements (4 for an fp32 C); the other dimensions are free (ragged tiles are zero-filled / clipped).
-bool gemm_bf16_tc_supported(int M, int N, int K, int trans_a, int trans_b, int c_dtype, int epilogue) {
+// A 16-bit C has the operands' type.
+bool gemm_tc_supported(int M, int N, int K, int trans_a, int trans_b, int dtype, int c_dtype, int epilogue) {
   if (M < 1 || N < 1 || K < 1) return false;
+  if (!is16(dtype)) return false;
   if ((trans_a ? M : K) % 8 != 0) return false;   // A stored [K][M] or [M][K]
   if ((trans_b ? K : N) % 8 != 0) return false;   // B stored [N][K] or [K][N]
-  if (c_dtype == VRR_BF16 ? (N % 8 != 0) : (N % 4 != 0)) return false;
-  if (c_dtype != VRR_F32 && c_dtype != VRR_BF16) return false;
-  if (epilogue >= VRR_EPI_BIAS_GELU && c_dtype != VRR_BF16) return false;
+  if (c_dtype == dtype ? (N % 8 != 0) : (N % 4 != 0)) return false;
+  if (c_dtype != VRR_F32 && c_dtype != dtype) return false;
+  if (epilogue >= VRR_EPI_BIAS_GELU && c_dtype != dtype) return false;
   if (epilogue != VRR_EPI_NONE && N % 8 != 0) return false;  // vector loads of the bias / the multiplier
   if ((long long)M * N >= (1ll << 40)) return false;
   return true;
 }
 
-int gemm_bf16_tc(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int trans_a,
-                 int trans_b, int c_dtype, int epilogue, int accumulate, cudaStream_t st, float* colsum) {
-  VRR_REQUIRE(colsum == nullptr || (c_dtype == VRR_BF16 && epilogue != VRR_EPI_BIAS_GELU && epilogue != VRR_EPI_BIAS_GELU_GRAD &&
+template <typename T>
+static int gemm_tc_t(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int trans_a,
+                     int trans_b, int c_f32, int epilogue, int accumulate, cudaStream_t st, float* colsum) {
+  const bool a_mn = trans_a != 0, b_mn = trans_b == 0;
+  if (!a_mn && !b_mn) return launch_store<T, false, false>(a, b, c, c2, bias, M, N, K, c_f32, epilogue, accumulate, colsum, st);
+  if (!a_mn && b_mn) return launch_store<T, false, true>(a, b, c, c2, bias, M, N, K, c_f32, epilogue, accumulate, colsum, st);
+  if (a_mn && b_mn) return launch_store<T, true, true>(a, b, c, c2, bias, M, N, K, c_f32, epilogue, accumulate, colsum, st);
+  return launch_store<T, true, false>(a, b, c, c2, bias, M, N, K, c_f32, epilogue, accumulate, colsum, st);
+}
+
+int gemm_tc(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int trans_a,
+            int trans_b, int dtype, int c_dtype, int epilogue, int accumulate, cudaStream_t st, float* colsum) {
+  VRR_REQUIRE(is16(dtype) && (c_dtype == VRR_F32 || c_dtype == dtype), VRR_ERR_UNSUPPORTED,
+              "gemm (tcgen05): operands must be bf16 or fp16 and C fp32 or the operands' type (got %d / %d)", dtype, c_dtype);
+  VRR_REQUIRE(colsum == nullptr || (c_dtype == dtype && epilogue != VRR_EPI_BIAS_GELU && epilogue != VRR_EPI_BIAS_GELU_GRAD &&
                                     epilogue != VRR_EPI_BIAS_GELU_ACT),
-              VRR_ERR_UNSUPPORTED, "gemm (tcgen05): column sums come with the bf16 plain / bias / multiply epilogues only");
+              VRR_ERR_UNSUPPORTED, "gemm (tcgen05): column sums come with the 16-bit plain / bias / multiply epilogues only");
   VRR_REQUIRE((((uintptr_t)a | (uintptr_t)b | (uintptr_t)c | (uintptr_t)c2) & 15) == 0, VRR_ERR_INVALID_ARG,
               "gemm (tcgen05): a / b / c must be 16-byte aligned");
   VRR_REQUIRE(epilogue == VRR_EPI_NONE || epilogue == VRR_EPI_MUL || (bias != nullptr && ((uintptr_t)bias & 15) == 0),
@@ -748,11 +764,9 @@ int gemm_bf16_tc(const void* a, const void* b, void* c, void* c2, const float* b
               "gemm (tcgen05): the two-output GELU epilogues and MUL need c2");
   VRR_REQUIRE(!accumulate || c_dtype == VRR_F32, VRR_ERR_UNSUPPORTED, "gemm (tcgen05): accumulate needs an fp32 C");
   const int c_f32 = c_dtype == VRR_F32;
-  const bool a_mn = trans_a != 0, b_mn = trans_b == 0;
-  if (!a_mn && !b_mn) return launch_store<false, false>(a, b, c, c2, bias, M, N, K, c_f32, epilogue, accumulate, colsum, st);
-  if (!a_mn && b_mn) return launch_store<false, true>(a, b, c, c2, bias, M, N, K, c_f32, epilogue, accumulate, colsum, st);
-  if (a_mn && b_mn) return launch_store<true, true>(a, b, c, c2, bias, M, N, K, c_f32, epilogue, accumulate, colsum, st);
-  return launch_store<true, false>(a, b, c, c2, bias, M, N, K, c_f32, epilogue, accumulate, colsum, st);
+  if (dtype == VRR_F16)
+    return gemm_tc_t<__half>(a, b, c, c2, bias, M, N, K, trans_a, trans_b, c_f32, epilogue, accumulate, st, colsum);
+  return gemm_tc_t<__nv_bfloat16>(a, b, c, c2, bias, M, N, K, trans_a, trans_b, c_f32, epilogue, accumulate, st, colsum);
 }
 
 // ---- QKV projection + RoPE epilogue on the CTA-pair kernel -----------------------------------------------
@@ -762,23 +776,32 @@ bool qkv_rope_fwd_tc_supported(int B, int N, int E, int H) {
   return true;
 }
 
+template <typename T>
+static int qkv_rope_fwd_tc2_t(const void* x, const void* w, const float* cos_tab, const float* sin_tab, const float* packed,
+                              void* planes, int B, int N, int E, int H, int rope_mode, cudaStream_t st) {
+  QkvRopeEpi2<T> epi{(T*)planes, cos_tab, sin_tab, reinterpret_cast<const float4*>(packed), B, N, E, H, rope_mode};
+  CUtensorMap tplanes;  // planes[3 B H][N][64] of T, box = [1][32 rows][64]
+  if (int rc = make_tmap_3d(&tplanes, planes, Elem16<T>::kTmap, 64, (uint64_t)N, (uint64_t)3 * B * H, 128, (uint64_t)N * 128,
+                            64, 32))
+    return rc;
+  // 64-column chunks are whole heads (3E = 192 H); a ragged last n-tile is clipped by the n0 < N test
+  if (3 * E > 128) return launch_pair<T, 256, false, false, QkvRopeEpi2<T>>(x, w, B * N, 3 * E, E, 1, tplanes, tplanes, epi, st);
+  return launch_pair<T, 128, false, false, QkvRopeEpi2<T>>(x, w, B * N, 3 * E, E, 1, tplanes, tplanes, epi, st);
+}
+
 int qkv_rope_fwd_tc2(const void* x, const void* w, const float* cos_tab, const float* sin_tab, const float* packed,
-                     void* planes, int B, int N, int E, int H, int rope_mode, cudaStream_t st) {
+                     void* planes, int B, int N, int E, int H, int rope_mode, int dtype, cudaStream_t st) {
   VRR_REQUIRE(((uintptr_t)x & 15) == 0 && ((uintptr_t)w & 15) == 0 && ((uintptr_t)planes & 15) == 0,
               VRR_ERR_INVALID_ARG, "qkv_rope_fwd (tcgen05): x / w / planes must be 16-byte aligned");
   if (rope_mode != VRR_ROPE_NONE)
     VRR_REQUIRE(((uintptr_t)cos_tab & 15) == 0 && ((uintptr_t)sin_tab & 15) == 0, VRR_ERR_INVALID_ARG,
                 "qkv_rope_fwd (tcgen05): cos / sin must be 16-byte aligned");
   VRR_REQUIRE(((uintptr_t)packed & 15) == 0, VRR_ERR_INVALID_ARG, "qkv_rope_fwd (tcgen05): packed table must be 16-byte aligned");
-  QkvRopeEpi2 epi{(__nv_bfloat16*)planes, cos_tab, sin_tab, reinterpret_cast<const float4*>(packed), B, N, E, H, rope_mode};
-  CUtensorMap tplanes;  // planes[3 B H][N][64] bf16, box = [1][32 rows][64]
-  if (int rc = make_tmap_3d_bf16(&tplanes, planes, 64, (uint64_t)N, (uint64_t)3 * B * H, 128, (uint64_t)N * 128, 64, 32)) return rc;
-  // 64-column chunks are whole heads (3E = 192 H); a ragged last n-tile is clipped by the n0 < N test
-  if (3 * E > 128) return launch_pair<256, false, false, QkvRopeEpi2>(x, w, B * N, 3 * E, E, 1, tplanes, tplanes, epi, st);
-  return launch_pair<128, false, false, QkvRopeEpi2>(x, w, B * N, 3 * E, E, 1, tplanes, tplanes, epi, st);
+  if (dtype == VRR_F16) return qkv_rope_fwd_tc2_t<__half>(x, w, cos_tab, sin_tab, packed, planes, B, N, E, H, rope_mode, st);
+  return qkv_rope_fwd_tc2_t<__nv_bfloat16>(x, w, cos_tab, sin_tab, packed, planes, B, N, E, H, rope_mode, st);
 }
 
-// ---- patch embedding: unfold pre-pass (fused fp32->bf16 cast) + the CTA-pair kernel ----------------------
+// ---- patch embedding: unfold pre-pass (fused fp32 -> 16-bit cast) + the CTA-pair kernel -------------------
 bool patch_embed_tc_supported(int B, int C, int Hi, int Wi, int P, int E) {
   const int K = C * P * P;
   if (P % 8 != 0 || Wi % 4 != 0 || K % 64 != 0 || E % 64 != 0) return false;
@@ -788,37 +811,54 @@ bool patch_embed_tc_supported(int B, int C, int Hi, int Wi, int P, int E) {
 size_t patch_embed_tc_workspace_bytes(int B, int C, int Hi, int Wi, int P) {
   return (size_t)B * (Hi / P) * (Wi / P) * C * P * P * 2;
 }
-int patch_unfold(const void* images, void* out, int B, int C, int Hi, int Wi, int P, int img_dtype, cudaStream_t st) {
+int patch_unfold(const void* images, void* out, int B, int C, int Hi, int Wi, int P, int img_dtype, int out_dtype,
+                 cudaStream_t st) {
   const int gw = Wi / P, Np = (Hi / P) * gw;
   VRR_REQUIRE(P % 8 == 0 && Wi % 4 == 0, VRR_ERR_UNSUPPORTED, "patch_unfold: needs P %% 8 == 0 and Wi %% 4 == 0");
   VRR_REQUIRE(((uintptr_t)images & 15) == 0 && ((uintptr_t)out & 15) == 0, VRR_ERR_INVALID_ARG,
               "patch_unfold: pointers must be 16-byte aligned");
+  VRR_REQUIRE(is16(out_dtype) && (img_dtype == VRR_F32 || img_dtype == out_dtype), VRR_ERR_INVALID_ARG,
+              "patch_unfold: images %d cannot be unfolded into dtype %d", img_dtype, out_dtype);
   const size_t total = (size_t)B * Np * (C * P * P / 8);
   const unsigned blocks = (unsigned)((total + 255) / 256);
-  if (img_dtype == VRR_F32)
-    patch_unfold_kernel<float><<<blocks, 256, 0, st>>>((const float*)images, (__nv_bfloat16*)out, B, C, Hi, Wi, P, gw, Np);
-  else
-    patch_unfold_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>((const __nv_bfloat16*)images, (__nv_bfloat16*)out, B, C,
-                                                              Hi, Wi, P, gw, Np);
+  if (out_dtype == VRR_BF16) {
+    if (img_dtype == VRR_F32)
+      patch_unfold_kernel<float, __nv_bfloat16><<<blocks, 256, 0, st>>>((const float*)images, (__nv_bfloat16*)out, B, C, Hi,
+                                                                         Wi, P, gw, Np);
+    else
+      patch_unfold_kernel<__nv_bfloat16, __nv_bfloat16><<<blocks, 256, 0, st>>>((const __nv_bfloat16*)images,
+                                                                                 (__nv_bfloat16*)out, B, C, Hi, Wi, P, gw, Np);
+  } else {
+    if (img_dtype == VRR_F32)
+      patch_unfold_kernel<float, __half><<<blocks, 256, 0, st>>>((const float*)images, (__half*)out, B, C, Hi, Wi, P, gw, Np);
+    else
+      patch_unfold_kernel<__half, __half><<<blocks, 256, 0, st>>>((const __half*)images, (__half*)out, B, C, Hi, Wi, P, gw, Np);
+  }
   VRR_LAUNCHED();
   return VRR_OK;
 }
-int patch_embed_fwd_tc(const void* images, const void* weight, const void* bias, const void* pos, void* tokens,
-                       void* workspace, int B, int C, int Hi, int Wi, int P, int E, int img_dtype, int tok_dtype,
-                       cudaStream_t st) {
-  const int Np = (Hi / P) * (Wi / P), K = C * P * P, M = B * Np;
-  if (int rc = patch_unfold(images, workspace, B, C, Hi, Wi, P, img_dtype, st)) return rc;
+
+template <typename T, typename TT>
+static int patch_embed_gemm(const void* workspace, const void* weight, const void* bias, const void* pos, void* tokens, int M,
+                            int E, int K, int Np, cudaStream_t st) {
   CUtensorMap dummy;  // PatchEmbedEpi2 stores its rows directly: no C map
   memset(&dummy, 0, sizeof(dummy));
-  if (tok_dtype == VRR_F32) {
-    PatchEmbedEpi2<float> epi{(float*)tokens, (const __nv_bfloat16*)bias, (const float*)pos, Np, E};
-    if (E > 128) return launch_pair<256, false, false, PatchEmbedEpi2<float>>(workspace, weight, M, E, K, 1, dummy, dummy, epi, st);
-    return launch_pair<128, false, false, PatchEmbedEpi2<float>>(workspace, weight, M, E, K, 1, dummy, dummy, epi, st);
+  PatchEmbedEpi2<T, TT> epi{(TT*)tokens, (const T*)bias, (const TT*)pos, Np, E};
+  if (E > 128) return launch_pair<T, 256, false, false, PatchEmbedEpi2<T, TT>>(workspace, weight, M, E, K, 1, dummy, dummy, epi, st);
+  return launch_pair<T, 128, false, false, PatchEmbedEpi2<T, TT>>(workspace, weight, M, E, K, 1, dummy, dummy, epi, st);
+}
+
+int patch_embed_fwd_tc(const void* images, const void* weight, const void* bias, const void* pos, void* tokens,
+                       void* workspace, int B, int C, int Hi, int Wi, int P, int E, int img_dtype, int dtype, int tok_dtype,
+                       cudaStream_t st) {
+  const int Np = (Hi / P) * (Wi / P), K = C * P * P, M = B * Np;
+  if (int rc = patch_unfold(images, workspace, B, C, Hi, Wi, P, img_dtype, dtype, st)) return rc;
+  if (dtype == VRR_F16) {
+    if (tok_dtype == VRR_F32) return patch_embed_gemm<__half, float>(workspace, weight, bias, pos, tokens, M, E, K, Np, st);
+    return patch_embed_gemm<__half, __half>(workspace, weight, bias, pos, tokens, M, E, K, Np, st);
   }
-  PatchEmbedEpi2<__nv_bfloat16> epi{(__nv_bfloat16*)tokens, (const __nv_bfloat16*)bias, (const __nv_bfloat16*)pos, Np, E};
-  if (E > 128)
-    return launch_pair<256, false, false, PatchEmbedEpi2<__nv_bfloat16>>(workspace, weight, M, E, K, 1, dummy, dummy, epi, st);
-  return launch_pair<128, false, false, PatchEmbedEpi2<__nv_bfloat16>>(workspace, weight, M, E, K, 1, dummy, dummy, epi, st);
+  if (tok_dtype == VRR_F32) return patch_embed_gemm<__nv_bfloat16, float>(workspace, weight, bias, pos, tokens, M, E, K, Np, st);
+  return patch_embed_gemm<__nv_bfloat16, __nv_bfloat16>(workspace, weight, bias, pos, tokens, M, E, K, Np, st);
 }
 
 }  // namespace vrr

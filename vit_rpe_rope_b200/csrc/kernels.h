@@ -13,30 +13,32 @@ int attn_bwd_simt(const void* planes, const vrr_bias_desc* bias, const void* out
                   const float* lse, void* d_planes, float* d_bias_param, float* delta, float* d_lut_ws, int B,
                   int H, int N, int Dh, float scale, int dtype, cudaStream_t st);
 
-// attn_tc.cu (tcgen05 / TMEM, bf16, Dh == 64; tiled over 64-key tiles): without bias attn_fwd_tc4_kernel (four CTAs
+// The tcgen05 launchers below take `dtype` VRR_BF16 or VRR_F16 (the operands' and the 16-bit outputs' element type).
+
+// attn_tc.cu (tcgen05 / TMEM, Dh == 64; tiled over 64-key tiles): without bias attn_fwd_tc4_kernel (four CTAs
 // per SM), with a bias attn_fwd_tc2_kernel (two CTAs per SM)
 bool attn_fwd_tc_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bias);
 void attn_fwd_tc_set_debug(long long* buf);
 int attn_fwd_tc(const void* planes, const vrr_bias_desc* bias, void* out, float* lse, int B, int H, int N,
-                int Dh, float scale, cudaStream_t st);
+                int Dh, float scale, int dtype, cudaStream_t st);
 
 // attn_fwd_ws.cu (whole-sequence forward with a bias for N <= 256: persistent, one round trip per (image, head))
 bool attn_fwd_ws_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bias);
 int attn_fwd_ws(const void* planes, const vrr_bias_desc* bias, void* out, float* lse, int B, int H, int N, int Dh,
-                float scale, cudaStream_t st);
+                float scale, int dtype, cudaStream_t st);
 
 // attn_bwd_tc2.cu (dQ and dK/dV kernels: issuer warp, double-buffered 32-row tiles; every case attn_bwd_ws.cu does
 // not take)
 bool attn_bwd_tc2_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bias);
 int attn_bwd_tc2(const void* planes, const vrr_bias_desc* bias, const void* out, const void* d_out, const float* lse,
                  void* d_planes, float* d_bias_param, float* delta, int B, int H, int N, int Dh, float scale,
-                 cudaStream_t st);
+                 int dtype, cudaStream_t st);
 
 // attn_bwd_ws.cu (whole-sequence fused backward for N <= 256, no bias: one persistent kernel, operands read once)
 bool attn_bwd_ws_supported(int B, int H, int N, int Dh, const vrr_bias_desc* bias);
 void attn_bwd_ws_set_debug(long long* buf);
 int attn_bwd_ws(const void* planes, const void* out, const void* d_out, const float* lse, void* d_planes, int B, int H,
-                int N, int Dh, float scale, cudaStream_t st);
+                int N, int Dh, float scale, int dtype, cudaStream_t st);
 
 // gemm_simt.cu
 void layernorm_set_option(int which, int value);  // 0: ln_reg, 1: ln_bwd_minb
@@ -56,21 +58,23 @@ int patch_embed_bwd_simt(const void* images, const void* d_tokens, float* d_weig
 int patch_cls_rows(void* tokens, const void* cls, int B, int Np, int E, int tok_dtype, cudaStream_t st);
 
 // gemm_tc2.cu (tcgen05 CTA pairs, cta_group::2: every operand layout, TMA-store epilogues)
-bool gemm_bf16_tc_supported(int M, int N, int K, int trans_a, int trans_b, int c_dtype, int epilogue);
-int gemm_bf16_tc(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int trans_a,
-                 int trans_b, int c_dtype, int epilogue, int accumulate, cudaStream_t st, float* colsum = nullptr);
-// colsum (bf16 C, plain / bias / multiply epilogues): colsum[n] += sum_m C[m][n] of the values as stored; zeroed by the caller
+bool gemm_tc_supported(int M, int N, int K, int trans_a, int trans_b, int dtype, int c_dtype, int epilogue);
+int gemm_tc(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int trans_a,
+            int trans_b, int dtype, int c_dtype, int epilogue, int accumulate, cudaStream_t st, float* colsum = nullptr);
+// colsum (16-bit C, plain / bias / multiply epilogues): colsum[n] += sum_m C[m][n] of the values as stored; zeroed by the caller
 int rope_pack_tables(const float* cos_tab, const float* sin_tab, float* packed, int heads, int rows, int hd, cudaStream_t st);
 bool qkv_rope_fwd_tc_supported(int B, int N, int E, int H);
 // `packed`: optional output of rope_pack_tables for the same tables (NULL: the epilogue reads cos_tab / sin_tab)
 int qkv_rope_fwd_tc2(const void* x, const void* w, const float* cos_tab, const float* sin_tab, const float* packed, void* planes, int B, int N,
-                     int E, int H, int rope_mode, cudaStream_t st);
+                     int E, int H, int rope_mode, int dtype, cudaStream_t st);
 
 bool patch_embed_tc_supported(int B, int C, int Hi, int Wi, int P, int E);
 size_t patch_embed_tc_workspace_bytes(int B, int C, int Hi, int Wi, int P);
-int patch_unfold(const void* images, void* out, int B, int C, int Hi, int Wi, int P, int img_dtype, cudaStream_t st);
+// out_dtype: VRR_BF16 or VRR_F16; images fp32 or of out_dtype
+int patch_unfold(const void* images, void* out, int B, int C, int Hi, int Wi, int P, int img_dtype, int out_dtype,
+                 cudaStream_t st);
 int patch_embed_fwd_tc(const void* images, const void* weight, const void* bias, const void* pos, void* tokens,
-                       void* workspace, int B, int C, int Hi, int Wi, int P, int E, int img_dtype, int tok_dtype,
+                       void* workspace, int B, int C, int Hi, int Wi, int P, int E, int img_dtype, int dtype, int tok_dtype,
                        cudaStream_t st);
 
 // layernorm.cu

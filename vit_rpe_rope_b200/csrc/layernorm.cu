@@ -588,6 +588,8 @@ int layernorm_fwd(const void* x, const float* gamma, const float* beta, void* y,
   if (x_dtype == VRR_F32 && y_dtype == VRR_BF16) return ln_fwd_t<float, __nv_bfloat16>(x, gamma, beta, y, mean, rstd, M, E, eps, st);
   if (x_dtype == VRR_BF16 && y_dtype == VRR_BF16)
     return ln_fwd_t<__nv_bfloat16, __nv_bfloat16>(x, gamma, beta, y, mean, rstd, M, E, eps, st);
+  if (x_dtype == VRR_F32 && y_dtype == VRR_F16) return ln_fwd_t<float, __half>(x, gamma, beta, y, mean, rstd, M, E, eps, st);
+  if (x_dtype == VRR_F16 && y_dtype == VRR_F16) return ln_fwd_t<__half, __half>(x, gamma, beta, y, mean, rstd, M, E, eps, st);
   set_error("layernorm_fwd: unsupported dtype combination (x %d, y %d)", x_dtype, y_dtype);
   return VRR_ERR_UNSUPPORTED;
 }
@@ -601,6 +603,10 @@ int layernorm_bwd(const void* dy, const void* x, const float* gamma, const float
     return ln_bwd_t<float, __nv_bfloat16>(dy, x, gamma, mean, rstd, dx, dgamma, dbeta, M, E, st);
   if (x_dtype == VRR_BF16 && y_dtype == VRR_BF16)
     return ln_bwd_t<__nv_bfloat16, __nv_bfloat16>(dy, x, gamma, mean, rstd, dx, dgamma, dbeta, M, E, st);
+  if (x_dtype == VRR_F32 && y_dtype == VRR_F16)
+    return ln_bwd_t<float, __half>(dy, x, gamma, mean, rstd, dx, dgamma, dbeta, M, E, st);
+  if (x_dtype == VRR_F16 && y_dtype == VRR_F16)
+    return ln_bwd_t<__half, __half>(dy, x, gamma, mean, rstd, dx, dgamma, dbeta, M, E, st);
   set_error("layernorm_bwd: unsupported dtype combination (x %d, y %d)", x_dtype, y_dtype);
   return VRR_ERR_UNSUPPORTED;
 }
@@ -614,6 +620,8 @@ int add_layernorm_fwd(const void* x, const void* branch, void* x_new, const floa
   if (branch_dtype == VRR_F32 && y_dtype == VRR_F32) return add_ln_fwd_t<float, float>(ARGS);
   if (branch_dtype == VRR_BF16 && y_dtype == VRR_BF16) return add_ln_fwd_t<__nv_bfloat16, __nv_bfloat16>(ARGS);
   if (branch_dtype == VRR_F32 && y_dtype == VRR_BF16) return add_ln_fwd_t<float, __nv_bfloat16>(ARGS);
+  if (branch_dtype == VRR_F16 && y_dtype == VRR_F16) return add_ln_fwd_t<__half, __half>(ARGS);
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_F16) return add_ln_fwd_t<float, __half>(ARGS);
 #undef ARGS
   set_error("add_layernorm_fwd: unsupported dtype combination (branch %d, y %d)", branch_dtype, y_dtype);
   return VRR_ERR_UNSUPPORTED;
@@ -628,6 +636,8 @@ int add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new, con
   if (branch_dtype == VRR_F32 && y_dtype == VRR_F32) return add_ln_bwd_t<float, float>(ARGS);
   if (branch_dtype == VRR_BF16 && y_dtype == VRR_BF16) return add_ln_bwd_t<__nv_bfloat16, __nv_bfloat16>(ARGS);
   if (branch_dtype == VRR_F32 && y_dtype == VRR_BF16) return add_ln_bwd_t<float, __nv_bfloat16>(ARGS);
+  if (branch_dtype == VRR_F16 && y_dtype == VRR_F16) return add_ln_bwd_t<__half, __half>(ARGS);
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_F16) return add_ln_bwd_t<float, __half>(ARGS);
 #undef ARGS
   set_error("add_layernorm_bwd: unsupported dtype combination (branch %d, y %d)", branch_dtype, y_dtype);
   return VRR_ERR_UNSUPPORTED;

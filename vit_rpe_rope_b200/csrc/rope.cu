@@ -47,6 +47,29 @@ struct VecIO<__nv_bfloat16, 8> {
     *reinterpret_cast<uint4*>(p) = x;
   }
 };
+template <>
+struct VecIO<__half, 8> {
+  using Raw = uint4;
+  static __device__ __forceinline__ void cvt(const uint4& x, float (&v)[8]) {
+    const uint32_t w[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&w[e]));
+      v[2 * e] = f.x; v[2 * e + 1] = f.y;
+    }
+  }
+  static __device__ __forceinline__ void ld(const __half* p, float (&v)[8]) {
+    cvt(*reinterpret_cast<const uint4*>(p), v);
+  }
+  static __device__ __forceinline__ void st(__half* p, const float (&v)[8]) {
+    uint4 x;
+    __half2 a = __floats2half2_rn(v[0], v[1]), b = __floats2half2_rn(v[2], v[3]);
+    __half2 c = __floats2half2_rn(v[4], v[5]), d = __floats2half2_rn(v[6], v[7]);
+    x.x = *reinterpret_cast<uint32_t*>(&a); x.y = *reinterpret_cast<uint32_t*>(&b);
+    x.z = *reinterpret_cast<uint32_t*>(&c); x.w = *reinterpret_cast<uint32_t*>(&d);
+    *reinterpret_cast<uint4*>(p) = x;
+  }
+};
 
 template <typename T, int VEC>
 __global__ void qkv_rope_bwd_kernel(const T* __restrict__ d_planes, const T* __restrict__ planes,
@@ -152,10 +175,13 @@ int qkv_rope_bwd(const void* d_planes, const void* planes, const float* cos_tab,
     qkv_rope_bwd_kernel<float, 4><<<grid, threads, 0, st>>>((const float*)d_planes, (const float*)planes, cos_tab,
                                                            sin_tab, (float*)d_qkv, d_cos, d_sin, B, N, E, H, Dh,
                                                            rope_mode, b_chunk);
-  else
+  else if (dtype == VRR_BF16)
     qkv_rope_bwd_kernel<__nv_bfloat16, 8><<<grid, threads, 0, st>>>(
         (const __nv_bfloat16*)d_planes, (const __nv_bfloat16*)planes, cos_tab, sin_tab,
         (__nv_bfloat16*)d_qkv, d_cos, d_sin, B, N, E, H, Dh, rope_mode, b_chunk);
+  else
+    qkv_rope_bwd_kernel<__half, 8><<<grid, threads, 0, st>>>((const __half*)d_planes, (const __half*)planes, cos_tab, sin_tab,
+                                                            (__half*)d_qkv, d_cos, d_sin, B, N, E, H, Dh, rope_mode, b_chunk);
   VRR_LAUNCHED();
   return VRR_OK;
 }
@@ -216,10 +242,13 @@ int rope_apply(const void* q_in, const void* k_in, const float* cos_tab, const f
   if (dtype == VRR_F32)
     rope_apply_kernel<float><<<blocks, threads, 0, st>>>((const float*)q_in, (const float*)k_in, cos_tab, sin_tab,
                                                         (float*)q_out, (float*)k_out, B, H, Nr, Dh, rope_mode, inverse);
-  else
+  else if (dtype == VRR_BF16)
     rope_apply_kernel<__nv_bfloat16><<<blocks, threads, 0, st>>>(
         (const __nv_bfloat16*)q_in, (const __nv_bfloat16*)k_in, cos_tab, sin_tab, (__nv_bfloat16*)q_out,
         (__nv_bfloat16*)k_out, B, H, Nr, Dh, rope_mode, inverse);
+  else
+    rope_apply_kernel<__half><<<blocks, threads, 0, st>>>((const __half*)q_in, (const __half*)k_in, cos_tab, sin_tab,
+                                                         (__half*)q_out, (__half*)k_out, B, H, Nr, Dh, rope_mode, inverse);
   VRR_LAUNCHED();
   return VRR_OK;
 }
@@ -259,10 +288,13 @@ int rope_table_grad(const void* q_in, const void* k_in, const void* dq, const vo
   if (dtype == VRR_F32)
     rope_table_grad_kernel<float><<<blocks, threads, 0, st>>>((const float*)q_in, (const float*)k_in, (const float*)dq,
                                                              (const float*)dk, d_cos, d_sin, B, H, Nr, Dh, rope_mode);
-  else
+  else if (dtype == VRR_BF16)
     rope_table_grad_kernel<__nv_bfloat16><<<blocks, threads, 0, st>>>(
         (const __nv_bfloat16*)q_in, (const __nv_bfloat16*)k_in, (const __nv_bfloat16*)dq, (const __nv_bfloat16*)dk,
         d_cos, d_sin, B, H, Nr, Dh, rope_mode);
+  else
+    rope_table_grad_kernel<__half><<<blocks, threads, 0, st>>>((const __half*)q_in, (const __half*)k_in, (const __half*)dq,
+                                                              (const __half*)dk, d_cos, d_sin, B, H, Nr, Dh, rope_mode);
   VRR_LAUNCHED();
   return VRR_OK;
 }

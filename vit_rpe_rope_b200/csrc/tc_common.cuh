@@ -6,6 +6,7 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -146,11 +147,11 @@ __device__ __forceinline__ uint64_t smem_desc_sw128(uint32_t smem_addr) {
   d |= (uint64_t)2 << 61;            // SWIZZLE_128B
   return d;
 }
-// Instruction descriptor for kind::f16 with bf16 A/B and fp32 accumulation.
-//   [4,6) D fmt (1 = f32)  [7,10) A fmt (1 = bf16)  [10,13) B fmt (1 = bf16)
+// Instruction descriptor for kind::f16 with 16-bit A/B (`fmt`: 0 = f16, 1 = bf16) and fp32 accumulation.
+//   [4,6) D fmt (1 = f32)  [7,10) A fmt  [10,13) B fmt
 //   [15] A major (0 = K)   [16] B major (0 = K, 1 = MN)   [17,23) N >> 3   [24,29) M >> 4
-__host__ __device__ constexpr uint32_t idesc_bf16(int M, int N, int a_mn_major, int b_mn_major) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
+__host__ __device__ constexpr uint32_t idesc_f16kind(uint32_t fmt, int M, int N, int a_mn_major, int b_mn_major) {
+  return (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
          ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
@@ -324,8 +325,8 @@ __device__ __forceinline__ float ex2(float x) {
   return y;
 }
 // 2^x for two values WITHOUT the MUFU unit: x = n + f with n = round(x) (magic-number add), f in [-0.5, 0.5];
-// 2^f by a degree-3 minimax polynomial (relative error 7.5e-5 - P is rounded to bf16, 3.9e-3, right after) and n
-// added into the exponent field.  ~5 FMA-pipe instructions per value on the packed fp32x2 pipe: MUFU.EX2 issues 16
+// 2^f by a degree-3 minimax polynomial (relative error 7.5e-5 - P is rounded right after, to bf16 (unit roundoff
+// 3.9e-3, a 50x margin) or to fp16 (4.9e-4, a 6x margin)) and n added into the exponent field.  ~5 FMA-pipe instructions per value on the packed fp32x2 pipe: MUFU.EX2 issues 16
 // per clock per SM against 32 softmax elements per clock the tensor pipe could consume at head dim 64, so a share
 // of the exponentials computed here raises the kernel's MUFU-bound ceiling.
 __device__ __forceinline__ float2 ex2_poly2(float2 x) {
@@ -347,17 +348,50 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
   return *reinterpret_cast<uint32_t*>(&v);
 }
 
+// The 16-bit element type of a tensor-core kernel: bf16 or fp16 operands, P / dS in TMEM, and the 16-bit stores.
+// Everything that depends on it goes through this struct, so the two instantiations differ only here.
+// The conversions round to nearest and overflow to +-inf (never a clamped finite value): a GradScaler step relies
+// on an overflowing fp16 gradient becoming non-finite.
+template <typename T>
+struct Elem16;
+template <>
+struct Elem16<__nv_bfloat16> {
+  static constexpr uint32_t kFmt = 1;  // instruction-descriptor A/B format
+  static constexpr CUtensorMapDataType kTmap = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+  static __device__ __forceinline__ uint32_t pack2(float lo, float hi) { return pack_bf16(lo, hi); }
+  static __device__ __forceinline__ float2 unpack2(uint32_t w) {
+    return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&w));
+  }
+  static __device__ __forceinline__ float round(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
+};
+template <>
+struct Elem16<__half> {
+  static constexpr uint32_t kFmt = 0;
+  static constexpr CUtensorMapDataType kTmap = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+  static __device__ __forceinline__ uint32_t pack2(float lo, float hi) {
+    __half2 v = __floats2half2_rn(lo, hi);
+    return *reinterpret_cast<uint32_t*>(&v);
+  }
+  static __device__ __forceinline__ float2 unpack2(uint32_t w) { return __half22float2(*reinterpret_cast<const __half2*>(&w)); }
+  static __device__ __forceinline__ float round(float x) { return __half2float(__float2half_rn(x)); }
+};
+template <typename T>
+__host__ __device__ constexpr uint32_t idesc_16(int M, int N, int a_mn_major, int b_mn_major) {
+  return idesc_f16kind(Elem16<T>::kFmt, M, N, a_mn_major, b_mn_major);
+}
+
 }  // namespace tc
 
-// Host: 2-D tensor map over a row-major [rows][cols] buffer: `elem_bytes` 2 (bf16) or 4 (fp32);
-// box = [box_rows][box_cols], box_cols * elem_bytes <= 128; 128-byte swizzle.
-int make_tmap_2d(CUtensorMap* map, const void* base, int elem_bytes, uint64_t rows, uint64_t cols,
+// Host: 2-D tensor map over a row-major [rows][cols] buffer of `dtype` (bf16, fp16 or fp32);
+// box = [box_rows][box_cols], box_cols * element bytes <= 128; 128-byte swizzle.
+int make_tmap_2d(CUtensorMap* map, const void* base, CUtensorMapDataType dtype, uint64_t rows, uint64_t cols,
                  uint64_t row_stride_bytes, uint32_t box_rows, uint32_t box_cols);
 
-// 3-D bf16 map over [d2][d1][d0] (d0 innermost, contiguous), box = [1][box1][box0], box0 * 2 <= 128 bytes, 128-byte
-// swizzle (or none: plain [box1][box0] staging).  Used for [B][N][E] activations and [planes][N][64] head planes: a
-// box never crosses an image / head, rows past N are clipped by the hardware (coordinates must not be negative).
-int make_tmap_3d_bf16(CUtensorMap* map, const void* base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t stride1_bytes,
-                      uint64_t stride2_bytes, uint32_t box0, uint32_t box1, int swizzle128 = 1);
+// 3-D map of a 16-bit `dtype` over [d2][d1][d0] (d0 innermost, contiguous), box = [1][box1][box0], box0 * 2 <= 128
+// bytes, 128-byte swizzle (or none: plain [box1][box0] staging).  Used for [B][N][E] activations and [planes][N][64]
+// head planes: a box never crosses an image / head, rows past N are clipped by the hardware (coordinates must not be
+// negative).
+int make_tmap_3d(CUtensorMap* map, const void* base, CUtensorMapDataType dtype, uint64_t d0, uint64_t d1, uint64_t d2,
+                 uint64_t stride1_bytes, uint64_t stride2_bytes, uint32_t box0, uint32_t box1, int swizzle128 = 1);
 
 }  // namespace vrr

@@ -94,7 +94,12 @@ bool first_use_on_device(std::atomic<unsigned char>* flags) {
   return flags[dev].exchange(1, std::memory_order_acq_rel) == 0;
 }
 
-static bool dtype_ok(int d) { return d == VRR_F32 || d == VRR_BF16; }
+static bool dtype_ok(int d) { return d == VRR_F32 || d == VRR_BF16 || d == VRR_F16; }
+// bf16 and fp16 never meet in one call (each pairs with fp32 only)
+static bool no_mix(int a, int b, int c = VRR_F32) {
+  const bool bf = a == VRR_BF16 || b == VRR_BF16 || c == VRR_BF16, hf = a == VRR_F16 || b == VRR_F16 || c == VRR_F16;
+  return !(bf && hf);
+}
 static bool gemm_ptrs_aligned16(const void* a, const void* b, const void* c, const void* c2, const void* bias) {
   return (((uintptr_t)a | (uintptr_t)b | (uintptr_t)c | (uintptr_t)c2 | (uintptr_t)bias) & 15) == 0;
 }
@@ -152,7 +157,7 @@ int vrr_set_option(const char* name, int value) {
 }
 
 size_t vrr_patch_embed_workspace_bytes(int B, int C, int Hi, int Wi, int P, int E, int dtype) {
-  if (dtype != VRR_BF16 || P <= 0 || !patch_embed_tc_supported(B, C, Hi, Wi, P, E)) return 0;
+  if (!is16(dtype) || P <= 0 || !patch_embed_tc_supported(B, C, Hi, Wi, P, E)) return 0;
   return patch_embed_tc_workspace_bytes(B, C, Hi, Wi, P);
 }
 
@@ -160,24 +165,24 @@ int vrr_patch_embed_fwd(const void* images, const void* weight, const void* bias
                         const void* pos_embed, void* tokens, void* workspace, size_t workspace_bytes, int B, int C,
                         int Hi, int Wi, int P, int E, int img_dtype, int dtype, int tok_dtype, void* stream) {
   VRR_REQUIRE(images && weight && bias && cls_token && tokens, VRR_ERR_INVALID_ARG, "patch_embed_fwd: NULL pointer");
-  VRR_REQUIRE(dtype_ok(dtype) && dtype_ok(tok_dtype) && dtype_ok(img_dtype), VRR_ERR_INVALID_ARG,
-              "patch_embed_fwd: bad dtype %d/%d/%d", img_dtype, dtype, tok_dtype);
+  VRR_REQUIRE(dtype_ok(dtype) && dtype_ok(tok_dtype) && dtype_ok(img_dtype) && no_mix(img_dtype, dtype, tok_dtype),
+              VRR_ERR_INVALID_ARG, "patch_embed_fwd: bad dtype %d/%d/%d", img_dtype, dtype, tok_dtype);
   VRR_REQUIRE(B > 0 && C > 0 && P > 0 && E > 0 && Hi >= P && Wi >= P, VRR_ERR_INVALID_ARG,
               "patch_embed_fwd: bad sizes B=%d C=%d Hi=%d Wi=%d P=%d E=%d", B, C, Hi, Wi, P, E);
   if (int rc = require_device()) return rc;
   const int impl = g_impl.load();
-  if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && patch_embed_tc_supported(B, C, Hi, Wi, P, E)) {
+  if (is16(dtype) && impl != VRR_IMPL_SIMT && patch_embed_tc_supported(B, C, Hi, Wi, P, E)) {
     const size_t need = patch_embed_tc_workspace_bytes(B, C, Hi, Wi, P);
     VRR_REQUIRE(workspace && workspace_bytes >= need, VRR_ERR_WORKSPACE,
                 "patch_embed_fwd: workspace %zu < %zu bytes (vrr_patch_embed_workspace_bytes)", workspace_bytes, need);
     VRR_REQUIRE(((uintptr_t)workspace & 255) == 0, VRR_ERR_INVALID_ARG, "patch_embed_fwd: workspace must be 256-byte aligned");
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
     if (int rc = patch_embed_fwd_tc(images, weight, bias, pos_embed, tokens, workspace, B, C, Hi, Wi, P, E, img_dtype,
-                                    tok_dtype, (cudaStream_t)stream))
+                                    dtype, tok_dtype, (cudaStream_t)stream))
       return rc;
     return patch_cls_rows(tokens, cls_token, B, (Hi / P) * (Wi / P), E, tok_dtype, (cudaStream_t)stream);
   }
-  VRR_REQUIRE(impl != VRR_IMPL_TCGEN05 || dtype != VRR_BF16, VRR_ERR_UNSUPPORTED,
+  VRR_REQUIRE(impl != VRR_IMPL_TCGEN05 || !is16(dtype), VRR_ERR_UNSUPPORTED,
               "patch_embed_fwd: tcgen05 kernel forced but shape unsupported (P %% 8, C*P*P %% 64, E %% 64)");
   VRR_COUNT_FAMILY(VRR_IMPL_SIMT);
   return patch_embed_fwd_simt(images, weight, bias, cls_token, pos_embed, tokens, B, C, Hi, Wi, P, E, img_dtype, dtype,
@@ -186,18 +191,28 @@ int vrr_patch_embed_fwd(const void* images, const void* weight, const void* bias
 
 int vrr_patch_unfold(const void* images, void* out, int B, int C, int Hi, int Wi, int P, int img_dtype, void* stream) {
   VRR_REQUIRE(images && out, VRR_ERR_INVALID_ARG, "patch_unfold: NULL pointer");
-  VRR_REQUIRE(dtype_ok(img_dtype), VRR_ERR_INVALID_ARG, "patch_unfold: bad dtype %d", img_dtype);
+  VRR_REQUIRE(img_dtype == VRR_F32 || img_dtype == VRR_BF16, VRR_ERR_INVALID_ARG, "patch_unfold: bad dtype %d", img_dtype);
   VRR_REQUIRE(B > 0 && C > 0 && P > 0 && Hi >= P && Wi >= P, VRR_ERR_INVALID_ARG, "patch_unfold: bad sizes");
   if (int rc = require_device()) return rc;
-  return patch_unfold(images, out, B, C, Hi, Wi, P, img_dtype, (cudaStream_t)stream);
+  return patch_unfold(images, out, B, C, Hi, Wi, P, img_dtype, VRR_BF16, (cudaStream_t)stream);
+}
+
+int vrr_patch_unfold_ex(const void* images, void* out, int B, int C, int Hi, int Wi, int P, int img_dtype, int out_dtype,
+                        void* stream) {
+  VRR_REQUIRE(images && out, VRR_ERR_INVALID_ARG, "patch_unfold_ex: NULL pointer");
+  VRR_REQUIRE(is16(out_dtype) && (img_dtype == VRR_F32 || img_dtype == out_dtype), VRR_ERR_INVALID_ARG,
+              "patch_unfold_ex: bad dtype %d -> %d", img_dtype, out_dtype);
+  VRR_REQUIRE(B > 0 && C > 0 && P > 0 && Hi >= P && Wi >= P, VRR_ERR_INVALID_ARG, "patch_unfold_ex: bad sizes");
+  if (int rc = require_device()) return rc;
+  return patch_unfold(images, out, B, C, Hi, Wi, P, img_dtype, out_dtype, (cudaStream_t)stream);
 }
 
 int vrr_patch_embed_bwd(const void* images, const void* d_tokens, void* d_weight, void* d_bias, void* d_cls,
                         void* d_pos, int B, int C, int Hi, int Wi, int P, int E, int img_dtype, int dtype,
                         int tok_dtype, void* stream) {
   VRR_REQUIRE(images && d_tokens && d_bias && d_cls, VRR_ERR_INVALID_ARG, "patch_embed_bwd: NULL pointer");
-  VRR_REQUIRE(dtype_ok(dtype) && dtype_ok(tok_dtype) && dtype_ok(img_dtype), VRR_ERR_INVALID_ARG,
-              "patch_embed_bwd: bad dtype %d/%d/%d", img_dtype, dtype, tok_dtype);
+  VRR_REQUIRE(dtype_ok(dtype) && dtype_ok(tok_dtype) && dtype_ok(img_dtype) && no_mix(img_dtype, dtype, tok_dtype),
+              VRR_ERR_INVALID_ARG, "patch_embed_bwd: bad dtype %d/%d/%d", img_dtype, dtype, tok_dtype);
   VRR_REQUIRE(B > 0 && C > 0 && P > 0 && E > 0 && Hi >= P && Wi >= P, VRR_ERR_INVALID_ARG,
               "patch_embed_bwd: bad sizes");
   if (int rc = require_device()) return rc;
@@ -231,12 +246,12 @@ int vrr_qkv_rope_fwd_packed(const void* x, const void* w_qkv, const float* cos_t
   VRR_REQUIRE(dh_ok(E / H), VRR_ERR_UNSUPPORTED, "qkv_rope_fwd: head dim %d unsupported (16, 32, 64)", E / H);
   if (int rc = require_device()) return rc;
   const int impl = g_impl.load();
-  if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && qkv_rope_fwd_tc_supported(B, N, E, H)) {
+  if (is16(dtype) && impl != VRR_IMPL_SIMT && qkv_rope_fwd_tc_supported(B, N, E, H)) {
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
-    return qkv_rope_fwd_tc2(x, w_qkv, cos_tab, sin_tab, packed, planes, B, N, E, H, rope_mode, (cudaStream_t)stream);
+    return qkv_rope_fwd_tc2(x, w_qkv, cos_tab, sin_tab, packed, planes, B, N, E, H, rope_mode, dtype, (cudaStream_t)stream);
   }
   VRR_REQUIRE(impl != VRR_IMPL_TCGEN05, VRR_ERR_UNSUPPORTED,
-              "qkv_rope_fwd: tcgen05 kernel forced but shape/dtype unsupported (bf16, Dh=64, E%%64==0)");
+              "qkv_rope_fwd: tcgen05 kernel forced but shape/dtype unsupported (bf16 or fp16, Dh=64, E%%64==0)");
   VRR_COUNT_FAMILY(VRR_IMPL_SIMT);
   return qkv_rope_fwd_simt(x, w_qkv, cos_tab, sin_tab, planes, B, N, E, H, rope_mode, dtype, (cudaStream_t)stream);
 }
@@ -287,7 +302,8 @@ int vrr_gemm(const void* a, const void* b, void* c, int M, int N, int K, int tra
              int c_dtype, void* stream) {
   VRR_REQUIRE(a && b && c, VRR_ERR_INVALID_ARG, "gemm: NULL pointer");
   VRR_REQUIRE(M > 0 && N > 0 && K > 0, VRR_ERR_INVALID_ARG, "gemm: bad sizes");
-  VRR_REQUIRE(dtype_ok(dtype) && dtype_ok(c_dtype), VRR_ERR_INVALID_ARG, "gemm: bad dtype %d/%d", dtype, c_dtype);
+  VRR_REQUIRE(dtype_ok(dtype) && dtype_ok(c_dtype) && no_mix(dtype, c_dtype), VRR_ERR_INVALID_ARG, "gemm: bad dtype %d/%d",
+              dtype, c_dtype);
   if (int rc = require_device()) return rc;
   return gemm_simt(a, b, c, M, N, K, trans_a, trans_b, dtype, c_dtype, (cudaStream_t)stream);
 }
@@ -296,7 +312,8 @@ int vrr_gemm_ex(const void* a, const void* b, void* c, void* c2, const float* bi
                 int trans_b, int dtype, int c_dtype, int epilogue, int accumulate, void* stream) {
   VRR_REQUIRE(a && b && c, VRR_ERR_INVALID_ARG, "gemm_ex: NULL pointer");
   VRR_REQUIRE(M > 0 && N > 0 && K > 0, VRR_ERR_INVALID_ARG, "gemm_ex: bad sizes");
-  VRR_REQUIRE(dtype_ok(dtype) && dtype_ok(c_dtype), VRR_ERR_INVALID_ARG, "gemm_ex: bad dtype %d/%d", dtype, c_dtype);
+  VRR_REQUIRE(dtype_ok(dtype) && dtype_ok(c_dtype) && no_mix(dtype, c_dtype), VRR_ERR_INVALID_ARG, "gemm_ex: bad dtype %d/%d",
+              dtype, c_dtype);
   VRR_REQUIRE(epilogue >= VRR_EPI_NONE && epilogue <= VRR_EPI_BIAS_GELU_ACT, VRR_ERR_INVALID_ARG, "gemm_ex: bad epilogue %d",
               epilogue);
   VRR_REQUIRE(epilogue == VRR_EPI_NONE || epilogue == VRR_EPI_MUL || bias, VRR_ERR_INVALID_ARG,
@@ -309,12 +326,11 @@ int vrr_gemm_ex(const void* a, const void* b, void* c, void* c2, const float* bi
   const bool uses_c2 = epilogue == VRR_EPI_BIAS_GELU || epilogue == VRR_EPI_BIAS_GELU_GRAD || epilogue == VRR_EPI_MUL;
   const bool uses_bias = epilogue != VRR_EPI_NONE && epilogue != VRR_EPI_MUL;
   const bool aligned = gemm_ptrs_aligned16(a, b, c, uses_c2 ? c2 : nullptr, uses_bias ? bias : nullptr);
-  if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && aligned &&
-      gemm_bf16_tc_supported(M, N, K, trans_a, trans_b, c_dtype, epilogue)) {
+  if (is16(dtype) && impl != VRR_IMPL_SIMT && aligned && gemm_tc_supported(M, N, K, trans_a, trans_b, dtype, c_dtype, epilogue)) {
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
-    return gemm_bf16_tc(a, b, c, c2, bias, M, N, K, trans_a, trans_b, c_dtype, epilogue, accumulate, (cudaStream_t)stream);
+    return gemm_tc(a, b, c, c2, bias, M, N, K, trans_a, trans_b, dtype, c_dtype, epilogue, accumulate, (cudaStream_t)stream);
   }
-  VRR_REQUIRE(impl != VRR_IMPL_TCGEN05 || dtype != VRR_BF16, VRR_ERR_UNSUPPORTED,
+  VRR_REQUIRE(impl != VRR_IMPL_TCGEN05 || !is16(dtype), VRR_ERR_UNSUPPORTED,
               "gemm_ex: tcgen05 kernel forced but M=%d N=%d K=%d (trans %d/%d) needs N %% 8 == 0, K %% 8 == 0 "
               "(M %% 8 == 0 when trans_a) and 16-byte aligned pointers", M, N, K, trans_a, trans_b);
   VRR_REQUIRE(!accumulate, VRR_ERR_UNSUPPORTED, "gemm_ex: accumulate is implemented by the tcgen05 kernel only");
@@ -343,12 +359,12 @@ int vrr_gemm_mul_colsum(const void* a, const void* b, void* c, const void* mul, 
   VRR_REQUIRE(dtype_ok(dtype), VRR_ERR_INVALID_ARG, "gemm_mul_colsum: bad dtype %d", dtype);
   if (int rc = require_device()) return rc;
   const int impl = g_impl.load();
-  if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && gemm_ptrs_aligned16(a, b, c, mul, nullptr) &&
-      gemm_bf16_tc_supported(M, N, K, trans_a, trans_b, VRR_BF16, VRR_EPI_MUL)) {
+  if (is16(dtype) && impl != VRR_IMPL_SIMT && gemm_ptrs_aligned16(a, b, c, mul, nullptr) &&
+      gemm_tc_supported(M, N, K, trans_a, trans_b, dtype, dtype, VRR_EPI_MUL)) {
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
     VRR_CUDA(cudaMemsetAsync(col_sums, 0, (size_t)N * sizeof(float), (cudaStream_t)stream));
-    return gemm_bf16_tc(a, b, c, const_cast<void*>(mul), nullptr, M, N, K, trans_a, trans_b, VRR_BF16, VRR_EPI_MUL, 0,
-                        (cudaStream_t)stream, col_sums);
+    return gemm_tc(a, b, c, const_cast<void*>(mul), nullptr, M, N, K, trans_a, trans_b, dtype, dtype, VRR_EPI_MUL, 0,
+                   (cudaStream_t)stream, col_sums);
   }
   if (int rc = vrr_gemm_ex(a, b, c, const_cast<void*>(mul), nullptr, M, N, K, trans_a, trans_b, dtype, dtype, VRR_EPI_MUL, 0, stream))
     return rc;
@@ -364,15 +380,15 @@ int vrr_attn_fwd(const void* planes, const vrr_bias_desc* bias, void* out, float
   if (int rc = check_bias(bias, H, N)) return rc;
   if (int rc = require_device()) return rc;
   const int impl = g_impl.load();
-  if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && attn_fwd_tc_supported(B, H, N, Dh, bias)) {
+  if (is16(dtype) && impl != VRR_IMPL_SIMT && attn_fwd_tc_supported(B, H, N, Dh, bias)) {
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
     // with a bias, N <= 256: the whole-sequence kernel; otherwise the tiled kernels (four CTAs per SM without bias)
     if (attn_fwd_ws_supported(B, H, N, Dh, bias))
-      return attn_fwd_ws(planes, bias, out, lse, B, H, N, Dh, scale, (cudaStream_t)stream);
-    return attn_fwd_tc(planes, bias, out, lse, B, H, N, Dh, scale, (cudaStream_t)stream);
+      return attn_fwd_ws(planes, bias, out, lse, B, H, N, Dh, scale, dtype, (cudaStream_t)stream);
+    return attn_fwd_tc(planes, bias, out, lse, B, H, N, Dh, scale, dtype, (cudaStream_t)stream);
   }
   VRR_REQUIRE(impl != VRR_IMPL_TCGEN05, VRR_ERR_UNSUPPORTED,
-              "attn_fwd: tcgen05 kernel forced but shape/dtype unsupported (bf16, Dh=64)");
+              "attn_fwd: tcgen05 kernel forced but shape/dtype unsupported (bf16 or fp16, Dh=64)");
   VRR_COUNT_FAMILY(VRR_IMPL_SIMT);
   return attn_fwd_simt(planes, bias, out, lse, B, H, N, Dh, scale, dtype, (cudaStream_t)stream);
 }
@@ -402,17 +418,17 @@ int vrr_attn_bwd(const void* planes, const vrr_bias_desc* bias, const void* out,
   size_t delta_bytes = (((size_t)B * H * N * sizeof(float) + 255) / 256) * 256;
   float* d_lut = (float*)((char*)workspace + delta_bytes);
   const int impl = g_impl.load();
-  if (dtype == VRR_BF16 && impl != VRR_IMPL_SIMT && attn_bwd_tc2_supported(B, H, N, Dh, bias)) {
+  if (is16(dtype) && impl != VRR_IMPL_SIMT && attn_bwd_tc2_supported(B, H, N, Dh, bias)) {
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
     if (attn_bwd_ws_supported(B, H, N, Dh, bias))  // short sequences, no bias: the whole-sequence kernel
-      return attn_bwd_ws(planes, out, d_out, lse, d_planes, B, H, N, Dh, scale, (cudaStream_t)stream);
-    return attn_bwd_tc2(planes, bias, out, d_out, lse, d_planes, d_bias_param, delta, B, H, N, Dh, scale,
+      return attn_bwd_ws(planes, out, d_out, lse, d_planes, B, H, N, Dh, scale, dtype, (cudaStream_t)stream);
+    return attn_bwd_tc2(planes, bias, out, d_out, lse, d_planes, d_bias_param, delta, B, H, N, Dh, scale, dtype,
                         (cudaStream_t)stream);
   }
   // e.g. polynomial degree > 3 (the tcgen05 kernel keeps 4 power sums per thread): explicit under
   // VRR_IMPL_TCGEN05, and visible to AUTO callers through vrr_family_count(VRR_IMPL_SIMT)
   VRR_REQUIRE(impl != VRR_IMPL_TCGEN05, VRR_ERR_UNSUPPORTED,
-              "attn_bwd: tcgen05 kernel forced but shape/dtype unsupported (bf16, Dh=64, poly degree <= 3)");
+              "attn_bwd: tcgen05 kernel forced but shape/dtype unsupported (bf16 or fp16, Dh=64, poly degree <= 3)");
   VRR_COUNT_FAMILY(VRR_IMPL_SIMT);
   return attn_bwd_simt(planes, bias, out, d_out, lse, d_planes, d_bias_param, delta, d_lut, B, H, N, Dh, scale,
                        dtype, (cudaStream_t)stream);
@@ -421,7 +437,7 @@ int vrr_attn_bwd(const void* planes, const vrr_bias_desc* bias, const void* out,
 int vrr_layernorm_fwd(const void* x, const float* gamma, const float* beta, void* y, float* mean, float* rstd, int M,
                       int E, float eps, int x_dtype, int y_dtype, void* stream) {
   VRR_REQUIRE(x && gamma && beta && y && mean && rstd, VRR_ERR_INVALID_ARG, "layernorm_fwd: NULL pointer");
-  VRR_REQUIRE(dtype_ok(x_dtype) && dtype_ok(y_dtype), VRR_ERR_INVALID_ARG, "layernorm_fwd: bad dtype");
+  VRR_REQUIRE(dtype_ok(x_dtype) && dtype_ok(y_dtype) && no_mix(x_dtype, y_dtype), VRR_ERR_INVALID_ARG, "layernorm_fwd: bad dtype");
   VRR_REQUIRE(M > 0 && E > 0, VRR_ERR_INVALID_ARG, "layernorm_fwd: bad sizes");
   VRR_REQUIRE((((uintptr_t)x | (uintptr_t)y | (uintptr_t)gamma | (uintptr_t)beta) & 15) == 0, VRR_ERR_INVALID_ARG,
               "layernorm_fwd: pointers must be 16-byte aligned");
@@ -432,7 +448,7 @@ int vrr_layernorm_fwd(const void* x, const float* gamma, const float* beta, void
 int vrr_layernorm_bwd(const void* dy, const void* x, const float* gamma, const float* mean, const float* rstd,
                       void* dx, float* dgamma, float* dbeta, int M, int E, int x_dtype, int y_dtype, void* stream) {
   VRR_REQUIRE(dy && x && gamma && mean && rstd && dx && dgamma && dbeta, VRR_ERR_INVALID_ARG, "layernorm_bwd: NULL pointer");
-  VRR_REQUIRE(dtype_ok(x_dtype) && dtype_ok(y_dtype), VRR_ERR_INVALID_ARG, "layernorm_bwd: bad dtype");
+  VRR_REQUIRE(dtype_ok(x_dtype) && dtype_ok(y_dtype) && no_mix(x_dtype, y_dtype), VRR_ERR_INVALID_ARG, "layernorm_bwd: bad dtype");
   VRR_REQUIRE(M > 0 && E > 0, VRR_ERR_INVALID_ARG, "layernorm_bwd: bad sizes");
   VRR_REQUIRE((((uintptr_t)x | (uintptr_t)dy | (uintptr_t)dx | (uintptr_t)gamma) & 15) == 0, VRR_ERR_INVALID_ARG,
               "layernorm_bwd: pointers must be 16-byte aligned");
@@ -444,7 +460,8 @@ int vrr_add_layernorm_fwd(const void* x, const void* branch, void* x_new, const 
                           void* y, float* mean, float* rstd, int M, int E, float eps, int branch_dtype, int y_dtype,
                           void* stream) {
   VRR_REQUIRE(x && branch && x_new && gamma && beta && y && mean && rstd, VRR_ERR_INVALID_ARG, "add_layernorm_fwd: NULL pointer");
-  VRR_REQUIRE(dtype_ok(branch_dtype) && dtype_ok(y_dtype), VRR_ERR_INVALID_ARG, "add_layernorm_fwd: bad dtype");
+  VRR_REQUIRE(dtype_ok(branch_dtype) && dtype_ok(y_dtype) && no_mix(branch_dtype, y_dtype), VRR_ERR_INVALID_ARG,
+              "add_layernorm_fwd: bad dtype");
   VRR_REQUIRE(M > 0 && E > 0, VRR_ERR_INVALID_ARG, "add_layernorm_fwd: bad sizes");
   VRR_REQUIRE((((uintptr_t)x | (uintptr_t)branch | (uintptr_t)x_new | (uintptr_t)y | (uintptr_t)gamma | (uintptr_t)beta) & 15) == 0,
               VRR_ERR_INVALID_ARG, "add_layernorm_fwd: pointers must be 16-byte aligned");
@@ -458,7 +475,8 @@ int vrr_add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new,
                           int branch_dtype, int y_dtype, void* stream) {
   VRR_REQUIRE(dy && x_new && gamma && mean && rstd && dx && d_branch && dgamma && dbeta, VRR_ERR_INVALID_ARG,
               "add_layernorm_bwd: NULL pointer");
-  VRR_REQUIRE(dtype_ok(branch_dtype) && dtype_ok(y_dtype), VRR_ERR_INVALID_ARG, "add_layernorm_bwd: bad dtype");
+  VRR_REQUIRE(dtype_ok(branch_dtype) && dtype_ok(y_dtype) && no_mix(branch_dtype, y_dtype), VRR_ERR_INVALID_ARG,
+              "add_layernorm_bwd: bad dtype");
   VRR_REQUIRE(M > 0 && E > 0, VRR_ERR_INVALID_ARG, "add_layernorm_bwd: bad sizes");
   VRR_REQUIRE((((uintptr_t)dy | (uintptr_t)d_xnew | (uintptr_t)x_new | (uintptr_t)dx | (uintptr_t)d_branch | (uintptr_t)gamma) & 15) == 0,
               VRR_ERR_INVALID_ARG, "add_layernorm_bwd: pointers must be 16-byte aligned");

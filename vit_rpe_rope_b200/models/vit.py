@@ -179,7 +179,7 @@ class VisionTransformer(nn.Module):
         ``forward`` only needs the cls row of the sum."""
         B, C, H, W = x.shape
         h, w = H // self.patch_size, W // self.patch_size
-        if x.is_cuda:  # one multi-tensor refresh of the bf16 weight copies per forward (no-op in fp32)
+        if x.is_cuda:  # one multi-tensor refresh of the 16-bit weight copies per forward (no-op in fp32)
             ops.refresh_lp_weights(self._gemm_weights(), ops.compute_dtype(x))
         abs_table = self.pos_embed.pos_embed if self.use_pos_embed_in_forward else None
         # (under autocast the token stream comes back fp32, like the reference's cat with the fp32 cls token)

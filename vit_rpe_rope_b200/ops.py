@@ -18,15 +18,18 @@ import torch
 
 from . import _lib
 
-_DT = {torch.float32: _lib.VRR_F32, torch.bfloat16: _lib.VRR_BF16}
+_DT = {torch.float32: _lib.VRR_F32, torch.bfloat16: _lib.VRR_BF16, torch.float16: _lib.VRR_F16}
+# the 16-bit compute dtypes: both run the same kernels (tcgen05 where the shape allows) and the same fusions
+_LP16 = (torch.bfloat16, torch.float16)
 
 
 def compute_dtype(x: torch.Tensor) -> torch.dtype:
-    """Element type the kernels run in: the autocast dtype inside ``torch.autocast('cuda')``
-    (how the build defines "bf16 training", SURVEY.md row O4), else the tensor's own dtype."""
+    """Element type the kernels run in: the autocast dtype inside ``torch.autocast('cuda')`` (bf16, or fp16 - the
+    default of ``torch.autocast('cuda')``; how the build defines "bf16 training", SURVEY.md row O4), else the tensor's
+    own dtype."""
     dt = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else x.dtype
     if dt not in _DT:
-        raise TypeError(f"vit_rpe_rope_b200 kernels support float32 and bfloat16, got {dt}")
+        raise TypeError(f"vit_rpe_rope_b200 kernels support float32, bfloat16 and float16, got {dt}")
     return dt
 
 
@@ -51,8 +54,8 @@ def _f32c(t):
 
 
 # ---- low-precision weight cache ---------------------------------------------------------------------
-# Under autocast the reference re-casts every fp32 weight to bf16 in every forward (~60 small cast kernels per
-# ViT-B step).  Here the model asks once per forward: the bf16 copies of all its GEMM weights are refreshed by
+# Under autocast the reference re-casts every fp32 weight to bf16 / fp16 in every forward (~60 small cast kernels per
+# ViT-B step).  Here the model asks once per forward: the 16-bit copies of all its GEMM weights are refreshed by
 # ONE multi-tensor copy, and only when a master weight changed (its version counter moved) - i.e. once per
 # optimizer step.  The GEMM Functions take the fp32 master (it receives the fp32 weight gradient straight from
 # the dW GEMM) plus this copy.
@@ -116,7 +119,7 @@ class PatchEmbedFn(torch.autograd.Function):
 
     weight / bias carry the conv dtype; cls_token / pos_embed / tokens the token-stream dtype (fp32
     under autocast, like the reference's cat with the fp32 cls token); images may stay fp32 when the
-    conv runs in bf16 - the rounding is fused into the kernel's load."""
+    conv runs in bf16 / fp16 - the rounding is fused into the kernel's load."""
 
     @staticmethod
     def forward(ctx, images, weight, bias, cls_token, pos_embed, patch):
@@ -127,7 +130,7 @@ class PatchEmbedFn(torch.autograd.Function):
         idt, dt, tdt = images.dtype, weight.dtype, cls_token.dtype
         if bias.dtype != dt or (pos_embed is not None and pos_embed.dtype != tdt):
             raise TypeError("patch_embed: weight/bias must share a dtype, cls_token/pos_embed another")
-        if idt != dt and not (idt == torch.float32 and dt == torch.bfloat16):
+        if idt != dt and not (idt == torch.float32 and dt in _LP16):
             raise TypeError(f"patch_embed: images {idt} with weights {dt} is not supported")
         images = images.contiguous()
         w = weight.detach().contiguous()
@@ -148,7 +151,7 @@ class PatchEmbedFn(torch.autograd.Function):
                                                _DT[tdt], _stream()), "vrr_patch_embed_fwd")
         if ctx.needs_input_grad[0]:
             ctx.w_for_dimg = w
-        # the tcgen05 path's workspace IS unfold(images) [B*Np][C*P*P] bf16: the weight-gradient GEMM reuses it
+        # the tcgen05 path's workspace IS unfold(images) [B*Np][C*P*P] in dt: the weight-gradient GEMM reuses it
         ctx.unfolded = ws if (ws is not None and ws_bytes == B * Np * C * patch * patch * 2) else None
         ctx.save_for_backward(images)
         ctx.meta = (B, C, Hi, Wi, patch, E, Np, pos_embed.shape if pos_embed is not None else None,
@@ -163,9 +166,9 @@ class PatchEmbedFn(torch.autograd.Function):
         d_tokens = d_tokens.contiguous()
         dev = images.device
         K = C * patch * patch
-        # bf16: the weight gradient is the GEMM d_tokens^T . unfold(images) on the tcgen05 kernel (fp32 result,
+        # bf16 / fp16: the weight gradient is the GEMM d_tokens^T . unfold(images) on the tcgen05 kernel (fp32 result,
         # split over the B*Np rows); fp32: the library's FFMA split-K GEMM with the unfold fused in.
-        own_dw = not (dt == torch.bfloat16 and patch % 8 == 0 and Wi % 4 == 0 and E % 8 == 0)
+        own_dw = not (dt in _LP16 and patch % 8 == 0 and Wi % 4 == 0 and E % 8 == 0)
         d_w = torch.empty(E, K, device=dev, dtype=torch.float32) if own_dw else None
         d_b = torch.empty(E, device=dev, dtype=torch.float32)
         d_cls = torch.empty(E, device=dev, dtype=torch.float32)
@@ -176,13 +179,13 @@ class PatchEmbedFn(torch.autograd.Function):
                                                _stream()), "vrr_patch_embed_bwd")
             if not own_dw:
                 if ctx.unfolded is not None:
-                    unf = ctx.unfolded.view(torch.bfloat16).view(B * Np, K)
+                    unf = ctx.unfolded.view(dt).view(B * Np, K)
                 else:
-                    unf = torch.empty(B * Np, K, device=dev, dtype=torch.bfloat16)
-                    _lib.check(lib.vrr_patch_unfold(_ptr(images), _ptr(unf), B, C, Hi, Wi, patch, _DT[idt], _stream()),
-                               "vrr_patch_unfold")
-                # cast first: one strided read + packed bf16 write (reshaping the fp32 slice first copied 154 MB twice)
-                g = d_tokens[:, 1:, :].to(torch.bfloat16).reshape(B * Np, E)
+                    unf = torch.empty(B * Np, K, device=dev, dtype=dt)
+                    _lib.check(lib.vrr_patch_unfold_ex(_ptr(images), _ptr(unf), B, C, Hi, Wi, patch, _DT[idt], _DT[dt],
+                                                       _stream()), "vrr_patch_unfold_ex")
+                # cast first: one strided read + packed 16-bit write (reshaping the fp32 slice first copied 154 MB twice)
+                g = d_tokens[:, 1:, :].to(dt).reshape(B * Np, E)
                 d_w = _gemm(g, unf, True, False, torch.float32, name="patch_dw")
         d_pos = None
         if pos_shape is not None:
@@ -194,10 +197,10 @@ class PatchEmbedFn(torch.autograd.Function):
 def patch_embed(images, weight, bias, cls_token, pos_embed, patch):
     """Conv weights are cast to the compute dtype (autograd-tracked casts keep fp32 master grads);
     under autocast the token stream (cls, pos, output) stays fp32 as in the reference, and fp32 images
-    are passed as they are (rounded to bf16 inside the kernel)."""
+    are passed as they are (rounded to bf16 / fp16 inside the kernel)."""
     dt = compute_dtype(images)
     tdt = torch.float32 if torch.is_autocast_enabled("cuda") else dt
-    if not (images.dtype == torch.float32 and dt == torch.bfloat16):
+    if not (images.dtype == torch.float32 and dt in _LP16):
         images = images.to(dt)
     return PatchEmbedFn.apply(images, weight.to(dt), bias.to(dt), cls_token.to(tdt),
                               None if pos_embed is None else pos_embed.to(tdt), patch)
@@ -254,7 +257,7 @@ class QkvRopeFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, w_qkv, cos, sin, num_heads, w_lp=None):
         """``w_qkv`` receives the gradient (fp32 master weight or a tensor already in x's dtype); ``w_lp`` is an
-        optional ready-made copy of it in x's dtype (the model's bf16 weight cache)."""
+        optional ready-made copy of it in x's dtype (the model's 16-bit weight cache)."""
         _require_cuda(x, w_qkv, cos, sin)
         lib = _lib.load()
         B, N, E = x.shape
@@ -267,7 +270,7 @@ class QkvRopeFn(torch.autograd.Function):
         planes = torch.empty(3, B, H, N, Dh, device=x.device, dtype=x.dtype)
         with torch.cuda.device(x.device):
             packed = None
-            if mode != _lib.ROPE_NONE and x.dtype == torch.bfloat16 and Dh == 64:  # the tcgen05 epilogue's table layout
+            if mode != _lib.ROPE_NONE and x.dtype in _LP16 and Dh == 64:  # the tcgen05 epilogue's table layout
                 packed = _packed_tables(cos32, sin32)
             with _timed("qkv_rope_fwd"):
                 _lib.check(lib.vrr_qkv_rope_fwd_packed(_ptr(x), _ptr(w), _ptr(cos32), _ptr(sin32), _ptr(packed), _ptr(planes),
@@ -306,9 +309,9 @@ class QkvRopeFn(torch.autograd.Function):
 def _gemm(a, b, trans_a, trans_b, out_dtype, bias=None, epilogue=_lib.EPI_NONE, out2=False, name="gemm", aux=None):
     """C = op(A) . op(B) in the library's kernels (``vrr_gemm_ex``) - no cuBLAS anywhere on the path.
 
-    op(A) is [M][K] (trans_a: A stored [K][M]); op(B) is [K][N] (trans_b: B stored [N][K]).  bf16 operands
-    run the tcgen05 CTA-pair kernel (fp32 accumulation; result in ``out_dtype``: bf16, or fp32 for weight
-    gradients), fp32 operands the exact-fp32 FFMA kernel (no TF32).  ``epilogue``: fused ``+ bias`` or
+    op(A) is [M][K] (trans_a: A stored [K][M]); op(B) is [K][N] (trans_b: B stored [N][K]).  bf16 / fp16 operands
+    run the tcgen05 CTA-pair kernel (fp32 accumulation; result in ``out_dtype``: the operands' type, or fp32 for
+    weight gradients), fp32 operands the exact-fp32 FFMA kernel (no TF32).  ``epilogue``: fused ``+ bias`` or
     ``+ bias, GELU`` (``out2``: second output - gelu(C) for EPI_BIAS_GELU; EPI_BIAS_GELU_GRAD returns
     (gelu(h), gelu'(h)) instead; EPI_BIAS_GELU_ACT returns gelu(h) alone); ``aux``: the [M][N] multiplier of EPI_MUL."""
     lib = _lib.load()
@@ -503,13 +506,13 @@ def add_layer_norm(x, branch, norm: torch.nn.LayerNorm):
 
 def layer_norm(x, norm: torch.nn.LayerNorm):
     """``norm(x)`` for an ``nn.LayerNorm`` over the last dimension, output in the compute dtype
-    (bf16 under autocast: the reference's LayerNorm-then-cast, fused).  Falls through to the module
+    (bf16 / fp16 under autocast: the reference's LayerNorm-then-cast, fused).  Falls through to the module
     itself for anything that is not a plain affine last-dim LayerNorm (a caller-supplied norm_layer)."""
     if (type(norm) is not torch.nn.LayerNorm or not norm.elementwise_affine or norm.bias is None
             or tuple(norm.normalized_shape) != (x.shape[-1],)):
         return norm(x)
     out_dtype = compute_dtype(x)
-    if x.dtype == torch.bfloat16 and out_dtype == torch.float32:
+    if x.dtype in _LP16 and out_dtype != x.dtype:
         x = x.float()
     return LayerNormFn.apply(x, norm.weight, norm.bias, norm.eps, out_dtype)
 
@@ -524,7 +527,7 @@ def _colsum(t2d):
 
 
 class LinearFn(torch.autograd.Function):
-    """y = x W^T + b (out-proj / head, models/vit.py:91,285).  bf16: forward GEMM with the bias in its
+    """y = x W^T + b (out-proj / head, models/vit.py:91,285).  bf16 / fp16: forward GEMM with the bias in its
     epilogue, dX and dW (fp32, straight into the master-weight gradient) on the tcgen05 CTA-pair kernel;
     bias gradient on the column-sum kernel.  ``w`` / ``b`` receive the gradients (fp32 masters or tensors in
     x's dtype); ``w_lp`` is an optional ready-made copy of ``w`` in x's dtype."""

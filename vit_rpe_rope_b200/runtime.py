@@ -151,12 +151,16 @@ class GraphedTrainStep:
 
 
 class GraphedInference:
-    """``model(images)`` under ``no_grad`` (and bf16 autocast) captured once and replayed with one launch: at small
-    batches the ~90 launches of a ViT-B forward cost more than the kernels (batch 1 at 1025 tokens: 4.5 ms eager).
-    ``run(images)`` copies the batch into the graph's static input and returns the static output tensor."""
+    """``model(images)`` under ``no_grad`` (and autocast to ``amp_dtype``, bf16 by default) captured once and replayed
+    with one launch: at small batches the ~90 launches of a ViT-B forward cost more than the kernels (batch 1 at 1025
+    tokens: 4.5 ms eager).  ``bf16=False`` runs without autocast (fp32).  ``run(images)`` copies the batch into the
+    graph's static input and returns the static output tensor."""
 
-    def __init__(self, model, images_shape, device, bf16: bool = True, use_graph: bool = True, warmup: int = 3):
-        self.model, self.bf16, self.device = model, bf16, device
+    def __init__(self, model, images_shape, device, bf16: bool = True, use_graph: bool = True, warmup: int = 3,
+                 amp_dtype: torch.dtype = torch.bfloat16):
+        if amp_dtype not in (torch.bfloat16, torch.float16):
+            raise ValueError(f"GraphedInference: amp_dtype must be torch.bfloat16 or torch.float16, got {amp_dtype}")
+        self.model, self.bf16, self.amp_dtype, self.device = model, bf16, amp_dtype, device
         self.static_images = torch.zeros(images_shape, device=device, dtype=torch.float32)
         self.static_out = None
         self.graph = None
@@ -177,7 +181,7 @@ class GraphedInference:
             torch.cuda.synchronize()
 
     def _eager(self):
-        with torch.no_grad(), torch.autocast("cuda", dtype=torch.bfloat16, enabled=self.bf16):
+        with torch.no_grad(), torch.autocast("cuda", dtype=self.amp_dtype, enabled=self.bf16):
             return self.model(self.static_images)
 
     def run(self, images=None):
