@@ -92,6 +92,23 @@ typedef struct {
   const float* param;  /* fp32 [heads][len]; NULL when mode == NONE                      */
 } vrr_bias_desc;
 
+/* Element dropout and stochastic depth (timm DropPath) applied inside the kernels that already read the data.
+ * Random numbers are Philox4x32-10 with key = *seed (low word = key[0]) and counter {g lo32, g hi32, site, stream}:
+ *   element (m, n) of an [M][E] site (E % 8 == 0): stream 0, g = (m E + n) / 8, 16-bit half (n & 1) (low half first)
+ *     of output word (n % 8) >> 1; kept iff that value < round((1 - p) 65536);
+ *   image b (rows b N .. b N + N - 1, N = rows_per_sample): stream 1, counter {b, 0, site, 1}; kept iff the low 16
+ *     bits of word 0 < round((1 - p_path) 65536).
+ * An element's factor is f = keep * keep_path(b) * s with s = (1 / (1 - p)) * (1 / (1 - p_path)) formed in fp32.
+ * A probability of 0 draws nothing for it.  The seed is read on the device, so a captured CUDA graph that refills
+ * it before the kernels gets fresh masks on every replay.  oracle/philox_np.py restates the masks. */
+typedef struct {
+  float p;                  /* element dropout probability, [0, 1)                            */
+  float p_path;             /* stochastic-depth probability per image, [0, 1); 0 where unused  */
+  int32_t rows_per_sample;  /* token rows per image (N): image of row m = m / rows_per_sample   */
+  int32_t site;             /* Philox counter word 2                                          */
+  const uint64_t* seed;     /* DEVICE pointer to the 64-bit Philox key                        */
+} vrr_drop_desc;
+
 /* ---- library ------------------------------------------------------------------------------- */
 int vrr_abi_version(void);
 const char* vrr_last_error(void);          /* thread-local, valid until the next call           */
@@ -251,6 +268,36 @@ int vrr_add_layernorm_fwd(const void* x, const void* branch, void* x_new, const 
 int vrr_add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new, const float* gamma,
                           const float* mean, const float* rstd, void* dx, void* d_branch, float* dgamma,
                           float* dbeta, int M, int E, int branch_dtype, int y_dtype, void* stream);
+
+/* The same with dropout / stochastic depth on the branch (Block with proj_drop / Mlp drop2 and DropPath):
+ *   forward : x_new = x + f * branch (the product rounded to fp32, never contracted into the add), so x_new, y,
+ *             mean and rstd are bit-identical to vrr_add_layernorm_fwd fed the fp32 branch f * branch;
+ *   backward: dx as vrr_add_layernorm_bwd; d_branch = round_to_branch_dtype(dx * f), the masks regenerated from the
+ *             same desc (nothing is stored between the passes).
+ * The element masks are indexed by (row, column) of the [M][E] stream (E % 8 == 0 when p > 0).  `drop` NULL, or
+ * p == p_path == 0, is exactly the entry point above. */
+int vrr_add_layernorm_drop_fwd(const void* x, const void* branch, void* x_new, const float* gamma,
+                               const float* beta, void* y, float* mean, float* rstd, int M, int E, float eps,
+                               int branch_dtype, int y_dtype, const vrr_drop_desc* drop, void* stream);
+int vrr_add_layernorm_drop_bwd(const void* dy, const void* d_xnew, const void* x_new, const float* gamma,
+                               const float* mean, const float* rstd, void* dx, void* d_branch, float* dgamma,
+                               float* dbeta, int M, int E, int branch_dtype, int y_dtype,
+                               const vrr_drop_desc* drop, void* stream);
+
+/* vrr_gemm_ex with element dropout on the GELU outputs (fc1 of an Mlp with drop1 > 0), for the epilogues
+ * VRR_EPI_BIAS_GELU_GRAD (C = T(T(gelu(h)) * f), C2 = T(T(gelu'(h)) * f)) and VRR_EPI_BIAS_GELU_ACT
+ * (C = T(T(gelu(h)) * f)), T = `dtype`; `drop->p_path` must be 0.  The mask is indexed by (m, n) of C (N % 8 == 0).
+ * This is torch's rounding of Dropout on a 16-bit tensor, and fc2's dX through VRR_EPI_MUL then yields
+ * (dy . W2) * gelu'(h) * f: Dropout's backward.  The tcgen05 kernel takes the Linear-forward layout (trans_a 0,
+ * trans_b 1) under the vrr_gemm_ex conditions; everything else runs the SIMT route. */
+int vrr_gemm_ex_drop(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K,
+                     int trans_a, int trans_b, int dtype, int c_dtype, int epilogue, int accumulate,
+                     const vrr_drop_desc* drop, void* stream);
+
+/* The decisions the kernels above take for `drop`: keep_u8 [M][E] (1 kept, 0 dropped; the element mask alone) and
+ * keep_path_u8 [ceil(M / rows_per_sample)] (the stochastic-depth decision per image); either may be NULL.  A
+ * probability of 0 writes all ones. */
+int vrr_dropout_mask(const vrr_drop_desc* drop, void* keep_u8, void* keep_path_u8, int M, int E, void* stream);
 
 /* fc2's input gradient with the GELU backward and fc1's bias gradient fused (autograd of timm Mlp, vit.py:118):
  *   c[m][n] = (op(a) . op(b))[m][n] * mul[m][n]   (`dtype`, as VRR_EPI_MUL)

@@ -14,6 +14,8 @@ Additions (all off by default, so a reference command line behaves like the refe
   --synthetic        class-conditional synthetic images instead of MNIST / CIFAR-10.  Chosen automatically when the
                      dataset is not on disk: this repository never downloads anything.
   --max_steps N      stop every epoch after N batches (smoke runs)
+  --drop_rate P      dropout on every block's attention projection and Mlp (timm's drop_rate)
+  --drop_path_rate P stochastic depth, linearly from 0 at the first block to P at the last (timm's drop_path_rate)
 There is no CPU path: a CUDA sm_100 device is required.
 """
 import argparse
@@ -61,6 +63,9 @@ def get_args(argv=None):
     p.add_argument("--max_steps", type=int, default=0)
     p.add_argument("--data_root", type=str, default="./data")
     p.add_argument("--seed", type=int, default=0)
+    p.add_argument("--drop_rate", type=float, default=0.0, help="proj / Mlp dropout of every block")
+    p.add_argument("--drop_path_rate", type=float, default=0.0,
+                   help="stochastic depth of the last block (linearly from 0 over the depth, timm's rule)")
     return p.parse_args(argv)
 
 
@@ -152,7 +157,8 @@ def main(argv=None):
     model = VisionTransformer(img_size=args.img_size, patch_size=args.patch_size, in_chans=in_chans, num_classes=num_classes,
                               embed_dim=args.embed_dim, depth=args.depth, num_heads=args.num_heads,
                               pos_encoding=args.pos_encoding, rope_theta=args.rope_theta, poly_degree=args.poly_degree,
-                              poly_shared_heads=args.poly_shared_heads).to(device)
+                              poly_shared_heads=args.poly_shared_heads, drop_rate=args.drop_rate,
+                              drop_path_rate=args.drop_path_rate).to(device)
     criterion = nn.CrossEntropyLoss()
     optimizer = torch.optim.AdamW(model.parameters(), lr=args.lr, weight_decay=args.weight_decay)
     scheduler = torch.optim.lr_scheduler.CosineAnnealingLR(optimizer, T_max=args.epochs)

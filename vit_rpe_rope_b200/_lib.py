@@ -29,6 +29,12 @@ class BiasDesc(Structure):
                 ("param", c_void_p)]
 
 
+class DropDesc(Structure):
+    """``vrr_drop_desc`` of include/vrr.h (``seed``: device pointer to the 64-bit Philox key)."""
+    _fields_ = [("p", c_float), ("p_path", c_float), ("rows_per_sample", c_int32), ("site", c_int32),
+                ("seed", c_void_p)]
+
+
 # name -> (restype, argtypes); must list every function include/vrr.h declares
 # (tests/test_c_abi.py parses the header and checks this table and the .so against it).
 SIGNATURES = {
@@ -57,6 +63,11 @@ SIGNATURES = {
     "vrr_layernorm_bwd": (c_int, [c_void_p] * 8 + [c_int] * 4 + [c_void_p]),
     "vrr_add_layernorm_fwd": (c_int, [c_void_p] * 8 + [c_int, c_int, c_float, c_int, c_int, c_void_p]),
     "vrr_add_layernorm_bwd": (c_int, [c_void_p] * 10 + [c_int] * 4 + [c_void_p]),
+    "vrr_add_layernorm_drop_fwd": (c_int, [c_void_p] * 8 + [c_int, c_int, c_float, c_int, c_int, POINTER(DropDesc),
+                                                           c_void_p]),
+    "vrr_add_layernorm_drop_bwd": (c_int, [c_void_p] * 10 + [c_int] * 4 + [POINTER(DropDesc), c_void_p]),
+    "vrr_gemm_ex_drop": (c_int, [c_void_p] * 5 + [c_int] * 9 + [POINTER(DropDesc), c_void_p]),
+    "vrr_dropout_mask": (c_int, [POINTER(DropDesc), c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "vrr_colsum": (c_int, [c_void_p] * 2 + [c_int] * 3 + [c_void_p]),
     "vrr_gemm_mul_colsum": (c_int, [c_void_p] * 5 + [c_int] * 6 + [c_void_p]),
     "vrr_gelu_bwd": (c_int, [c_void_p] * 4 + [c_int] * 3 + [c_void_p]),

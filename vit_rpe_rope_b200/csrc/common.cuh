@@ -112,6 +112,69 @@ __device__ __forceinline__ void st4(__half* p, float4 v) {
   *reinterpret_cast<uint2*>(p) = raw;
 }
 
+// ---- counter-based randomness for dropout / stochastic depth (vrr_drop_desc) ----------------------------
+// Philox4x32-10 (Salmon et al., SC'11; the Random123 constants).  Counter {g lo, g hi, site, stream}, key = the 64-bit
+// seed (low word first).  Element (m, n) of an [M][E] site (E % 8 == 0) is group g = (m E + n) / 8 of stream 0 and
+// uses 16-bit half (n & 1) of output word (n % 8) >> 1; image b's stochastic-depth decision is the low half of word
+// 0 of counter {b, 0, site, 1}.  Kept iff the 16 bits are below the threshold t = round((1 - p) 65536).
+// oracle/philox_np.py restates all of it.
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    if (r) {
+      k.x += 0x9E3779B9u;
+      k.y += 0xBB67AE85u;
+    }
+    const uint32_t lo0 = 0xD2511F53u * c.x, hi0 = __umulhi(0xD2511F53u, c.x);
+    const uint32_t lo1 = 0xCD9E8D57u * c.z, hi1 = __umulhi(0xCD9E8D57u, c.z);
+    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+  }
+  return c;
+}
+
+// Device-side view of vrr_drop_desc.  A threshold of 65536 keeps everything and draws nothing.
+struct DropView {
+  const unsigned long long* seed;
+  uint32_t t, t_path;     // element / stochastic-depth keep thresholds
+  float s;                // (1 / (1 - p)) * (1 / (1 - p_path)), formed in fp32
+  int rows_per_sample, site;
+  __device__ __forceinline__ uint2 key() const {
+    const unsigned long long k = *seed;
+    return make_uint2((uint32_t)k, (uint32_t)(k >> 32));
+  }
+  // factor of row m before the element mask: s, or 0 when the row's image is dropped
+  __device__ __forceinline__ float row_factor(uint2 k, int m) const {
+    if (t_path >= 65536u) return s;
+    const uint4 r = philox4x32_10(make_uint4((uint32_t)(m / rows_per_sample), 0u, (uint32_t)site, 1u), k);
+    return (r.x & 0xFFFFu) < t_path ? s : 0.f;
+  }
+  __device__ __forceinline__ uint4 bits(uint2 k, unsigned long long g) const {
+    return philox4x32_10(make_uint4((uint32_t)g, (uint32_t)(g >> 32), (uint32_t)site, 0u), k);
+  }
+  // factors of elements (m, n .. n + 3), n % 4 == 0, given the row factor fr
+  __device__ __forceinline__ float4 factor4(uint2 k, int m, int n, int E, float fr) const {
+    if (t >= 65536u) return make_float4(fr, fr, fr, fr);
+    const uint4 r = bits(k, ((unsigned long long)m * E + n) >> 3);
+    const uint32_t w0 = (n & 4) ? r.z : r.x, w1 = (n & 4) ? r.w : r.y;
+    return make_float4((w0 & 0xFFFFu) < t ? fr : 0.f, (w0 >> 16) < t ? fr : 0.f, (w1 & 0xFFFFu) < t ? fr : 0.f,
+                       (w1 >> 16) < t ? fr : 0.f);
+  }
+  __device__ __forceinline__ float factor(uint2 k, int m, int n, int E, float fr) const {
+    if (t >= 65536u) return fr;
+    const uint4 r = bits(k, ((unsigned long long)m * E + n) >> 3);
+    const int j = n & 7;
+    const uint32_t w = j < 2 ? r.x : (j < 4 ? r.y : (j < 6 ? r.z : r.w));
+    return ((j & 1) ? (w >> 16) : (w & 0xFFFFu)) < t ? fr : 0.f;
+  }
+};
+__device__ __forceinline__ float4 mul4_rn(float4 a, float4 f) {
+  return make_float4(__fmul_rn(a.x, f.x), __fmul_rn(a.y, f.y), __fmul_rn(a.z, f.z), __fmul_rn(a.w, f.w));
+}
+
+// vrr_drop_desc -> DropView (validated); `*active` = false when the desc draws nothing (NULL, or both
+// probabilities 0): the caller then runs the plain kernels.
+int drop_view(const vrr_drop_desc* d, int M, int E, DropView* v, bool* active);
+
 // ---- logit bias evaluated on the fly -------------------------------------------------------------
 // Device-side view of vrr_bias_desc for one head.  `lut` lives in shared memory:
 //   TABLE: the head's table row, lut[i - j + N - 1]

@@ -208,7 +208,66 @@ __global__ void mul_inplace_kernel(T* __restrict__ c, const T* __restrict__ m, s
     Elem<T>::st(c + i, Elem<T>::ld(c + i) * Elem<T>::ld(m + i));
 }
 
+// One thread per group of 8 elements (one Philox call).  c <- T(c * f); c2 (h on entry) <- T(T(gelu'(h)) * f).
+template <typename T>
+__global__ void drop_gelu_kernel(T* __restrict__ c, T* __restrict__ c2, int M, int N, const DropView dv) {
+  const uint2 key = dv.key();
+  const size_t groups = (size_t)M * N / 8;
+  for (size_t gi = (size_t)blockIdx.x * blockDim.x + threadIdx.x; gi < groups; gi += (size_t)gridDim.x * blockDim.x) {
+    const int m = (int)(gi * 8 / N), n = (int)(gi * 8 - (size_t)m * N);
+    const float4 f0 = dv.factor4(key, m, n, N, dv.s), f1 = dv.factor4(key, m, n + 4, N, dv.s);
+    const float f[8] = {f0.x, f0.y, f0.z, f0.w, f1.x, f1.y, f1.z, f1.w};
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      T* pc = c + gi * 8 + j;
+      Elem<T>::st(pc, Elem<T>::ld(pc) * f[j]);
+      if (c2) {
+        T* p2 = c2 + gi * 8 + j;
+        Elem<T>::st(p2, Elem<T>::round(gelu_grad(Elem<T>::ld(p2))) * f[j]);
+      }
+    }
+  }
+}
+
+// keep[m][n] (element mask alone) and keep_path[b] (stochastic depth per image), 1 = kept
+__global__ void dropout_mask_kernel(const DropView dv, uint8_t* __restrict__ keep, uint8_t* __restrict__ keep_path,
+                                    int M, int E, int images) {
+  const uint2 key = dv.key();
+  const size_t groups = keep ? (size_t)M * E / 8 : 0;
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t gi = (size_t)blockIdx.x * blockDim.x + threadIdx.x; gi < groups; gi += stride) {
+    const int m = (int)(gi * 8 / E), n = (int)(gi * 8 - (size_t)m * E);
+    const float4 f0 = dv.factor4(key, m, n, E, 1.f), f1 = dv.factor4(key, m, n + 4, E, 1.f);
+    uint2 w;
+    w.x = (f0.x != 0.f ? 1u : 0u) | (f0.y != 0.f ? 1u << 8 : 0u) | (f0.z != 0.f ? 1u << 16 : 0u) | (f0.w != 0.f ? 1u << 24 : 0u);
+    w.y = (f1.x != 0.f ? 1u : 0u) | (f1.y != 0.f ? 1u << 8 : 0u) | (f1.z != 0.f ? 1u << 16 : 0u) | (f1.w != 0.f ? 1u << 24 : 0u);
+    *reinterpret_cast<uint2*>(keep + gi * 8) = w;
+  }
+  if (keep_path)
+    for (size_t b = (size_t)blockIdx.x * blockDim.x + threadIdx.x; b < (size_t)images; b += stride)
+      keep_path[b] = dv.row_factor(key, (int)b * dv.rows_per_sample) != 0.f ? 1 : 0;
+}
+
 }  // namespace
+
+int drop_gelu_inplace(void* c, void* c2, int M, int N, int dtype, const DropView& dv, cudaStream_t st) {
+  const size_t groups = (size_t)M * N / 8;
+  const int grid = (int)((groups + 255) / 256 < 148 * 8 ? (groups + 255) / 256 : 148 * 8);
+  if (dtype == VRR_F32) drop_gelu_kernel<float><<<grid, 256, 0, st>>>((float*)c, (float*)c2, M, N, dv);
+  else if (dtype == VRR_BF16) drop_gelu_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>((__nv_bfloat16*)c, (__nv_bfloat16*)c2, M, N, dv);
+  else drop_gelu_kernel<__half><<<grid, 256, 0, st>>>((__half*)c, (__half*)c2, M, N, dv);
+  VRR_LAUNCHED();
+  return VRR_OK;
+}
+
+int dropout_mask(const DropView& dv, uint8_t* keep, uint8_t* keep_path, int M, int E, cudaStream_t st) {
+  const int images = dv.rows_per_sample > 0 ? ceil_div(M, dv.rows_per_sample) : 0;
+  const size_t work = keep ? (size_t)M * E / 8 : (size_t)images;
+  const int grid = (int)((work + 255) / 256 < 148 * 8 ? (work + 255) / 256 : 148 * 8);
+  dropout_mask_kernel<<<grid, 256, 0, st>>>(dv, keep, keep_path, M, E, keep_path ? images : 0);
+  VRR_LAUNCHED();
+  return VRR_OK;
+}
 
 int gelu_grad_inplace(void* h, size_t n, int dtype, cudaStream_t st) {
   const int grid = (int)((n + 255) / 256 < 148 * 8 ? (n + 255) / 256 : 148 * 8);

@@ -61,6 +61,7 @@ template <typename T>
 struct QkvRopeEpi2 {
   static constexpr bool kTma = false;
   static constexpr bool kPlaneStore = true;
+  static constexpr bool kDrop = false;
   T* planes;
   const float *cos_tab, *sin_tab;
   const float4* packed;  // rope_pack_tables layout [heads][16][N-1], or null
@@ -111,6 +112,7 @@ template <typename T, typename TT>
 struct PatchEmbedEpi2 {
   static constexpr bool kTma = false;
   static constexpr bool kPlaneStore = false;
+  static constexpr bool kDrop = false;
   TT* tokens;
   const T* bias;
   const TT* pos;  // may be null
@@ -142,6 +144,7 @@ template <typename T>
 struct StoreEpi {
   static constexpr bool kTma = true;
   static constexpr bool kPlaneStore = false;
+  static constexpr bool kDrop = false;
   const float* bias;  // fp32 [N] or null; rounded to T first for either C type (autocast casts the bias)
   int out_f32;        // C element type: 0 T, 1 fp32
   int reduce;         // fp32 only: C += tile via TMA reduce-add (split-K partial sums / gradient accumulation)
@@ -150,6 +153,14 @@ struct StoreEpi {
                       //         3: C = T(gelu(h)) only (inference): its own code path, one TMA store per chunk
   const T* mul;       // T C only, or null: C = T(acc * mul[m][n]) (mul is [M][N] like C): d_act * gelu'(h)
   float* colsum;      // T plain / bias / mul paths, or null: colsum[n] += sum_m C[m][n] (values as stored; atomics)
+};
+
+// fc1 with element dropout (vrr_gemm_ex_drop): gelu 2 or 3 as above, every output then T(T(value) * f).  A type of its
+// own, so that its epilogue branch is compiled into its own kernels and leaves the registers of the others alone.
+template <typename T>
+struct StoreEpiDrop : StoreEpi<T> {
+  static constexpr bool kDrop = true;
+  DropView dv;
 };
 
 // gelu(h) and d gelu / dh for TWO values at a time on the packed fp32x2 pipe (fma.rn.f32x2, sm_100): the epilogue of
@@ -340,7 +351,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         // will use (its previous TMA store has been read: bulk_wait_read<1>).
         [[maybe_unused]] uint4 mv[8];
         [[maybe_unused]] bool with_mul = false;
-        if constexpr (Epi::kTma) {
+        if constexpr (Epi::kTma && !Epi::kDrop) {
           with_mul = epi.mul != nullptr;
           if (with_mul) {
             const int n0m = n_blk * BN + chalf * (BN / 2) + c * 64;
@@ -355,7 +366,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         __syncwarp();  // tcgen05.ld is .sync.aligned
         tmem_ld32(trow + c * 64, *reinterpret_cast<uint32_t(*)[32]>(&v[0]));
         tmem_ld32(trow + c * 64 + 32, *reinterpret_cast<uint32_t(*)[32]>(&v[32]));
-        if constexpr (Epi::kTma) {
+        if constexpr (Epi::kTma && !Epi::kDrop) {
           if (with_mul) {
             const uint32_t tbuf = stage_u32 + (chunk_counter & 1u) * 4096u;
             if (lane == 0) bulk_wait_read<1>();
@@ -423,9 +434,67 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           const bool store_ok = (n0 < g.N) && (m_warp0 < g.M);
           const uint32_t sw = (uint32_t)(lane & 7);
           const uint32_t row_base = stage_u32 + (uint32_t)lane * 128u;
-          if (!epi.out_f32) {
+          if (Epi::kDrop || !epi.out_f32) {
             // ---- 16-bit C (T) ----
-            if (epi.gelu == 3) {
+            if constexpr (Epi::kDrop) {
+              // fc1 with dropout: (gelu(h), gelu'(h)) or gelu(h) alone, each rounded to T and multiplied by the keep
+              // factor of its element; one Philox call per 8 columns covers a group of the mask.  Computed in two
+              // halves of 32 columns, as in the two-output branch below.
+              const uint2 key = epi.dv.key();
+              const bool two = epi.gelu == 2;
+#pragma unroll
+              for (int hf = 0; hf < 2; ++hf) {
+                uint32_t o0[16], o1[16];
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                  const int c8 = hf * 4 + q;
+                  const int nb = min(n0 + c8 * 8, g.N - 8);
+                  const float4 b0 = __ldg(reinterpret_cast<const float4*>(epi.bias + nb));
+                  const float4 b1 = __ldg(reinterpret_cast<const float4*>(epi.bias + nb + 4));
+                  const uint32_t br[4] = {Elem16<T>::pack2(b0.x, b0.y), Elem16<T>::pack2(b0.z, b0.w), Elem16<T>::pack2(b1.x, b1.y), Elem16<T>::pack2(b1.z, b1.w)};
+                  const uint4 r = epi.dv.bits(key, ((unsigned long long)m * (unsigned)g.N + (unsigned)nb) >> 3);
+                  const uint32_t rw[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+                  for (int j = 0; j < 4; ++j) {
+                    const float2 bb = Elem16<T>::unpack2(br[j]);
+                    const float2 hs = __fadd2_rn(make_float2(f[c8 * 8 + 2 * j], f[c8 * 8 + 2 * j + 1]), bb);
+                    const float2 hr = Elem16<T>::unpack2(Elem16<T>::pack2(hs.x, hs.y));
+                    const float f0 = (rw[j] & 0xFFFFu) < epi.dv.t ? epi.dv.s : 0.f;
+                    const float f1 = (rw[j] >> 16) < epi.dv.t ? epi.dv.s : 0.f;
+                    if (two) {
+                      float2 gl, dg;
+                      gelu_and_grad2(hr, gl, dg);
+                      const float2 gr = Elem16<T>::unpack2(Elem16<T>::pack2(gl.x, gl.y));
+                      const float2 dr = Elem16<T>::unpack2(Elem16<T>::pack2(dg.x, dg.y));
+                      o0[q * 4 + j] = Elem16<T>::pack2(__fmul_rn(gr.x, f0), __fmul_rn(gr.y, f1));
+                      o1[q * 4 + j] = Elem16<T>::pack2(__fmul_rn(dr.x, f0), __fmul_rn(dr.y, f1));
+                    } else {
+                      const float2 gr = Elem16<T>::unpack2(gelu_only2<T>(hr));
+                      o0[q * 4 + j] = Elem16<T>::pack2(__fmul_rn(gr.x, f0), __fmul_rn(gr.y, f1));
+                    }
+                  }
+                }
+                if (hf == 0) {
+                  if (lane == 0) bulk_wait_read<0>();
+                  __syncwarp();
+                }
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                  const uint32_t off = (((uint32_t)(hf * 4 + q) ^ sw) << 4);
+                  st_shared_v4(row_base + off, o0[q * 4], o0[q * 4 + 1], o0[q * 4 + 2], o0[q * 4 + 3]);
+                  if (two) st_shared_v4(row_base + 4096u + off, o1[q * 4], o1[q * 4 + 1], o1[q * 4 + 2], o1[q * 4 + 3]);
+                }
+              }
+              fence_proxy_async_smem();
+              __syncwarp();
+              if (lane == 0) {
+                if (store_ok) {
+                  tma_store_2d(&tmap_c, my_stage, n0, m_warp0);
+                  if (two) tma_store_2d(&tmap_c2, my_stage + 4096, n0, m_warp0);
+                }
+                bulk_commit();
+              }
+            } else if (epi.gelu == 3) {
               // inference: gelu(h) alone.  Its own branch - folding it into the two-output code below cost that path
               // 50 us per launch (register allocation of the o0 / o1 arrays).
               uint32_t o0[32];
@@ -703,6 +772,22 @@ int launch_store(const void* a, const void* b, void* c, void* c2, const float* b
   return launch_pair<T, 128, A_MN, B_MN, StoreEpi<T>>(a, b, M, N, K, splits, tc_, tc2_, epi, st);
 }
 
+template <typename T>
+int launch_store_drop(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int epilogue,
+                      const DropView& dv, cudaStream_t st) {
+  StoreEpiDrop<T> epi = {};
+  epi.bias = bias;
+  epi.gelu = epilogue == VRR_EPI_BIAS_GELU_GRAD ? 2 : 3;
+  epi.dv = dv;
+  CUtensorMap tc_, tc2_;
+  if (int rc = make_tmap_2d(&tc_, c, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)N, (uint64_t)N * 2, 32, 64)) return rc;
+  tc2_ = tc_;
+  if (epi.gelu == 2)
+    if (int rc = make_tmap_2d(&tc2_, c2, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)N, (uint64_t)N * 2, 32, 64)) return rc;
+  if (N > 128) return launch_pair<T, 256, false, false, StoreEpiDrop<T>>(a, b, M, N, K, 1, tc_, tc2_, epi, st);
+  return launch_pair<T, 128, false, false, StoreEpiDrop<T>>(a, b, M, N, K, 1, tc_, tc2_, epi, st);
+}
+
 // unfold(images)[m][k], m = b*Np + py*gw + px, k = c*P*P + i*P + j  ->  TO (bf16 / fp16); 8 consecutive j per thread
 template <typename TI, typename TO>
 __global__ void patch_unfold_kernel(const TI* __restrict__ img, TO* __restrict__ out, int B, int C, int Hi,
@@ -767,6 +852,16 @@ int gemm_tc(const void* a, const void* b, void* c, void* c2, const float* bias, 
   if (dtype == VRR_F16)
     return gemm_tc_t<__half>(a, b, c, c2, bias, M, N, K, trans_a, trans_b, c_f32, epilogue, accumulate, st, colsum);
   return gemm_tc_t<__nv_bfloat16>(a, b, c, c2, bias, M, N, K, trans_a, trans_b, c_f32, epilogue, accumulate, st, colsum);
+}
+
+int gemm_tc_drop(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int dtype,
+                 int epilogue, const DropView& dv, cudaStream_t st) {
+  VRR_REQUIRE(is16(dtype) && (epilogue == VRR_EPI_BIAS_GELU_GRAD || epilogue == VRR_EPI_BIAS_GELU_ACT), VRR_ERR_UNSUPPORTED,
+              "gemm (tcgen05, dropout): 16-bit operands and the BIAS_GELU_GRAD / BIAS_GELU_ACT epilogues only");
+  VRR_REQUIRE(gemm_tc_supported(M, N, K, 0, 1, dtype, dtype, epilogue), VRR_ERR_UNSUPPORTED,
+              "gemm (tcgen05, dropout): unsupported shape M=%d N=%d K=%d", M, N, K);
+  if (dtype == VRR_F16) return launch_store_drop<__half>(a, b, c, c2, bias, M, N, K, epilogue, dv, st);
+  return launch_store_drop<__nv_bfloat16>(a, b, c, c2, bias, M, N, K, epilogue, dv, st);
 }
 
 // ---- QKV projection + RoPE epilogue on the CTA-pair kernel -----------------------------------------------

@@ -6,6 +6,8 @@
 
 namespace vrr {
 
+struct DropView;  // common.cuh
+
 // attn_simt.cu
 int attn_fwd_simt(const void* planes, const vrr_bias_desc* bias, void* out, float* lse, int B, int H, int N,
                   int Dh, float scale, int dtype, cudaStream_t st);
@@ -61,6 +63,9 @@ int patch_cls_rows(void* tokens, const void* cls, int B, int Np, int E, int tok_
 bool gemm_tc_supported(int M, int N, int K, int trans_a, int trans_b, int dtype, int c_dtype, int epilogue);
 int gemm_tc(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int trans_a,
             int trans_b, int dtype, int c_dtype, int epilogue, int accumulate, cudaStream_t st, float* colsum = nullptr);
+// fc1 with element dropout on the GELU outputs (VRR_EPI_BIAS_GELU_GRAD / _ACT, trans_a 0, trans_b 1, C of dtype)
+int gemm_tc_drop(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int dtype,
+                 int epilogue, const DropView& dv, cudaStream_t st);
 // colsum (16-bit C, plain / bias / multiply epilogues): colsum[n] += sum_m C[m][n] of the values as stored; zeroed by the caller
 int rope_pack_tables(const float* cos_tab, const float* sin_tab, float* packed, int heads, int rows, int hd, cudaStream_t st);
 bool qkv_rope_fwd_tc_supported(int B, int N, int E, int H);
@@ -83,18 +88,22 @@ int layernorm_fwd(const void* x, const float* gamma, const float* beta, void* y,
 int layernorm_bwd(const void* dy, const void* x, const float* gamma, const float* mean, const float* rstd, void* dx,
                   float* dgamma, float* dbeta, int M, int E, int x_dtype, int y_dtype, cudaStream_t st);
 
+// drop: NULL or a desc that draws nothing runs the plain kernels
 int add_layernorm_fwd(const void* x, const void* branch, void* x_new, const float* gamma, const float* beta, void* y,
                       float* mean, float* rstd, int M, int E, float eps, int branch_dtype, int y_dtype,
-                      cudaStream_t st);
+                      const vrr_drop_desc* drop, cudaStream_t st);
 int add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new, const float* gamma, const float* mean,
                       const float* rstd, void* dx, void* d_branch, float* dgamma, float* dbeta, int M, int E,
-                      int branch_dtype, int y_dtype, cudaStream_t st);
+                      int branch_dtype, int y_dtype, const vrr_drop_desc* drop, cudaStream_t st);
 
 // elementwise.cu
 int colsum(const void* x, float* out, int M, int C, int dtype, cudaStream_t st);
 int gelu_bwd_colsum(const void* dy, const void* h, void* dh, float* db, int M, int C, int dtype, cudaStream_t st);
 int gelu_grad_inplace(void* h, size_t n, int dtype, cudaStream_t st);            // h <- d gelu / dh (h)
 int mul_inplace(void* c, const void* m, size_t n, int dtype, cudaStream_t st);  // c <- c * m
+// c <- T(c * f) and, when c2 is given, c2 <- T(T(gelu'(c2)) * f) (SIMT route of vrr_gemm_ex_drop); c, c2 [M][N]
+int drop_gelu_inplace(void* c, void* c2, int M, int N, int dtype, const DropView& dv, cudaStream_t st);
+int dropout_mask(const DropView& dv, uint8_t* keep, uint8_t* keep_path, int M, int E, cudaStream_t st);
 
 // rope.cu
 int qkv_rope_bwd(const void* d_planes, const void* planes, const float* cos_tab, const float* sin_tab,

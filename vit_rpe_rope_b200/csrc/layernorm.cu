@@ -36,6 +36,19 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+// DROP (add+LayerNorm): 0 plain; 1 stochastic depth only (one factor per row); 2 element masks (and stochastic depth).
+// Factors of elements (m, n .. n + 3) / (m, n) given the row factor fr.
+template <int DROP>
+__device__ __forceinline__ float4 drop_f4(const DropView& dv, uint2 k, int m, int n, int E, float fr) {
+  if constexpr (DROP == 1) return make_float4(fr, fr, fr, fr);
+  else return dv.factor4(k, m, n, E, fr);
+}
+template <int DROP>
+__device__ __forceinline__ float drop_f1(const DropView& dv, uint2 k, int m, int n, int E, float fr) {
+  if constexpr (DROP == 1) return fr;
+  else return dv.factor(k, m, n, E, fr);
+}
+
 // VEC = 4: E % 128 == 0, 16-byte (fp32) / 8-byte (bf16) accesses; VEC = 1: any E.
 template <typename TX, typename TY, int VEC>
 __global__ void __launch_bounds__(kLnWarps * 32)
@@ -216,29 +229,44 @@ int ln_bwd_t(const void* dy, const void* x, const float* gamma, const float* mea
 // forward : reads x (fp32) and branch, writes x_new (fp32) and y.
 // backward: dx = d_xnew + LN'(dy) written as fp32 (gradient of the residual input) AND in the branch's
 //           dtype (gradient of the branch: the same values) - the autograd add and the cast disappear.
-template <typename TB, typename TY, int VEC>
+// DROP != 0: the branch is multiplied by its dropout / stochastic-depth factor f (DropView) as it is read, in every pass.
+template <typename TB, typename TY, int VEC, int DROP>
 __global__ void __launch_bounds__(kLnWarps * 32)
 add_ln_fwd_kernel(const float* __restrict__ x, const TB* __restrict__ branch, float* __restrict__ x_new,
                   const float* __restrict__ gamma, const float* __restrict__ beta, TY* __restrict__ y,
-                  float* __restrict__ mean_out, float* __restrict__ rstd_out, int M, int E, float eps) {
+                  float* __restrict__ mean_out, float* __restrict__ rstd_out, int M, int E, float eps, const DropView dv) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const float inv_e = 1.f / (float)E;
+  [[maybe_unused]] uint2 key;
+  if constexpr (DROP) key = dv.key();
   for (int row = blockIdx.x * kLnWarps + warp; row < M; row += gridDim.x * kLnWarps) {
     const float* xr = x + (size_t)row * E;
     const TB* br = branch + (size_t)row * E;
     float* nr = x_new + (size_t)row * E;
     TY* yr = y + (size_t)row * E;
+    [[maybe_unused]] float fr = 1.f;
+    if constexpr (DROP) fr = dv.row_factor(key, row);
+    auto ldb4 = [&](int c) {
+      float4 b = ld4(br + c);
+      if constexpr (DROP) b = mul4_rn(b, drop_f4<DROP>(dv, key, row, c, E, fr));
+      return b;
+    };
+    auto ldb1 = [&](int c) {
+      float b = Elem<TB>::ld(br + c);
+      if constexpr (DROP) b = __fmul_rn(b, drop_f1<DROP>(dv, key, row, c, E, fr));
+      return b;
+    };
     float s = 0.f;
     if (VEC == 4) {
       for (int c = lane * 4; c < E; c += 128) {
-        const float4 a = ld4(xr + c), b = ld4(br + c);
+        const float4 a = ld4(xr + c), b = ldb4(c);
         const float4 v = make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);
         st4(nr + c, v);
         s += (v.x + v.y) + (v.z + v.w);
       }
     } else {
       for (int c = lane; c < E; c += 32) {
-        const float v = xr[c] + Elem<TB>::ld(br + c);
+        const float v = xr[c] + ldb1(c);
         nr[c] = v;
         s += v;
       }
@@ -247,20 +275,20 @@ add_ln_fwd_kernel(const float* __restrict__ x, const TB* __restrict__ branch, fl
     float q = 0.f;
     if (VEC == 4) {
       for (int c = lane * 4; c < E; c += 128) {
-        const float4 a = ld4(xr + c), b = ld4(br + c);
+        const float4 a = ld4(xr + c), b = ldb4(c);
         const float d0 = a.x + b.x - mean, d1 = a.y + b.y - mean, d2 = a.z + b.z - mean, d3 = a.w + b.w - mean;
         q += (d0 * d0 + d1 * d1) + (d2 * d2 + d3 * d3);
       }
     } else {
       for (int c = lane; c < E; c += 32) {
-        const float d = xr[c] + Elem<TB>::ld(br + c) - mean;
+        const float d = xr[c] + ldb1(c) - mean;
         q += d * d;
       }
     }
     const float rstd = rsqrtf(warp_sum(q) * inv_e + eps);
     if (VEC == 4) {
       for (int c = lane * 4; c < E; c += 128) {
-        const float4 a = ld4(xr + c), b = ld4(br + c), g = ld4(gamma + c), bt = ld4(beta + c);
+        const float4 a = ld4(xr + c), b = ldb4(c), g = ld4(gamma + c), bt = ld4(beta + c);
         float4 o;
         o.x = (a.x + b.x - mean) * rstd * g.x + bt.x;
         o.y = (a.y + b.y - mean) * rstd * g.y + bt.y;
@@ -270,7 +298,7 @@ add_ln_fwd_kernel(const float* __restrict__ x, const TB* __restrict__ branch, fl
       }
     } else {
       for (int c = lane; c < E; c += 32)
-        Elem<TY>::st(yr + c, (xr[c] + Elem<TB>::ld(br + c) - mean) * rstd * gamma[c] + beta[c]);
+        Elem<TY>::st(yr + c, (xr[c] + ldb1(c) - mean) * rstd * gamma[c] + beta[c]);
     }
     if (lane == 0) {
       mean_out[row] = mean;
@@ -279,12 +307,13 @@ add_ln_fwd_kernel(const float* __restrict__ x, const TB* __restrict__ branch, fl
   }
 }
 
-template <typename TB, typename TY, int VEC>
+// DROP != 0: d_branch = dx * f (the factor of the forward, regenerated)
+template <typename TB, typename TY, int VEC, int DROP>
 __global__ void __launch_bounds__(kLnWarps * 32)
 add_ln_bwd_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, const float* __restrict__ x_new,
                   const float* __restrict__ gamma, const float* __restrict__ mean_in,
                   const float* __restrict__ rstd_in, float* __restrict__ dx, TB* __restrict__ d_branch,
-                  float* __restrict__ dgamma, float* __restrict__ dbeta, int M, int E) {
+                  float* __restrict__ dgamma, float* __restrict__ dbeta, int M, int E, const DropView dv) {
   extern __shared__ __align__(16) float ln_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   float* pg = ln_smem + (size_t)warp * E;
@@ -295,10 +324,14 @@ add_ln_bwd_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, c
   }
   __syncwarp();
   const float inv_e = 1.f / (float)E;
+  [[maybe_unused]] uint2 key;
+  if constexpr (DROP) key = dv.key();
   for (int row = blockIdx.x * kLnWarps + warp; row < M; row += gridDim.x * kLnWarps) {
     const TY* gr = dy + (size_t)row * E;
     const float* xr = x_new + (size_t)row * E;
     const float* rr = d_xnew ? d_xnew + (size_t)row * E : nullptr;
+    [[maybe_unused]] float fr = 1.f;
+    if constexpr (DROP) fr = dv.row_factor(key, row);
     float* dr = dx + (size_t)row * E;
     TB* br = d_branch + (size_t)row * E;
     const float mean = mean_in[row], rstd = rstd_in[row];
@@ -339,7 +372,8 @@ add_ln_bwd_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, c
         }
         const float4 ov = make_float4(o[0], o[1], o[2], o[3]);
         st4(dr + c, ov);
-        st4(br + c, ov);
+        if constexpr (DROP) st4(br + c, mul4_rn(ov, drop_f4<DROP>(dv, key, row, c, E, fr)));
+        else st4(br + c, ov);
         *reinterpret_cast<float4*>(pg + c) = make_float4(agv[0], agv[1], agv[2], agv[3]);
         *reinterpret_cast<float4*>(pb + c) = make_float4(abv[0], abv[1], abv[2], abv[3]);
       }
@@ -348,7 +382,8 @@ add_ln_bwd_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, c
         const float g = Elem<TY>::ld(gr + c), xh = (xr[c] - mean) * rstd;
         const float o = (rr ? rr[c] : 0.f) + rstd * (g * gamma[c] - c1 - xh * c2);
         dr[c] = o;
-        Elem<TB>::st(br + c, o);
+        if constexpr (DROP) Elem<TB>::st(br + c, __fmul_rn(o, drop_f1<DROP>(dv, key, row, c, E, fr)));
+        else Elem<TB>::st(br + c, o);
         pg[c] = fmaf(g, xh, pg[c]);
         pb[c] += g;
       }
@@ -374,11 +409,11 @@ add_ln_bwd_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, c
 // passes and its slice of the dgamma / dbeta partial sums in registers across ROWS (a lane owns the same columns
 // for every row), touching shared memory once per CTA for the cross-warp reduction.  Same operation order per
 // element as the generic kernels, so the results are bit-identical to them.
-template <typename TB, typename TY, int NV>
+template <typename TB, typename TY, int NV, int DROP>
 __global__ void __launch_bounds__(kLnWarps * 32)
 add_ln_fwd_reg_kernel(const float* __restrict__ x, const TB* __restrict__ branch, float* __restrict__ x_new,
                       const float* __restrict__ gamma, const float* __restrict__ beta, TY* __restrict__ y,
-                      float* __restrict__ mean_out, float* __restrict__ rstd_out, int M, float eps) {
+                      float* __restrict__ mean_out, float* __restrict__ rstd_out, int M, float eps, const DropView dv) {
   constexpr int E = NV * 128;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const float inv_e = 1.f / (float)E;
@@ -388,6 +423,8 @@ add_ln_fwd_reg_kernel(const float* __restrict__ x, const TB* __restrict__ branch
     g[i] = ld4(gamma + lane * 4 + i * 128);
     bt[i] = ld4(beta + lane * 4 + i * 128);
   }
+  [[maybe_unused]] uint2 key;
+  if constexpr (DROP) key = dv.key();
   for (int row = blockIdx.x * kLnWarps + warp; row < M; row += gridDim.x * kLnWarps) {
     const float* xr = x + (size_t)row * E + lane * 4;
     const TB* br = branch + (size_t)row * E + lane * 4;
@@ -395,9 +432,13 @@ add_ln_fwd_reg_kernel(const float* __restrict__ x, const TB* __restrict__ branch
     TY* yr = y + (size_t)row * E + lane * 4;
     float4 v[NV];
     float s = 0.f;
+    [[maybe_unused]] float fr = 1.f;
+    if constexpr (DROP) fr = dv.row_factor(key, row);
 #pragma unroll
     for (int i = 0; i < NV; ++i) {
-      const float4 a = ld4(xr + i * 128), b = ld4(br + i * 128);
+      const float4 a = ld4(xr + i * 128);
+      float4 b = ld4(br + i * 128);
+      if constexpr (DROP) b = mul4_rn(b, drop_f4<DROP>(dv, key, row, lane * 4 + i * 128, E, fr));
       v[i] = make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);
     }
 #pragma unroll
@@ -429,12 +470,12 @@ add_ln_fwd_reg_kernel(const float* __restrict__ x, const TB* __restrict__ branch
   }
 }
 
-template <typename TB, typename TY, int NV, int WARPS, int MINB>
+template <typename TB, typename TY, int NV, int WARPS, int MINB, int DROP>
 __global__ void __launch_bounds__(WARPS * 32, MINB)
 add_ln_bwd_reg_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, const float* __restrict__ x_new,
                       const float* __restrict__ gamma, const float* __restrict__ mean_in, const float* __restrict__ rstd_in,
                       float* __restrict__ dx, TB* __restrict__ d_branch, float* __restrict__ dgamma,
-                      float* __restrict__ dbeta, int M) {
+                      float* __restrict__ dbeta, int M, const DropView dv) {
   constexpr int E = NV * 128;
   extern __shared__ __align__(16) float ln_smem[];  // [2][WARPS][E], used once at the end
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -442,6 +483,8 @@ add_ln_bwd_reg_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xne
   float4 pg[NV], pb[NV];
 #pragma unroll
   for (int i = 0; i < NV; ++i) pg[i] = pb[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+  [[maybe_unused]] uint2 key;
+  if constexpr (DROP) key = dv.key();
   for (int row = blockIdx.x * WARPS + warp; row < M; row += gridDim.x * WARPS) {
     const TY* gr = dy + (size_t)row * E + lane * 4;
     const float* xr = x_new + (size_t)row * E + lane * 4;
@@ -454,6 +497,18 @@ add_ln_bwd_reg_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xne
     for (int i = 0; i < NV; ++i) {
       g[i] = ld4(gr + i * 128);
       xh[i] = ld4(xr + i * 128);
+    }
+    // the row's factor and (DROP == 2) keep bits (4 per float4), drawn while its loads are in flight: at one CTA of
+    // 12 warps per SM the Philox rounds were exposed when they ran in the output loop
+    [[maybe_unused]] float fr = 1.f;
+    if constexpr (DROP) fr = dv.row_factor(key, row);
+    [[maybe_unused]] uint32_t kb = 0;
+    if constexpr (DROP == 2) {
+#pragma unroll
+      for (int i = 0; i < NV; ++i) {
+        const float4 f = dv.factor4(key, row, lane * 4 + i * 128, E, 1.f);
+        kb |= ((f.x != 0.f ? 1u : 0u) | (f.y != 0.f ? 2u : 0u) | (f.z != 0.f ? 4u : 0u) | (f.w != 0.f ? 8u : 0u)) << (4 * i);
+      }
     }
     float s1 = 0.f, s2 = 0.f;
 #pragma unroll
@@ -479,7 +534,14 @@ add_ln_bwd_reg_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xne
       o.z = r.z + rstd * (g[i].z * w.z - c1 - xh[i].z * c2);
       o.w = r.w + rstd * (g[i].w * w.w - c1 - xh[i].w * c2);
       st4(dr + i * 128, o);
-      st4(br + i * 128, o);
+      if constexpr (DROP == 1) {
+        st4(br + i * 128, mul4_rn(o, make_float4(fr, fr, fr, fr)));
+      } else if constexpr (DROP == 2) {
+        const uint32_t b4 = kb >> (4 * i);
+        st4(br + i * 128, mul4_rn(o, make_float4(b4 & 1u ? fr : 0.f, b4 & 2u ? fr : 0.f, b4 & 4u ? fr : 0.f, b4 & 8u ? fr : 0.f)));
+      } else {
+        st4(br + i * 128, o);
+      }
       pg[i].x = fmaf(g[i].x, xh[i].x, pg[i].x);
       pg[i].y = fmaf(g[i].y, xh[i].y, pg[i].y);
       pg[i].z = fmaf(g[i].z, xh[i].z, pg[i].z);
@@ -508,45 +570,45 @@ add_ln_bwd_reg_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xne
   }
 }
 
-template <typename TB, typename TY>
+template <typename TB, typename TY, int DROP>
 int add_ln_fwd_t(const float* x, const void* branch, float* x_new, const float* gamma, const float* beta, void* y,
-                 float* mean, float* rstd, int M, int E, float eps, cudaStream_t st) {
+                 float* mean, float* rstd, int M, int E, float eps, const DropView& dv, cudaStream_t st) {
   const int grid = min(ceil_div(M, kLnWarps), 8 * sm_count());
 #define VRR_LN_REG(NV)                                                                                                \
   if (g_ln_reg && E == NV * 128) { \
     const int g2 = min(ceil_div(M, kLnWarps), 4 * sm_count());                                                        \
-    add_ln_fwd_reg_kernel<TB, TY, NV><<<g2, kLnWarps * 32, 0, st>>>(x, (const TB*)branch, x_new, gamma, beta, (TY*)y, \
-                                                                    mean, rstd, M, eps);                              \
+    add_ln_fwd_reg_kernel<TB, TY, NV, DROP><<<g2, kLnWarps * 32, 0, st>>>(x, (const TB*)branch, x_new, gamma, beta,  \
+                                                                          (TY*)y, mean, rstd, M, eps, dv);            \
     VRR_LAUNCHED();                                                                                                   \
     return VRR_OK;                                                                                                    \
   }
   VRR_LN_REG(6) VRR_LN_REG(8) VRR_LN_REG(4) VRR_LN_REG(2)
 #undef VRR_LN_REG
   if (E % 128 == 0)
-    add_ln_fwd_kernel<TB, TY, 4><<<grid, kLnWarps * 32, 0, st>>>(x, (const TB*)branch, x_new, gamma, beta, (TY*)y, mean, rstd, M, E, eps);
+    add_ln_fwd_kernel<TB, TY, 4, DROP><<<grid, kLnWarps * 32, 0, st>>>(x, (const TB*)branch, x_new, gamma, beta, (TY*)y, mean, rstd, M, E, eps, dv);
   else
-    add_ln_fwd_kernel<TB, TY, 1><<<grid, kLnWarps * 32, 0, st>>>(x, (const TB*)branch, x_new, gamma, beta, (TY*)y, mean, rstd, M, E, eps);
+    add_ln_fwd_kernel<TB, TY, 1, DROP><<<grid, kLnWarps * 32, 0, st>>>(x, (const TB*)branch, x_new, gamma, beta, (TY*)y, mean, rstd, M, E, eps, dv);
   VRR_LAUNCHED();
   return VRR_OK;
 }
 
-template <typename TB, typename TY, int VEC>
+template <typename TB, typename TY, int VEC, int DROP>
 int add_ln_bwd_launch(const void* dy, const float* d_xnew, const float* x_new, const float* gamma, const float* mean,
                       const float* rstd, float* dx, void* d_branch, float* dgamma, float* dbeta, int M, int E,
-                      cudaStream_t st) {
+                      const DropView& dv, cudaStream_t st) {
   const size_t smem = (size_t)2 * kLnWarps * E * sizeof(float);
-  auto kern = add_ln_bwd_kernel<TB, TY, VEC>;
+  auto kern = add_ln_bwd_kernel<TB, TY, VEC, DROP>;
   VRR_SMEM_ATTR_ONCE(kern, 160 * 1024);
   const int grid = min(ceil_div(M, kLnWarps), ln_bwd_ctas_per_sm(E) * sm_count());
-  kern<<<grid, kLnWarps * 32, smem, st>>>((const TY*)dy, d_xnew, x_new, gamma, mean, rstd, dx, (TB*)d_branch, dgamma, dbeta, M, E);
+  kern<<<grid, kLnWarps * 32, smem, st>>>((const TY*)dy, d_xnew, x_new, gamma, mean, rstd, dx, (TB*)d_branch, dgamma, dbeta, M, E, dv);
   VRR_LAUNCHED();
   return VRR_OK;
 }
 
-template <typename TB, typename TY>
+template <typename TB, typename TY, int DROP>
 int add_ln_bwd_t(const void* dy, const float* d_xnew, const float* x_new, const float* gamma, const float* mean,
                  const float* rstd, float* dx, void* d_branch, float* dgamma, float* dbeta, int M, int E,
-                 cudaStream_t st) {
+                 const DropView& dv, cudaStream_t st) {
   if (dbeta == dgamma + E) {  // the two rows of one [2][E] buffer (what ops.py allocates): one memset node instead of two
     VRR_CUDA(cudaMemsetAsync(dgamma, 0, (size_t)2 * E * sizeof(float), st));
   } else {
@@ -554,11 +616,11 @@ int add_ln_bwd_t(const void* dy, const float* d_xnew, const float* x_new, const 
     VRR_CUDA(cudaMemsetAsync(dbeta, 0, (size_t)E * sizeof(float), st));
   }
 #define VRR_LN_BWD_GO(NV, W, B)                                                                                          \
-  auto kern = add_ln_bwd_reg_kernel<TB, TY, NV, W, B>;                                                                 \
+  auto kern = add_ln_bwd_reg_kernel<TB, TY, NV, W, B, DROP>;                                                           \
   VRR_SMEM_ATTR_ONCE(kern, 160 * 1024);                                                                                \
   const int grid = min(ceil_div(M, W), B * sm_count());                                                                \
   kern<<<grid, W * 32, (size_t)2 * W * E * sizeof(float), st>>>((const TY*)dy, d_xnew, x_new, gamma, mean, rstd, dx,   \
-                                                                (TB*)d_branch, dgamma, dbeta, M);
+                                                                (TB*)d_branch, dgamma, dbeta, M, dv);
 #define VRR_LN_REG(NV)                                                                                                  \
   if (g_ln_reg && E == NV * 128) { \
     if (NV <= 4 || g_ln_bwd_minb == 2) {                                                                                \
@@ -574,8 +636,8 @@ int add_ln_bwd_t(const void* dy, const float* d_xnew, const float* x_new, const 
   VRR_LN_REG(6) VRR_LN_REG(8) VRR_LN_REG(4) VRR_LN_REG(2)
 #undef VRR_LN_REG
   if (E % 128 == 0)
-    return add_ln_bwd_launch<TB, TY, 4>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, st);
-  return add_ln_bwd_launch<TB, TY, 1>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, st);
+    return add_ln_bwd_launch<TB, TY, 4, DROP>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, dv, st);
+  return add_ln_bwd_launch<TB, TY, 1, DROP>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, dv, st);
 }
 
 }  // namespace
@@ -611,36 +673,68 @@ int layernorm_bwd(const void* dy, const void* x, const float* gamma, const float
   return VRR_ERR_UNSUPPORTED;
 }
 
-int add_layernorm_fwd(const void* x, const void* branch, void* x_new, const float* gamma, const float* beta, void* y,
-                      float* mean, float* rstd, int M, int E, float eps, int branch_dtype, int y_dtype,
-                      cudaStream_t st) {
+template <int DROP>
+static int add_layernorm_fwd_d(const void* x, const void* branch, void* x_new, const float* gamma, const float* beta,
+                               void* y, float* mean, float* rstd, int M, int E, float eps, int branch_dtype, int y_dtype,
+                               const DropView& dv, cudaStream_t st) {
   VRR_REQUIRE((size_t)2 * kLnWarps * E * sizeof(float) <= 160 * 1024, VRR_ERR_UNSUPPORTED,
               "add_layernorm: E = %d too large (max 2560)", E);
-#define ARGS (const float*)x, branch, (float*)x_new, gamma, beta, y, mean, rstd, M, E, eps, st
-  if (branch_dtype == VRR_F32 && y_dtype == VRR_F32) return add_ln_fwd_t<float, float>(ARGS);
-  if (branch_dtype == VRR_BF16 && y_dtype == VRR_BF16) return add_ln_fwd_t<__nv_bfloat16, __nv_bfloat16>(ARGS);
-  if (branch_dtype == VRR_F32 && y_dtype == VRR_BF16) return add_ln_fwd_t<float, __nv_bfloat16>(ARGS);
-  if (branch_dtype == VRR_F16 && y_dtype == VRR_F16) return add_ln_fwd_t<__half, __half>(ARGS);
-  if (branch_dtype == VRR_F32 && y_dtype == VRR_F16) return add_ln_fwd_t<float, __half>(ARGS);
+#define ARGS (const float*)x, branch, (float*)x_new, gamma, beta, y, mean, rstd, M, E, eps, dv, st
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_F32) return add_ln_fwd_t<float, float, DROP>(ARGS);
+  if (branch_dtype == VRR_BF16 && y_dtype == VRR_BF16) return add_ln_fwd_t<__nv_bfloat16, __nv_bfloat16, DROP>(ARGS);
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_BF16) return add_ln_fwd_t<float, __nv_bfloat16, DROP>(ARGS);
+  if (branch_dtype == VRR_F16 && y_dtype == VRR_F16) return add_ln_fwd_t<__half, __half, DROP>(ARGS);
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_F16) return add_ln_fwd_t<float, __half, DROP>(ARGS);
 #undef ARGS
   set_error("add_layernorm_fwd: unsupported dtype combination (branch %d, y %d)", branch_dtype, y_dtype);
   return VRR_ERR_UNSUPPORTED;
 }
 
-int add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new, const float* gamma, const float* mean,
-                      const float* rstd, void* dx, void* d_branch, float* dgamma, float* dbeta, int M, int E,
-                      int branch_dtype, int y_dtype, cudaStream_t st) {
+template <int DROP>
+static int add_layernorm_bwd_d(const void* dy, const void* d_xnew, const void* x_new, const float* gamma,
+                               const float* mean, const float* rstd, void* dx, void* d_branch, float* dgamma,
+                               float* dbeta, int M, int E, int branch_dtype, int y_dtype, const DropView& dv,
+                               cudaStream_t st) {
   VRR_REQUIRE((size_t)2 * kLnWarps * E * sizeof(float) <= 160 * 1024, VRR_ERR_UNSUPPORTED,
               "add_layernorm: E = %d too large (max 2560)", E);
-#define ARGS dy, (const float*)d_xnew, (const float*)x_new, gamma, mean, rstd, (float*)dx, d_branch, dgamma, dbeta, M, E, st
-  if (branch_dtype == VRR_F32 && y_dtype == VRR_F32) return add_ln_bwd_t<float, float>(ARGS);
-  if (branch_dtype == VRR_BF16 && y_dtype == VRR_BF16) return add_ln_bwd_t<__nv_bfloat16, __nv_bfloat16>(ARGS);
-  if (branch_dtype == VRR_F32 && y_dtype == VRR_BF16) return add_ln_bwd_t<float, __nv_bfloat16>(ARGS);
-  if (branch_dtype == VRR_F16 && y_dtype == VRR_F16) return add_ln_bwd_t<__half, __half>(ARGS);
-  if (branch_dtype == VRR_F32 && y_dtype == VRR_F16) return add_ln_bwd_t<float, __half>(ARGS);
+#define ARGS dy, (const float*)d_xnew, (const float*)x_new, gamma, mean, rstd, (float*)dx, d_branch, dgamma, dbeta, M, E, dv, st
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_F32) return add_ln_bwd_t<float, float, DROP>(ARGS);
+  if (branch_dtype == VRR_BF16 && y_dtype == VRR_BF16) return add_ln_bwd_t<__nv_bfloat16, __nv_bfloat16, DROP>(ARGS);
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_BF16) return add_ln_bwd_t<float, __nv_bfloat16, DROP>(ARGS);
+  if (branch_dtype == VRR_F16 && y_dtype == VRR_F16) return add_ln_bwd_t<__half, __half, DROP>(ARGS);
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_F16) return add_ln_bwd_t<float, __half, DROP>(ARGS);
 #undef ARGS
   set_error("add_layernorm_bwd: unsupported dtype combination (branch %d, y %d)", branch_dtype, y_dtype);
   return VRR_ERR_UNSUPPORTED;
+}
+
+int add_layernorm_fwd(const void* x, const void* branch, void* x_new, const float* gamma, const float* beta, void* y,
+                      float* mean, float* rstd, int M, int E, float eps, int branch_dtype, int y_dtype,
+                      const vrr_drop_desc* drop, cudaStream_t st) {
+  DropView dv = {};
+  bool active = false;
+  if (int rc = drop_view(drop, M, E, &dv, &active)) return rc;
+  if (active && dv.t < 65536u)
+    return add_layernorm_fwd_d<2>(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, dv, st);
+  if (active)
+    return add_layernorm_fwd_d<1>(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, dv, st);
+  return add_layernorm_fwd_d<0>(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, dv, st);
+}
+
+int add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new, const float* gamma, const float* mean,
+                      const float* rstd, void* dx, void* d_branch, float* dgamma, float* dbeta, int M, int E,
+                      int branch_dtype, int y_dtype, const vrr_drop_desc* drop, cudaStream_t st) {
+  DropView dv = {};
+  bool active = false;
+  if (int rc = drop_view(drop, M, E, &dv, &active)) return rc;
+  if (active && dv.t < 65536u)
+    return add_layernorm_bwd_d<2>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
+                                  y_dtype, dv, st);
+  if (active)
+    return add_layernorm_bwd_d<1>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
+                                  y_dtype, dv, st);
+  return add_layernorm_bwd_d<0>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
+                                    y_dtype, dv, st);
 }
 
 void layernorm_set_option(int which, int value) {

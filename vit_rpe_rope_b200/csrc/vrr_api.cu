@@ -124,6 +124,30 @@ static int check_bias(const vrr_bias_desc* b, int H, int N) {
   return VRR_OK;
 }
 
+static uint32_t keep_threshold(float p) { return (uint32_t)llrint((1.0 - (double)p) * 65536.0); }
+
+int drop_view(const vrr_drop_desc* d, int M, int E, DropView* v, bool* active) {
+  (void)M;
+  *active = false;
+  if (!d) return VRR_OK;
+  VRR_REQUIRE(d->p >= 0.f && d->p < 1.f && d->p_path >= 0.f && d->p_path < 1.f, VRR_ERR_INVALID_ARG,
+              "drop desc: probabilities must lie in [0, 1) (p %g, p_path %g)", (double)d->p, (double)d->p_path);
+  if (d->p == 0.f && d->p_path == 0.f) return VRR_OK;
+  VRR_REQUIRE(d->seed != nullptr && ((uintptr_t)d->seed & 7) == 0, VRR_ERR_INVALID_ARG,
+              "drop desc: seed must be an 8-byte aligned device pointer");
+  VRR_REQUIRE(d->p == 0.f || E % 8 == 0, VRR_ERR_UNSUPPORTED, "drop desc: element dropout needs E %% 8 == 0 (E = %d)", E);
+  VRR_REQUIRE(d->p_path == 0.f || d->rows_per_sample > 0, VRR_ERR_INVALID_ARG,
+              "drop desc: stochastic depth needs rows_per_sample > 0");
+  v->seed = reinterpret_cast<const unsigned long long*>(d->seed);
+  v->t = keep_threshold(d->p);
+  v->t_path = keep_threshold(d->p_path);
+  v->s = (1.f / (1.f - d->p)) * (1.f / (1.f - d->p_path));
+  v->rows_per_sample = d->rows_per_sample > 0 ? d->rows_per_sample : 1;
+  v->site = d->site;
+  *active = true;
+  return VRR_OK;
+}
+
 }  // namespace vrr
 
 using namespace vrr;
@@ -352,6 +376,44 @@ int vrr_gemm_ex(const void* a, const void* b, void* c, void* c2, const float* bi
   return gemm_simt(a, b, c, M, N, K, trans_a, trans_b, dtype, c_dtype, (cudaStream_t)stream);
 }
 
+int vrr_gemm_ex_drop(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K,
+                     int trans_a, int trans_b, int dtype, int c_dtype, int epilogue, int accumulate,
+                     const vrr_drop_desc* drop, void* stream) {
+  VRR_REQUIRE(epilogue == VRR_EPI_BIAS_GELU_GRAD || epilogue == VRR_EPI_BIAS_GELU_ACT, VRR_ERR_INVALID_ARG,
+              "gemm_ex_drop: epilogue %d (only BIAS_GELU_GRAD and BIAS_GELU_ACT take dropout)", epilogue);
+  VRR_REQUIRE(!drop || drop->p_path == 0.f, VRR_ERR_INVALID_ARG, "gemm_ex_drop: p_path must be 0");
+  DropView dv = {};
+  bool active = false;
+  if (int rc = drop_view(drop, M, N, &dv, &active)) return rc;
+  if (!active) return vrr_gemm_ex(a, b, c, c2, bias, M, N, K, trans_a, trans_b, dtype, c_dtype, epilogue, accumulate, stream);
+  VRR_REQUIRE(a && b && c && bias, VRR_ERR_INVALID_ARG, "gemm_ex_drop: NULL pointer");
+  VRR_REQUIRE(epilogue == VRR_EPI_BIAS_GELU_ACT || c2, VRR_ERR_INVALID_ARG, "gemm_ex_drop: BIAS_GELU_GRAD needs `c2`");
+  VRR_REQUIRE(M > 0 && N > 0 && K > 0, VRR_ERR_INVALID_ARG, "gemm_ex_drop: bad sizes");
+  VRR_REQUIRE(dtype_ok(dtype) && c_dtype == dtype, VRR_ERR_INVALID_ARG, "gemm_ex_drop: bad dtype %d/%d (C has the operands' type)",
+              dtype, c_dtype);
+  VRR_REQUIRE(!accumulate, VRR_ERR_UNSUPPORTED, "gemm_ex_drop: accumulate needs an fp32 C");
+  if (int rc = require_device()) return rc;
+  const int impl = g_impl.load();
+  const bool grad = epilogue == VRR_EPI_BIAS_GELU_GRAD;
+  const bool aligned = gemm_ptrs_aligned16(a, b, c, grad ? c2 : nullptr, bias);
+  const bool tc_ok = is16(dtype) && aligned && trans_a == 0 && trans_b == 1 &&
+                     gemm_tc_supported(M, N, K, trans_a, trans_b, dtype, c_dtype, epilogue);
+  if (impl != VRR_IMPL_SIMT && tc_ok) {
+    VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
+    return gemm_tc_drop(a, b, c, grad ? c2 : nullptr, bias, M, N, K, dtype, epilogue, dv, (cudaStream_t)stream);
+  }
+  VRR_REQUIRE(impl != VRR_IMPL_TCGEN05 || !is16(dtype), VRR_ERR_UNSUPPORTED,
+              "gemm_ex_drop: tcgen05 kernel forced but the case needs trans_a 0, trans_b 1, N %% 8 == 0, K %% 8 == 0 "
+              "and 16-byte aligned pointers");
+  VRR_COUNT_FAMILY(VRR_IMPL_SIMT);
+  if (grad) {  // (h, gelu(h)) into (c2, c); then c <- T(c f), c2 <- T(T(gelu'(h)) f)
+    if (int rc = gemm_simt_bias(a, b, c2, c, bias, M, N, K, trans_a, trans_b, dtype, 1, (cudaStream_t)stream)) return rc;
+  } else {
+    if (int rc = gemm_simt_bias(a, b, c, nullptr, bias, M, N, K, trans_a, trans_b, dtype, 2, (cudaStream_t)stream)) return rc;
+  }
+  return drop_gelu_inplace(c, grad ? c2 : nullptr, M, N, dtype, dv, (cudaStream_t)stream);
+}
+
 int vrr_gemm_mul_colsum(const void* a, const void* b, void* c, const void* mul, float* col_sums, int M, int N, int K,
                         int trans_a, int trans_b, int dtype, void* stream) {
   VRR_REQUIRE(a && b && c && mul && col_sums, VRR_ERR_INVALID_ARG, "gemm_mul_colsum: NULL pointer");
@@ -466,7 +528,21 @@ int vrr_add_layernorm_fwd(const void* x, const void* branch, void* x_new, const 
   VRR_REQUIRE((((uintptr_t)x | (uintptr_t)branch | (uintptr_t)x_new | (uintptr_t)y | (uintptr_t)gamma | (uintptr_t)beta) & 15) == 0,
               VRR_ERR_INVALID_ARG, "add_layernorm_fwd: pointers must be 16-byte aligned");
   if (int rc = require_device()) return rc;
-  return add_layernorm_fwd(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype,
+  return add_layernorm_fwd(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, nullptr,
+                           (cudaStream_t)stream);
+}
+
+int vrr_add_layernorm_drop_fwd(const void* x, const void* branch, void* x_new, const float* gamma, const float* beta,
+                               void* y, float* mean, float* rstd, int M, int E, float eps, int branch_dtype, int y_dtype,
+                               const vrr_drop_desc* drop, void* stream) {
+  VRR_REQUIRE(x && branch && x_new && gamma && beta && y && mean && rstd, VRR_ERR_INVALID_ARG, "add_layernorm_drop_fwd: NULL pointer");
+  VRR_REQUIRE(dtype_ok(branch_dtype) && dtype_ok(y_dtype) && no_mix(branch_dtype, y_dtype), VRR_ERR_INVALID_ARG,
+              "add_layernorm_drop_fwd: bad dtype");
+  VRR_REQUIRE(M > 0 && E > 0, VRR_ERR_INVALID_ARG, "add_layernorm_drop_fwd: bad sizes");
+  VRR_REQUIRE((((uintptr_t)x | (uintptr_t)branch | (uintptr_t)x_new | (uintptr_t)y | (uintptr_t)gamma | (uintptr_t)beta) & 15) == 0,
+              VRR_ERR_INVALID_ARG, "add_layernorm_drop_fwd: pointers must be 16-byte aligned");
+  if (int rc = require_device()) return rc;
+  return add_layernorm_fwd(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, drop,
                            (cudaStream_t)stream);
 }
 
@@ -482,7 +558,44 @@ int vrr_add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new,
               VRR_ERR_INVALID_ARG, "add_layernorm_bwd: pointers must be 16-byte aligned");
   if (int rc = require_device()) return rc;
   return add_layernorm_bwd(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
-                           y_dtype, (cudaStream_t)stream);
+                           y_dtype, nullptr, (cudaStream_t)stream);
+}
+
+int vrr_add_layernorm_drop_bwd(const void* dy, const void* d_xnew, const void* x_new, const float* gamma,
+                               const float* mean, const float* rstd, void* dx, void* d_branch, float* dgamma,
+                               float* dbeta, int M, int E, int branch_dtype, int y_dtype, const vrr_drop_desc* drop,
+                               void* stream) {
+  VRR_REQUIRE(dy && x_new && gamma && mean && rstd && dx && d_branch && dgamma && dbeta, VRR_ERR_INVALID_ARG,
+              "add_layernorm_drop_bwd: NULL pointer");
+  VRR_REQUIRE(dtype_ok(branch_dtype) && dtype_ok(y_dtype) && no_mix(branch_dtype, y_dtype), VRR_ERR_INVALID_ARG,
+              "add_layernorm_drop_bwd: bad dtype");
+  VRR_REQUIRE(M > 0 && E > 0, VRR_ERR_INVALID_ARG, "add_layernorm_drop_bwd: bad sizes");
+  VRR_REQUIRE((((uintptr_t)dy | (uintptr_t)d_xnew | (uintptr_t)x_new | (uintptr_t)dx | (uintptr_t)d_branch | (uintptr_t)gamma) & 15) == 0,
+              VRR_ERR_INVALID_ARG, "add_layernorm_drop_bwd: pointers must be 16-byte aligned");
+  if (int rc = require_device()) return rc;
+  return add_layernorm_bwd(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
+                           y_dtype, drop, (cudaStream_t)stream);
+}
+
+int vrr_dropout_mask(const vrr_drop_desc* drop, void* keep_u8, void* keep_path_u8, int M, int E, void* stream) {
+  VRR_REQUIRE(drop && drop->seed, VRR_ERR_INVALID_ARG, "dropout_mask: NULL desc or seed");
+  VRR_REQUIRE(M > 0 && E > 0 && E % 8 == 0, VRR_ERR_INVALID_ARG, "dropout_mask: bad sizes (E %% 8 == 0)");
+  VRR_REQUIRE(!keep_path_u8 || drop->rows_per_sample > 0, VRR_ERR_INVALID_ARG,
+              "dropout_mask: keep_path needs rows_per_sample > 0");
+  VRR_REQUIRE(((uintptr_t)keep_u8 & 7) == 0, VRR_ERR_INVALID_ARG, "dropout_mask: keep_u8 must be 8-byte aligned");
+  DropView dv = {};
+  bool active = false;
+  if (int rc = drop_view(drop, M, E, &dv, &active)) return rc;
+  if (!active) {  // nothing dropped: the same DropView with thresholds that keep everything
+    dv.seed = reinterpret_cast<const unsigned long long*>(drop->seed);
+    dv.t = dv.t_path = 65536u;
+    dv.s = 1.f;
+    dv.rows_per_sample = drop->rows_per_sample > 0 ? drop->rows_per_sample : 1;
+    dv.site = drop->site;
+  }
+  if (int rc = require_device()) return rc;
+  if (!keep_u8 && !keep_path_u8) return VRR_OK;
+  return dropout_mask(dv, (uint8_t*)keep_u8, (uint8_t*)keep_path_u8, M, E, (cudaStream_t)stream);
 }
 
 int vrr_colsum(const void* x, float* out, int M, int C, int dtype, void* stream) {

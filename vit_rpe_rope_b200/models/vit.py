@@ -13,6 +13,10 @@ construction (citations: /root/reference/models/vit.py).  What changes is undern
 LayerNorm (fused with the residual adds), the output projection, the MLP (bias + GELU in the fc1 GEMM epilogue)
 and the head run library kernels too (SURVEY.md section 8(f) N1): the forward and backward contain no cuBLAS
 GEMM.  CUDA sm_100 only: CPU inputs raise; there is no fallback path.
+
+Regularisers of a ViT training recipe (``VisionTransformer(drop_rate, drop_path_rate)``, timm's names): inside the
+fused block loop, proj_drop / drop2 and stochastic depth are applied by the add+LayerNorm kernels that read the
+branch anyway, and drop1 by fc1's GELU epilogue, all from one Philox key drawn per training forward.
 """
 import torch
 import torch.nn as nn
@@ -22,8 +26,42 @@ from .positional_encoding import (AbsolutePositionalEncoding, NoPositionalEncodi
                                   RelativePositionalEncoding, RoPEAxial, RoPEMixed)
 
 
+def drop_path(x, drop_prob: float = 0., training: bool = False, scale_by_keep: bool = True):
+    """timm's stochastic depth on its own (torch ops): each sample of the batch is kept with probability
+    1 - drop_prob and scaled by 1 / (1 - drop_prob)."""
+    if drop_prob == 0. or not training:
+        return x
+    keep_prob = 1 - drop_prob
+    shape = (x.shape[0],) + (1,) * (x.ndim - 1)
+    random_tensor = x.new_empty(shape).bernoulli_(keep_prob)
+    if keep_prob > 0.0 and scale_by_keep:
+        random_tensor.div_(keep_prob)
+    return x * random_tensor
+
+
+class DropPath(nn.Module):
+    """Stochastic depth per sample (timm.layers.DropPath).  Inside ``VisionTransformer``'s fused block loop the
+    decision is taken by the add+LayerNorm kernels instead (same probability and scale, Philox draws)."""
+
+    def __init__(self, drop_prob: float = 0., scale_by_keep: bool = True):
+        super().__init__()
+        self.drop_prob = drop_prob
+        self.scale_by_keep = scale_by_keep
+
+    def forward(self, x):
+        return drop_path(x, self.drop_prob, self.training, self.scale_by_keep)
+
+    def extra_repr(self):
+        return f'drop_prob={round(self.drop_prob, 3):0.3f}'
+
+
+def _drop_p(m):
+    return m.p if isinstance(m, nn.Dropout) else 0.
+
+
 class Mlp(nn.Module):
-    """fc1 -> GELU -> fc2 with timm's parameter names (the reference takes it from timm, vit.py:9,118)."""
+    """fc1 -> GELU -> fc2 with timm's parameter names (the reference takes it from timm, vit.py:9,118).  In training
+    mode drop1 runs in fc1's GEMM epilogue (a Philox key drawn per call) and drop2 as ``nn.Dropout``."""
 
     def __init__(self, in_features, hidden_features=None, out_features=None, act_layer=nn.GELU, drop=0.):
         super().__init__()
@@ -36,10 +74,18 @@ class Mlp(nn.Module):
         self.drop2 = nn.Dropout(drop)
 
     def forward(self, x):
+        drop1 = None
+        if self.training and _drop_p(self.drop1) > 0 and x.is_cuda:
+            drop1 = (_drop_p(self.drop1), 0., 1, 0, ops.new_seed(x.device))
+        return self.drop2(self._branch(x, drop1))
+
+    def _branch(self, x, drop1=None):
+        """fc2(drop1(gelu(fc1(x)))) without drop2; ``drop1``: the dropout site of fc1's epilogue (training), or None."""
         if ops.can_fuse_mlp(x, self):
             dt = ops.compute_dtype(x)
-            return ops.mlp(x, self.fc1, self.fc2, ops.lp_weight(self.fc1.weight, dt), ops.lp_weight(self.fc2.weight, dt))
-        return self.drop2(self.fc2(self.drop1(self.act(self.fc1(x)))))
+            return ops.mlp(x, self.fc1, self.fc2, ops.lp_weight(self.fc1.weight, dt), ops.lp_weight(self.fc2.weight, dt),
+                           drop1)
+        return self.fc2(self.drop1(self.act(self.fc1(x))))
 
 
 class Attention(nn.Module):
@@ -63,6 +109,10 @@ class Attention(nn.Module):
         self.pos_encoding = None
 
     def forward(self, x, freqs_cis=None):
+        return self.proj_drop(self._branch(x, freqs_cis))
+
+    def _branch(self, x, freqs_cis=None):
+        """The attention output before proj_drop (the fused block loop applies it in the next add+LayerNorm)."""
         pe = self.pos_encoding
         cos = sin = None
         bias_mode, bias_param, bias_grid = _lib.BIAS_NONE, None, 0
@@ -75,7 +125,7 @@ class Attention(nn.Module):
         dt = ops.compute_dtype(x)
         planes = ops.qkv_rope(x, self.qkv.weight, cos, sin, self.num_heads, ops.lp_weight(self.qkv.weight, dt))
         out = ops.fused_attention(planes, self.scale, bias_mode, bias_param, bias_grid)
-        return self.proj_drop(ops.linear(out, self.proj, ops.lp_weight(self.proj.weight, dt)))
+        return ops.linear(out, self.proj, ops.lp_weight(self.proj.weight, dt))
 
     def set_pos_encoding(self, pos_encoding):
         self.pos_encoding = pos_encoding  # registers the shared PE module as a child (state_dict dups)
@@ -87,11 +137,9 @@ class Block(nn.Module):
     def __init__(self, dim, num_heads, mlp_ratio=4., qkv_bias=False, drop=0., attn_drop=0.,
                  drop_path=0., act_layer=nn.GELU, norm_layer=nn.LayerNorm):
         super().__init__()
-        if drop_path > 0.:
-            raise NotImplementedError("drop_path is always 0 in the reference (vit.py:200)")
         self.norm1 = norm_layer(dim)
         self.attn = Attention(dim, num_heads=num_heads, qkv_bias=qkv_bias, attn_drop=attn_drop, proj_drop=drop)
-        self.drop_path = nn.Identity()
+        self.drop_path = DropPath(drop_path) if drop_path > 0. else nn.Identity()
         self.norm2 = norm_layer(dim)
         self.mlp = Mlp(in_features=dim, hidden_features=int(dim * mlp_ratio), act_layer=act_layer, drop=drop)
 
@@ -108,13 +156,15 @@ class VisionTransformer(nn.Module):
     """ViT with selectable positional encoding (reference vit.py:131-285).
 
     ``pos_encoding`` is one of ``none | absolute | relative | polynomial | rope-axial | rope-mixed``;
-    anything else raises ``ValueError`` (vit.py:196).
+    anything else raises ``ValueError`` (vit.py:196).  ``drop_rate`` is every block's proj_drop / Mlp dropout,
+    ``drop_path_rate`` the stochastic-depth rate of the last block (timm's rule: block i of d gets
+    ``linspace(0, drop_path_rate, d)[i]``); both default to 0, the reference's values.
     """
 
     def __init__(self, img_size=32, patch_size=4, in_chans=3, num_classes=10,
                  embed_dim=192, depth=6, num_heads=6, mlp_ratio=4.,
                  pos_encoding='absolute', rope_theta=100.0,
-                 poly_degree=3, poly_shared_heads=True):
+                 poly_degree=3, poly_shared_heads=True, drop_rate=0., drop_path_rate=0.):
         super().__init__()
         self.num_classes = num_classes
         self.embed_dim = embed_dim
@@ -146,7 +196,9 @@ class VisionTransformer(nn.Module):
         else:
             raise ValueError(f"Unknown positional encoding type: {pos_encoding}")
 
-        self.blocks = nn.ModuleList([Block(embed_dim, num_heads, mlp_ratio) for _ in range(depth)])
+        dpr = [r.item() for r in torch.linspace(0, drop_path_rate, depth)]  # draws no random numbers
+        self.blocks = nn.ModuleList([Block(embed_dim, num_heads, mlp_ratio, drop=drop_rate, drop_path=dpr[i])
+                                     for i in range(depth)])
         if not self.use_pos_embed_in_forward:
             for blk in self.blocks:
                 blk.set_pos_encoding(self.pos_embed)  # one shared module, referenced by every block
@@ -171,12 +223,32 @@ class VisionTransformer(nn.Module):
 
     def forward_features(self, x):
         """[B, C, H, W] -> [B, N, E] with N = (H/P)(W/P) + 1 taken from the input (vit.py:235-271)."""
-        x, m = self._features(x)
-        return x if m is None else x + m
+        x, m, drop = self._features(x)
+        if m is None:
+            return x
+        if drop is None:
+            return x + m
+        return x + m.float() * ops.branch_factor(drop, *m.shape)
+
+    def _drop_sites(self, x):
+        """Per block (attention branch, fc1's activation, MLP branch): the dropout sites of one training forward, all
+        keyed by one seed drawn here, or None where a rate is 0.  Sites 3i, 3i+1, 3i+2 of block i."""
+        rates = []
+        for blk in self.blocks:
+            pp = blk.drop_path.drop_prob if isinstance(blk.drop_path, DropPath) else 0.
+            rates.append((_drop_p(blk.attn.proj_drop), pp, _drop_p(blk.mlp.drop1), _drop_p(blk.mlp.drop2)))
+        if not self.training or not any(any(r) for r in rates):
+            return None
+        seed = ops.new_seed(x.device)
+        self._drop_seed = seed  # the key of the last training forward (tests replay its masks)
+        N = x.shape[1]
+        site = lambda p, pp, i: (p, pp, N, i, seed) if (p > 0 or pp > 0) else None
+        return [(site(pa, pp, 3 * i), site(p1, 0., 3 * i + 1), site(p2, pp, 3 * i + 2))
+                for i, (pa, pp, p1, p2) in enumerate(rates)]
 
     def _features(self, x):
-        """The token stream before the LAST residual add and that add's branch (or the finished stream and None):
-        ``forward`` only needs the cls row of the sum."""
+        """The token stream before the LAST residual add, that add's branch and its dropout site (or the finished
+        stream, None, None): ``forward`` only needs the cls row of the sum."""
         B, C, H, W = x.shape
         h, w = H // self.patch_size, W // self.patch_size
         if x.is_cuda:  # one multi-tensor refresh of the 16-bit weight copies per forward (no-op in fp32)
@@ -192,19 +264,21 @@ class VisionTransformer(nn.Module):
         if not self._fusable(x):
             for blk in self.blocks:
                 x = blk(x, freqs_cis=freqs_cis)
-            return x, None
+            return x, None, None
         # Same arithmetic as the loop above (vit.py:120-125 per block), with every residual add fused with
         # the LayerNorm that follows it - also across block boundaries:
-        #   x = x + attn(norm1(x));  x = x + mlp(norm2(x))
+        #   x = x + drop_path(proj_drop(attn(norm1(x))));  x = x + drop_path(drop2(mlp(norm2(x))))
         blocks = self.blocks
+        sites = self._drop_sites(x)
         y = ops.layer_norm(x, blocks[0].norm1)
-        m = None
+        m = d_mlp = None
         for i, blk in enumerate(blocks):
-            x, y = ops.add_layer_norm(x, blk.attn(y, freqs_cis=freqs_cis), blk.norm2)
-            m = blk.mlp(y)
+            d_attn, d_fc1, d_mlp = sites[i] if sites is not None else (None, None, None)
+            x, y = ops.add_layer_norm(x, blk.attn._branch(y, freqs_cis=freqs_cis), blk.norm2, drop=d_attn)
+            m = blk.mlp._branch(y, d_fc1)
             if i + 1 < len(blocks):
-                x, y = ops.add_layer_norm(x, m, blocks[i + 1].norm1)
-        return x, m
+                x, y = ops.add_layer_norm(x, m, blocks[i + 1].norm1, drop=d_mlp)
+        return x, m, d_mlp
 
     def _gemm_weights(self):
         ws = [self.head.weight]
@@ -216,14 +290,21 @@ class VisionTransformer(nn.Module):
 
     def _fusable(self, x):
         return len(self.blocks) > 0 and all(
-            type(blk) is Block and isinstance(blk.drop_path, nn.Identity)
+            type(blk) is Block and type(blk.drop_path) in (nn.Identity, DropPath) and type(blk.mlp) is Mlp
+            and type(blk.attn.proj_drop) is nn.Dropout and type(blk.mlp.drop2) is nn.Dropout
             and ops.can_fuse_add_layer_norm(x, blk.norm1) and ops.can_fuse_add_layer_norm(x, blk.norm2)
             for blk in self.blocks)
 
     def forward(self, x):
-        x, m = self._features(x)
+        x, m, drop = self._features(x)
         # LayerNorm is per token and only the cls token reaches the head (vit.py:284-285): the last residual
-        # add and the final norm of that row alone give identical logits and gradients
-        cls = x[:, 0] if m is None else x[:, 0] + m[:, 0]
+        # add and the final norm of that row alone give identical logits and gradients (with dropout: the factors
+        # of token rows b*N, the same arithmetic as forward_features)
+        if m is None:
+            cls = x[:, 0]
+        elif drop is None:
+            cls = x[:, 0] + m[:, 0]
+        else:
+            cls = x[:, 0] + m[:, 0].float() * ops.branch_factor(drop, *m.shape, cls_only=True)[:, 0]
         y = ops.layer_norm(cls, self.norm)
         return ops.linear(y, self.head, ops.lp_weight(self.head.weight, ops.compute_dtype(y)))

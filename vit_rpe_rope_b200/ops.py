@@ -306,14 +306,16 @@ class QkvRopeFn(torch.autograd.Function):
         return dx, dw, d_cos, d_sin, None, None
 
 
-def _gemm(a, b, trans_a, trans_b, out_dtype, bias=None, epilogue=_lib.EPI_NONE, out2=False, name="gemm", aux=None):
+def _gemm(a, b, trans_a, trans_b, out_dtype, bias=None, epilogue=_lib.EPI_NONE, out2=False, name="gemm", aux=None,
+          drop=None):
     """C = op(A) . op(B) in the library's kernels (``vrr_gemm_ex``) - no cuBLAS anywhere on the path.
 
     op(A) is [M][K] (trans_a: A stored [K][M]); op(B) is [K][N] (trans_b: B stored [N][K]).  bf16 / fp16 operands
     run the tcgen05 CTA-pair kernel (fp32 accumulation; result in ``out_dtype``: the operands' type, or fp32 for
     weight gradients), fp32 operands the exact-fp32 FFMA kernel (no TF32).  ``epilogue``: fused ``+ bias`` or
     ``+ bias, GELU`` (``out2``: second output - gelu(C) for EPI_BIAS_GELU; EPI_BIAS_GELU_GRAD returns
-    (gelu(h), gelu'(h)) instead; EPI_BIAS_GELU_ACT returns gelu(h) alone); ``aux``: the [M][N] multiplier of EPI_MUL."""
+    (gelu(h), gelu'(h)) instead; EPI_BIAS_GELU_ACT returns gelu(h) alone); ``aux``: the [M][N] multiplier of EPI_MUL;
+    ``drop``: element dropout on the GELU outputs of those two epilogues (``vrr_gemm_ex_drop``)."""
     lib = _lib.load()
     M = a.shape[1] if trans_a else a.shape[0]
     K = a.shape[0] if trans_a else a.shape[1]
@@ -323,8 +325,14 @@ def _gemm(a, b, trans_a, trans_b, out_dtype, bias=None, epilogue=_lib.EPI_NONE, 
     c2 = torch.empty_like(c) if out2 else (aux.contiguous() if aux is not None else None)
     bias32 = _f32c(bias) if bias is not None and epilogue != _lib.EPI_NONE else None
     with _timed(name):
-        _lib.check(lib.vrr_gemm_ex(_ptr(a), _ptr(b), _ptr(c), _ptr(c2), _ptr(bias32), M, N, K, int(trans_a), int(trans_b),
-                                   _DT[a.dtype], _DT[out_dtype], int(epilogue), 0, _stream()), "vrr_gemm_ex")
+        if drop is None:
+            _lib.check(lib.vrr_gemm_ex(_ptr(a), _ptr(b), _ptr(c), _ptr(c2), _ptr(bias32), M, N, K, int(trans_a), int(trans_b),
+                                       _DT[a.dtype], _DT[out_dtype], int(epilogue), 0, _stream()), "vrr_gemm_ex")
+        else:
+            d = _drop_desc(drop)
+            _lib.check(lib.vrr_gemm_ex_drop(_ptr(a), _ptr(b), _ptr(c), _ptr(c2), _ptr(bias32), M, N, K, int(trans_a),
+                                            int(trans_b), _DT[a.dtype], _DT[out_dtype], int(epilogue), 0, ctypes.byref(d),
+                                            _stream()), "vrr_gemm_ex_drop")
     return (c, c2) if out2 else c
 
 
@@ -437,13 +445,66 @@ class LayerNormFn(torch.autograd.Function):
         return dx.view(shape), dg.to(w_dtype), db.to(b_dtype), None, None
 
 
+# ------------------------------------------------------------------------------------------------
+# Dropout / stochastic depth inside the kernels (vrr_drop_desc).  A site is described by the tuple
+# ``(p, p_path, rows_per_sample, site, seed)``: element probability, per-image probability, token rows per image, the
+# Philox counter word naming the site within one forward, and the int64 device tensor holding the key.  None = off.
+def new_seed(device):
+    """One 64-bit Philox key drawn on the device from torch's CUDA generator (graph-safe: a captured step draws a
+    fresh key on every replay)."""
+    return torch.randint(-2 ** 63, 2 ** 63 - 1, (1,), device=device, dtype=torch.int64)
+
+
+def _drop_desc(drop):
+    p, p_path, rows, site, seed = drop
+    d = _lib.DropDesc()
+    d.p, d.p_path, d.rows_per_sample, d.site = float(p), float(p_path), int(rows), int(site)
+    d.seed = seed.data_ptr()
+    return d
+
+
+def drop_scale(p, p_path):
+    """The kernels' factor of a kept element: (1 / (1 - p)) * (1 / (1 - p_path)) formed in fp32."""
+    one = torch.ones((), dtype=torch.float32)
+    return ((one / (one - torch.tensor(p, dtype=torch.float32))) * (one / (one - torch.tensor(p_path, dtype=torch.float32)))).item()
+
+
+def dropout_mask(drop, M, E):
+    """(keep [M, E] uint8 or None when p == 0, keep_path [ceil(M / rows)] uint8 or None when p_path == 0): the
+    decisions the kernels take for ``drop`` (``vrr_dropout_mask``)."""
+    p, p_path, rows, site, seed = drop
+    dev = seed.device
+    keep = torch.empty(M, E, device=dev, dtype=torch.uint8) if p > 0 else None
+    keep_path = torch.empty(-(-M // rows), device=dev, dtype=torch.uint8) if p_path > 0 else None
+    d = _drop_desc(drop)
+    with torch.cuda.device(dev):
+        _lib.check(_lib.load().vrr_dropout_mask(ctypes.byref(d), _ptr(keep), _ptr(keep_path), M, E, _stream()),
+                   "vrr_dropout_mask")
+    return keep, keep_path
+
+
+def branch_factor(drop, B, N, E, cls_only=False):
+    """f [B, N, E] fp32 (cls_only: [B, 1, E], token rows b*N): the factor each element of a [B*N, E] branch gets at
+    site ``drop`` (keep * keep_path * s), for the residual add the kernels do not take (the model's last one)."""
+    p, p_path = drop[0], drop[1]
+    keep, keep_path = dropout_mask(drop, B * N, E)
+    f = torch.full((B, 1 if cls_only else N, E), drop_scale(p, p_path), device=drop[4].device, dtype=torch.float32)
+    if keep is not None:
+        k = keep.view(B, N, E)
+        f = f * (k[:, :1] if cls_only else k)
+    if keep_path is not None:
+        f = f * keep_path[:B].view(B, 1, 1)
+    return f
+
+
 class AddLayerNormFn(torch.autograd.Function):
     """(x_new, y) = (x + branch, LayerNorm(x + branch)): the residual add of one sub-block fused with the
     LayerNorm that opens the next one; the backward emits the residual-stream gradient (fp32) and the
-    branch gradient (branch dtype) from a single pass."""
+    branch gradient (branch dtype) from a single pass.  ``drop``: the branch's dropout / stochastic-depth site
+    (x_new = x + f * branch; the masks are regenerated in the backward), or None."""
 
     @staticmethod
-    def forward(ctx, x, branch, weight, bias, eps, out_dtype):
+    def forward(ctx, x, branch, weight, bias, eps, out_dtype, drop=None):
         _require_cuda(x, branch, weight, bias)
         lib = _lib.load()
         E = x.shape[-1]
@@ -456,9 +517,17 @@ class AddLayerNormFn(torch.autograd.Function):
         mean = torch.empty(M, device=x.device, dtype=torch.float32)
         rstd = torch.empty(M, device=x.device, dtype=torch.float32)
         with torch.cuda.device(x.device), _timed("add_layernorm_fwd"):
-            _lib.check(lib.vrr_add_layernorm_fwd(_ptr(x2), _ptr(b2), _ptr(x_new), _ptr(w32), _ptr(b32), _ptr(y),
-                                                 _ptr(mean), _ptr(rstd), M, E, float(eps), _DT[b2.dtype],
-                                                 _DT[out_dtype], _stream()), "vrr_add_layernorm_fwd")
+            if drop is None:
+                _lib.check(lib.vrr_add_layernorm_fwd(_ptr(x2), _ptr(b2), _ptr(x_new), _ptr(w32), _ptr(b32), _ptr(y),
+                                                     _ptr(mean), _ptr(rstd), M, E, float(eps), _DT[b2.dtype],
+                                                     _DT[out_dtype], _stream()), "vrr_add_layernorm_fwd")
+            else:
+                d = _drop_desc(drop)
+                _lib.check(lib.vrr_add_layernorm_drop_fwd(_ptr(x2), _ptr(b2), _ptr(x_new), _ptr(w32), _ptr(b32), _ptr(y),
+                                                          _ptr(mean), _ptr(rstd), M, E, float(eps), _DT[b2.dtype],
+                                                          _DT[out_dtype], ctypes.byref(d), _stream()),
+                           "vrr_add_layernorm_drop_fwd")
+        ctx.drop = drop  # holds the seed tensor: the backward regenerates the masks from it
         ctx.save_for_backward(x_new, w32, mean, rstd)
         ctx.meta = (x.shape, weight.dtype, bias.dtype, out_dtype, b2.dtype)
         return x_new.view(x.shape), y.view(x.shape)
@@ -484,10 +553,17 @@ class AddLayerNormFn(torch.autograd.Function):
         dgb = torch.empty(2, E, device=x_new.device, dtype=torch.float32)  # one buffer: the library zeroes both rows with one memset
         dg, db = dgb[0], dgb[1]
         with torch.cuda.device(x_new.device), _timed("add_layernorm_bwd"):
-            _lib.check(lib.vrr_add_layernorm_bwd(_ptr(dy2), _ptr(dr2), _ptr(x_new), _ptr(w32), _ptr(mean), _ptr(rstd),
-                                                 _ptr(dx), _ptr(d_branch), _ptr(dg), _ptr(db), M, E, _DT[br_dtype],
-                                                 _DT[out_dtype], _stream()), "vrr_add_layernorm_bwd")
-        return dx.view(shape), d_branch.view(shape), dg.to(w_dtype), db.to(b_dtype), None, None
+            if ctx.drop is None:
+                _lib.check(lib.vrr_add_layernorm_bwd(_ptr(dy2), _ptr(dr2), _ptr(x_new), _ptr(w32), _ptr(mean), _ptr(rstd),
+                                                     _ptr(dx), _ptr(d_branch), _ptr(dg), _ptr(db), M, E, _DT[br_dtype],
+                                                     _DT[out_dtype], _stream()), "vrr_add_layernorm_bwd")
+            else:
+                d = _drop_desc(ctx.drop)
+                _lib.check(lib.vrr_add_layernorm_drop_bwd(_ptr(dy2), _ptr(dr2), _ptr(x_new), _ptr(w32), _ptr(mean),
+                                                          _ptr(rstd), _ptr(dx), _ptr(d_branch), _ptr(dg), _ptr(db), M, E,
+                                                          _DT[br_dtype], _DT[out_dtype], ctypes.byref(d), _stream()),
+                           "vrr_add_layernorm_drop_bwd")
+        return dx.view(shape), d_branch.view(shape), dg.to(w_dtype), db.to(b_dtype), None, None, None
 
 
 def can_fuse_add_layer_norm(x, norm) -> bool:
@@ -496,12 +572,13 @@ def can_fuse_add_layer_norm(x, norm) -> bool:
             and norm.bias is not None and tuple(norm.normalized_shape) == (x.shape[-1],))
 
 
-def add_layer_norm(x, branch, norm: torch.nn.LayerNorm):
-    """``x_new = x + branch; y = norm(x_new)`` in one kernel (see :class:`AddLayerNormFn`)."""
+def add_layer_norm(x, branch, norm: torch.nn.LayerNorm, drop=None):
+    """``x_new = x + f * branch; y = norm(x_new)`` in one kernel (see :class:`AddLayerNormFn`); f = 1 when ``drop`` is
+    None."""
     out_dtype = compute_dtype(x)
     if branch.dtype not in (torch.float32, out_dtype):
         branch = branch.to(out_dtype)
-    return AddLayerNormFn.apply(x, branch, norm.weight, norm.bias, norm.eps, out_dtype)
+    return AddLayerNormFn.apply(x, branch, norm.weight, norm.bias, norm.eps, out_dtype, drop)
 
 
 def layer_norm(x, norm: torch.nn.LayerNorm):
@@ -573,17 +650,20 @@ class MlpFn(torch.autograd.Function):
     (dh = (dy . W2) * gelu'(h)), the two bias gradients are column sums."""
 
     @staticmethod
-    def forward(ctx, x, w1, b1, w2, b2, w1_lp=None, w2_lp=None):
+    def forward(ctx, x, w1, b1, w2, b2, w1_lp=None, w2_lp=None, drop1=None):
+        """``drop1``: element dropout on the GELU output (a site with p_path 0), applied in fc1's epilogue to gelu(h)
+        and gelu'(h) alike - the backward below is then Dropout's backward unchanged."""
         _require_cuda(x, w1, b1, w2, b2)
         dt = x.dtype
         w1l = (w1_lp if w1_lp is not None else w1.detach().to(dt)).detach()
         w2l = (w2_lp if w2_lp is not None else w2.detach().to(dt)).detach()
         x2 = x.reshape(-1, x.shape[-1])
         if not any(ctx.needs_input_grad):  # inference: the activation alone - one output stream instead of two
-            a = _gemm(x2, w1l, False, True, dt, bias=b1, epilogue=_lib.EPI_BIAS_GELU_ACT, name="fc1_fwd")
+            a = _gemm(x2, w1l, False, True, dt, bias=b1, epilogue=_lib.EPI_BIAS_GELU_ACT, name="fc1_fwd", drop=drop1)
             y = _gemm(a, w2l, False, True, dt, bias=b2, epilogue=_lib.EPI_BIAS, name="fc2_fwd")
             return y.view(*x.shape[:-1], w2l.shape[0])
-        a, gp = _gemm(x2, w1l, False, True, dt, bias=b1, epilogue=_lib.EPI_BIAS_GELU_GRAD, out2=True, name="fc1_fwd")
+        a, gp = _gemm(x2, w1l, False, True, dt, bias=b1, epilogue=_lib.EPI_BIAS_GELU_GRAD, out2=True, name="fc1_fwd",
+                      drop=drop1)
         y = _gemm(a, w2l, False, True, dt, bias=b2, epilogue=_lib.EPI_BIAS, name="fc2_fwd")
         ctx.save_for_backward(x2, gp, a, w1l, w2l)
         ctx.meta = (x.shape, w1.dtype, b1.dtype, w2.dtype, b2.dtype)
@@ -617,7 +697,7 @@ class MlpFn(torch.autograd.Function):
                 db2 = _colsum(dy2).to(b2_dt)
             dx = _gemm(dh, w1l, False, False, x2.dtype, name="fc1_dx").view(x_shape)
             dw1 = _gemm(dh, x2, True, False, w1_dt, name="fc1_dw")
-        return dx, dw1, db1, dw2, db2, None, None
+        return dx, dw1, db1, dw2, db2, None, None, None
 
 
 def linear(x, lin: torch.nn.Linear, w_lp=None):
@@ -630,18 +710,22 @@ def linear(x, lin: torch.nn.Linear, w_lp=None):
     return LinearFn.apply(x.to(dt), lin.weight, lin.bias, w_lp)
 
 
-def mlp(x, fc1: torch.nn.Linear, fc2: torch.nn.Linear, w1_lp=None, w2_lp=None):
+def mlp(x, fc1: torch.nn.Linear, fc2: torch.nn.Linear, w1_lp=None, w2_lp=None, drop1=None):
     dt = compute_dtype(x)
     if w1_lp is not None and (w1_lp.dtype != dt or w2_lp is None or w2_lp.dtype != dt):
         w1_lp = w2_lp = None
-    return MlpFn.apply(x.to(dt), fc1.weight, fc1.bias, fc2.weight, fc2.bias, w1_lp, w2_lp)
+    return MlpFn.apply(x.to(dt), fc1.weight, fc1.bias, fc2.weight, fc2.bias, w1_lp, w2_lp, drop1)
 
 
 def can_fuse_mlp(x, m) -> bool:
+    """fc1 -> exact GELU -> fc2 with biases; fc1's dropout (drop1) runs in its epilogue when its hidden width is a
+    multiple of 8 (the mask's groups), and the caller applies drop2 (nn.Dropout, or the next add+LayerNorm)."""
     act = getattr(m, "act", None)
+    p1 = getattr(m.drop1, "p", 0.0) if isinstance(m.drop1, torch.nn.Dropout) else None
     return (x.is_cuda and x.dtype in _DT and type(act) is torch.nn.GELU and getattr(act, "approximate", "none") == "none"
             and m.fc1.bias is not None and m.fc2.bias is not None and m.fc1.out_features % 4 == 0
-            and m.fc2.out_features % 4 == 0 and getattr(m.drop1, "p", 0.0) == 0.0 and getattr(m.drop2, "p", 0.0) == 0.0)
+            and m.fc2.out_features % 4 == 0 and p1 is not None and (p1 == 0.0 or m.fc1.out_features % 8 == 0)
+            and isinstance(m.drop2, (torch.nn.Dropout, torch.nn.Identity)))
 
 
 # ------------------------------------------------------------------------------------------------
