@@ -23,9 +23,13 @@
  *   - there is no CPU path: on a machine without an sm_100 device every compute entry point
  *     returns VRR_ERR_NO_DEVICE.
  *
- * Token / head geometry: B images, N tokens per image (token 0 is the cls token, tokens 1..N-1 are
- * the g*g patches in raster order), E = H * Dh channels, H heads of Dh channels.  Dh must be one of
- * 16, 32, 64 (the tcgen05 bf16 / fp16 kernels need Dh == 64).
+ * Token / head geometry: B images, N tokens per image, E = H * Dh channels, H heads of Dh channels.  Dh must be
+ * one of 16, 32, 64 (the tcgen05 bf16 / fp16 kernels need Dh == 64).  An image's token stream is
+ *   [cls, reg_0 .. reg_{R-1}, patch_0 .. patch_{Np-1}]      (timm / DINOv2 order, n_prefix = 1 + R, N = n_prefix + Np)
+ * with the Np patches in raster order.  The n_prefix prefix tokens (the cls token and R register tokens) get no
+ * absolute position embedding and are never rotated; patch p sits at token row n_prefix + p.  The *_prefix entry
+ * points take n_prefix (1 <= n_prefix <= N, else VRR_ERR_INVALID_ARG); the others are those entry points at
+ * n_prefix = 1 (no registers: token 0 is the cls token, tokens 1..N-1 the patches).
  *
  * "qkv planes": one buffer [3][B][H][N][Dh] holding q (rotated when RoPE is on), k (likewise), v.
  */
@@ -54,9 +58,10 @@ typedef enum {
  * with a loss scaler detects the overflow from them). */
 typedef enum { VRR_F32 = 0, VRR_BF16 = 1, VRR_F16 = 2 } vrr_dtype;
 
-/* RoPE variants of models/vit.py:51-68.  AXIAL: cos/sin are [N-1][Dh/2] shared by all heads
- * (positional_encoding.py:216-245).  MIXED: cos/sin are [H][N-1][Dh/2]
- * (positional_encoding.py:313-351).  Token 0 (cls) is never rotated (vit.py:56-57). */
+/* RoPE variants of models/vit.py:51-68.  AXIAL: cos/sin are [N-n_prefix][Dh/2] shared by all heads
+ * (positional_encoding.py:216-245).  MIXED: cos/sin are [H][N-n_prefix][Dh/2]
+ * (positional_encoding.py:313-351).  Prefix tokens (cls, registers) are never rotated (vit.py:56-57); token row
+ * t >= n_prefix is rotated by table row t - n_prefix. */
 typedef enum { VRR_ROPE_NONE = 0, VRR_ROPE_AXIAL = 1, VRR_ROPE_MIXED = 2 } vrr_rope_mode;
 
 /* Additive logit bias of models/vit.py:73-81.
@@ -148,6 +153,15 @@ int vrr_patch_embed_fwd(const void* images, const void* weight, const void* bias
                         const void* cls_token, const void* pos_embed, void* tokens, void* workspace,
                         size_t workspace_bytes, int B, int C, int Hi, int Wi, int P, int E,
                         int img_dtype, int dtype, int tok_dtype, void* stream);
+/* The same with n_prefix prefix tokens (cls, then registers):
+ *   tokens[b][t][:]          = prefix_tokens[t][:]                 for t < n_prefix
+ *   tokens[b][n_prefix+p][:] = the patch row p above (+ pos_embed[p])
+ * prefix_tokens [n_prefix][E] and tokens [B][n_prefix+Np][E] are of `tok_dtype`.  n_prefix = 1 is
+ * vrr_patch_embed_fwd. */
+int vrr_patch_embed_fwd_prefix(const void* images, const void* weight, const void* bias, const void* prefix_tokens,
+                               int n_prefix, const void* pos_embed, void* tokens, void* workspace,
+                               size_t workspace_bytes, int B, int C, int Hi, int Wi, int P, int E, int img_dtype,
+                               int dtype, int tok_dtype, void* stream);
 /* out[b*Np + p][c*P*P + i*P + j] = bf16(images[b][c][py*P+i][px*P+j]): the im2col matrix of the
  * stride-P convolution (needs P % 8 == 0).  Used by the forward above and by callers that take the
  * weight gradient with a plain library GEMM. */
@@ -163,9 +177,15 @@ int vrr_patch_unfold_ex(const void* images, void* out, int B, int C, int Hi, int
 int vrr_patch_embed_bwd(const void* images, const void* d_tokens, void* d_weight, void* d_bias,
                         void* d_cls, void* d_pos, int B, int C, int Hi, int Wi, int P, int E,
                         int img_dtype, int dtype, int tok_dtype, void* stream);
+/* The same with n_prefix prefix tokens: d_tokens [B][n_prefix+Np][E]; d_prefix fp32 [n_prefix][E] with
+ * d_prefix[t] = sum_b d_tokens[b][t]; d_pos, d_bias and d_weight come from the rows t >= n_prefix.  n_prefix = 1 is
+ * vrr_patch_embed_bwd. */
+int vrr_patch_embed_bwd_prefix(const void* images, const void* d_tokens, void* d_weight, void* d_bias, void* d_prefix,
+                               int n_prefix, void* d_pos, int B, int C, int Hi, int Wi, int P, int E, int img_dtype,
+                               int dtype, int tok_dtype, void* stream);
 
 /* ---- (a) QKV projection with RoPE epilogue: models/vit.py:47-68, rope_utils.py:3-37 -------- */
-/* planes = split_heads(x . w_qkv^T) with q,k rows 1.. rotated by (cos,sin) in the epilogue.
+/* planes = split_heads(x . w_qkv^T) with q,k rows 1.. rotated by (cos,sin) in the epilogue (n_prefix = 1).
  * x [B*N][E], w_qkv [3E][E] (row order (3,H,Dh), vit.py:47), cos/sin fp32 (see vrr_rope_mode),
  * planes [3][B][H][N][Dh]. */
 int vrr_qkv_rope_fwd(const void* x, const void* w_qkv, const float* cos_tab, const float* sin_tab,
@@ -173,7 +193,7 @@ int vrr_qkv_rope_fwd(const void* x, const void* w_qkv, const float* cos_tab, con
                      void* stream);
 /* Optional fast path for the tables: `packed` = vrr_rope_pack_tables(cos_tab, sin_tab) of the SAME tables,
  * [heads][half_dim/2][rows] float4 {cos[2q], sin[2q], cos[2q+1], sin[2q+1]} (heads = H for rope-mixed, 1 for
- * rope-axial; rows = N-1; half_dim = Dh/2).  In the tcgen05 epilogue a lane is a token row: with the row-major tables
+ * rope-axial; rows = N-n_prefix; half_dim = Dh/2).  In the tcgen05 epilogue a lane is a token row: with the row-major tables
  * one load instruction touches 32 cache lines, with the packed table 4 (ViT-B rope-mixed: 189 -> ~140 us).  Results
  * are bit-identical.  `packed` may be NULL (= vrr_qkv_rope_fwd); cos_tab / sin_tab are still required (the SIMT
  * family reads them). */
@@ -182,6 +202,11 @@ int vrr_rope_pack_tables(const float* cos_tab, const float* sin_tab, float* pack
 int vrr_qkv_rope_fwd_packed(const void* x, const void* w_qkv, const float* cos_tab, const float* sin_tab,
                             const float* packed, void* planes, int B, int N, int E, int H, int rope_mode,
                             int dtype, void* stream);
+/* vrr_qkv_rope_fwd_packed with n_prefix prefix tokens: q,k rows t >= n_prefix are rotated by table row t - n_prefix
+ * (cos/sin and `packed` have N - n_prefix rows); rows t < n_prefix and all of v are stored as computed. */
+int vrr_qkv_rope_fwd_prefix(const void* x, const void* w_qkv, const float* cos_tab, const float* sin_tab,
+                            const float* packed, void* planes, int B, int N, int E, int H, int n_prefix, int rope_mode,
+                            int dtype, void* stream);
 /* Backward of the epilogue: un-rotates d_planes into token layout and reduces the table grads.
  * d_planes [3][B][H][N][Dh] (grads w.r.t. rotated q,k and v), planes = forward output,
  * d_qkv [B*N][3E] (gradient of x . w_qkv^T, ready for the two plain GEMMs dX = d_qkv . W and
@@ -189,6 +214,11 @@ int vrr_qkv_rope_fwd_packed(const void* x, const void* w_qkv, const float* cos_t
 int vrr_qkv_rope_bwd(const void* d_planes, const void* planes, const float* cos_tab,
                      const float* sin_tab, void* d_qkv, float* d_cos, float* d_sin, int B, int N,
                      int E, int H, int rope_mode, int dtype, void* stream);
+/* The same with n_prefix prefix tokens: rows t >= n_prefix are un-rotated with table row t - n_prefix and feed
+ * d_cos / d_sin there ([..][N-n_prefix][Dh/2]); prefix rows pass through. */
+int vrr_qkv_rope_bwd_prefix(const void* d_planes, const void* planes, const float* cos_tab, const float* sin_tab,
+                            void* d_qkv, float* d_cos, float* d_sin, int B, int N, int E, int H, int n_prefix,
+                            int rope_mode, int dtype, void* stream);
 
 /* Stand-alone rotate-half of rope_utils.py:3-37 (the public apply_rotary_emb): q,k [B][H][Nr][Dh]
  * dense, cos/sin fp32 [Nr][Dh/2] (AXIAL) or [H][Nr][Dh/2] (MIXED); every row is rotated.

@@ -16,6 +16,7 @@ Additions (all off by default, so a reference command line behaves like the refe
   --max_steps N      stop every epoch after N batches (smoke runs)
   --drop_rate P      dropout on every block's attention projection and Mlp (timm's drop_rate)
   --drop_path_rate P stochastic depth, linearly from 0 at the first block to P at the last (timm's drop_path_rate)
+  --reg_tokens R     R register tokens after the cls token (timm's reg_tokens; not with relative / polynomial)
 There is no CPU path: a CUDA sm_100 device is required.
 """
 import argparse
@@ -66,6 +67,7 @@ def get_args(argv=None):
     p.add_argument("--drop_rate", type=float, default=0.0, help="proj / Mlp dropout of every block")
     p.add_argument("--drop_path_rate", type=float, default=0.0,
                    help="stochastic depth of the last block (linearly from 0 over the depth, timm's rule)")
+    p.add_argument("--reg_tokens", type=int, default=0, help="register tokens after the cls token")
     return p.parse_args(argv)
 
 
@@ -158,7 +160,7 @@ def main(argv=None):
                               embed_dim=args.embed_dim, depth=args.depth, num_heads=args.num_heads,
                               pos_encoding=args.pos_encoding, rope_theta=args.rope_theta, poly_degree=args.poly_degree,
                               poly_shared_heads=args.poly_shared_heads, drop_rate=args.drop_rate,
-                              drop_path_rate=args.drop_path_rate).to(device)
+                              drop_path_rate=args.drop_path_rate, reg_tokens=args.reg_tokens).to(device)
     criterion = nn.CrossEntropyLoss()
     optimizer = torch.optim.AdamW(model.parameters(), lr=args.lr, weight_decay=args.weight_decay)
     scheduler = torch.optim.lr_scheduler.CosineAnnealingLR(optimizer, T_max=args.epochs)

@@ -51,10 +51,15 @@ SIGNATURES = {
     "vrr_patch_unfold": (c_int, [c_void_p] * 2 + [c_int] * 6 + [c_void_p]),
     "vrr_patch_unfold_ex": (c_int, [c_void_p] * 2 + [c_int] * 7 + [c_void_p]),
     "vrr_patch_embed_bwd": (c_int, [c_void_p] * 6 + [c_int] * 9 + [c_void_p]),
+    "vrr_patch_embed_fwd_prefix": (c_int, [c_void_p] * 4 + [c_int] + [c_void_p] * 3 + [c_size_t] + [c_int] * 9
+                                   + [c_void_p]),
+    "vrr_patch_embed_bwd_prefix": (c_int, [c_void_p] * 5 + [c_int] + [c_void_p] + [c_int] * 9 + [c_void_p]),
     "vrr_qkv_rope_fwd": (c_int, [c_void_p] * 5 + [c_int] * 6 + [c_void_p]),
     "vrr_qkv_rope_fwd_packed": (c_int, [c_void_p] * 6 + [c_int] * 6 + [c_void_p]),
     "vrr_rope_pack_tables": (c_int, [c_void_p] * 3 + [c_int] * 3 + [c_void_p]),
     "vrr_qkv_rope_bwd": (c_int, [c_void_p] * 7 + [c_int] * 6 + [c_void_p]),
+    "vrr_qkv_rope_fwd_prefix": (c_int, [c_void_p] * 6 + [c_int] * 7 + [c_void_p]),
+    "vrr_qkv_rope_bwd_prefix": (c_int, [c_void_p] * 7 + [c_int] * 7 + [c_void_p]),
     "vrr_rope_apply": (c_int, [c_void_p] * 6 + [c_int] * 7 + [c_void_p]),
     "vrr_rope_table_grad": (c_int, [c_void_p] * 6 + [c_int] * 6 + [c_void_p]),
     "vrr_gemm": (c_int, [c_void_p] * 3 + [c_int] * 7 + [c_void_p]),

@@ -53,15 +53,15 @@ struct Im2colOperand {
   }
 };
 
-// A'[e][m] = d_tokens[b][1+p][e] for the patch-embed weight gradient (m = b*Np + p)
+// A'[e][m] = d_tokens[b][npre+p][e] for the patch-embed weight gradient (m = b*Np + p)
 template <typename T>
 struct PatchGradOperand {
   static constexpr bool kVec = false;
   const T* dtok;
-  int Np, E;
+  int Np, E, rows;  // rows = npre + Np token rows per image; dtok points at row npre of image 0
   __device__ __forceinline__ float operator()(int e, int m) const {
     int b = m / Np, p = m - b * Np;
-    return Elem<T>::ld(dtok + ((long long)b * (Np + 1) + 1 + p) * E + e);
+    return Elem<T>::ld(dtok + ((long long)b * rows + p) * E + e);
   }
 };
 
@@ -115,12 +115,13 @@ struct QkvRopeEpilogue {
   T* planes;
   const float *cos_tab, *sin_tab;
   int B, N, E, H, Dh, rope_mode;
+  int npre, rows;  // prefix tokens (never rotated); row t >= npre uses table row t - npre of rows = N - npre
   __device__ __forceinline__ void operator()(int m, int n, float v, const float* crow, int n0) const {
     const int which = n / E, r = n - which * E, h = r / Dh, d = r - h * Dh;
     const int b = m / N, t = m - b * N;
-    if (rope_mode != VRR_ROPE_NONE && which < 2 && t >= 1) {
+    if (rope_mode != VRR_ROPE_NONE && which < 2 && t >= npre) {
       const int hd = Dh >> 1, dd = d < hd ? d : d - hd;
-      const size_t idx = ((size_t)(rope_mode == VRR_ROPE_MIXED ? h * (N - 1) : 0) + (t - 1)) * hd + dd;
+      const size_t idx = ((size_t)(rope_mode == VRR_ROPE_MIXED ? h * rows : 0) + (t - npre)) * hd + dd;
       const float c = cos_tab[idx], s = sin_tab[idx];
       const float other = crow[(d < hd ? n + hd : n - hd) - n0];
       v = d < hd ? v * c - other * s : other * s + v * c;
@@ -130,7 +131,7 @@ struct QkvRopeEpilogue {
 };
 
 // T: element type of images / weight / bias (the conv arithmetic); TT: element type of the token
-// stream (cls_token, pos_embed, tokens).  Under autocast T = bf16 and TT = fp32, which reproduces
+// stream (prefix tokens, pos_embed, tokens).  Under autocast T = bf16 and TT = fp32, which reproduces
 // the reference's semantics: conv output rounded to bf16, then cat with the fp32 cls token promotes
 // to fp32 and the absolute table is added in fp32 (vit.py:248-258).
 template <typename T, typename TT>
@@ -138,14 +139,14 @@ struct PatchEmbedEpilogue {
   TT* tokens;
   const T* bias;
   const TT* pos;  // may be null
-  int Np, E;
+  int Np, E, npre;
   __device__ __forceinline__ void operator()(int m, int n, float v, const float*, int) const {
     const int b = m / Np, p = m - b * Np;
     T rounded;
     Elem<T>::st(&rounded, v + Elem<T>::ld(bias + n));  // conv (+bias) in the conv dtype
     float out = Elem<T>::ld(&rounded);
     if (pos) out += Elem<TT>::ld(pos + (size_t)p * E + n);
-    Elem<TT>::st(tokens + ((size_t)b * (Np + 1) + 1 + p) * E + n, out);
+    Elem<TT>::st(tokens + ((size_t)b * (Np + npre) + npre + p) * E + n, out);
   }
 };
 
@@ -381,18 +382,18 @@ static int launch_gemm(AOp A, BOp Bop, Epi epi, int M, int N, int K, int splits,
 // ---- QKV projection + RoPE epilogue -----------------------------------------------------------
 template <typename T>
 static int qkv_rope_fwd_t(const void* x, const void* w, const float* cos_tab, const float* sin_tab,
-                          void* planes, int B, int N, int E, int H, int rope_mode, cudaStream_t st) {
+                          void* planes, int B, int N, int E, int H, int npre, int rope_mode, cudaStream_t st) {
   StridedOperand<T> A{(const T*)x, E, 1}, W{(const T*)w, E, 1};
-  QkvRopeEpilogue<T> epi{(T*)planes, cos_tab, sin_tab, B, N, E, H, E / H, rope_mode};
+  QkvRopeEpilogue<T> epi{(T*)planes, cos_tab, sin_tab, B, N, E, H, E / H, rope_mode, npre, N - npre};
   return launch_gemm<StridedOperand<T>, StridedOperand<T>, QkvRopeEpilogue<T>, true, true>(
       A, W, epi, B * N, 3 * E, E, 1, st);
 }
 int qkv_rope_fwd_simt(const void* x, const void* w, const float* cos_tab, const float* sin_tab,
-                      void* planes, int B, int N, int E, int H, int rope_mode, int dtype,
+                      void* planes, int B, int N, int E, int H, int npre, int rope_mode, int dtype,
                       cudaStream_t st) {
-  if (dtype == VRR_F32) return qkv_rope_fwd_t<float>(x, w, cos_tab, sin_tab, planes, B, N, E, H, rope_mode, st);
-  if (dtype == VRR_BF16) return qkv_rope_fwd_t<__nv_bfloat16>(x, w, cos_tab, sin_tab, planes, B, N, E, H, rope_mode, st);
-  return qkv_rope_fwd_t<__half>(x, w, cos_tab, sin_tab, planes, B, N, E, H, rope_mode, st);
+  if (dtype == VRR_F32) return qkv_rope_fwd_t<float>(x, w, cos_tab, sin_tab, planes, B, N, E, H, npre, rope_mode, st);
+  if (dtype == VRR_BF16) return qkv_rope_fwd_t<__nv_bfloat16>(x, w, cos_tab, sin_tab, planes, B, N, E, H, npre, rope_mode, st);
+  return qkv_rope_fwd_t<__half>(x, w, cos_tab, sin_tab, planes, B, N, E, H, npre, rope_mode, st);
 }
 
 // ---- plain GEMM -------------------------------------------------------------------------------
@@ -463,45 +464,48 @@ int gemm_simt(const void* a, const void* b, void* c, int M, int N, int K, int ta
 }
 
 // ---- patch embedding --------------------------------------------------------------------------
-int patch_cls_rows(void* tokens, const void* cls, int B, int Np, int E, int tok_dtype, cudaStream_t st);
+int patch_prefix_rows(void* tokens, const void* prefix, int B, int Np, int E, int npre, int tok_dtype, cudaStream_t st);
+// tokens[b][t][:] = prefix[t][:] for the npre prefix rows (cls, then the registers) of every image
 template <typename T>
-__global__ void cls_rows_kernel(T* tokens, const T* cls, int B, int Np, int E) {
+__global__ void prefix_rows_kernel(T* tokens, const T* prefix, int B, int Np, int E, int npre) {
   int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= B * E) return;
-  int b = idx / E, e = idx - b * E;
-  tokens[(size_t)b * (Np + 1) * E + e] = cls[e];
+  if (idx >= B * npre * E) return;
+  int b = idx / (npre * E), r = idx - b * (npre * E);
+  tokens[(size_t)b * (Np + npre) * E + r] = prefix[r];
 }
 
 template <typename TI, typename T, typename TT>
-static int patch_fwd_t(const void* images, const void* weight, const void* bias, const void* cls,
-                       const void* pos, void* tokens, int B, int C, int Hi, int Wi, int P, int E,
+static int patch_fwd_t(const void* images, const void* weight, const void* bias, const void* prefix,
+                       const void* pos, void* tokens, int B, int C, int Hi, int Wi, int P, int E, int npre,
                        cudaStream_t st) {
   constexpr bool kRound = sizeof(TI) == 4 && sizeof(T) == 2;
   using AOp = Im2colOperand<TI, kRound, T>;
   const int gh = Hi / P, gw = Wi / P, Np = gh * gw, Kd = C * P * P;
   AOp A{(const TI*)images, C, Hi, Wi, P, gw, Np};
   StridedOperand<T> W{(const T*)weight, Kd, 1};
-  PatchEmbedEpilogue<T, TT> epi{(TT*)tokens, (const T*)bias, (const TT*)pos, Np, E};
+  PatchEmbedEpilogue<T, TT> epi{(TT*)tokens, (const T*)bias, (const TT*)pos, Np, E, npre};
   int rc = launch_gemm<AOp, StridedOperand<T>, PatchEmbedEpilogue<T, TT>, true, true>(
       A, W, epi, B * Np, E, Kd, 1, st);
   if (rc) return rc;
-  return patch_cls_rows(tokens, cls, B, Np, E, sizeof(TT) == 4 ? VRR_F32 : (std::is_same<TT, __half>::value ? VRR_F16 : VRR_BF16),
+  return patch_prefix_rows(tokens, prefix, B, Np, E, npre, sizeof(TT) == 4 ? VRR_F32 : (std::is_same<TT, __half>::value ? VRR_F16 : VRR_BF16),
                         st);
 }
-int patch_cls_rows(void* tokens, const void* cls, int B, int Np, int E, int tok_dtype, cudaStream_t st) {
+int patch_prefix_rows(void* tokens, const void* prefix, int B, int Np, int E, int npre, int tok_dtype, cudaStream_t st) {
+  const int blocks = ceil_div(B * npre * E, 256);
   if (tok_dtype == VRR_F32)
-    cls_rows_kernel<float><<<ceil_div(B * E, 256), 256, 0, st>>>((float*)tokens, (const float*)cls, B, Np, E);
+    prefix_rows_kernel<float><<<blocks, 256, 0, st>>>((float*)tokens, (const float*)prefix, B, Np, E, npre);
   else if (tok_dtype == VRR_BF16)
-    cls_rows_kernel<__nv_bfloat16><<<ceil_div(B * E, 256), 256, 0, st>>>((__nv_bfloat16*)tokens, (const __nv_bfloat16*)cls, B, Np, E);
+    prefix_rows_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>((__nv_bfloat16*)tokens, (const __nv_bfloat16*)prefix, B, Np, E,
+                                                              npre);
   else
-    cls_rows_kernel<__half><<<ceil_div(B * E, 256), 256, 0, st>>>((__half*)tokens, (const __half*)cls, B, Np, E);
+    prefix_rows_kernel<__half><<<blocks, 256, 0, st>>>((__half*)tokens, (const __half*)prefix, B, Np, E, npre);
   VRR_LAUNCHED();
   return VRR_OK;
 }
-int patch_embed_fwd_simt(const void* images, const void* weight, const void* bias, const void* cls,
-                         const void* pos, void* tokens, int B, int C, int Hi, int Wi, int P, int E,
+int patch_embed_fwd_simt(const void* images, const void* weight, const void* bias, const void* prefix,
+                         const void* pos, void* tokens, int B, int C, int Hi, int Wi, int P, int E, int npre,
                          int img_dtype, int dtype, int tok_dtype, cudaStream_t st) {
-#define ARGS images, weight, bias, cls, pos, tokens, B, C, Hi, Wi, P, E, st
+#define ARGS images, weight, bias, prefix, pos, tokens, B, C, Hi, Wi, P, E, npre, st
   if (img_dtype == VRR_F32 && dtype == VRR_F32 && tok_dtype == VRR_F32) return patch_fwd_t<float, float, float>(ARGS);
   if (img_dtype == VRR_F32 && dtype == VRR_BF16 && tok_dtype == VRR_F32) return patch_fwd_t<float, __nv_bfloat16, float>(ARGS);
   if (img_dtype == VRR_BF16 && dtype == VRR_BF16 && tok_dtype == VRR_F32) return patch_fwd_t<__nv_bfloat16, __nv_bfloat16, float>(ARGS);
@@ -515,35 +519,36 @@ int patch_embed_fwd_simt(const void* images, const void* weight, const void* bia
   return VRR_ERR_UNSUPPORTED;
 }
 
-// s[t][e] = sum_b d_tokens[b][t][e]  ->  d_cls (t == 0), d_pos (t >= 1), d_bias (sum over t >= 1)
+// s[t][e] = sum_b d_tokens[b][t][e]  ->  d_prefix (t < npre), d_pos (t >= npre), d_bias (sum over t >= npre)
 template <typename T>
-__global__ void token_batch_sum_kernel(const T* __restrict__ dtok, float* d_bias, float* d_cls,
-                                       float* d_pos, int B, int Np, int E) {
+__global__ void token_batch_sum_kernel(const T* __restrict__ dtok, float* d_bias, float* d_prefix,
+                                       float* d_pos, int B, int Np, int E, int npre) {
   int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= (Np + 1) * E) return;
+  if (idx >= (Np + npre) * E) return;
   int t = idx / E, e = idx - t * E;
   float s = 0.f;
-  for (int b = 0; b < B; ++b) s += Elem<T>::ld(dtok + ((size_t)b * (Np + 1) + t) * E + e);
-  if (t == 0) {
-    d_cls[e] = s;
+  for (int b = 0; b < B; ++b) s += Elem<T>::ld(dtok + ((size_t)b * (Np + npre) + t) * E + e);
+  if (t < npre) {
+    d_prefix[idx] = s;
   } else {
-    if (d_pos) d_pos[(size_t)(t - 1) * E + e] = s;
+    if (d_pos) d_pos[(size_t)(t - npre) * E + e] = s;
     atomicAdd(d_bias + e, s);
   }
 }
 
 template <typename TI, bool ROUND, typename TT, typename TR>
 static int patch_bwd_t(const void* images, const void* d_tokens, float* d_weight, float* d_bias,
-                       float* d_cls, float* d_pos, int B, int C, int Hi, int Wi, int P, int E,
+                       float* d_prefix, float* d_pos, int B, int C, int Hi, int Wi, int P, int E, int npre,
                        cudaStream_t st) {
   const int gh = Hi / P, gw = Wi / P, Np = gh * gw, Kd = C * P * P, Mtok = B * Np;
   VRR_CUDA(cudaMemsetAsync(d_bias, 0, (size_t)E * sizeof(float), st));
-  token_batch_sum_kernel<TT><<<ceil_div((Np + 1) * E, 256), 256, 0, st>>>((const TT*)d_tokens, d_bias, d_cls, d_pos, B, Np, E);
+  token_batch_sum_kernel<TT><<<ceil_div((Np + npre) * E, 256), 256, 0, st>>>((const TT*)d_tokens, d_bias, d_prefix, d_pos, B,
+                                                                              Np, E, npre);
   VRR_LAUNCHED();
   if (!d_weight) return VRR_OK;  // caller computes the weight gradient itself (plain library GEMM)
   // d_weight[e][k] = sum_m d_tokens[m][e] * unfold(images)[m][k]   (reduction over m = tokens)
   using BOp = SwapArgs<Im2colOperand<TI, ROUND, TR>>;
-  PatchGradOperand<TT> A{(const TT*)d_tokens, Np, E};
+  PatchGradOperand<TT> A{(const TT*)d_tokens + (size_t)npre * E, Np, E, Np + npre};
   BOp Bo{Im2colOperand<TI, ROUND, TR>{(const TI*)images, C, Hi, Wi, P, gw, Np}};
   const int tiles = ceil_div(E, BM) * ceil_div(Kd, BN);
   int splits = max(1, min(ceil_div(2 * sm_count(), tiles), Mtok / (4 * BK)));
@@ -552,9 +557,9 @@ static int patch_bwd_t(const void* images, const void* d_tokens, float* d_weight
       A, Bo, AtomicEpilogue{d_weight, Kd}, E, Kd, Mtok, splits, st);
 }
 int patch_embed_bwd_simt(const void* images, const void* d_tokens, float* d_weight, float* d_bias,
-                         float* d_cls, float* d_pos, int B, int C, int Hi, int Wi, int P, int E,
+                         float* d_prefix, float* d_pos, int B, int C, int Hi, int Wi, int P, int E, int npre,
                          int img_dtype, int dtype, int tok_dtype, cudaStream_t st) {
-#define ARGS images, d_tokens, d_weight, d_bias, d_cls, d_pos, B, C, Hi, Wi, P, E, st
+#define ARGS images, d_tokens, d_weight, d_bias, d_prefix, d_pos, B, C, Hi, Wi, P, E, npre, st
   using bf16 = __nv_bfloat16;
   if (img_dtype == VRR_F32 && dtype == VRR_F32 && tok_dtype == VRR_F32) return patch_bwd_t<float, false, float, float>(ARGS);
   if (img_dtype == VRR_F32 && dtype == VRR_BF16 && tok_dtype == VRR_F32) return patch_bwd_t<float, true, float, bf16>(ARGS);

@@ -64,26 +64,27 @@ struct QkvRopeEpi2 {
   static constexpr bool kDrop = false;
   T* planes;
   const float *cos_tab, *sin_tab;
-  const float4* packed;  // rope_pack_tables layout [heads][16][N-1], or null
+  const float4* packed;  // rope_pack_tables layout [heads][16][N - npre], or null
   int B, N, E, H, rope_mode;
+  int npre;  // prefix tokens (cls, registers): rows t >= npre are rotated by table row t - npre
   __device__ __forceinline__ void rotate(int m, int n0, float (&f)[64]) const {
     const int hd = 32;
     const int b = m / N, t = m - b * N;
     const int which = n0 / E, h = (n0 - which * E) >> 6;
-    if (rope_mode != VRR_ROPE_NONE && which < 2 && t >= 1 && b < B && packed != nullptr) {
+    if (rope_mode != VRR_ROPE_NONE && which < 2 && t >= npre && b < B && packed != nullptr) {
       // lanes = consecutive token rows = consecutive float4 of the packed table: coalesced 512-byte requests
-      const float4* pk = packed + (size_t)(rope_mode == VRR_ROPE_MIXED ? h * 16 : 0) * (N - 1) + (t - 1);
+      const float4* pk = packed + (size_t)(rope_mode == VRR_ROPE_MIXED ? h * 16 : 0) * (N - npre) + (t - npre);
 #pragma unroll
       for (int q = 0; q < 16; ++q) {
-        const float4 v = __ldg(pk + (size_t)q * (N - 1));  // {cos[2q], sin[2q], cos[2q+1], sin[2q+1]}
+        const float4 v = __ldg(pk + (size_t)q * (N - npre));  // {cos[2q], sin[2q], cos[2q+1], sin[2q+1]}
         const float x1 = f[2 * q], x2 = f[2 * q + hd], y1 = f[2 * q + 1], y2 = f[2 * q + 1 + hd];
         f[2 * q] = x1 * v.x - x2 * v.y;
         f[2 * q + hd] = x1 * v.y + x2 * v.x;
         f[2 * q + 1] = y1 * v.z - y2 * v.w;
         f[2 * q + 1 + hd] = y1 * v.w + y2 * v.z;
       }
-    } else if (rope_mode != VRR_ROPE_NONE && which < 2 && t >= 1 && b < B) {
-      const size_t base = ((size_t)(rope_mode == VRR_ROPE_MIXED ? h * (N - 1) : 0) + (t - 1)) * hd;
+    } else if (rope_mode != VRR_ROPE_NONE && which < 2 && t >= npre && b < B) {
+      const size_t base = ((size_t)(rope_mode == VRR_ROPE_MIXED ? h * (N - npre) : 0) + (t - npre)) * hd;
       const float4* c4 = reinterpret_cast<const float4*>(cos_tab + base);
       const float4* s4 = reinterpret_cast<const float4*>(sin_tab + base);
 #pragma unroll
@@ -107,7 +108,7 @@ struct QkvRopeEpi2 {
   }
 };
 
-// tokens[b][1+p][n] = round_T(acc + bias[n]) (+ pos[p][n]); TT = token-stream type
+// tokens[b][npre+p][n] = round_T(acc + bias[n]) (+ pos[p][n]); TT = token-stream type
 template <typename T, typename TT>
 struct PatchEmbedEpi2 {
   static constexpr bool kTma = false;
@@ -117,9 +118,10 @@ struct PatchEmbedEpi2 {
   const T* bias;
   const TT* pos;  // may be null
   int Np, E;
+  int rows;  // token rows per image (npre + Np); `tokens` points at row npre of image 0
   __device__ __forceinline__ void operator()(int m, int n0, float (&f)[64]) const {
     const int b = m / Np, p = m - b * Np;
-    TT* dst = tokens + ((size_t)b * (Np + 1) + 1 + p) * E + n0;
+    TT* dst = tokens + ((size_t)b * rows + p) * E + n0;
     const TT* prow = pos ? pos + (size_t)p * E + n0 : nullptr;
 #pragma unroll
     for (int v4 = 0; v4 < 16; ++v4) {
@@ -873,8 +875,8 @@ bool qkv_rope_fwd_tc_supported(int B, int N, int E, int H) {
 
 template <typename T>
 static int qkv_rope_fwd_tc2_t(const void* x, const void* w, const float* cos_tab, const float* sin_tab, const float* packed,
-                              void* planes, int B, int N, int E, int H, int rope_mode, cudaStream_t st) {
-  QkvRopeEpi2<T> epi{(T*)planes, cos_tab, sin_tab, reinterpret_cast<const float4*>(packed), B, N, E, H, rope_mode};
+                              void* planes, int B, int N, int E, int H, int npre, int rope_mode, cudaStream_t st) {
+  QkvRopeEpi2<T> epi{(T*)planes, cos_tab, sin_tab, reinterpret_cast<const float4*>(packed), B, N, E, H, rope_mode, npre};
   CUtensorMap tplanes;  // planes[3 B H][N][64] of T, box = [1][32 rows][64]
   if (int rc = make_tmap_3d(&tplanes, planes, Elem16<T>::kTmap, 64, (uint64_t)N, (uint64_t)3 * B * H, 128, (uint64_t)N * 128,
                             64, 32))
@@ -885,15 +887,15 @@ static int qkv_rope_fwd_tc2_t(const void* x, const void* w, const float* cos_tab
 }
 
 int qkv_rope_fwd_tc2(const void* x, const void* w, const float* cos_tab, const float* sin_tab, const float* packed,
-                     void* planes, int B, int N, int E, int H, int rope_mode, int dtype, cudaStream_t st) {
+                     void* planes, int B, int N, int E, int H, int npre, int rope_mode, int dtype, cudaStream_t st) {
   VRR_REQUIRE(((uintptr_t)x & 15) == 0 && ((uintptr_t)w & 15) == 0 && ((uintptr_t)planes & 15) == 0,
               VRR_ERR_INVALID_ARG, "qkv_rope_fwd (tcgen05): x / w / planes must be 16-byte aligned");
   if (rope_mode != VRR_ROPE_NONE)
     VRR_REQUIRE(((uintptr_t)cos_tab & 15) == 0 && ((uintptr_t)sin_tab & 15) == 0, VRR_ERR_INVALID_ARG,
                 "qkv_rope_fwd (tcgen05): cos / sin must be 16-byte aligned");
   VRR_REQUIRE(((uintptr_t)packed & 15) == 0, VRR_ERR_INVALID_ARG, "qkv_rope_fwd (tcgen05): packed table must be 16-byte aligned");
-  if (dtype == VRR_F16) return qkv_rope_fwd_tc2_t<__half>(x, w, cos_tab, sin_tab, packed, planes, B, N, E, H, rope_mode, st);
-  return qkv_rope_fwd_tc2_t<__nv_bfloat16>(x, w, cos_tab, sin_tab, packed, planes, B, N, E, H, rope_mode, st);
+  if (dtype == VRR_F16) return qkv_rope_fwd_tc2_t<__half>(x, w, cos_tab, sin_tab, packed, planes, B, N, E, H, npre, rope_mode, st);
+  return qkv_rope_fwd_tc2_t<__nv_bfloat16>(x, w, cos_tab, sin_tab, packed, planes, B, N, E, H, npre, rope_mode, st);
 }
 
 // ---- patch embedding: unfold pre-pass (fused fp32 -> 16-bit cast) + the CTA-pair kernel -------------------
@@ -935,25 +937,25 @@ int patch_unfold(const void* images, void* out, int B, int C, int Hi, int Wi, in
 
 template <typename T, typename TT>
 static int patch_embed_gemm(const void* workspace, const void* weight, const void* bias, const void* pos, void* tokens, int M,
-                            int E, int K, int Np, cudaStream_t st) {
+                            int E, int K, int Np, int npre, cudaStream_t st) {
   CUtensorMap dummy;  // PatchEmbedEpi2 stores its rows directly: no C map
   memset(&dummy, 0, sizeof(dummy));
-  PatchEmbedEpi2<T, TT> epi{(TT*)tokens, (const T*)bias, (const TT*)pos, Np, E};
+  PatchEmbedEpi2<T, TT> epi{(TT*)tokens + (size_t)npre * E, (const T*)bias, (const TT*)pos, Np, E, Np + npre};
   if (E > 128) return launch_pair<T, 256, false, false, PatchEmbedEpi2<T, TT>>(workspace, weight, M, E, K, 1, dummy, dummy, epi, st);
   return launch_pair<T, 128, false, false, PatchEmbedEpi2<T, TT>>(workspace, weight, M, E, K, 1, dummy, dummy, epi, st);
 }
 
 int patch_embed_fwd_tc(const void* images, const void* weight, const void* bias, const void* pos, void* tokens,
-                       void* workspace, int B, int C, int Hi, int Wi, int P, int E, int img_dtype, int dtype, int tok_dtype,
-                       cudaStream_t st) {
+                       void* workspace, int B, int C, int Hi, int Wi, int P, int E, int npre, int img_dtype, int dtype,
+                       int tok_dtype, cudaStream_t st) {
   const int Np = (Hi / P) * (Wi / P), K = C * P * P, M = B * Np;
   if (int rc = patch_unfold(images, workspace, B, C, Hi, Wi, P, img_dtype, dtype, st)) return rc;
   if (dtype == VRR_F16) {
-    if (tok_dtype == VRR_F32) return patch_embed_gemm<__half, float>(workspace, weight, bias, pos, tokens, M, E, K, Np, st);
-    return patch_embed_gemm<__half, __half>(workspace, weight, bias, pos, tokens, M, E, K, Np, st);
+    if (tok_dtype == VRR_F32) return patch_embed_gemm<__half, float>(workspace, weight, bias, pos, tokens, M, E, K, Np, npre, st);
+    return patch_embed_gemm<__half, __half>(workspace, weight, bias, pos, tokens, M, E, K, Np, npre, st);
   }
-  if (tok_dtype == VRR_F32) return patch_embed_gemm<__nv_bfloat16, float>(workspace, weight, bias, pos, tokens, M, E, K, Np, st);
-  return patch_embed_gemm<__nv_bfloat16, __nv_bfloat16>(workspace, weight, bias, pos, tokens, M, E, K, Np, st);
+  if (tok_dtype == VRR_F32) return patch_embed_gemm<__nv_bfloat16, float>(workspace, weight, bias, pos, tokens, M, E, K, Np, npre, st);
+  return patch_embed_gemm<__nv_bfloat16, __nv_bfloat16>(workspace, weight, bias, pos, tokens, M, E, K, Np, npre, st);
 }
 
 }  // namespace vrr

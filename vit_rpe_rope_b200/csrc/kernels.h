@@ -45,19 +45,21 @@ int attn_bwd_ws(const void* planes, const void* out, const void* d_out, const fl
 // gemm_simt.cu
 void layernorm_set_option(int which, int value);  // 0: ln_reg, 1: ln_bwd_minb
 void gemm_simt_set_tile(int v);  // 128 (default): 128 x 128 double-buffered kernel for problems with a full tile; 64: 64 x 64 always
+// npre: prefix tokens per image (token rows 0..npre-1: cls, then registers); they are never rotated, and the patch
+// rows t >= npre use table row t - npre
 int qkv_rope_fwd_simt(const void* x, const void* w, const float* cos_tab, const float* sin_tab, void* planes,
-                      int B, int N, int E, int H, int rope_mode, int dtype, cudaStream_t st);
+                      int B, int N, int E, int H, int npre, int rope_mode, int dtype, cudaStream_t st);
 int gemm_simt(const void* a, const void* b, void* c, int M, int N, int K, int ta, int tb, int dtype,
               int c_dtype, cudaStream_t st);
 int gemm_simt_bias(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int ta, int tb,
                    int dtype, int gelu, cudaStream_t st);
-int patch_embed_fwd_simt(const void* images, const void* weight, const void* bias, const void* cls,
-                         const void* pos, void* tokens, int B, int C, int Hi, int Wi, int P, int E, int img_dtype,
-                         int dtype, int tok_dtype, cudaStream_t st);
-int patch_embed_bwd_simt(const void* images, const void* d_tokens, float* d_weight, float* d_bias, float* d_cls,
-                         float* d_pos, int B, int C, int Hi, int Wi, int P, int E, int img_dtype, int dtype,
+int patch_embed_fwd_simt(const void* images, const void* weight, const void* bias, const void* prefix,
+                         const void* pos, void* tokens, int B, int C, int Hi, int Wi, int P, int E, int npre,
+                         int img_dtype, int dtype, int tok_dtype, cudaStream_t st);
+int patch_embed_bwd_simt(const void* images, const void* d_tokens, float* d_weight, float* d_bias, float* d_prefix,
+                         float* d_pos, int B, int C, int Hi, int Wi, int P, int E, int npre, int img_dtype, int dtype,
                          int tok_dtype, cudaStream_t st);
-int patch_cls_rows(void* tokens, const void* cls, int B, int Np, int E, int tok_dtype, cudaStream_t st);
+int patch_prefix_rows(void* tokens, const void* prefix, int B, int Np, int E, int npre, int tok_dtype, cudaStream_t st);
 
 // gemm_tc2.cu (tcgen05 CTA pairs, cta_group::2: every operand layout, TMA-store epilogues)
 bool gemm_tc_supported(int M, int N, int K, int trans_a, int trans_b, int dtype, int c_dtype, int epilogue);
@@ -71,7 +73,7 @@ int rope_pack_tables(const float* cos_tab, const float* sin_tab, float* packed, 
 bool qkv_rope_fwd_tc_supported(int B, int N, int E, int H);
 // `packed`: optional output of rope_pack_tables for the same tables (NULL: the epilogue reads cos_tab / sin_tab)
 int qkv_rope_fwd_tc2(const void* x, const void* w, const float* cos_tab, const float* sin_tab, const float* packed, void* planes, int B, int N,
-                     int E, int H, int rope_mode, int dtype, cudaStream_t st);
+                     int E, int H, int npre, int rope_mode, int dtype, cudaStream_t st);
 
 bool patch_embed_tc_supported(int B, int C, int Hi, int Wi, int P, int E);
 size_t patch_embed_tc_workspace_bytes(int B, int C, int Hi, int Wi, int P);
@@ -79,8 +81,8 @@ size_t patch_embed_tc_workspace_bytes(int B, int C, int Hi, int Wi, int P);
 int patch_unfold(const void* images, void* out, int B, int C, int Hi, int Wi, int P, int img_dtype, int out_dtype,
                  cudaStream_t st);
 int patch_embed_fwd_tc(const void* images, const void* weight, const void* bias, const void* pos, void* tokens,
-                       void* workspace, int B, int C, int Hi, int Wi, int P, int E, int img_dtype, int dtype, int tok_dtype,
-                       cudaStream_t st);
+                       void* workspace, int B, int C, int Hi, int Wi, int P, int E, int npre, int img_dtype, int dtype,
+                       int tok_dtype, cudaStream_t st);
 
 // layernorm.cu
 int layernorm_fwd(const void* x, const float* gamma, const float* beta, void* y, float* mean, float* rstd, int M, int E,
@@ -107,7 +109,7 @@ int dropout_mask(const DropView& dv, uint8_t* keep, uint8_t* keep_path, int M, i
 
 // rope.cu
 int qkv_rope_bwd(const void* d_planes, const void* planes, const float* cos_tab, const float* sin_tab,
-                 void* d_qkv, float* d_cos, float* d_sin, int B, int N, int E, int H, int rope_mode, int dtype,
+                 void* d_qkv, float* d_cos, float* d_sin, int B, int N, int E, int H, int npre, int rope_mode, int dtype,
                  cudaStream_t st);
 int rope_apply(const void* q_in, const void* k_in, const float* cos_tab, const float* sin_tab, void* q_out,
                void* k_out, int B, int H, int Nr, int Dh, int rope_mode, int inverse, int dtype, cudaStream_t st);

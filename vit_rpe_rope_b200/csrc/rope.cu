@@ -75,20 +75,20 @@ template <typename T, int VEC>
 __global__ void qkv_rope_bwd_kernel(const T* __restrict__ d_planes, const T* __restrict__ planes,
                                     const float* __restrict__ cos_tab, const float* __restrict__ sin_tab,
                                     T* __restrict__ d_qkv, float* d_cos, float* d_sin, int B, int N,
-                                    int E, int H, int Dh, int rope_mode, int b_chunk) {
+                                    int E, int H, int Dh, int npre, int rope_mode, int b_chunk) {
   const int hd = Dh >> 1, nv = hd / VEC;
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= H * N * nv) return;
   const int dd = (idx % nv) * VEC, t = (idx / nv) % N, h = idx / (nv * N);
   const int b0 = blockIdx.y * b_chunk, b1 = min(B, b0 + b_chunk);
   const size_t plane = (size_t)B * H * N * Dh;
-  const bool rot = rope_mode != VRR_ROPE_NONE && t >= 1;
+  const bool rot = rope_mode != VRR_ROPE_NONE && t >= npre;  // prefix rows (cls, registers) are never rotated
   float c[VEC], s[VEC], acc_c[VEC], acc_s[VEC];
   size_t tab = 0;
 #pragma unroll
   for (int e = 0; e < VEC; ++e) { c[e] = 1.f; s[e] = 0.f; acc_c[e] = 0.f; acc_s[e] = 0.f; }
   if (rot) {
-    tab = ((size_t)(rope_mode == VRR_ROPE_MIXED ? h * (N - 1) : 0) + (t - 1)) * hd + dd;
+    tab = ((size_t)(rope_mode == VRR_ROPE_MIXED ? h * (N - npre) : 0) + (t - npre)) * hd + dd;
 #pragma unroll
     for (int e = 0; e < VEC; ++e) { c[e] = cos_tab[tab + e]; s[e] = sin_tab[tab + e]; }
   }
@@ -149,12 +149,12 @@ __global__ void qkv_rope_bwd_kernel(const T* __restrict__ d_planes, const T* __r
 }
 
 int qkv_rope_bwd(const void* d_planes, const void* planes, const float* cos_tab, const float* sin_tab,
-                 void* d_qkv, float* d_cos, float* d_sin, int B, int N, int E, int H, int rope_mode,
+                 void* d_qkv, float* d_cos, float* d_sin, int B, int N, int E, int H, int npre, int rope_mode,
                  int dtype, cudaStream_t st) {
   const int Dh = E / H, hd = Dh / 2;
   if (rope_mode == VRR_ROPE_NONE) d_cos = d_sin = nullptr;
   if (d_cos) {
-    size_t n = (size_t)(rope_mode == VRR_ROPE_MIXED ? H : 1) * (N - 1) * hd * sizeof(float);
+    size_t n = (size_t)(rope_mode == VRR_ROPE_MIXED ? H : 1) * (N - npre) * hd * sizeof(float);
     if (reinterpret_cast<char*>(d_sin) == reinterpret_cast<char*>(d_cos) + n) {  // halves of one buffer: one memset node
       VRR_CUDA(cudaMemsetAsync(d_cos, 0, 2 * n, st));
     } else {
@@ -174,14 +174,15 @@ int qkv_rope_bwd(const void* d_planes, const void* planes, const float* cos_tab,
   if (dtype == VRR_F32)
     qkv_rope_bwd_kernel<float, 4><<<grid, threads, 0, st>>>((const float*)d_planes, (const float*)planes, cos_tab,
                                                            sin_tab, (float*)d_qkv, d_cos, d_sin, B, N, E, H, Dh,
-                                                           rope_mode, b_chunk);
+                                                           npre, rope_mode, b_chunk);
   else if (dtype == VRR_BF16)
     qkv_rope_bwd_kernel<__nv_bfloat16, 8><<<grid, threads, 0, st>>>(
         (const __nv_bfloat16*)d_planes, (const __nv_bfloat16*)planes, cos_tab, sin_tab,
-        (__nv_bfloat16*)d_qkv, d_cos, d_sin, B, N, E, H, Dh, rope_mode, b_chunk);
+        (__nv_bfloat16*)d_qkv, d_cos, d_sin, B, N, E, H, Dh, npre, rope_mode, b_chunk);
   else
     qkv_rope_bwd_kernel<__half, 8><<<grid, threads, 0, st>>>((const __half*)d_planes, (const __half*)planes, cos_tab, sin_tab,
-                                                            (__half*)d_qkv, d_cos, d_sin, B, N, E, H, Dh, rope_mode, b_chunk);
+                                                            (__half*)d_qkv, d_cos, d_sin, B, N, E, H, Dh, npre, rope_mode,
+                                                            b_chunk);
   VRR_LAUNCHED();
   return VRR_OK;
 }

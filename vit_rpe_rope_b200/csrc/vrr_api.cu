@@ -104,6 +104,10 @@ static bool gemm_ptrs_aligned16(const void* a, const void* b, const void* c, con
   return (((uintptr_t)a | (uintptr_t)b | (uintptr_t)c | (uintptr_t)c2 | (uintptr_t)bias) & 15) == 0;
 }
 static bool dh_ok(int dh) { return dh == 16 || dh == 32 || dh == 64; }
+// 1 <= n_prefix <= N, and the prefix rows of the batch indexable by the 32-bit index of the prefix-rows kernel
+static bool prefix_ok(int n_prefix, long long N, int B, int E) {
+  return n_prefix >= 1 && n_prefix <= N && (long long)B * n_prefix * E < (1ll << 31);
+}
 
 static int check_bias(const vrr_bias_desc* b, int H, int N) {
   if (!b || b->mode == VRR_BIAS_NONE) return VRR_OK;
@@ -188,11 +192,22 @@ size_t vrr_patch_embed_workspace_bytes(int B, int C, int Hi, int Wi, int P, int 
 int vrr_patch_embed_fwd(const void* images, const void* weight, const void* bias, const void* cls_token,
                         const void* pos_embed, void* tokens, void* workspace, size_t workspace_bytes, int B, int C,
                         int Hi, int Wi, int P, int E, int img_dtype, int dtype, int tok_dtype, void* stream) {
-  VRR_REQUIRE(images && weight && bias && cls_token && tokens, VRR_ERR_INVALID_ARG, "patch_embed_fwd: NULL pointer");
+  return vrr_patch_embed_fwd_prefix(images, weight, bias, cls_token, 1, pos_embed, tokens, workspace, workspace_bytes, B, C,
+                                    Hi, Wi, P, E, img_dtype, dtype, tok_dtype, stream);
+}
+
+int vrr_patch_embed_fwd_prefix(const void* images, const void* weight, const void* bias, const void* prefix_tokens,
+                               int n_prefix, const void* pos_embed, void* tokens, void* workspace, size_t workspace_bytes,
+                               int B, int C, int Hi, int Wi, int P, int E, int img_dtype, int dtype, int tok_dtype,
+                               void* stream) {
+  VRR_REQUIRE(images && weight && bias && prefix_tokens && tokens, VRR_ERR_INVALID_ARG, "patch_embed_fwd: NULL pointer");
   VRR_REQUIRE(dtype_ok(dtype) && dtype_ok(tok_dtype) && dtype_ok(img_dtype) && no_mix(img_dtype, dtype, tok_dtype),
               VRR_ERR_INVALID_ARG, "patch_embed_fwd: bad dtype %d/%d/%d", img_dtype, dtype, tok_dtype);
   VRR_REQUIRE(B > 0 && C > 0 && P > 0 && E > 0 && Hi >= P && Wi >= P, VRR_ERR_INVALID_ARG,
               "patch_embed_fwd: bad sizes B=%d C=%d Hi=%d Wi=%d P=%d E=%d", B, C, Hi, Wi, P, E);
+  const int Np = (Hi / P) * (Wi / P);
+  VRR_REQUIRE(prefix_ok(n_prefix, Np + (long long)n_prefix, B, E), VRR_ERR_INVALID_ARG,
+              "patch_embed_fwd: n_prefix %d must lie in [1, N] (N = n_prefix + %d patches)", n_prefix, Np);
   if (int rc = require_device()) return rc;
   const int impl = g_impl.load();
   if (is16(dtype) && impl != VRR_IMPL_SIMT && patch_embed_tc_supported(B, C, Hi, Wi, P, E)) {
@@ -201,16 +216,16 @@ int vrr_patch_embed_fwd(const void* images, const void* weight, const void* bias
                 "patch_embed_fwd: workspace %zu < %zu bytes (vrr_patch_embed_workspace_bytes)", workspace_bytes, need);
     VRR_REQUIRE(((uintptr_t)workspace & 255) == 0, VRR_ERR_INVALID_ARG, "patch_embed_fwd: workspace must be 256-byte aligned");
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
-    if (int rc = patch_embed_fwd_tc(images, weight, bias, pos_embed, tokens, workspace, B, C, Hi, Wi, P, E, img_dtype,
-                                    dtype, tok_dtype, (cudaStream_t)stream))
+    if (int rc = patch_embed_fwd_tc(images, weight, bias, pos_embed, tokens, workspace, B, C, Hi, Wi, P, E, n_prefix,
+                                    img_dtype, dtype, tok_dtype, (cudaStream_t)stream))
       return rc;
-    return patch_cls_rows(tokens, cls_token, B, (Hi / P) * (Wi / P), E, tok_dtype, (cudaStream_t)stream);
+    return patch_prefix_rows(tokens, prefix_tokens, B, Np, E, n_prefix, tok_dtype, (cudaStream_t)stream);
   }
   VRR_REQUIRE(impl != VRR_IMPL_TCGEN05 || !is16(dtype), VRR_ERR_UNSUPPORTED,
               "patch_embed_fwd: tcgen05 kernel forced but shape unsupported (P %% 8, C*P*P %% 64, E %% 64)");
   VRR_COUNT_FAMILY(VRR_IMPL_SIMT);
-  return patch_embed_fwd_simt(images, weight, bias, cls_token, pos_embed, tokens, B, C, Hi, Wi, P, E, img_dtype, dtype,
-                              tok_dtype, (cudaStream_t)stream);
+  return patch_embed_fwd_simt(images, weight, bias, prefix_tokens, pos_embed, tokens, B, C, Hi, Wi, P, E, n_prefix,
+                              img_dtype, dtype, tok_dtype, (cudaStream_t)stream);
 }
 
 int vrr_patch_unfold(const void* images, void* out, int B, int C, int Hi, int Wi, int P, int img_dtype, void* stream) {
@@ -234,14 +249,24 @@ int vrr_patch_unfold_ex(const void* images, void* out, int B, int C, int Hi, int
 int vrr_patch_embed_bwd(const void* images, const void* d_tokens, void* d_weight, void* d_bias, void* d_cls,
                         void* d_pos, int B, int C, int Hi, int Wi, int P, int E, int img_dtype, int dtype,
                         int tok_dtype, void* stream) {
-  VRR_REQUIRE(images && d_tokens && d_bias && d_cls, VRR_ERR_INVALID_ARG, "patch_embed_bwd: NULL pointer");
+  return vrr_patch_embed_bwd_prefix(images, d_tokens, d_weight, d_bias, d_cls, 1, d_pos, B, C, Hi, Wi, P, E, img_dtype,
+                                    dtype, tok_dtype, stream);
+}
+
+int vrr_patch_embed_bwd_prefix(const void* images, const void* d_tokens, void* d_weight, void* d_bias, void* d_prefix,
+                               int n_prefix, void* d_pos, int B, int C, int Hi, int Wi, int P, int E, int img_dtype,
+                               int dtype, int tok_dtype, void* stream) {
+  VRR_REQUIRE(images && d_tokens && d_bias && d_prefix, VRR_ERR_INVALID_ARG, "patch_embed_bwd: NULL pointer");
   VRR_REQUIRE(dtype_ok(dtype) && dtype_ok(tok_dtype) && dtype_ok(img_dtype) && no_mix(img_dtype, dtype, tok_dtype),
               VRR_ERR_INVALID_ARG, "patch_embed_bwd: bad dtype %d/%d/%d", img_dtype, dtype, tok_dtype);
   VRR_REQUIRE(B > 0 && C > 0 && P > 0 && E > 0 && Hi >= P && Wi >= P, VRR_ERR_INVALID_ARG,
               "patch_embed_bwd: bad sizes");
+  const int Np = (Hi / P) * (Wi / P);
+  VRR_REQUIRE(prefix_ok(n_prefix, Np + (long long)n_prefix, B, E), VRR_ERR_INVALID_ARG,
+              "patch_embed_bwd: n_prefix %d must lie in [1, N] (N = n_prefix + %d patches)", n_prefix, Np);
   if (int rc = require_device()) return rc;
-  return patch_embed_bwd_simt(images, d_tokens, (float*)d_weight, (float*)d_bias, (float*)d_cls, (float*)d_pos, B,
-                              C, Hi, Wi, P, E, img_dtype, dtype, tok_dtype, (cudaStream_t)stream);
+  return patch_embed_bwd_simt(images, d_tokens, (float*)d_weight, (float*)d_bias, (float*)d_prefix, (float*)d_pos, B,
+                              C, Hi, Wi, P, E, n_prefix, img_dtype, dtype, tok_dtype, (cudaStream_t)stream);
 }
 
 int vrr_qkv_rope_fwd(const void* x, const void* w_qkv, const float* cos_tab, const float* sin_tab, void* planes,
@@ -260,6 +285,12 @@ int vrr_rope_pack_tables(const float* cos_tab, const float* sin_tab, float* pack
 int vrr_qkv_rope_fwd_packed(const void* x, const void* w_qkv, const float* cos_tab, const float* sin_tab,
                             const float* packed, void* planes, int B, int N, int E, int H, int rope_mode, int dtype,
                             void* stream) {
+  return vrr_qkv_rope_fwd_prefix(x, w_qkv, cos_tab, sin_tab, packed, planes, B, N, E, H, 1, rope_mode, dtype, stream);
+}
+
+int vrr_qkv_rope_fwd_prefix(const void* x, const void* w_qkv, const float* cos_tab, const float* sin_tab,
+                            const float* packed, void* planes, int B, int N, int E, int H, int n_prefix, int rope_mode,
+                            int dtype, void* stream) {
   VRR_REQUIRE(x && w_qkv && planes, VRR_ERR_INVALID_ARG, "qkv_rope_fwd: NULL pointer");
   VRR_REQUIRE(dtype_ok(dtype), VRR_ERR_INVALID_ARG, "qkv_rope_fwd: bad dtype %d", dtype);
   VRR_REQUIRE(rope_mode >= VRR_ROPE_NONE && rope_mode <= VRR_ROPE_MIXED, VRR_ERR_INVALID_ARG,
@@ -267,22 +298,32 @@ int vrr_qkv_rope_fwd_packed(const void* x, const void* w_qkv, const float* cos_t
   VRR_REQUIRE(rope_mode == VRR_ROPE_NONE || (cos_tab && sin_tab), VRR_ERR_INVALID_ARG,
               "qkv_rope_fwd: cos/sin required for rope_mode %d", rope_mode);
   VRR_REQUIRE(B > 0 && N > 0 && H > 0 && E > 0 && E % H == 0, VRR_ERR_INVALID_ARG, "qkv_rope_fwd: bad sizes");
+  VRR_REQUIRE(n_prefix >= 1 && n_prefix <= N, VRR_ERR_INVALID_ARG, "qkv_rope_fwd: n_prefix %d must lie in [1, N = %d]",
+              n_prefix, N);
   VRR_REQUIRE(dh_ok(E / H), VRR_ERR_UNSUPPORTED, "qkv_rope_fwd: head dim %d unsupported (16, 32, 64)", E / H);
   if (int rc = require_device()) return rc;
   const int impl = g_impl.load();
   if (is16(dtype) && impl != VRR_IMPL_SIMT && qkv_rope_fwd_tc_supported(B, N, E, H)) {
     VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
-    return qkv_rope_fwd_tc2(x, w_qkv, cos_tab, sin_tab, packed, planes, B, N, E, H, rope_mode, dtype, (cudaStream_t)stream);
+    return qkv_rope_fwd_tc2(x, w_qkv, cos_tab, sin_tab, packed, planes, B, N, E, H, n_prefix, rope_mode, dtype,
+                            (cudaStream_t)stream);
   }
   VRR_REQUIRE(impl != VRR_IMPL_TCGEN05, VRR_ERR_UNSUPPORTED,
               "qkv_rope_fwd: tcgen05 kernel forced but shape/dtype unsupported (bf16 or fp16, Dh=64, E%%64==0)");
   VRR_COUNT_FAMILY(VRR_IMPL_SIMT);
-  return qkv_rope_fwd_simt(x, w_qkv, cos_tab, sin_tab, planes, B, N, E, H, rope_mode, dtype, (cudaStream_t)stream);
+  return qkv_rope_fwd_simt(x, w_qkv, cos_tab, sin_tab, planes, B, N, E, H, n_prefix, rope_mode, dtype, (cudaStream_t)stream);
 }
 
 int vrr_qkv_rope_bwd(const void* d_planes, const void* planes, const float* cos_tab, const float* sin_tab,
                      void* d_qkv, float* d_cos, float* d_sin, int B, int N, int E, int H, int rope_mode,
                      int dtype, void* stream) {
+  return vrr_qkv_rope_bwd_prefix(d_planes, planes, cos_tab, sin_tab, d_qkv, d_cos, d_sin, B, N, E, H, 1, rope_mode, dtype,
+                                 stream);
+}
+
+int vrr_qkv_rope_bwd_prefix(const void* d_planes, const void* planes, const float* cos_tab, const float* sin_tab,
+                            void* d_qkv, float* d_cos, float* d_sin, int B, int N, int E, int H, int n_prefix,
+                            int rope_mode, int dtype, void* stream) {
   VRR_REQUIRE(d_planes && planes && d_qkv, VRR_ERR_INVALID_ARG, "qkv_rope_bwd: NULL pointer");
   VRR_REQUIRE(dtype_ok(dtype), VRR_ERR_INVALID_ARG, "qkv_rope_bwd: bad dtype %d", dtype);
   VRR_REQUIRE(rope_mode >= VRR_ROPE_NONE && rope_mode <= VRR_ROPE_MIXED, VRR_ERR_INVALID_ARG,
@@ -293,8 +334,10 @@ int vrr_qkv_rope_bwd(const void* d_planes, const void* planes, const float* cos_
               "qkv_rope_bwd: d_cos and d_sin must both be given or both NULL");
   VRR_REQUIRE(B > 0 && N > 0 && H > 0 && E > 0 && E % H == 0 && dh_ok(E / H), VRR_ERR_INVALID_ARG,
               "qkv_rope_bwd: bad sizes");
+  VRR_REQUIRE(n_prefix >= 1 && n_prefix <= N, VRR_ERR_INVALID_ARG, "qkv_rope_bwd: n_prefix %d must lie in [1, N = %d]",
+              n_prefix, N);
   if (int rc = require_device()) return rc;
-  return qkv_rope_bwd(d_planes, planes, cos_tab, sin_tab, d_qkv, d_cos, d_sin, B, N, E, H, rope_mode, dtype,
+  return qkv_rope_bwd(d_planes, planes, cos_tab, sin_tab, d_qkv, d_cos, d_sin, B, N, E, H, n_prefix, rope_mode, dtype,
                       (cudaStream_t)stream);
 }
 

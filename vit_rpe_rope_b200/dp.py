@@ -6,8 +6,8 @@ exchange and the single collective is the gradient mean before ``optimizer.step`
 
 * parameters are grouped into flat fp32 buckets (~``bucket_mb`` each) in *reverse registration
   order* - the order backward produces their gradients; parameters whose gradient only completes
-  at the very end of backward (the shared PE parameter that every block feeds, the cls token,
-  the patch projection, an absolute table) go into the last bucket;
+  at the very end of backward (the shared PE parameter that every block feeds, the cls and
+  register tokens, the patch projection, an absolute table) go into the last bucket;
 * default (``dp.zero_grad()``): ``param.grad`` is dropped, autograd then ADOPTS the gradient tensors the backward
   kernels produce (no ``grad += dW`` pass, no zero-fill of 345 MB per step: ~220 small ATen launches and ~0.9 ms of
   a 38 ms ViT-B step); when the last parameter of a bucket has its gradient, ONE multi-tensor copy gathers them
@@ -87,7 +87,7 @@ class BucketedDataParallel(torch.nn.Module):
         """Parameters whose gradient is complete only when backward reaches the stem."""
         late = set()
         for name, p in module.named_parameters():
-            if name.startswith(("pos_embed.", "patch_embed.")) or name == "cls_token":
+            if name.startswith(("pos_embed.", "patch_embed.")) or name in ("cls_token", "reg_token"):
                 late.add(id(p))
         return late
 

@@ -17,6 +17,11 @@ GEMM.  CUDA sm_100 only: CPU inputs raise; there is no fallback path.
 Regularisers of a ViT training recipe (``VisionTransformer(drop_rate, drop_path_rate)``, timm's names): inside the
 fused block loop, proj_drop / drop2 and stochastic depth are applied by the add+LayerNorm kernels that read the
 branch anyway, and drop1 by fc1's GELU epilogue, all from one Philox key drawn per training forward.
+
+Register tokens (``VisionTransformer(reg_tokens=R)``, timm's name; DINOv2-with-registers, DINOv3): R learnable tokens
+between the cls token and the patches, ``[cls, reg_0 .. reg_{R-1}, patch_0 ..]``.  Like the cls token they get no
+absolute position embedding and are never rotated; the patch-embedding kernel writes them and the QKV+RoPE epilogue
+skips them (``num_prefix_tokens = 1 + R``).
 """
 import torch
 import torch.nn as nn
@@ -107,6 +112,7 @@ class Attention(nn.Module):
         self.proj = nn.Linear(dim, dim)
         self.proj_drop = nn.Dropout(proj_drop)
         self.pos_encoding = None
+        self.num_prefix_tokens = 1  # leading tokens RoPE leaves alone (cls + registers; VisionTransformer sets it)
 
     def forward(self, x, freqs_cis=None):
         return self.proj_drop(self._branch(x, freqs_cis))
@@ -123,7 +129,8 @@ class Attention(nn.Module):
         elif isinstance(pe, PolynomialRPE):
             bias_mode, bias_param, bias_grid = _lib.BIAS_POLY, pe.coefficients, pe.grid_size
         dt = ops.compute_dtype(x)
-        planes = ops.qkv_rope(x, self.qkv.weight, cos, sin, self.num_heads, ops.lp_weight(self.qkv.weight, dt))
+        planes = ops.qkv_rope(x, self.qkv.weight, cos, sin, self.num_heads, ops.lp_weight(self.qkv.weight, dt),
+                              self.num_prefix_tokens)
         out = ops.fused_attention(planes, self.scale, bias_mode, bias_param, bias_grid)
         return ops.linear(out, self.proj, ops.lp_weight(self.proj.weight, dt))
 
@@ -159,13 +166,23 @@ class VisionTransformer(nn.Module):
     anything else raises ``ValueError`` (vit.py:196).  ``drop_rate`` is every block's proj_drop / Mlp dropout,
     ``drop_path_rate`` the stochastic-depth rate of the last block (timm's rule: block i of d gets
     ``linspace(0, drop_path_rate, d)[i]``); both default to 0, the reference's values.
+
+    ``reg_tokens`` adds that many register tokens after the cls token (parameter ``reg_token`` [1, R, E], present
+    only when R > 0, initialised ``normal_(std=1e-6)`` as timm does, drawn after every other parameter so the rest of
+    a seeded model is unchanged).  The relative and polynomial biases are defined against a single cls token and
+    raise ``ValueError`` with registers.
     """
 
     def __init__(self, img_size=32, patch_size=4, in_chans=3, num_classes=10,
                  embed_dim=192, depth=6, num_heads=6, mlp_ratio=4.,
                  pos_encoding='absolute', rope_theta=100.0,
-                 poly_degree=3, poly_shared_heads=True, drop_rate=0., drop_path_rate=0.):
+                 poly_degree=3, poly_shared_heads=True, drop_rate=0., drop_path_rate=0., reg_tokens=0):
         super().__init__()
+        if reg_tokens < 0:
+            raise ValueError(f"reg_tokens must be >= 0, got {reg_tokens}")
+        if reg_tokens > 0 and pos_encoding in ('relative', 'polynomial'):
+            raise ValueError(f"reg_tokens > 0 is not supported with pos_encoding={pos_encoding!r}: its attention bias "
+                             "is defined against a single cls token")
         self.num_classes = num_classes
         self.embed_dim = embed_dim
         self.patch_size = patch_size
@@ -173,6 +190,8 @@ class VisionTransformer(nn.Module):
         self.head_dim = embed_dim // num_heads
         self.num_heads = num_heads
         self.num_patches = (img_size // patch_size) ** 2
+        self.num_reg_tokens = reg_tokens
+        self.num_prefix_tokens = 1 + reg_tokens
 
         # parameter holder for the patch projection; the forward pass runs the unfold+GEMM kernel
         self.patch_embed = nn.Conv2d(in_chans, embed_dim, kernel_size=patch_size, stride=patch_size)
@@ -202,10 +221,15 @@ class VisionTransformer(nn.Module):
         if not self.use_pos_embed_in_forward:
             for blk in self.blocks:
                 blk.set_pos_encoding(self.pos_embed)  # one shared module, referenced by every block
+        for blk in self.blocks:
+            blk.attn.num_prefix_tokens = self.num_prefix_tokens
 
         self.norm = nn.LayerNorm(embed_dim)
         self.head = nn.Linear(embed_dim, num_classes)
         self.apply(self._init_weights)
+        if reg_tokens > 0:  # drawn last: every other tensor matches a model built with the same seed and no registers
+            self.reg_token = nn.Parameter(torch.zeros(1, reg_tokens, embed_dim))
+            nn.init.normal_(self.reg_token, std=1e-6)
 
     def _init_weights(self, m):
         """Same initialisers as the reference (vit.py:216-233); PE parameters are left alone."""
@@ -222,7 +246,7 @@ class VisionTransformer(nn.Module):
                 nn.init.constant_(m.bias, 0)
 
     def forward_features(self, x):
-        """[B, C, H, W] -> [B, N, E] with N = (H/P)(W/P) + 1 taken from the input (vit.py:235-271)."""
+        """[B, C, H, W] -> [B, N, E] with N = (H/P)(W/P) + num_prefix_tokens taken from the input (vit.py:235-271)."""
         x, m, drop = self._features(x)
         if m is None:
             return x
@@ -255,8 +279,8 @@ class VisionTransformer(nn.Module):
             ops.refresh_lp_weights(self._gemm_weights(), ops.compute_dtype(x))
         abs_table = self.pos_embed.pos_embed if self.use_pos_embed_in_forward else None
         # (under autocast the token stream comes back fp32, like the reference's cat with the fp32 cls token)
-        x = ops.patch_embed(x, self.patch_embed.weight, self.patch_embed.bias, self.cls_token,
-                            abs_table, self.patch_size)
+        prefix = self.cls_token if self.num_reg_tokens == 0 else torch.cat((self.cls_token, self.reg_token), 1)
+        x = ops.patch_embed(x, self.patch_embed.weight, self.patch_embed.bias, prefix, abs_table, self.patch_size)
 
         freqs_cis = None
         if self.use_rope:

@@ -3,7 +3,7 @@
 Each ``torch.autograd.Function`` here is the product implementation of one stretch of the
 reference's ``Attention.forward`` / ``forward_features`` (citations: /root/reference):
 
-* :class:`PatchEmbedFn`      - models/vit.py:164,248-258 (conv patch embed, cls concat, absolute add)
+* :class:`PatchEmbedFn`      - models/vit.py:164,248-258 (conv patch embed, cls / register concat, absolute add)
 * :class:`QkvRopeFn`         - models/vit.py:47-68 + models/rope_utils.py:22-35
 * :class:`FusedAttentionFn`  - models/vit.py:71-88
 
@@ -115,54 +115,58 @@ class _timed:
 
 # ------------------------------------------------------------------------------------------------
 class PatchEmbedFn(torch.autograd.Function):
-    """tokens[B, Np+1, E] from images: unfold + GEMM + bias (+ absolute pos_embed) + cls row.
+    """tokens[B, P+Np, E] from images: the P prefix rows (cls, then register tokens) + unfold + GEMM + bias
+    (+ absolute pos_embed on the patch rows).
 
-    weight / bias carry the conv dtype; cls_token / pos_embed / tokens the token-stream dtype (fp32
-    under autocast, like the reference's cat with the fp32 cls token); images may stay fp32 when the
-    conv runs in bf16 / fp16 - the rounding is fused into the kernel's load."""
+    weight / bias carry the conv dtype; prefix_tokens ([..., P, E], e.g. the [1, 1, E] cls token) / pos_embed / tokens
+    the token-stream dtype (fp32 under autocast, like the reference's cat with the fp32 cls token); images may stay
+    fp32 when the conv runs in bf16 / fp16 - the rounding is fused into the kernel's load."""
 
     @staticmethod
-    def forward(ctx, images, weight, bias, cls_token, pos_embed, patch):
-        _require_cuda(images, weight, bias, cls_token, pos_embed)
+    def forward(ctx, images, weight, bias, prefix_tokens, pos_embed, patch):
+        _require_cuda(images, weight, bias, prefix_tokens, pos_embed)
         lib = _lib.load()
         B, C, Hi, Wi = images.shape
         E = weight.shape[0]
-        idt, dt, tdt = images.dtype, weight.dtype, cls_token.dtype
+        idt, dt, tdt = images.dtype, weight.dtype, prefix_tokens.dtype
         if bias.dtype != dt or (pos_embed is not None and pos_embed.dtype != tdt):
-            raise TypeError("patch_embed: weight/bias must share a dtype, cls_token/pos_embed another")
+            raise TypeError("patch_embed: weight/bias must share a dtype, prefix_tokens/pos_embed another")
         if idt != dt and not (idt == torch.float32 and dt in _LP16):
             raise TypeError(f"patch_embed: images {idt} with weights {dt} is not supported")
+        if prefix_tokens.numel() == 0 or prefix_tokens.numel() % E or prefix_tokens.shape[-1] != E:
+            raise RuntimeError(f"patch_embed: prefix tokens {tuple(prefix_tokens.shape)} are not [..., n_prefix, {E}]")
         images = images.contiguous()
         w = weight.detach().contiguous()
         b = bias.detach().contiguous()
-        cls = cls_token.detach().reshape(-1).contiguous()
+        prefix = prefix_tokens.detach().reshape(-1, E).contiguous()
+        n_prefix = prefix.shape[0]
         Np = (Hi // patch) * (Wi // patch)
         pos = None
         if pos_embed is not None:
             if pos_embed.shape[-2] < Np:
                 raise RuntimeError(f"absolute pos_embed has {pos_embed.shape[-2]} rows, need {Np}")
             pos = pos_embed.detach().reshape(-1, E).contiguous()
-        tokens = torch.empty(B, Np + 1, E, device=images.device, dtype=tdt)
+        tokens = torch.empty(B, n_prefix + Np, E, device=images.device, dtype=tdt)
         ws_bytes = int(lib.vrr_patch_embed_workspace_bytes(B, C, Hi, Wi, patch, E, _DT[dt]))
         ws = torch.empty(ws_bytes, device=images.device, dtype=torch.uint8) if ws_bytes else None
         with torch.cuda.device(images.device), _timed("patch_embed_fwd"):
-            _lib.check(lib.vrr_patch_embed_fwd(_ptr(images), _ptr(w), _ptr(b), _ptr(cls), _ptr(pos), _ptr(tokens),
-                                               _ptr(ws), ws_bytes, B, C, Hi, Wi, patch, E, _DT[idt], _DT[dt],
-                                               _DT[tdt], _stream()), "vrr_patch_embed_fwd")
+            _lib.check(lib.vrr_patch_embed_fwd_prefix(_ptr(images), _ptr(w), _ptr(b), _ptr(prefix), n_prefix, _ptr(pos),
+                                                      _ptr(tokens), _ptr(ws), ws_bytes, B, C, Hi, Wi, patch, E, _DT[idt],
+                                                      _DT[dt], _DT[tdt], _stream()), "vrr_patch_embed_fwd_prefix")
         if ctx.needs_input_grad[0]:
             ctx.w_for_dimg = w
         # the tcgen05 path's workspace IS unfold(images) [B*Np][C*P*P] in dt: the weight-gradient GEMM reuses it
         ctx.unfolded = ws if (ws is not None and ws_bytes == B * Np * C * patch * patch * 2) else None
         ctx.save_for_backward(images)
-        ctx.meta = (B, C, Hi, Wi, patch, E, Np, pos_embed.shape if pos_embed is not None else None,
-                    weight.shape, cls_token.shape, idt, dt, tdt)
+        ctx.meta = (B, C, Hi, Wi, patch, E, Np, n_prefix, pos_embed.shape if pos_embed is not None else None,
+                    weight.shape, prefix_tokens.shape, idt, dt, tdt)
         return tokens
 
     @staticmethod
     def backward(ctx, d_tokens):
         lib = _lib.load()
         (images,) = ctx.saved_tensors
-        B, C, Hi, Wi, patch, E, Np, pos_shape, w_shape, cls_shape, idt, dt, tdt = ctx.meta
+        B, C, Hi, Wi, patch, E, Np, n_prefix, pos_shape, w_shape, prefix_shape, idt, dt, tdt = ctx.meta
         d_tokens = d_tokens.contiguous()
         dev = images.device
         K = C * patch * patch
@@ -171,12 +175,12 @@ class PatchEmbedFn(torch.autograd.Function):
         own_dw = not (dt in _LP16 and patch % 8 == 0 and Wi % 4 == 0 and E % 8 == 0)
         d_w = torch.empty(E, K, device=dev, dtype=torch.float32) if own_dw else None
         d_b = torch.empty(E, device=dev, dtype=torch.float32)
-        d_cls = torch.empty(E, device=dev, dtype=torch.float32)
+        d_prefix = torch.empty(n_prefix, E, device=dev, dtype=torch.float32)
         d_pos_rows = torch.empty(Np, E, device=dev, dtype=torch.float32) if pos_shape is not None else None
         with torch.cuda.device(dev), _timed("patch_embed_bwd"):
-            _lib.check(lib.vrr_patch_embed_bwd(_ptr(images), _ptr(d_tokens), _ptr(d_w), _ptr(d_b), _ptr(d_cls),
-                                               _ptr(d_pos_rows), B, C, Hi, Wi, patch, E, _DT[idt], _DT[dt], _DT[tdt],
-                                               _stream()), "vrr_patch_embed_bwd")
+            _lib.check(lib.vrr_patch_embed_bwd_prefix(_ptr(images), _ptr(d_tokens), _ptr(d_w), _ptr(d_b), _ptr(d_prefix),
+                                                      n_prefix, _ptr(d_pos_rows), B, C, Hi, Wi, patch, E, _DT[idt], _DT[dt],
+                                                      _DT[tdt], _stream()), "vrr_patch_embed_bwd_prefix")
             if not own_dw:
                 if ctx.unfolded is not None:
                     unf = ctx.unfolded.view(dt).view(B * Np, K)
@@ -185,43 +189,47 @@ class PatchEmbedFn(torch.autograd.Function):
                     _lib.check(lib.vrr_patch_unfold_ex(_ptr(images), _ptr(unf), B, C, Hi, Wi, patch, _DT[idt], _DT[dt],
                                                        _stream()), "vrr_patch_unfold_ex")
                 # cast first: one strided read + packed 16-bit write (reshaping the fp32 slice first copied 154 MB twice)
-                g = d_tokens[:, 1:, :].to(dt).reshape(B * Np, E)
+                g = d_tokens[:, n_prefix:, :].to(dt).reshape(B * Np, E)
                 d_w = _gemm(g, unf, True, False, torch.float32, name="patch_dw")
         d_pos = None
         if pos_shape is not None:
             d_pos = torch.zeros(pos_shape, device=dev, dtype=tdt)
             d_pos.view(-1, E)[:Np] = d_pos_rows.to(tdt)
-        return (None, d_w.view(w_shape).to(dt), d_b.to(dt), d_cls.view(cls_shape).to(tdt), d_pos, None)
+        return (None, d_w.view(w_shape).to(dt), d_b.to(dt), d_prefix.view(prefix_shape).to(tdt), d_pos, None)
 
 
-def patch_embed(images, weight, bias, cls_token, pos_embed, patch):
+def patch_embed(images, weight, bias, prefix_tokens, pos_embed, patch):
     """Conv weights are cast to the compute dtype (autograd-tracked casts keep fp32 master grads);
-    under autocast the token stream (cls, pos, output) stays fp32 as in the reference, and fp32 images
-    are passed as they are (rounded to bf16 / fp16 inside the kernel)."""
+    under autocast the token stream (prefix tokens, pos, output) stays fp32 as in the reference, and fp32 images
+    are passed as they are (rounded to bf16 / fp16 inside the kernel).  ``prefix_tokens``: ``[1, n_prefix, E]``, the
+    cls token followed by the register tokens (``torch.cat((cls_token, reg_token), 1)``); its gradient is the batch
+    sum of the prefix rows' gradients."""
     dt = compute_dtype(images)
     tdt = torch.float32 if torch.is_autocast_enabled("cuda") else dt
     if not (images.dtype == torch.float32 and dt in _LP16):
         images = images.to(dt)
-    return PatchEmbedFn.apply(images, weight.to(dt), bias.to(dt), cls_token.to(tdt),
+    return PatchEmbedFn.apply(images, weight.to(dt), bias.to(dt), prefix_tokens.to(tdt),
                               None if pos_embed is None else pos_embed.to(tdt), patch)
 
 
 # ------------------------------------------------------------------------------------------------
-def _rope_args(cos, sin, H, N, Dh):
-    """Classify the (cos, sin) pair the way ``reshape_for_broadcast`` does (rope_utils.py:39-66)."""
+def _rope_args(cos, sin, H, N, Dh, n_prefix=1):
+    """Classify the (cos, sin) pair the way ``reshape_for_broadcast`` does (rope_utils.py:39-66).  The tables cover
+    the N - n_prefix patch tokens; the prefix tokens (cls, registers) are not rotated."""
     if cos is None:
         return _lib.ROPE_NONE
     if cos.shape != sin.shape:
         raise RuntimeError(f"cos {tuple(cos.shape)} and sin {tuple(sin.shape)} differ")
+    rows = N - n_prefix
     if cos.ndim == 2:
-        mode, want = _lib.ROPE_AXIAL, (N - 1, Dh // 2)
+        mode, want = _lib.ROPE_AXIAL, (rows, Dh // 2)
     elif cos.ndim == 3:
-        mode, want = _lib.ROPE_MIXED, (H, N - 1, Dh // 2)
+        mode, want = _lib.ROPE_MIXED, (H, rows, Dh // 2)
     else:
-        raise ValueError(f"Unexpected tensor shapes: {cos.shape} vs {(1, H, N - 1, Dh)}")
+        raise ValueError(f"Unexpected tensor shapes: {cos.shape} vs {(1, H, rows, Dh)}")
     if tuple(cos.shape) != want:
         raise RuntimeError(f"RoPE table shape {tuple(cos.shape)} does not broadcast against the "
-                           f"{N - 1} patch tokens x {H} heads x {Dh} channels (expected {want})")
+                           f"{rows} patch tokens x {H} heads x {Dh} channels (expected {want})")
     return mode
 
 
@@ -252,17 +260,18 @@ def _packed_tables(cos32, sin32):
 
 
 class QkvRopeFn(torch.autograd.Function):
-    """planes[3, B, H, N, Dh] = split_heads(x @ w_qkv^T), q/k rows 1.. rotated in the GEMM epilogue."""
+    """planes[3, B, H, N, Dh] = split_heads(x @ w_qkv^T), q/k rows n_prefix.. rotated in the GEMM epilogue."""
 
     @staticmethod
-    def forward(ctx, x, w_qkv, cos, sin, num_heads, w_lp=None):
+    def forward(ctx, x, w_qkv, cos, sin, num_heads, w_lp=None, n_prefix=1):
         """``w_qkv`` receives the gradient (fp32 master weight or a tensor already in x's dtype); ``w_lp`` is an
-        optional ready-made copy of it in x's dtype (the model's 16-bit weight cache)."""
+        optional ready-made copy of it in x's dtype (the model's 16-bit weight cache).  ``n_prefix``: the leading
+        token rows that are never rotated (cls and register tokens); row t >= n_prefix uses table row t - n_prefix."""
         _require_cuda(x, w_qkv, cos, sin)
         lib = _lib.load()
         B, N, E = x.shape
         H, Dh = num_heads, E // num_heads
-        mode = _rope_args(cos, sin, H, N, Dh)
+        mode = _rope_args(cos, sin, H, N, Dh, n_prefix)
         x = x.contiguous()
         w = (w_lp if w_lp is not None else w_qkv.detach().to(x.dtype)).detach().contiguous()
         ctx.w_grad_dtype = w_qkv.dtype
@@ -273,17 +282,18 @@ class QkvRopeFn(torch.autograd.Function):
             if mode != _lib.ROPE_NONE and x.dtype in _LP16 and Dh == 64:  # the tcgen05 epilogue's table layout
                 packed = _packed_tables(cos32, sin32)
             with _timed("qkv_rope_fwd"):
-                _lib.check(lib.vrr_qkv_rope_fwd_packed(_ptr(x), _ptr(w), _ptr(cos32), _ptr(sin32), _ptr(packed), _ptr(planes),
-                                                       B, N, E, H, mode, _DT[x.dtype], _stream()), "vrr_qkv_rope_fwd_packed")
+                _lib.check(lib.vrr_qkv_rope_fwd_prefix(_ptr(x), _ptr(w), _ptr(cos32), _ptr(sin32), _ptr(packed), _ptr(planes),
+                                                       B, N, E, H, n_prefix, mode, _DT[x.dtype], _stream()),
+                           "vrr_qkv_rope_fwd_prefix")
         ctx.save_for_backward(x, w, planes, cos32, sin32)
-        ctx.meta = (B, N, E, H, mode, None if cos is None else (cos.dtype, sin.dtype))
+        ctx.meta = (B, N, E, H, n_prefix, mode, None if cos is None else (cos.dtype, sin.dtype))
         return planes
 
     @staticmethod
     def backward(ctx, d_planes):
         lib = _lib.load()
         x, w, planes, cos32, sin32 = ctx.saved_tensors
-        B, N, E, H, mode, cs_dtypes = ctx.meta
+        B, N, E, H, n_prefix, mode, cs_dtypes = ctx.meta
         d_planes = d_planes.contiguous()
         dev, dt = x.device, x.dtype
         need_cs = mode != _lib.ROPE_NONE and (ctx.needs_input_grad[2] or ctx.needs_input_grad[3])
@@ -293,9 +303,9 @@ class QkvRopeFn(torch.autograd.Function):
             d_cos, d_sin = d_cs[0], d_cs[1]
         d_qkv = torch.empty(B * N, 3 * E, device=dev, dtype=dt)
         with torch.cuda.device(dev):
-            _lib.check(lib.vrr_qkv_rope_bwd(_ptr(d_planes), _ptr(planes), _ptr(cos32), _ptr(sin32), _ptr(d_qkv),
-                                            _ptr(d_cos), _ptr(d_sin), B, N, E, H, mode, _DT[dt], _stream()),
-                       "vrr_qkv_rope_bwd")
+            _lib.check(lib.vrr_qkv_rope_bwd_prefix(_ptr(d_planes), _ptr(planes), _ptr(cos32), _ptr(sin32), _ptr(d_qkv),
+                                                   _ptr(d_cos), _ptr(d_sin), B, N, E, H, n_prefix, mode, _DT[dt], _stream()),
+                       "vrr_qkv_rope_bwd_prefix")
             dx = dw = None
             if ctx.needs_input_grad[0]:
                 dx = _gemm(d_qkv, w, False, False, dt, name="qkv_dx").view(B, N, E)            # [BN,3E] . [3E,E]
@@ -303,7 +313,7 @@ class QkvRopeFn(torch.autograd.Function):
                 dw = _gemm(d_qkv, x.view(B * N, E), True, False, ctx.w_grad_dtype, name="qkv_dw")  # [3E,BN] . [BN,E]
         if need_cs:
             d_cos, d_sin = d_cos.to(cs_dtypes[0]), d_sin.to(cs_dtypes[1])
-        return dx, dw, d_cos, d_sin, None, None
+        return dx, dw, d_cos, d_sin, None, None, None
 
 
 def _gemm(a, b, trans_a, trans_b, out_dtype, bias=None, epilogue=_lib.EPI_NONE, out2=False, name="gemm", aux=None,
@@ -336,11 +346,12 @@ def _gemm(a, b, trans_a, trans_b, out_dtype, bias=None, epilogue=_lib.EPI_NONE, 
     return (c, c2) if out2 else c
 
 
-def qkv_rope(x, w_qkv, cos, sin, num_heads, w_lp=None):
+def qkv_rope(x, w_qkv, cos, sin, num_heads, w_lp=None, n_prefix=1):
+    """``n_prefix``: the leading token rows that RoPE leaves alone (the cls token and any register tokens)."""
     dt = compute_dtype(x)
     if w_lp is not None and w_lp.dtype != dt:
         w_lp = None
-    return QkvRopeFn.apply(x.to(dt), w_qkv, cos, sin, num_heads, w_lp)
+    return QkvRopeFn.apply(x.to(dt), w_qkv, cos, sin, num_heads, w_lp, n_prefix)
 
 
 # ------------------------------------------------------------------------------------------------
