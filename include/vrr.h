@@ -314,6 +314,29 @@ int vrr_add_layernorm_drop_bwd(const void* dy, const void* d_xnew, const void* x
                                float* dbeta, int M, int E, int branch_dtype, int y_dtype,
                                const vrr_drop_desc* drop, void* stream);
 
+/* The same with LayerScale on the branch (timm's LayerScale, Block(init_values): x = x + drop_path(ls * branch)).
+ * ls fp32 [E].  f is the factor of `drop` as above; without a desc (drop NULL) no f product is taken.  Every product
+ * is rounded to fp32 and never contracted into the add:
+ *   forward : b' = fl(fl(f * branch) * ls[c]); x_new = x + b'; y = LayerNorm(x_new).  x_new, y, mean and rstd are
+ *             bit-identical to vrr_add_layernorm_fwd fed the fp32 branch b'.  Without dropout b' = fl(branch * ls),
+ *             torch's product of a 16-bit tensor and an fp32 parameter;
+ *   backward: dx as vrr_add_layernorm_bwd; d_branch = round_to_branch_dtype(fl(fl(dx * f) * ls[c]));
+ *             d_ls[c] = sum_m fl(dx * f)[m][c] * float(branch[m][c]), an fp32 column sum (written, not accumulated;
+ *             like dgamma / dbeta its summation order is not fixed).  `branch` is the forward's branch input
+ *             (`branch_dtype`); it is read only when d_ls is not NULL.
+ * d_ls non-NULL needs ls and branch (VRR_ERR_INVALID_ARG otherwise).  ls NULL is exactly the _drop_ entry points
+ * (branch and d_ls are then not used).  With ls the backward keeps a third [warps][E] partial in shared memory:
+ * E <= 1706 (VRR_ERR_UNSUPPORTED beyond). */
+int vrr_add_layernorm_ls_fwd(const void* x, const void* branch, void* x_new, const float* gamma,
+                             const float* beta, void* y, float* mean, float* rstd, int M, int E, float eps,
+                             int branch_dtype, int y_dtype, const vrr_drop_desc* drop, const float* ls,
+                             void* stream);
+int vrr_add_layernorm_ls_bwd(const void* dy, const void* d_xnew, const void* x_new, const float* gamma,
+                             const float* mean, const float* rstd, void* dx, void* d_branch, float* dgamma,
+                             float* dbeta, int M, int E, int branch_dtype, int y_dtype,
+                             const vrr_drop_desc* drop, const float* ls, const void* branch, float* d_ls,
+                             void* stream);
+
 /* vrr_gemm_ex with element dropout on the GELU outputs (fc1 of an Mlp with drop1 > 0), for the epilogues
  * VRR_EPI_BIAS_GELU_GRAD (C = T(T(gelu(h)) * f), C2 = T(T(gelu'(h)) * f)) and VRR_EPI_BIAS_GELU_ACT
  * (C = T(T(gelu(h)) * f)), T = `dtype`; `drop->p_path` must be 0.  The mask is indexed by (m, n) of C (N % 8 == 0).

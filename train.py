@@ -17,6 +17,7 @@ Additions (all off by default, so a reference command line behaves like the refe
   --drop_rate P      dropout on every block's attention projection and Mlp (timm's drop_rate)
   --drop_path_rate P stochastic depth, linearly from 0 at the first block to P at the last (timm's drop_path_rate)
   --reg_tokens R     R register tokens after the cls token (timm's reg_tokens; not with relative / polynomial)
+  --init_values V    LayerScale in every block, gamma initialised to V (timm's init_values, e.g. 1e-5 as in DeiT III)
 There is no CPU path: a CUDA sm_100 device is required.
 """
 import argparse
@@ -68,6 +69,7 @@ def get_args(argv=None):
     p.add_argument("--drop_path_rate", type=float, default=0.0,
                    help="stochastic depth of the last block (linearly from 0 over the depth, timm's rule)")
     p.add_argument("--reg_tokens", type=int, default=0, help="register tokens after the cls token")
+    p.add_argument("--init_values", type=float, default=None, help="LayerScale initial value (default: no LayerScale)")
     return p.parse_args(argv)
 
 
@@ -160,7 +162,8 @@ def main(argv=None):
                               embed_dim=args.embed_dim, depth=args.depth, num_heads=args.num_heads,
                               pos_encoding=args.pos_encoding, rope_theta=args.rope_theta, poly_degree=args.poly_degree,
                               poly_shared_heads=args.poly_shared_heads, drop_rate=args.drop_rate,
-                              drop_path_rate=args.drop_path_rate, reg_tokens=args.reg_tokens).to(device)
+                              drop_path_rate=args.drop_path_rate, reg_tokens=args.reg_tokens,
+                              init_values=args.init_values).to(device)
     criterion = nn.CrossEntropyLoss()
     optimizer = torch.optim.AdamW(model.parameters(), lr=args.lr, weight_decay=args.weight_decay)
     scheduler = torch.optim.lr_scheduler.CosineAnnealingLR(optimizer, T_max=args.epochs)

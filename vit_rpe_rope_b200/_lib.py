@@ -71,6 +71,9 @@ SIGNATURES = {
     "vrr_add_layernorm_drop_fwd": (c_int, [c_void_p] * 8 + [c_int, c_int, c_float, c_int, c_int, POINTER(DropDesc),
                                                            c_void_p]),
     "vrr_add_layernorm_drop_bwd": (c_int, [c_void_p] * 10 + [c_int] * 4 + [POINTER(DropDesc), c_void_p]),
+    "vrr_add_layernorm_ls_fwd": (c_int, [c_void_p] * 8 + [c_int, c_int, c_float, c_int, c_int, POINTER(DropDesc),
+                                                         c_void_p, c_void_p]),
+    "vrr_add_layernorm_ls_bwd": (c_int, [c_void_p] * 10 + [c_int] * 4 + [POINTER(DropDesc)] + [c_void_p] * 4),
     "vrr_gemm_ex_drop": (c_int, [c_void_p] * 5 + [c_int] * 9 + [POINTER(DropDesc), c_void_p]),
     "vrr_dropout_mask": (c_int, [POINTER(DropDesc), c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "vrr_colsum": (c_int, [c_void_p] * 2 + [c_int] * 3 + [c_void_p]),

@@ -90,13 +90,15 @@ int layernorm_fwd(const void* x, const float* gamma, const float* beta, void* y,
 int layernorm_bwd(const void* dy, const void* x, const float* gamma, const float* mean, const float* rstd, void* dx,
                   float* dgamma, float* dbeta, int M, int E, int x_dtype, int y_dtype, cudaStream_t st);
 
-// drop: NULL or a desc that draws nothing runs the plain kernels
+// drop: NULL or a desc that draws nothing runs the plain kernels; ls: NULL runs the kernels without LayerScale
+// (branch and d_ls are then ignored); d_ls NULL: no LayerScale gradient (branch is not read)
 int add_layernorm_fwd(const void* x, const void* branch, void* x_new, const float* gamma, const float* beta, void* y,
                       float* mean, float* rstd, int M, int E, float eps, int branch_dtype, int y_dtype,
-                      const vrr_drop_desc* drop, cudaStream_t st);
+                      const vrr_drop_desc* drop, const float* ls, cudaStream_t st);
 int add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new, const float* gamma, const float* mean,
                       const float* rstd, void* dx, void* d_branch, float* dgamma, float* dbeta, int M, int E,
-                      int branch_dtype, int y_dtype, const vrr_drop_desc* drop, cudaStream_t st);
+                      int branch_dtype, int y_dtype, const vrr_drop_desc* drop, const float* ls, const void* branch,
+                      float* d_ls, cudaStream_t st);
 
 // elementwise.cu
 int colsum(const void* x, float* out, int M, int C, int dtype, cudaStream_t st);

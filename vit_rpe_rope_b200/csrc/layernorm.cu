@@ -23,9 +23,9 @@ constexpr int kLnWarps = 8;
 static int g_ln_bwd_minb = 3;  // register-resident add_ln_bwd at E >= 768: 3 = 12 warps x 1 CTA/SM (E = 768), 1 = 8 x 1, 2 = 8 x 2 (spills)
 static int g_ln_reg = 1;       // 0: generic multi-pass kernels only (option "ln_reg")
 
-// resident CTAs per SM the backward's shared-memory partials allow (2 x warps x E floats per CTA)
-static inline int ln_bwd_ctas_per_sm(int E) {
-  const size_t per_cta = (size_t)2 * kLnWarps * E * sizeof(float) + 1024;
+// resident CTAs per SM the backward's shared-memory partials allow (`rows` x warps x E floats per CTA)
+static inline int ln_bwd_ctas_per_sm(int E, int rows = 2) {
+  const size_t per_cta = (size_t)rows * kLnWarps * E * sizeof(float) + 1024;
   int n = (int)((200 * 1024) / per_cta);
   return n < 1 ? 1 : (n > 6 ? 6 : n);
 }
@@ -230,11 +230,15 @@ int ln_bwd_t(const void* dy, const void* x, const float* gamma, const float* mea
 // backward: dx = d_xnew + LN'(dy) written as fp32 (gradient of the residual input) AND in the branch's
 //           dtype (gradient of the branch: the same values) - the autograd add and the cast disappear.
 // DROP != 0: the branch is multiplied by its dropout / stochastic-depth factor f (DropView) as it is read, in every pass.
-template <typename TB, typename TY, int VEC, int DROP>
-__global__ void __launch_bounds__(kLnWarps * 32)
+// LS: then by the LayerScale vector ls[E], b' = fl(fl(f * branch) * ls[c]) (each product rounded, never contracted).
+// The LS kernels declare one resident CTA per SM as the minimum (a minimum of 0 is no declaration, today's kernels):
+// without it ptxas aims at a lower register count and spills a few bytes in some of them.
+template <typename TB, typename TY, int VEC, int DROP, bool LS>
+__global__ void __launch_bounds__(kLnWarps * 32, LS ? 1 : 0)
 add_ln_fwd_kernel(const float* __restrict__ x, const TB* __restrict__ branch, float* __restrict__ x_new,
                   const float* __restrict__ gamma, const float* __restrict__ beta, TY* __restrict__ y,
-                  float* __restrict__ mean_out, float* __restrict__ rstd_out, int M, int E, float eps, const DropView dv) {
+                  float* __restrict__ mean_out, float* __restrict__ rstd_out, int M, int E, float eps, const DropView dv,
+                  const float* __restrict__ ls) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const float inv_e = 1.f / (float)E;
   [[maybe_unused]] uint2 key;
@@ -249,11 +253,13 @@ add_ln_fwd_kernel(const float* __restrict__ x, const TB* __restrict__ branch, fl
     auto ldb4 = [&](int c) {
       float4 b = ld4(br + c);
       if constexpr (DROP) b = mul4_rn(b, drop_f4<DROP>(dv, key, row, c, E, fr));
+      if constexpr (LS) b = mul4_rn(b, ld4(ls + c));
       return b;
     };
     auto ldb1 = [&](int c) {
       float b = Elem<TB>::ld(br + c);
       if constexpr (DROP) b = __fmul_rn(b, drop_f1<DROP>(dv, key, row, c, E, fr));
+      if constexpr (LS) b = __fmul_rn(b, ls[c]);
       return b;
     };
     float s = 0.f;
@@ -308,19 +314,23 @@ add_ln_fwd_kernel(const float* __restrict__ x, const TB* __restrict__ branch, fl
 }
 
 // DROP != 0: d_branch = dx * f (the factor of the forward, regenerated)
-template <typename TB, typename TY, int VEC, int DROP>
+// LS: d_branch = fl(fl(dx * f) * ls[c]); with d_ls, d_ls[c] = sum_rows fl(dx * f) * branch (a third [warps][E] partial)
+template <typename TB, typename TY, int VEC, int DROP, bool LS>
 __global__ void __launch_bounds__(kLnWarps * 32)
 add_ln_bwd_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, const float* __restrict__ x_new,
                   const float* __restrict__ gamma, const float* __restrict__ mean_in,
                   const float* __restrict__ rstd_in, float* __restrict__ dx, TB* __restrict__ d_branch,
-                  float* __restrict__ dgamma, float* __restrict__ dbeta, int M, int E, const DropView dv) {
+                  float* __restrict__ dgamma, float* __restrict__ dbeta, int M, int E, const DropView dv,
+                  const float* __restrict__ ls, const TB* __restrict__ branch, float* __restrict__ d_ls) {
   extern __shared__ __align__(16) float ln_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   float* pg = ln_smem + (size_t)warp * E;
   float* pb = ln_smem + (size_t)(kLnWarps + warp) * E;
+  [[maybe_unused]] float* pl = ln_smem + (size_t)(2 * kLnWarps + warp) * E;  // LS: this warp's d_ls partial
   for (int c = lane; c < E; c += 32) {
     pg[c] = 0.f;
     pb[c] = 0.f;
+    if constexpr (LS) pl[c] = 0.f;
   }
   __syncwarp();
   const float inv_e = 1.f / (float)E;
@@ -334,6 +344,7 @@ add_ln_bwd_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, c
     if constexpr (DROP) fr = dv.row_factor(key, row);
     float* dr = dx + (size_t)row * E;
     TB* br = d_branch + (size_t)row * E;
+    [[maybe_unused]] const TB* xb = LS && d_ls ? branch + (size_t)row * E : nullptr;
     const float mean = mean_in[row], rstd = rstd_in[row];
     float s1 = 0.f, s2 = 0.f;
     if (VEC == 4) {
@@ -372,8 +383,19 @@ add_ln_bwd_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, c
         }
         const float4 ov = make_float4(o[0], o[1], o[2], o[3]);
         st4(dr + c, ov);
-        if constexpr (DROP) st4(br + c, mul4_rn(ov, drop_f4<DROP>(dv, key, row, c, E, fr)));
-        else st4(br + c, ov);
+        float4 t = ov;
+        if constexpr (DROP) t = mul4_rn(ov, drop_f4<DROP>(dv, key, row, c, E, fr));
+        if constexpr (LS) {
+          st4(br + c, mul4_rn(t, ld4(ls + c)));
+          if (xb) {
+            const float4 bv = ld4(xb + c);
+            float4 al = *reinterpret_cast<float4*>(pl + c);
+            al = make_float4(fmaf(t.x, bv.x, al.x), fmaf(t.y, bv.y, al.y), fmaf(t.z, bv.z, al.z), fmaf(t.w, bv.w, al.w));
+            *reinterpret_cast<float4*>(pl + c) = al;
+          }
+        } else {
+          st4(br + c, t);
+        }
         *reinterpret_cast<float4*>(pg + c) = make_float4(agv[0], agv[1], agv[2], agv[3]);
         *reinterpret_cast<float4*>(pb + c) = make_float4(abv[0], abv[1], abv[2], abv[3]);
       }
@@ -382,8 +404,14 @@ add_ln_bwd_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, c
         const float g = Elem<TY>::ld(gr + c), xh = (xr[c] - mean) * rstd;
         const float o = (rr ? rr[c] : 0.f) + rstd * (g * gamma[c] - c1 - xh * c2);
         dr[c] = o;
-        if constexpr (DROP) Elem<TB>::st(br + c, __fmul_rn(o, drop_f1<DROP>(dv, key, row, c, E, fr)));
-        else Elem<TB>::st(br + c, o);
+        float t = o;
+        if constexpr (DROP) t = __fmul_rn(o, drop_f1<DROP>(dv, key, row, c, E, fr));
+        if constexpr (LS) {
+          Elem<TB>::st(br + c, __fmul_rn(t, ls[c]));
+          if (xb) pl[c] = fmaf(t, Elem<TB>::ld(xb + c), pl[c]);
+        } else {
+          Elem<TB>::st(br + c, t);
+        }
         pg[c] = fmaf(g, xh, pg[c]);
         pb[c] += g;
       }
@@ -399,6 +427,14 @@ add_ln_bwd_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, c
     }
     atomicAdd(dgamma + c, sg);
     atomicAdd(dbeta + c, sb);
+    if constexpr (LS) {
+      if (d_ls) {
+        float sl = 0.f;
+#pragma unroll
+        for (int w = 0; w < kLnWarps; ++w) sl += ln_smem[(size_t)(2 * kLnWarps + w) * E + c];
+        atomicAdd(d_ls + c, sl);
+      }
+    }
   }
 }
 
@@ -409,19 +445,22 @@ add_ln_bwd_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, c
 // passes and its slice of the dgamma / dbeta partial sums in registers across ROWS (a lane owns the same columns
 // for every row), touching shared memory once per CTA for the cross-warp reduction.  Same operation order per
 // element as the generic kernels, so the results are bit-identical to them.
-template <typename TB, typename TY, int NV, int DROP>
-__global__ void __launch_bounds__(kLnWarps * 32)
+template <typename TB, typename TY, int NV, int DROP, bool LS>
+__global__ void __launch_bounds__(kLnWarps * 32, LS ? 1 : 0)  // see add_ln_fwd_kernel
 add_ln_fwd_reg_kernel(const float* __restrict__ x, const TB* __restrict__ branch, float* __restrict__ x_new,
                       const float* __restrict__ gamma, const float* __restrict__ beta, TY* __restrict__ y,
-                      float* __restrict__ mean_out, float* __restrict__ rstd_out, int M, float eps, const DropView dv) {
+                      float* __restrict__ mean_out, float* __restrict__ rstd_out, int M, float eps, const DropView dv,
+                      const float* __restrict__ ls) {
   constexpr int E = NV * 128;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const float inv_e = 1.f / (float)E;
   float4 g[NV], bt[NV];
+  [[maybe_unused]] float4 lsv[LS ? NV : 1];
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
     g[i] = ld4(gamma + lane * 4 + i * 128);
     bt[i] = ld4(beta + lane * 4 + i * 128);
+    if constexpr (LS) lsv[i] = ld4(ls + lane * 4 + i * 128);
   }
   [[maybe_unused]] uint2 key;
   if constexpr (DROP) key = dv.key();
@@ -439,6 +478,7 @@ add_ln_fwd_reg_kernel(const float* __restrict__ x, const TB* __restrict__ branch
       const float4 a = ld4(xr + i * 128);
       float4 b = ld4(br + i * 128);
       if constexpr (DROP) b = mul4_rn(b, drop_f4<DROP>(dv, key, row, lane * 4 + i * 128, E, fr));
+      if constexpr (LS) b = mul4_rn(b, lsv[i]);
       v[i] = make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);
     }
 #pragma unroll
@@ -470,19 +510,27 @@ add_ln_fwd_reg_kernel(const float* __restrict__ x, const TB* __restrict__ branch
   }
 }
 
-template <typename TB, typename TY, int NV, int WARPS, int MINB, int DROP>
+// LS: the d_ls partial of a lane's columns accumulates in that lane's slots of the third [WARPS][E] shared row (no
+// synchronisation: a lane owns the same columns for every row) - in registers it would not fit next to pg / pb at NV 8.
+template <typename TB, typename TY, int NV, int WARPS, int MINB, int DROP, bool LS>
 __global__ void __launch_bounds__(WARPS * 32, MINB)
 add_ln_bwd_reg_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xnew, const float* __restrict__ x_new,
                       const float* __restrict__ gamma, const float* __restrict__ mean_in, const float* __restrict__ rstd_in,
                       float* __restrict__ dx, TB* __restrict__ d_branch, float* __restrict__ dgamma,
-                      float* __restrict__ dbeta, int M, const DropView dv) {
+                      float* __restrict__ dbeta, int M, const DropView dv, const float* __restrict__ ls,
+                      const TB* __restrict__ branch, float* __restrict__ d_ls) {
   constexpr int E = NV * 128;
-  extern __shared__ __align__(16) float ln_smem[];  // [2][WARPS][E], used once at the end
+  extern __shared__ __align__(16) float ln_smem[];  // [2 (+1 LS)][WARPS][E]; pg / pb used once at the end
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const float inv_e = 1.f / (float)E;
   float4 pg[NV], pb[NV];
 #pragma unroll
   for (int i = 0; i < NV; ++i) pg[i] = pb[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+  [[maybe_unused]] float* pl = ln_smem + (size_t)(2 * WARPS + warp) * E + lane * 4;
+  if constexpr (LS) {
+#pragma unroll
+    for (int i = 0; i < NV; ++i) *reinterpret_cast<float4*>(pl + i * 128) = make_float4(0.f, 0.f, 0.f, 0.f);
+  }
   [[maybe_unused]] uint2 key;
   if constexpr (DROP) key = dv.key();
   for (int row = blockIdx.x * WARPS + warp; row < M; row += gridDim.x * WARPS) {
@@ -491,6 +539,7 @@ add_ln_bwd_reg_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xne
     const float* rr = d_xnew ? d_xnew + (size_t)row * E + lane * 4 : nullptr;
     float* dr = dx + (size_t)row * E + lane * 4;
     TB* br = d_branch + (size_t)row * E + lane * 4;
+    [[maybe_unused]] const TB* xb = LS && d_ls ? branch + (size_t)row * E + lane * 4 : nullptr;
     const float mean = mean_in[row], rstd = rstd_in[row];
     float4 g[NV], xh[NV];
 #pragma unroll
@@ -534,7 +583,22 @@ add_ln_bwd_reg_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xne
       o.z = r.z + rstd * (g[i].z * w.z - c1 - xh[i].z * c2);
       o.w = r.w + rstd * (g[i].w * w.w - c1 - xh[i].w * c2);
       st4(dr + i * 128, o);
-      if constexpr (DROP == 1) {
+      if constexpr (LS) {
+        float4 t = o;
+        if constexpr (DROP == 1) {
+          t = mul4_rn(o, make_float4(fr, fr, fr, fr));
+        } else if constexpr (DROP == 2) {
+          const uint32_t b4 = kb >> (4 * i);
+          t = mul4_rn(o, make_float4(b4 & 1u ? fr : 0.f, b4 & 2u ? fr : 0.f, b4 & 4u ? fr : 0.f, b4 & 8u ? fr : 0.f));
+        }
+        st4(br + i * 128, mul4_rn(t, __ldg(reinterpret_cast<const float4*>(ls + lane * 4 + i * 128))));
+        if (xb) {
+          const float4 bv = ld4(xb + i * 128);
+          float4 al = *reinterpret_cast<float4*>(pl + i * 128);
+          al = make_float4(fmaf(t.x, bv.x, al.x), fmaf(t.y, bv.y, al.y), fmaf(t.z, bv.z, al.z), fmaf(t.w, bv.w, al.w));
+          *reinterpret_cast<float4*>(pl + i * 128) = al;
+        }
+      } else if constexpr (DROP == 1) {
         st4(br + i * 128, mul4_rn(o, make_float4(fr, fr, fr, fr)));
       } else if constexpr (DROP == 2) {
         const uint32_t b4 = kb >> (4 * i);
@@ -567,63 +631,84 @@ add_ln_bwd_reg_kernel(const TY* __restrict__ dy, const float* __restrict__ d_xne
     }
     atomicAdd(dgamma + c, sg);
     atomicAdd(dbeta + c, sb);
+    if constexpr (LS) {
+      if (d_ls) {
+        float sl = 0.f;
+#pragma unroll
+        for (int w = 0; w < WARPS; ++w) sl += ln_smem[(size_t)(2 * WARPS + w) * E + c];
+        atomicAdd(d_ls + c, sl);
+      }
+    }
   }
 }
 
-template <typename TB, typename TY, int DROP>
+template <typename TB, typename TY, int DROP, bool LS>
 int add_ln_fwd_t(const float* x, const void* branch, float* x_new, const float* gamma, const float* beta, void* y,
-                 float* mean, float* rstd, int M, int E, float eps, const DropView& dv, cudaStream_t st) {
+                 float* mean, float* rstd, int M, int E, float eps, const DropView& dv, const float* ls, cudaStream_t st) {
   const int grid = min(ceil_div(M, kLnWarps), 8 * sm_count());
 #define VRR_LN_REG(NV)                                                                                                \
   if (g_ln_reg && E == NV * 128) { \
     const int g2 = min(ceil_div(M, kLnWarps), 4 * sm_count());                                                        \
-    add_ln_fwd_reg_kernel<TB, TY, NV, DROP><<<g2, kLnWarps * 32, 0, st>>>(x, (const TB*)branch, x_new, gamma, beta,  \
-                                                                          (TY*)y, mean, rstd, M, eps, dv);            \
+    add_ln_fwd_reg_kernel<TB, TY, NV, DROP, LS><<<g2, kLnWarps * 32, 0, st>>>(x, (const TB*)branch, x_new, gamma,     \
+                                                                              beta, (TY*)y, mean, rstd, M, eps, dv, ls); \
     VRR_LAUNCHED();                                                                                                   \
     return VRR_OK;                                                                                                    \
   }
   VRR_LN_REG(6) VRR_LN_REG(8) VRR_LN_REG(4) VRR_LN_REG(2)
 #undef VRR_LN_REG
   if (E % 128 == 0)
-    add_ln_fwd_kernel<TB, TY, 4, DROP><<<grid, kLnWarps * 32, 0, st>>>(x, (const TB*)branch, x_new, gamma, beta, (TY*)y, mean, rstd, M, E, eps, dv);
+    add_ln_fwd_kernel<TB, TY, 4, DROP, LS><<<grid, kLnWarps * 32, 0, st>>>(x, (const TB*)branch, x_new, gamma, beta, (TY*)y, mean, rstd, M, E, eps, dv, ls);
   else
-    add_ln_fwd_kernel<TB, TY, 1, DROP><<<grid, kLnWarps * 32, 0, st>>>(x, (const TB*)branch, x_new, gamma, beta, (TY*)y, mean, rstd, M, E, eps, dv);
+    add_ln_fwd_kernel<TB, TY, 1, DROP, LS><<<grid, kLnWarps * 32, 0, st>>>(x, (const TB*)branch, x_new, gamma, beta, (TY*)y, mean, rstd, M, E, eps, dv, ls);
   VRR_LAUNCHED();
   return VRR_OK;
 }
 
-template <typename TB, typename TY, int VEC, int DROP>
+template <typename TB, typename TY, int VEC, int DROP, bool LS>
 int add_ln_bwd_launch(const void* dy, const float* d_xnew, const float* x_new, const float* gamma, const float* mean,
                       const float* rstd, float* dx, void* d_branch, float* dgamma, float* dbeta, int M, int E,
-                      const DropView& dv, cudaStream_t st) {
-  const size_t smem = (size_t)2 * kLnWarps * E * sizeof(float);
-  auto kern = add_ln_bwd_kernel<TB, TY, VEC, DROP>;
+                      const DropView& dv, const float* ls, const void* branch, float* d_ls, cudaStream_t st) {
+  const size_t smem = (size_t)(LS ? 3 : 2) * kLnWarps * E * sizeof(float);
+  auto kern = add_ln_bwd_kernel<TB, TY, VEC, DROP, LS>;
   VRR_SMEM_ATTR_ONCE(kern, 160 * 1024);
-  const int grid = min(ceil_div(M, kLnWarps), ln_bwd_ctas_per_sm(E) * sm_count());
-  kern<<<grid, kLnWarps * 32, smem, st>>>((const TY*)dy, d_xnew, x_new, gamma, mean, rstd, dx, (TB*)d_branch, dgamma, dbeta, M, E, dv);
+  const int grid = min(ceil_div(M, kLnWarps), ln_bwd_ctas_per_sm(E, LS ? 3 : 2) * sm_count());
+  kern<<<grid, kLnWarps * 32, smem, st>>>((const TY*)dy, d_xnew, x_new, gamma, mean, rstd, dx, (TB*)d_branch, dgamma, dbeta, M, E, dv,
+                                          ls, (const TB*)branch, d_ls);
   VRR_LAUNCHED();
   return VRR_OK;
 }
 
-template <typename TB, typename TY, int DROP>
+template <typename TB, typename TY, int DROP, bool LS>
 int add_ln_bwd_t(const void* dy, const float* d_xnew, const float* x_new, const float* gamma, const float* mean,
                  const float* rstd, float* dx, void* d_branch, float* dgamma, float* dbeta, int M, int E,
-                 const DropView& dv, cudaStream_t st) {
-  if (dbeta == dgamma + E) {  // the two rows of one [2][E] buffer (what ops.py allocates): one memset node instead of two
-    VRR_CUDA(cudaMemsetAsync(dgamma, 0, (size_t)2 * E * sizeof(float), st));
+                 const DropView& dv, const float* ls, const void* branch, float* d_ls, cudaStream_t st) {
+  // the rows of one [2][E] (or, with d_ls, [3][E]) buffer (what ops.py allocates): one memset node
+  const bool three = d_ls && dbeta == dgamma + E && d_ls == dgamma + 2 * E;
+  if (dbeta == dgamma + E) {
+    VRR_CUDA(cudaMemsetAsync(dgamma, 0, (size_t)(three ? 3 : 2) * E * sizeof(float), st));
   } else {
     VRR_CUDA(cudaMemsetAsync(dgamma, 0, (size_t)E * sizeof(float), st));
     VRR_CUDA(cudaMemsetAsync(dbeta, 0, (size_t)E * sizeof(float), st));
   }
+  if (d_ls && !three) VRR_CUDA(cudaMemsetAsync(d_ls, 0, (size_t)E * sizeof(float), st));
 #define VRR_LN_BWD_GO(NV, W, B)                                                                                          \
-  auto kern = add_ln_bwd_reg_kernel<TB, TY, NV, W, B, DROP>;                                                           \
+  auto kern = add_ln_bwd_reg_kernel<TB, TY, NV, W, B, DROP, LS>;                                                       \
   VRR_SMEM_ATTR_ONCE(kern, 160 * 1024);                                                                                \
   const int grid = min(ceil_div(M, W), B * sm_count());                                                                \
-  kern<<<grid, W * 32, (size_t)2 * W * E * sizeof(float), st>>>((const TY*)dy, d_xnew, x_new, gamma, mean, rstd, dx,   \
-                                                                (TB*)d_branch, dgamma, dbeta, M, dv);
+  kern<<<grid, W * 32, (size_t)(LS ? 3 : 2) * W * E * sizeof(float), st>>>((const TY*)dy, d_xnew, x_new, gamma, mean,  \
+                                                                           rstd, dx, (TB*)d_branch, dgamma, dbeta, M,   \
+                                                                           dv, ls, (const TB*)branch, d_ls);
+  // LS: its own launch shape, the one that compiles without spills for every dtype and DROP (12 x 1 spills at NV 6 with
+  // an fp32 branch, 8 x 2 at NV >= 4); ln_bwd_minb does not apply
 #define VRR_LN_REG(NV)                                                                                                  \
   if (g_ln_reg && E == NV * 128) { \
-    if (NV <= 4 || g_ln_bwd_minb == 2) {                                                                                \
+    if constexpr (LS) {                                                                                                 \
+      if constexpr (NV <= 2) {                                                                                                  \
+        VRR_LN_BWD_GO(NV, 8, 2)                                                                                         \
+      } else {                                                                                                          \
+        VRR_LN_BWD_GO(NV, 8, 1)                                                                                         \
+      }                                                                                                                 \
+    } else if (NV <= 4 || g_ln_bwd_minb == 2) {                                                                                \
       VRR_LN_BWD_GO(NV, 8, 2)                                                                                              \
     } else if (g_ln_bwd_minb == 1 || NV > 6) {                                                                               \
       VRR_LN_BWD_GO(NV, 8, 1)                                                                                              \
@@ -636,8 +721,10 @@ int add_ln_bwd_t(const void* dy, const float* d_xnew, const float* x_new, const 
   VRR_LN_REG(6) VRR_LN_REG(8) VRR_LN_REG(4) VRR_LN_REG(2)
 #undef VRR_LN_REG
   if (E % 128 == 0)
-    return add_ln_bwd_launch<TB, TY, 4, DROP>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, dv, st);
-  return add_ln_bwd_launch<TB, TY, 1, DROP>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, dv, st);
+    return add_ln_bwd_launch<TB, TY, 4, DROP, LS>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, dv,
+                                                  ls, branch, d_ls, st);
+  return add_ln_bwd_launch<TB, TY, 1, DROP, LS>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, dv,
+                                                ls, branch, d_ls, st);
 }
 
 }  // namespace
@@ -673,68 +760,89 @@ int layernorm_bwd(const void* dy, const void* x, const float* gamma, const float
   return VRR_ERR_UNSUPPORTED;
 }
 
-template <int DROP>
+template <int DROP, bool LS>
 static int add_layernorm_fwd_d(const void* x, const void* branch, void* x_new, const float* gamma, const float* beta,
                                void* y, float* mean, float* rstd, int M, int E, float eps, int branch_dtype, int y_dtype,
-                               const DropView& dv, cudaStream_t st) {
+                               const DropView& dv, const float* ls, cudaStream_t st) {
   VRR_REQUIRE((size_t)2 * kLnWarps * E * sizeof(float) <= 160 * 1024, VRR_ERR_UNSUPPORTED,
               "add_layernorm: E = %d too large (max 2560)", E);
-#define ARGS (const float*)x, branch, (float*)x_new, gamma, beta, y, mean, rstd, M, E, eps, dv, st
-  if (branch_dtype == VRR_F32 && y_dtype == VRR_F32) return add_ln_fwd_t<float, float, DROP>(ARGS);
-  if (branch_dtype == VRR_BF16 && y_dtype == VRR_BF16) return add_ln_fwd_t<__nv_bfloat16, __nv_bfloat16, DROP>(ARGS);
-  if (branch_dtype == VRR_F32 && y_dtype == VRR_BF16) return add_ln_fwd_t<float, __nv_bfloat16, DROP>(ARGS);
-  if (branch_dtype == VRR_F16 && y_dtype == VRR_F16) return add_ln_fwd_t<__half, __half, DROP>(ARGS);
-  if (branch_dtype == VRR_F32 && y_dtype == VRR_F16) return add_ln_fwd_t<float, __half, DROP>(ARGS);
+#define ARGS (const float*)x, branch, (float*)x_new, gamma, beta, y, mean, rstd, M, E, eps, dv, ls, st
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_F32) return add_ln_fwd_t<float, float, DROP, LS>(ARGS);
+  if (branch_dtype == VRR_BF16 && y_dtype == VRR_BF16) return add_ln_fwd_t<__nv_bfloat16, __nv_bfloat16, DROP, LS>(ARGS);
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_BF16) return add_ln_fwd_t<float, __nv_bfloat16, DROP, LS>(ARGS);
+  if (branch_dtype == VRR_F16 && y_dtype == VRR_F16) return add_ln_fwd_t<__half, __half, DROP, LS>(ARGS);
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_F16) return add_ln_fwd_t<float, __half, DROP, LS>(ARGS);
 #undef ARGS
   set_error("add_layernorm_fwd: unsupported dtype combination (branch %d, y %d)", branch_dtype, y_dtype);
   return VRR_ERR_UNSUPPORTED;
 }
 
-template <int DROP>
+template <int DROP, bool LS>
 static int add_layernorm_bwd_d(const void* dy, const void* d_xnew, const void* x_new, const float* gamma,
                                const float* mean, const float* rstd, void* dx, void* d_branch, float* dgamma,
                                float* dbeta, int M, int E, int branch_dtype, int y_dtype, const DropView& dv,
-                               cudaStream_t st) {
-  VRR_REQUIRE((size_t)2 * kLnWarps * E * sizeof(float) <= 160 * 1024, VRR_ERR_UNSUPPORTED,
-              "add_layernorm: E = %d too large (max 2560)", E);
-#define ARGS dy, (const float*)d_xnew, (const float*)x_new, gamma, mean, rstd, (float*)dx, d_branch, dgamma, dbeta, M, E, dv, st
-  if (branch_dtype == VRR_F32 && y_dtype == VRR_F32) return add_ln_bwd_t<float, float, DROP>(ARGS);
-  if (branch_dtype == VRR_BF16 && y_dtype == VRR_BF16) return add_ln_bwd_t<__nv_bfloat16, __nv_bfloat16, DROP>(ARGS);
-  if (branch_dtype == VRR_F32 && y_dtype == VRR_BF16) return add_ln_bwd_t<float, __nv_bfloat16, DROP>(ARGS);
-  if (branch_dtype == VRR_F16 && y_dtype == VRR_F16) return add_ln_bwd_t<__half, __half, DROP>(ARGS);
-  if (branch_dtype == VRR_F32 && y_dtype == VRR_F16) return add_ln_bwd_t<float, __half, DROP>(ARGS);
+                               const float* ls, const void* branch, float* d_ls, cudaStream_t st) {
+  VRR_REQUIRE((size_t)(LS ? 3 : 2) * kLnWarps * E * sizeof(float) <= 160 * 1024, VRR_ERR_UNSUPPORTED,
+              "add_layernorm: E = %d too large (max %d)", E, LS ? 1706 : 2560);
+#define ARGS dy, (const float*)d_xnew, (const float*)x_new, gamma, mean, rstd, (float*)dx, d_branch, dgamma, dbeta, M, E, dv, \
+             ls, branch, d_ls, st
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_F32) return add_ln_bwd_t<float, float, DROP, LS>(ARGS);
+  if (branch_dtype == VRR_BF16 && y_dtype == VRR_BF16) return add_ln_bwd_t<__nv_bfloat16, __nv_bfloat16, DROP, LS>(ARGS);
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_BF16) return add_ln_bwd_t<float, __nv_bfloat16, DROP, LS>(ARGS);
+  if (branch_dtype == VRR_F16 && y_dtype == VRR_F16) return add_ln_bwd_t<__half, __half, DROP, LS>(ARGS);
+  if (branch_dtype == VRR_F32 && y_dtype == VRR_F16) return add_ln_bwd_t<float, __half, DROP, LS>(ARGS);
 #undef ARGS
   set_error("add_layernorm_bwd: unsupported dtype combination (branch %d, y %d)", branch_dtype, y_dtype);
   return VRR_ERR_UNSUPPORTED;
 }
 
-int add_layernorm_fwd(const void* x, const void* branch, void* x_new, const float* gamma, const float* beta, void* y,
-                      float* mean, float* rstd, int M, int E, float eps, int branch_dtype, int y_dtype,
-                      const vrr_drop_desc* drop, cudaStream_t st) {
+template <bool LS>
+static int add_layernorm_fwd_l(const void* x, const void* branch, void* x_new, const float* gamma, const float* beta,
+                               void* y, float* mean, float* rstd, int M, int E, float eps, int branch_dtype, int y_dtype,
+                               const vrr_drop_desc* drop, const float* ls, cudaStream_t st) {
   DropView dv = {};
   bool active = false;
   if (int rc = drop_view(drop, M, E, &dv, &active)) return rc;
-  if (active && dv.t < 65536u)
-    return add_layernorm_fwd_d<2>(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, dv, st);
-  if (active)
-    return add_layernorm_fwd_d<1>(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, dv, st);
-  return add_layernorm_fwd_d<0>(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, dv, st);
+#define ARGS x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, dv, ls, st
+  if (active && dv.t < 65536u) return add_layernorm_fwd_d<2, LS>(ARGS);
+  if (active) return add_layernorm_fwd_d<1, LS>(ARGS);
+  return add_layernorm_fwd_d<0, LS>(ARGS);
+#undef ARGS
+}
+
+template <bool LS>
+static int add_layernorm_bwd_l(const void* dy, const void* d_xnew, const void* x_new, const float* gamma,
+                               const float* mean, const float* rstd, void* dx, void* d_branch, float* dgamma,
+                               float* dbeta, int M, int E, int branch_dtype, int y_dtype, const vrr_drop_desc* drop,
+                               const float* ls, const void* branch, float* d_ls, cudaStream_t st) {
+  DropView dv = {};
+  bool active = false;
+  if (int rc = drop_view(drop, M, E, &dv, &active)) return rc;
+#define ARGS dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype, y_dtype, dv, ls, branch, d_ls, st
+  if (active && dv.t < 65536u) return add_layernorm_bwd_d<2, LS>(ARGS);
+  if (active) return add_layernorm_bwd_d<1, LS>(ARGS);
+  return add_layernorm_bwd_d<0, LS>(ARGS);
+#undef ARGS
+}
+
+int add_layernorm_fwd(const void* x, const void* branch, void* x_new, const float* gamma, const float* beta, void* y,
+                      float* mean, float* rstd, int M, int E, float eps, int branch_dtype, int y_dtype,
+                      const vrr_drop_desc* drop, const float* ls, cudaStream_t st) {
+  if (ls)
+    return add_layernorm_fwd_l<true>(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, drop, ls, st);
+  return add_layernorm_fwd_l<false>(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, drop,
+                                    nullptr, st);
 }
 
 int add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new, const float* gamma, const float* mean,
                       const float* rstd, void* dx, void* d_branch, float* dgamma, float* dbeta, int M, int E,
-                      int branch_dtype, int y_dtype, const vrr_drop_desc* drop, cudaStream_t st) {
-  DropView dv = {};
-  bool active = false;
-  if (int rc = drop_view(drop, M, E, &dv, &active)) return rc;
-  if (active && dv.t < 65536u)
-    return add_layernorm_bwd_d<2>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
-                                  y_dtype, dv, st);
-  if (active)
-    return add_layernorm_bwd_d<1>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
-                                  y_dtype, dv, st);
-  return add_layernorm_bwd_d<0>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
-                                    y_dtype, dv, st);
+                      int branch_dtype, int y_dtype, const vrr_drop_desc* drop, const float* ls, const void* branch,
+                      float* d_ls, cudaStream_t st) {
+  if (ls)
+    return add_layernorm_bwd_l<true>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
+                                     y_dtype, drop, ls, branch, d_ls, st);
+  return add_layernorm_bwd_l<false>(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
+                                    y_dtype, drop, nullptr, nullptr, nullptr, st);
 }
 
 void layernorm_set_option(int which, int value) {

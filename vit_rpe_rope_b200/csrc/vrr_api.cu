@@ -572,7 +572,7 @@ int vrr_add_layernorm_fwd(const void* x, const void* branch, void* x_new, const 
               VRR_ERR_INVALID_ARG, "add_layernorm_fwd: pointers must be 16-byte aligned");
   if (int rc = require_device()) return rc;
   return add_layernorm_fwd(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, nullptr,
-                           (cudaStream_t)stream);
+                           nullptr, (cudaStream_t)stream);
 }
 
 int vrr_add_layernorm_drop_fwd(const void* x, const void* branch, void* x_new, const float* gamma, const float* beta,
@@ -586,7 +586,7 @@ int vrr_add_layernorm_drop_fwd(const void* x, const void* branch, void* x_new, c
               VRR_ERR_INVALID_ARG, "add_layernorm_drop_fwd: pointers must be 16-byte aligned");
   if (int rc = require_device()) return rc;
   return add_layernorm_fwd(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, drop,
-                           (cudaStream_t)stream);
+                           nullptr, (cudaStream_t)stream);
 }
 
 int vrr_add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new, const float* gamma, const float* mean,
@@ -601,7 +601,7 @@ int vrr_add_layernorm_bwd(const void* dy, const void* d_xnew, const void* x_new,
               VRR_ERR_INVALID_ARG, "add_layernorm_bwd: pointers must be 16-byte aligned");
   if (int rc = require_device()) return rc;
   return add_layernorm_bwd(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
-                           y_dtype, nullptr, (cudaStream_t)stream);
+                           y_dtype, nullptr, nullptr, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 int vrr_add_layernorm_drop_bwd(const void* dy, const void* d_xnew, const void* x_new, const float* gamma,
@@ -617,7 +617,40 @@ int vrr_add_layernorm_drop_bwd(const void* dy, const void* d_xnew, const void* x
               VRR_ERR_INVALID_ARG, "add_layernorm_drop_bwd: pointers must be 16-byte aligned");
   if (int rc = require_device()) return rc;
   return add_layernorm_bwd(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
-                           y_dtype, drop, (cudaStream_t)stream);
+                           y_dtype, drop, nullptr, nullptr, nullptr, (cudaStream_t)stream);
+}
+
+int vrr_add_layernorm_ls_fwd(const void* x, const void* branch, void* x_new, const float* gamma, const float* beta,
+                             void* y, float* mean, float* rstd, int M, int E, float eps, int branch_dtype, int y_dtype,
+                             const vrr_drop_desc* drop, const float* ls, void* stream) {
+  VRR_REQUIRE(x && branch && x_new && gamma && beta && y && mean && rstd, VRR_ERR_INVALID_ARG, "add_layernorm_ls_fwd: NULL pointer");
+  VRR_REQUIRE(dtype_ok(branch_dtype) && dtype_ok(y_dtype) && no_mix(branch_dtype, y_dtype), VRR_ERR_INVALID_ARG,
+              "add_layernorm_ls_fwd: bad dtype");
+  VRR_REQUIRE(M > 0 && E > 0, VRR_ERR_INVALID_ARG, "add_layernorm_ls_fwd: bad sizes");
+  VRR_REQUIRE((((uintptr_t)x | (uintptr_t)branch | (uintptr_t)x_new | (uintptr_t)y | (uintptr_t)gamma | (uintptr_t)beta |
+                (uintptr_t)ls) & 15) == 0,
+              VRR_ERR_INVALID_ARG, "add_layernorm_ls_fwd: pointers must be 16-byte aligned");
+  if (int rc = require_device()) return rc;
+  return add_layernorm_fwd(x, branch, x_new, gamma, beta, y, mean, rstd, M, E, eps, branch_dtype, y_dtype, drop, ls,
+                           (cudaStream_t)stream);
+}
+
+int vrr_add_layernorm_ls_bwd(const void* dy, const void* d_xnew, const void* x_new, const float* gamma,
+                             const float* mean, const float* rstd, void* dx, void* d_branch, float* dgamma,
+                             float* dbeta, int M, int E, int branch_dtype, int y_dtype, const vrr_drop_desc* drop,
+                             const float* ls, const void* branch, float* d_ls, void* stream) {
+  VRR_REQUIRE(dy && x_new && gamma && mean && rstd && dx && d_branch && dgamma && dbeta, VRR_ERR_INVALID_ARG,
+              "add_layernorm_ls_bwd: NULL pointer");
+  VRR_REQUIRE(!d_ls || (ls && branch), VRR_ERR_INVALID_ARG, "add_layernorm_ls_bwd: d_ls needs ls and branch");
+  VRR_REQUIRE(dtype_ok(branch_dtype) && dtype_ok(y_dtype) && no_mix(branch_dtype, y_dtype), VRR_ERR_INVALID_ARG,
+              "add_layernorm_ls_bwd: bad dtype");
+  VRR_REQUIRE(M > 0 && E > 0, VRR_ERR_INVALID_ARG, "add_layernorm_ls_bwd: bad sizes");
+  VRR_REQUIRE((((uintptr_t)dy | (uintptr_t)d_xnew | (uintptr_t)x_new | (uintptr_t)dx | (uintptr_t)d_branch | (uintptr_t)gamma |
+                (uintptr_t)ls | (uintptr_t)branch) & 15) == 0,
+              VRR_ERR_INVALID_ARG, "add_layernorm_ls_bwd: pointers must be 16-byte aligned");
+  if (int rc = require_device()) return rc;
+  return add_layernorm_bwd(dy, d_xnew, x_new, gamma, mean, rstd, dx, d_branch, dgamma, dbeta, M, E, branch_dtype,
+                           y_dtype, drop, ls, branch, d_ls, (cudaStream_t)stream);
 }
 
 int vrr_dropout_mask(const vrr_drop_desc* drop, void* keep_u8, void* keep_path_u8, int M, int E, void* stream) {

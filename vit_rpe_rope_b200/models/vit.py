@@ -22,6 +22,10 @@ Register tokens (``VisionTransformer(reg_tokens=R)``, timm's name; DINOv2-with-r
 between the cls token and the patches, ``[cls, reg_0 .. reg_{R-1}, patch_0 ..]``.  Like the cls token they get no
 absolute position embedding and are never rotated; the patch-embedding kernel writes them and the QKV+RoPE epilogue
 skips them (``num_prefix_tokens = 1 + R``).
+
+LayerScale (``VisionTransformer(init_values=)``, timm's name; DeiT III, DINOv2, DINOv3): a learnable per-channel
+``gamma`` multiplies each residual branch before it is added.  Inside the fused block loop the add+LayerNorm kernels
+apply it in fp32 as they read the branch and reduce its gradient in the same backward pass.
 """
 import torch
 import torch.nn as nn
@@ -62,6 +66,22 @@ class DropPath(nn.Module):
 
 def _drop_p(m):
     return m.p if isinstance(m, nn.Dropout) else 0.
+
+
+def _gamma(ls):
+    return ls.gamma if isinstance(ls, LayerScale) else None
+
+
+class LayerScale(nn.Module):
+    """``x * gamma`` with ``gamma = init_values * ones(dim)`` (timm.layers.LayerScale without ``inplace``).  Inside
+    ``VisionTransformer``'s fused block loop the product is taken by the add+LayerNorm kernels instead."""
+
+    def __init__(self, dim, init_values=1e-5):
+        super().__init__()
+        self.gamma = nn.Parameter(init_values * torch.ones(dim))
+
+    def forward(self, x):
+        return x * self.gamma
 
 
 class Mlp(nn.Module):
@@ -139,20 +159,23 @@ class Attention(nn.Module):
 
 
 class Block(nn.Module):
-    """Pre-LN transformer block (reference vit.py:100-129)."""
+    """Pre-LN transformer block (reference vit.py:100-129); ``init_values`` adds timm's LayerScale ``ls1`` / ``ls2``
+    (None or 0: none, the reference's block)."""
 
     def __init__(self, dim, num_heads, mlp_ratio=4., qkv_bias=False, drop=0., attn_drop=0.,
-                 drop_path=0., act_layer=nn.GELU, norm_layer=nn.LayerNorm):
+                 drop_path=0., act_layer=nn.GELU, norm_layer=nn.LayerNorm, init_values=None):
         super().__init__()
         self.norm1 = norm_layer(dim)
         self.attn = Attention(dim, num_heads=num_heads, qkv_bias=qkv_bias, attn_drop=attn_drop, proj_drop=drop)
+        self.ls1 = LayerScale(dim, init_values) if init_values else nn.Identity()
         self.drop_path = DropPath(drop_path) if drop_path > 0. else nn.Identity()
         self.norm2 = norm_layer(dim)
         self.mlp = Mlp(in_features=dim, hidden_features=int(dim * mlp_ratio), act_layer=act_layer, drop=drop)
+        self.ls2 = LayerScale(dim, init_values) if init_values else nn.Identity()
 
     def forward(self, x, freqs_cis=None):
-        x = x + self.drop_path(self.attn(ops.layer_norm(x, self.norm1), freqs_cis=freqs_cis))
-        x = x + self.drop_path(self.mlp(ops.layer_norm(x, self.norm2)))
+        x = x + self.drop_path(self.ls1(self.attn(ops.layer_norm(x, self.norm1), freqs_cis=freqs_cis)))
+        x = x + self.drop_path(self.ls2(self.mlp(ops.layer_norm(x, self.norm2))))
         return x
 
     def set_pos_encoding(self, pos_encoding):
@@ -171,12 +194,16 @@ class VisionTransformer(nn.Module):
     only when R > 0, initialised ``normal_(std=1e-6)`` as timm does, drawn after every other parameter so the rest of
     a seeded model is unchanged).  The relative and polynomial biases are defined against a single cls token and
     raise ``ValueError`` with registers.
+
+    ``init_values`` gives every block LayerScale (``blocks.{i}.ls1.gamma`` / ``ls2.gamma`` [E], filled with the value;
+    no random numbers are drawn); None or 0, the default, means none.
     """
 
     def __init__(self, img_size=32, patch_size=4, in_chans=3, num_classes=10,
                  embed_dim=192, depth=6, num_heads=6, mlp_ratio=4.,
                  pos_encoding='absolute', rope_theta=100.0,
-                 poly_degree=3, poly_shared_heads=True, drop_rate=0., drop_path_rate=0., reg_tokens=0):
+                 poly_degree=3, poly_shared_heads=True, drop_rate=0., drop_path_rate=0., reg_tokens=0,
+                 init_values=None):
         super().__init__()
         if reg_tokens < 0:
             raise ValueError(f"reg_tokens must be >= 0, got {reg_tokens}")
@@ -216,8 +243,8 @@ class VisionTransformer(nn.Module):
             raise ValueError(f"Unknown positional encoding type: {pos_encoding}")
 
         dpr = [r.item() for r in torch.linspace(0, drop_path_rate, depth)]  # draws no random numbers
-        self.blocks = nn.ModuleList([Block(embed_dim, num_heads, mlp_ratio, drop=drop_rate, drop_path=dpr[i])
-                                     for i in range(depth)])
+        self.blocks = nn.ModuleList([Block(embed_dim, num_heads, mlp_ratio, drop=drop_rate, drop_path=dpr[i],
+                                           init_values=init_values) for i in range(depth)])
         if not self.use_pos_embed_in_forward:
             for blk in self.blocks:
                 blk.set_pos_encoding(self.pos_embed)  # one shared module, referenced by every block
@@ -247,12 +274,14 @@ class VisionTransformer(nn.Module):
 
     def forward_features(self, x):
         """[B, C, H, W] -> [B, N, E] with N = (H/P)(W/P) + num_prefix_tokens taken from the input (vit.py:235-271)."""
-        x, m, drop = self._features(x)
+        x, m, drop, ls = self._features(x)
         if m is None:
             return x
-        if drop is None:
-            return x + m
-        return x + m.float() * ops.branch_factor(drop, *m.shape)
+        if drop is not None:
+            m = m.float() * ops.branch_factor(drop, *m.shape)
+        if ls is not None:
+            m = m.float() * ls
+        return x + m
 
     def _drop_sites(self, x):
         """Per block (attention branch, fc1's activation, MLP branch): the dropout sites of one training forward, all
@@ -271,8 +300,8 @@ class VisionTransformer(nn.Module):
                 for i, (pa, pp, p1, p2) in enumerate(rates)]
 
     def _features(self, x):
-        """The token stream before the LAST residual add, that add's branch and its dropout site (or the finished
-        stream, None, None): ``forward`` only needs the cls row of the sum."""
+        """The token stream before the LAST residual add, that add's branch, its dropout site and its LayerScale gamma
+        (or the finished stream, None, None, None): ``forward`` only needs the cls row of the sum."""
         B, C, H, W = x.shape
         h, w = H // self.patch_size, W // self.patch_size
         if x.is_cuda:  # one multi-tensor refresh of the 16-bit weight copies per forward (no-op in fp32)
@@ -288,21 +317,22 @@ class VisionTransformer(nn.Module):
         if not self._fusable(x):
             for blk in self.blocks:
                 x = blk(x, freqs_cis=freqs_cis)
-            return x, None, None
+            return x, None, None, None
         # Same arithmetic as the loop above (vit.py:120-125 per block), with every residual add fused with
         # the LayerNorm that follows it - also across block boundaries:
-        #   x = x + drop_path(proj_drop(attn(norm1(x))));  x = x + drop_path(drop2(mlp(norm2(x))))
+        #   x = x + drop_path(ls1(proj_drop(attn(norm1(x)))));  x = x + drop_path(ls2(drop2(mlp(norm2(x)))))
         blocks = self.blocks
         sites = self._drop_sites(x)
         y = ops.layer_norm(x, blocks[0].norm1)
         m = d_mlp = None
         for i, blk in enumerate(blocks):
             d_attn, d_fc1, d_mlp = sites[i] if sites is not None else (None, None, None)
-            x, y = ops.add_layer_norm(x, blk.attn._branch(y, freqs_cis=freqs_cis), blk.norm2, drop=d_attn)
+            x, y = ops.add_layer_norm(x, blk.attn._branch(y, freqs_cis=freqs_cis), blk.norm2, drop=d_attn,
+                                      ls=_gamma(blk.ls1))
             m = blk.mlp._branch(y, d_fc1)
             if i + 1 < len(blocks):
-                x, y = ops.add_layer_norm(x, m, blocks[i + 1].norm1, drop=d_mlp)
-        return x, m, d_mlp
+                x, y = ops.add_layer_norm(x, m, blocks[i + 1].norm1, drop=d_mlp, ls=_gamma(blk.ls2))
+        return x, m, d_mlp, _gamma(blocks[-1].ls2)
 
     def _gemm_weights(self):
         ws = [self.head.weight]
@@ -315,20 +345,26 @@ class VisionTransformer(nn.Module):
     def _fusable(self, x):
         return len(self.blocks) > 0 and all(
             type(blk) is Block and type(blk.drop_path) in (nn.Identity, DropPath) and type(blk.mlp) is Mlp
+            and type(blk.ls1) in (nn.Identity, LayerScale) and type(blk.ls2) in (nn.Identity, LayerScale)
             and type(blk.attn.proj_drop) is nn.Dropout and type(blk.mlp.drop2) is nn.Dropout
             and ops.can_fuse_add_layer_norm(x, blk.norm1) and ops.can_fuse_add_layer_norm(x, blk.norm2)
             for blk in self.blocks)
 
     def forward(self, x):
-        x, m, drop = self._features(x)
+        x, m, drop, ls = self._features(x)
         # LayerNorm is per token and only the cls token reaches the head (vit.py:284-285): the last residual
         # add and the final norm of that row alone give identical logits and gradients (with dropout: the factors
-        # of token rows b*N, the same arithmetic as forward_features)
+        # of token rows b*N; with LayerScale: then times gamma - the same arithmetic as forward_features)
         if m is None:
             cls = x[:, 0]
-        elif drop is None:
+        elif drop is None and ls is None:
             cls = x[:, 0] + m[:, 0]
         else:
-            cls = x[:, 0] + m[:, 0].float() * ops.branch_factor(drop, *m.shape, cls_only=True)[:, 0]
+            b = m[:, 0]
+            if drop is not None:
+                b = b.float() * ops.branch_factor(drop, *m.shape, cls_only=True)[:, 0]
+            if ls is not None:
+                b = b.float() * ls
+            cls = x[:, 0] + b
         y = ops.layer_norm(cls, self.norm)
         return ops.linear(y, self.head, ops.lp_weight(self.head.weight, ops.compute_dtype(y)))

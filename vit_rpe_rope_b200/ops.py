@@ -512,10 +512,12 @@ class AddLayerNormFn(torch.autograd.Function):
     """(x_new, y) = (x + branch, LayerNorm(x + branch)): the residual add of one sub-block fused with the
     LayerNorm that opens the next one; the backward emits the residual-stream gradient (fp32) and the
     branch gradient (branch dtype) from a single pass.  ``drop``: the branch's dropout / stochastic-depth site
-    (x_new = x + f * branch; the masks are regenerated in the backward), or None."""
+    (x_new = x + f * branch; the masks are regenerated in the backward), or None.  ``ls``: a LayerScale vector [E]
+    (x_new = x + (f * branch) * ls, each product rounded to fp32), or None; its gradient is a column reduction of the
+    same pass, for which the branch is saved only when ``ls`` needs one."""
 
     @staticmethod
-    def forward(ctx, x, branch, weight, bias, eps, out_dtype, drop=None):
+    def forward(ctx, x, branch, weight, bias, eps, out_dtype, drop=None, ls=None):
         _require_cuda(x, branch, weight, bias)
         lib = _lib.load()
         E = x.shape[-1]
@@ -527,8 +529,15 @@ class AddLayerNormFn(torch.autograd.Function):
         y = torch.empty(M, E, device=x.device, dtype=out_dtype)
         mean = torch.empty(M, device=x.device, dtype=torch.float32)
         rstd = torch.empty(M, device=x.device, dtype=torch.float32)
+        ls32 = _f32c(ls)
         with torch.cuda.device(x.device), _timed("add_layernorm_fwd"):
-            if drop is None:
+            if ls is not None:
+                d = _drop_desc(drop) if drop is not None else None
+                _lib.check(lib.vrr_add_layernorm_ls_fwd(_ptr(x2), _ptr(b2), _ptr(x_new), _ptr(w32), _ptr(b32), _ptr(y),
+                                                        _ptr(mean), _ptr(rstd), M, E, float(eps), _DT[b2.dtype],
+                                                        _DT[out_dtype], ctypes.byref(d) if d is not None else None,
+                                                        _ptr(ls32), _stream()), "vrr_add_layernorm_ls_fwd")
+            elif drop is None:
                 _lib.check(lib.vrr_add_layernorm_fwd(_ptr(x2), _ptr(b2), _ptr(x_new), _ptr(w32), _ptr(b32), _ptr(y),
                                                      _ptr(mean), _ptr(rstd), M, E, float(eps), _DT[b2.dtype],
                                                      _DT[out_dtype], _stream()), "vrr_add_layernorm_fwd")
@@ -539,15 +548,16 @@ class AddLayerNormFn(torch.autograd.Function):
                                                           _DT[out_dtype], ctypes.byref(d), _stream()),
                            "vrr_add_layernorm_drop_fwd")
         ctx.drop = drop  # holds the seed tensor: the backward regenerates the masks from it
-        ctx.save_for_backward(x_new, w32, mean, rstd)
-        ctx.meta = (x.shape, weight.dtype, bias.dtype, out_dtype, b2.dtype)
+        ls_grad = ls is not None and ctx.needs_input_grad[7]
+        ctx.save_for_backward(x_new, w32, mean, rstd, ls32, b2 if ls_grad else None)
+        ctx.meta = (x.shape, weight.dtype, bias.dtype, out_dtype, b2.dtype, None if ls is None else ls.dtype)
         return x_new.view(x.shape), y.view(x.shape)
 
     @staticmethod
     def backward(ctx, d_xnew, d_y):
         lib = _lib.load()
-        x_new, w32, mean, rstd = ctx.saved_tensors
-        shape, w_dtype, b_dtype, out_dtype, br_dtype = ctx.meta
+        x_new, w32, mean, rstd, ls32, b2 = ctx.saved_tensors
+        shape, w_dtype, b_dtype, out_dtype, br_dtype, ls_dtype = ctx.meta
         M, E = x_new.shape
         if d_y is None:
             d_y = torch.zeros(M, E, device=x_new.device, dtype=out_dtype)
@@ -561,10 +571,19 @@ class AddLayerNormFn(torch.autograd.Function):
                 dr2 = dr2.float()
         dx = torch.empty_like(x_new)
         d_branch = torch.empty(M, E, device=x_new.device, dtype=br_dtype)
-        dgb = torch.empty(2, E, device=x_new.device, dtype=torch.float32)  # one buffer: the library zeroes both rows with one memset
+        # one buffer: the library zeroes its rows (gamma, beta and the LayerScale gradient) with one memset
+        dgb = torch.empty(2 if b2 is None else 3, E, device=x_new.device, dtype=torch.float32)
         dg, db = dgb[0], dgb[1]
+        d_ls = dgb[2] if b2 is not None else None
         with torch.cuda.device(x_new.device), _timed("add_layernorm_bwd"):
-            if ctx.drop is None:
+            if ls32 is not None:
+                d = _drop_desc(ctx.drop) if ctx.drop is not None else None
+                _lib.check(lib.vrr_add_layernorm_ls_bwd(_ptr(dy2), _ptr(dr2), _ptr(x_new), _ptr(w32), _ptr(mean),
+                                                        _ptr(rstd), _ptr(dx), _ptr(d_branch), _ptr(dg), _ptr(db), M, E,
+                                                        _DT[br_dtype], _DT[out_dtype],
+                                                        ctypes.byref(d) if d is not None else None, _ptr(ls32),
+                                                        _ptr(b2), _ptr(d_ls), _stream()), "vrr_add_layernorm_ls_bwd")
+            elif ctx.drop is None:
                 _lib.check(lib.vrr_add_layernorm_bwd(_ptr(dy2), _ptr(dr2), _ptr(x_new), _ptr(w32), _ptr(mean), _ptr(rstd),
                                                      _ptr(dx), _ptr(d_branch), _ptr(dg), _ptr(db), M, E, _DT[br_dtype],
                                                      _DT[out_dtype], _stream()), "vrr_add_layernorm_bwd")
@@ -574,7 +593,8 @@ class AddLayerNormFn(torch.autograd.Function):
                                                           _ptr(rstd), _ptr(dx), _ptr(d_branch), _ptr(dg), _ptr(db), M, E,
                                                           _DT[br_dtype], _DT[out_dtype], ctypes.byref(d), _stream()),
                            "vrr_add_layernorm_drop_bwd")
-        return dx.view(shape), d_branch.view(shape), dg.to(w_dtype), db.to(b_dtype), None, None, None
+        return (dx.view(shape), d_branch.view(shape), dg.to(w_dtype), db.to(b_dtype), None, None, None,
+                None if d_ls is None else d_ls.to(ls_dtype))
 
 
 def can_fuse_add_layer_norm(x, norm) -> bool:
@@ -583,13 +603,13 @@ def can_fuse_add_layer_norm(x, norm) -> bool:
             and norm.bias is not None and tuple(norm.normalized_shape) == (x.shape[-1],))
 
 
-def add_layer_norm(x, branch, norm: torch.nn.LayerNorm, drop=None):
-    """``x_new = x + f * branch; y = norm(x_new)`` in one kernel (see :class:`AddLayerNormFn`); f = 1 when ``drop`` is
-    None."""
+def add_layer_norm(x, branch, norm: torch.nn.LayerNorm, drop=None, ls=None):
+    """``x_new = x + (f * branch) * ls; y = norm(x_new)`` in one kernel (see :class:`AddLayerNormFn`); f = 1 when
+    ``drop`` is None, and no LayerScale product when ``ls`` (a LayerScale's ``gamma`` [E]) is None."""
     out_dtype = compute_dtype(x)
     if branch.dtype not in (torch.float32, out_dtype):
         branch = branch.to(out_dtype)
-    return AddLayerNormFn.apply(x, branch, norm.weight, norm.bias, norm.eps, out_dtype, drop)
+    return AddLayerNormFn.apply(x, branch, norm.weight, norm.bias, norm.eps, out_dtype, drop, ls)
 
 
 def layer_norm(x, norm: torch.nn.LayerNorm):
