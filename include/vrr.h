@@ -361,6 +361,30 @@ int vrr_dropout_mask(const vrr_drop_desc* drop, void* keep_u8, void* keep_path_u
 int vrr_gemm_mul_colsum(const void* a, const void* b, void* c, const void* mul, float* col_sums, int M, int N,
                         int K, int trans_a, int trans_b, int dtype, void* stream);
 
+/* fc1 of a packed SwiGLU Mlp (timm's SwiGLUPacked: fc2(silu(x W_g^T + b_g) * (x W_v^T + b_v))), T = `dtype`.
+ * x [M][K], w1 [2H][K] (fc1.weight: gate rows [0, H), then value rows [H, 2H)), b1 fp32 [2H]; act [M][H];
+ * aux [M][2H] or NULL (torch.no_grad: act only).  For output column j (rounding as torch on T tensors):
+ *   g = T(acc_j + T(b1[j])),  v = T(acc_{H+j} + T(b1[H+j]))                 (F.linear)
+ *   s = T(silu(g))                                                          (nn.SiLU)
+ *   act[m][j]     = T(T(s * v) * f)                                         (the product, then Dropout)
+ *   aux[m][j]     = T(fl(v * silu'(g)) * f)                                 (d act / d g)
+ *   aux[m][H + j] = T(s * f)                                                (d act / d v)
+ * Every product is an fp32 multiply rounded to nearest; silu and silu' carry the error bound documented in
+ * csrc/common.cuh (relative 2^-20 (1 + |g|), plus 2^-126 (1 + |g|) absolute where sigma underflows).  f is the factor of `drop` for element (m, j) of act [M][H] (as
+ * vrr_gemm_ex_drop: p_path must be 0, the mask groups need H % 8 == 0); drop NULL or p == 0: f = 1 and no product is
+ * taken.  bf16 / fp16 with H % 8 == 0, K % 8 == 0 and 16-byte aligned pointers run the tcgen05 kernel (gate and value
+ * columns paired in one accumulator tile); everything else, fp32 included, the FFMA kernel with the same arithmetic.
+ * vrr_set_impl / vrr_family_count as for vrr_gemm_ex.  No workspace. */
+int vrr_gemm_swiglu(const void* x, const void* w1, const float* b1, void* act, void* aux, int M, int H, int K,
+                    int dtype, const vrr_drop_desc* drop, void* stream);
+/* fc2's dX with the SwiGLU backward and fc1's bias gradient: dA = dy [M][K] . w2 [K][H] (fc2.weight) in fp32, then
+ *   dh [M][2H]:  dh[m][j] = T(dA[m][j] * aux[m][j]),  dh[m][H + j] = T(dA[m][j] * aux[m][H + j])
+ *   db1 fp32 [2H] = column sums of dh as stored (written; tcgen05: fp32 atomics, summation order not fixed).
+ * dh is then the gradient of fc1's output (dX = dh . w1 and dW1 = dh^T x are plain vrr_gemm_ex calls).  H % 2 == 0.
+ * Dispatch as vrr_gemm_swiglu; the FFMA route is the GEMM with the products in its epilogue, then vrr_colsum. */
+int vrr_gemm_swiglu_bwd(const void* dy, const void* w2, const void* aux, void* dh, float* db1, int M, int H,
+                        int K, int dtype, void* stream);
+
 /* Bias gradient of a Linear layer (out-proj vit.py:91, Mlp fc1/fc2 vit.py:118, head vit.py:285):
  * out[c] = sum_m x[m][c], fp32 [C] (written); x [M][C] `dtype`, C % 4 == 0, any element-aligned address (a view
  * at an offset into a larger buffer takes an element-wise kernel). */

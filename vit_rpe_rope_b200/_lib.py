@@ -79,6 +79,8 @@ SIGNATURES = {
     "vrr_colsum": (c_int, [c_void_p] * 2 + [c_int] * 3 + [c_void_p]),
     "vrr_gemm_mul_colsum": (c_int, [c_void_p] * 5 + [c_int] * 6 + [c_void_p]),
     "vrr_gelu_bwd": (c_int, [c_void_p] * 4 + [c_int] * 3 + [c_void_p]),
+    "vrr_gemm_swiglu": (c_int, [c_void_p] * 5 + [c_int] * 4 + [POINTER(DropDesc), c_void_p]),
+    "vrr_gemm_swiglu_bwd": (c_int, [c_void_p] * 5 + [c_int] * 4 + [c_void_p]),
     "vrr_attn_fwd": (c_int, [c_void_p, POINTER(BiasDesc), c_void_p, c_void_p] + [c_int] * 4
                      + [c_float, c_int, c_void_p]),
     "vrr_attn_bwd_workspace_bytes": (c_size_t, [c_int] * 4 + [POINTER(BiasDesc)]),

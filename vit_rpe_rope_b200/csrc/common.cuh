@@ -167,6 +167,21 @@ struct DropView {
     return ((j & 1) ? (w >> 16) : (w & 0xFFFFu)) < t ? fr : 0.f;
   }
 };
+// SiLU of a SwiGLU Mlp (vrr_gemm_swiglu) and its derivative, sigma = 1 / (1 + 2^(-g log2 e)) on the MUFU unit:
+//   s = silu(g) = g sigma,  ds = silu'(g) = sigma + s (1 - sigma).
+// ex2.approx (relative error <= 2^-22) of an argument rounded to fp32 (relative error of the exponential
+// <= |g| 2^-24) and rcp.approx (<= 1 ulp) give |s - silu(g)| <= 2^-20 (1 + |g|) |silu(g)| + 2^-126 (1 + |g|) and
+// |ds - silu'(g)| <= 2^-20 (1 + |g|) (sigma + |silu(g)| (1 - sigma)) + 2^-126 (1 + |g|) for finite g
+// (tests/test_swiglu_gpu.py); the absolute term is sigma flushed to zero below the fp32 normal range (g < -87.3).
+// g -> -inf: the exponential overflows to +inf, sigma = 0, s = -0, ds = 0.
+__device__ __forceinline__ void silu_and_grad(float g, float& s, float& ds) {
+  float e, sig;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(__fmul_rn(g, -1.4426950408889634f)));
+  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(sig) : "f"(__fadd_rn(e, 1.f)));
+  s = __fmul_rn(g, sig);
+  ds = __fmaf_rn(s, __fadd_rn(1.f, -sig), sig);
+}
+
 __device__ __forceinline__ float4 mul4_rn(float4 a, float4 f) {
   return make_float4(__fmul_rn(a.x, f.x), __fmul_rn(a.y, f.y), __fmul_rn(a.z, f.z), __fmul_rn(a.w, f.w));
 }

@@ -449,6 +449,107 @@ int gemm_simt_bias(const void* a, const void* b, void* c, void* c2, const float*
   return gemm_bias_t<__half>(a, b, c, c2, bias, M, N, K, ta, tb, gelu, st);
 }
 
+// ---- SwiGLU Mlp (vrr_gemm_swiglu / vrr_gemm_swiglu_bwd) ---------------------------------------------------
+// fc1: logical output column n of block n / 64 pairs gate row j = 32 (n / 64) + (n % 32) of w1 [2H][K] (n % 64 < 32)
+// with value row H + j (n % 64 >= 32), so every 64-column block of a tile (both tile widths are multiples of 64) holds
+// the g and v of 32 output columns; rows j >= H read as zeros.
+template <typename T>
+struct SwiGluPairOperand {
+  static constexpr bool kVec = true;
+  const T* w;
+  int H, K;
+  __device__ __forceinline__ int row(int n) const {
+    const int j = (n >> 6) * 32 + (n & 31);
+    return j < H ? ((n & 32) ? H + j : j) : -1;
+  }
+  __device__ __forceinline__ float operator()(int n, int k) const {
+    const int r = row(n);
+    return r < 0 ? 0.f : Elem<T>::ld(w + (long long)r * K + k);
+  }
+  __device__ __forceinline__ bool vec_ok() const { return (K & 3) == 0 && ((uintptr_t)w & 15) == 0; }
+  __device__ __forceinline__ float4 ld4k(int n, int k) const {
+    const int r = row(n);
+    return r < 0 ? make_float4(0.f, 0.f, 0.f, 0.f) : ld4(w + (long long)r * K + k);
+  }
+  __device__ __forceinline__ float4 ld4r(int n, int k) const {
+    return make_float4((*this)(n, k), (*this)(n + 1, k), (*this)(n + 2, k), (*this)(n + 3, k));
+  }
+  static constexpr long long s_k = 1, s_row = 0;  // k-contiguous (the launcher's vectorisation test)
+};
+// g = T(acc + T(b1[j])), v = T(acc' + T(b1[H + j])), s = T(silu(g)); act = T(T(s v) f); aux = [T(v silu'(g) f) | T(s f)]
+template <typename T>
+struct SwiGluEpilogue {
+  T* act;
+  T* aux;  // [M][2H] or null (act only)
+  const float* bias;
+  int H;
+  int drop;  // 0: f = 1, no product taken
+  DropView dv;
+  __device__ __forceinline__ void operator()(int m, int n, float acc, const float* crow, int n0) const {
+    if (n & 32) return;  // the value column: handled with its gate column
+    const int j = (n >> 6) * 32 + (n & 31);
+    if (j >= H) return;
+    const float g = Elem<T>::round(acc + Elem<T>::round(bias[j]));
+    const float v = Elem<T>::round(crow[n + 32 - n0] + Elem<T>::round(bias[H + j]));
+    float s, ds;
+    silu_and_grad(g, s, ds);
+    const float sr = Elem<T>::round(s);
+    float a = Elem<T>::round(__fmul_rn(sr, v)), lo = __fmul_rn(v, ds), hi = sr;
+    if (drop) {
+      const float f = dv.factor(dv.key(), m, j, H, dv.s);
+      a = __fmul_rn(a, f);
+      lo = __fmul_rn(lo, f);
+      hi = __fmul_rn(hi, f);
+    }
+    Elem<T>::st(act + (long long)m * H + j, a);
+    if (aux) {
+      Elem<T>::st(aux + (long long)m * 2 * H + j, lo);
+      Elem<T>::st(aux + (long long)m * 2 * H + H + j, hi);
+    }
+  }
+};
+// dh[m][j] = T(dA aux[m][j]), dh[m][H + j] = T(dA aux[m][H + j]) for the fp32 accumulator dA of (m, j)
+template <typename T>
+struct SwiGluBwdEpilogue {
+  T* dh;
+  const T* aux;
+  int H;
+  __device__ __forceinline__ void operator()(int m, int j, float acc, const float*, int) const {
+    const long long o = (long long)m * 2 * H + j;
+    Elem<T>::st(dh + o, __fmul_rn(acc, Elem<T>::ld(aux + o)));
+    Elem<T>::st(dh + o + H, __fmul_rn(acc, Elem<T>::ld(aux + o + H)));
+  }
+};
+
+template <typename T>
+static int swiglu_simt_t(const void* x, const void* w1, const float* b1, void* act, void* aux, int M, int H, int K,
+                         const DropView* dv, cudaStream_t st) {
+  StridedOperand<T> A{(const T*)x, K, 1};
+  SwiGluPairOperand<T> Bo{(const T*)w1, H, K};
+  SwiGluEpilogue<T> epi{(T*)act, (T*)aux, b1, H, dv != nullptr, dv ? *dv : DropView{}};
+  return launch_gemm<StridedOperand<T>, SwiGluPairOperand<T>, SwiGluEpilogue<T>, true, true>(A, Bo, epi, M, 64 * ceil_div(H, 32),
+                                                                                            K, 1, st);
+}
+int swiglu_simt(const void* x, const void* w1, const float* b1, void* act, void* aux, int M, int H, int K, int dtype,
+                const DropView* dv, cudaStream_t st) {
+  if (dtype == VRR_F32) return swiglu_simt_t<float>(x, w1, b1, act, aux, M, H, K, dv, st);
+  if (dtype == VRR_BF16) return swiglu_simt_t<__nv_bfloat16>(x, w1, b1, act, aux, M, H, K, dv, st);
+  return swiglu_simt_t<__half>(x, w1, b1, act, aux, M, H, K, dv, st);
+}
+
+template <typename T>
+static int swiglu_bwd_simt_t(const void* dy, const void* w2, const void* aux, void* dh, int M, int H, int K, cudaStream_t st) {
+  StridedOperand<T> A{(const T*)dy, K, 1};
+  StridedOperand<T> Bo{(const T*)w2, 1, H};  // op(B)[k][n] = w2[k][n]: fc2.weight [K][H]
+  SwiGluBwdEpilogue<T> epi{(T*)dh, (const T*)aux, H};
+  return launch_gemm<StridedOperand<T>, StridedOperand<T>, SwiGluBwdEpilogue<T>, true, false>(A, Bo, epi, M, H, K, 1, st);
+}
+int swiglu_bwd_simt(const void* dy, const void* w2, const void* aux, void* dh, int M, int H, int K, int dtype, cudaStream_t st) {
+  if (dtype == VRR_F32) return swiglu_bwd_simt_t<float>(dy, w2, aux, dh, M, H, K, st);
+  if (dtype == VRR_BF16) return swiglu_bwd_simt_t<__nv_bfloat16>(dy, w2, aux, dh, M, H, K, st);
+  return swiglu_bwd_simt_t<__half>(dy, w2, aux, dh, M, H, K, st);
+}
+
 void gemm_simt_set_tile(int v) { g_simt_tile.store(v == 64 ? 64 : 128); }
 
 int gemm_simt(const void* a, const void* b, void* c, int M, int N, int K, int ta, int tb, int dtype,

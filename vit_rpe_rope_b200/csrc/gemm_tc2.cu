@@ -27,6 +27,8 @@
 // bit for bit with biases off the bf16 grid.
 #include <string.h>
 
+#include <type_traits>
+
 #include "common.cuh"
 #include "kernels.h"
 #include "tc_common.cuh"
@@ -165,6 +167,42 @@ struct StoreEpiDrop : StoreEpi<T> {
   DropView dv;
 };
 
+// fc1 of a packed SwiGLU Mlp (vrr_gemm_swiglu).  The CTA pair stages gate rows (rank 0) and the matching value rows
+// (rank 1) of w1 through one 3-D map [2][H][K], so TMEM columns [0, BN/2) of the tile hold g and [BN/2, BN) hold v
+// for the same BN/2 output columns, and a ragged last tile is zero-filled within its half.  The epilogue writes act
+// (tmap_c) and the two halves of aux (tmap_c2 / tmap_c3: maps over aux[:, :H] / aux[:, H:], row stride 2H) - or act
+// alone when with_aux is 0.  Three [32 rows][128 B] staging buffers per warp.
+template <typename T, bool DROP>
+struct SwiGluEpi {
+  static constexpr int kSwiGlu = 1;
+  static constexpr int kStagingBytes = 12288;
+  static constexpr bool kDrop = DROP;
+  const float* bias;  // fp32 [2H]: gate biases, then value biases
+  int with_aux;
+  DropView dv;        // DROP only: mask of act [M][H]
+};
+
+// fc2's dX with the SwiGLU backward (vrr_gemm_swiglu_bwd): dA = dy . w2 stays in registers and is multiplied by the
+// two multiplier tiles aux[:, n..] and aux[:, H+n..] into the halves of dh (tmap_c / tmap_c2); fc1's bias gradient
+// is the column sums of both staged tiles (fp32 atomics, as StoreEpi::colsum).
+template <typename T>
+struct SwiGluBwdEpi {
+  static constexpr int kSwiGlu = 2;
+  const T* aux;   // [M][2H]
+  float* colsum;  // [2H], zeroed by the caller
+};
+
+// SwiGluKind<Epi>::value: 0 for the epilogues above these two, else their kSwiGlu.  Staging<Epi>::kBytes: shared
+// memory per epilogue warp.
+template <class E, class = void>
+struct SwiGluKind { static constexpr int value = 0; };
+template <class E>
+struct SwiGluKind<E, std::void_t<decltype(E::kSwiGlu)>> { static constexpr int value = E::kSwiGlu; };
+template <class E, class = void>
+struct Staging { static constexpr int kBytes = kWarpStaging; };
+template <class E>
+struct Staging<E, std::void_t<decltype(E::kStagingBytes)>> { static constexpr int kBytes = E::kStagingBytes; };
+
 // gelu(h) and d gelu / dh for TWO values at a time on the packed fp32x2 pipe (fma.rn.f32x2, sm_100): the epilogue of
 // fc1 is bound by its instruction count (128 x 256 outputs per CTA against ~6 100 tensor-clocks of MMA per tile), and
 // the scalar version (~20 FMA-pipe ops per element) made the GEMM run at half the speed of the plain one.
@@ -219,18 +257,21 @@ template <typename T, int BN, bool A_MN, bool B_MN, class Epi>
 __global__ void __launch_bounds__(kPairThreads, 1)
 gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                  const __grid_constant__ CUtensorMap tmap_c, const __grid_constant__ CUtensorMap tmap_c2,
-                 const PairShape g, const Epi epi) {
+                 const __grid_constant__ CUtensorMap tmap_c3, const PairShape g, const Epi epi) {
   constexpr int kBHalf = BN / 2;
   constexpr int kABytes = kPM * kPK * 2;
   constexpr int kBBytes = kBHalf * kPK * 2;
   constexpr int kStageBytes = kABytes + kBBytes;
-  constexpr int kStages = (kSmemBudget - 1024 - kEpiWarps * kWarpStaging - 512) / kStageBytes;
+  constexpr int kStg = Staging<Epi>::kBytes;
+  constexpr int kSwi = SwiGluKind<Epi>::value;
+  constexpr int kStages = (kSmemBudget - 1024 - kEpiWarps * kStg - 512) / kStageBytes;
   constexpr uint32_t kTmemCols = 2 * BN;  // two accumulator stages (256 or 512: powers of two)
   static_assert(kStages >= 3, "pipeline too shallow");
+  static_assert(kSwi != 1 || (BN == 256 && !A_MN && !B_MN), "the SwiGLU forward pairs 128 gate with 128 value columns");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* staging = smem + kStages * kStageBytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(staging + kEpiWarps * kWarpStaging);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(staging + kEpiWarps * kStg);
   uint64_t* bar_full = bars;                              // [kStages] leader's: both CTAs' TMA -> MMA
   uint64_t* bar_empty = bars + kStages;                   // [kStages] per CTA: MMA retired -> own TMA producer
   uint64_t* bar_acc_full = bars + 2 * kStages;            // [2] per CTA: accumulator ready -> own epilogue
@@ -272,7 +313,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         const int n_blk = t % g.tiles_n, m_blk = t / g.tiles_n;
         const int kb0 = (int)((long long)split * g.num_k / g.splits), kb1 = (int)((long long)(split + 1) * g.num_k / g.splits);
         const int m_row0 = m_blk * (2 * kPM) + (int)rank * kPM;
-        const int n_row0 = n_blk * BN + (int)rank * kBHalf;
+        [[maybe_unused]] const int n_row0 = n_blk * BN + (int)rank * kBHalf;
         for (int kb = kb0; kb < kb1; ++kb) {
           mbar_wait_cluster(&bar_empty[stage], phase ^ 1);
           const uint32_t full_leader = mapa(smem_u32(&bar_full[stage]), 0);
@@ -285,7 +326,9 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
 #pragma unroll
             for (int j = 0; j < kPM / 64; ++j) tma_load_2d_pair(sa + j * 8192, &tmap_a, full_leader, m_row0 + 64 * j, kb * kPK);
           }
-          if (!B_MN) {
+          if constexpr (kSwi == 1) {  // rank 0: gate rows, rank 1: the value rows of the same output columns
+            tma_load_3d_pair(sb, &tmap_b, full_leader, kb * kPK, n_blk * kBHalf, (int)rank);
+          } else if (!B_MN) {
             tma_load_2d_pair(sb, &tmap_b, full_leader, kb * kPK, n_row0);
           } else {
 #pragma unroll
@@ -324,6 +367,212 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         if (++acc == 2) { acc = 0; acc_phase ^= 1; }
       }
     }
+  } else if constexpr (kSwi == 1) {
+    // ============================ SwiGLU fc1 epilogue (both CTAs): act and aux from (g, v) ===============
+    // Warp half `chalf` takes output columns [64 chalf, 64 chalf + 64) of the tile: g at TMEM column c, v at
+    // BN/2 + c; two halves of 32 columns, every 8 columns stored to the three swizzled staging buffers as soon as
+    // they are computed (holding them for a later flush spilled registers).
+    const int ew = warp - 2, quad = warp & 3, chalf = ew >> 2;
+    uint8_t* my_stage = staging + ew * kStg;
+    const uint32_t sw = (uint32_t)(lane & 7);
+    const uint32_t row_base = smem_u32(my_stage) + (uint32_t)lane * 128u;
+    const int H = g.N;
+    [[maybe_unused]] uint2 key;
+    if constexpr (Epi::kDrop) key = epi.dv.key();
+    int acc = 0;
+    uint32_t acc_phase = 0;
+    for (int unit = cluster_id; unit < total_units; unit += num_clusters) {
+      const int n_blk = unit % g.tiles_n, m_blk = unit / g.tiles_n;  // one k-split
+      const int m_warp0 = m_blk * (2 * kPM) + (int)rank * kPM + quad * 32;
+      const int m = m_warp0 + lane;
+      const int n0 = n_blk * kBHalf + chalf * 64;
+      mbar_wait_cluster(&bar_acc_full[acc], acc_phase);
+      tc_fence_after();
+      const uint32_t tg = tmem_base + ((uint32_t)(quad * 32) << 16) + acc * BN + chalf * 64;
+      if (lane == 0) bulk_wait_read<0>();  // the previous unit's stores have left the staging buffers
+      __syncwarp();
+#pragma unroll 1
+      for (int hf = 0; hf < 2; ++hf) {
+        uint32_t v[64];
+        __syncwarp();
+        tmem_ld32(tg + hf * 32, *reinterpret_cast<uint32_t(*)[32]>(&v[0]));
+        tmem_ld32(tg + kBHalf + hf * 32, *reinterpret_cast<uint32_t(*)[32]>(&v[32]));
+        tmem_wait_ld();
+        if (hf == 1) {  // this warp has read everything it needs from the accumulator stage
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) mbar_arrive_cluster(mapa(smem_u32(&bar_acc_empty[acc]), 0));
+        }
+        const float* fa = reinterpret_cast<const float*>(v);
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          uint32_t oa[4], og[4], ov[4];
+          const int nb = max(min(n0 + hf * 32 + q * 8, H - 8), 0);  // H % 8 == 0; columns past H are clipped
+          const float4 bg0 = __ldg(reinterpret_cast<const float4*>(epi.bias + nb));
+          const float4 bg1 = __ldg(reinterpret_cast<const float4*>(epi.bias + nb + 4));
+          const float4 bv0 = __ldg(reinterpret_cast<const float4*>(epi.bias + H + nb));
+          const float4 bv1 = __ldg(reinterpret_cast<const float4*>(epi.bias + H + nb + 4));
+          // the biases as T (F.linear's cast), packed in pairs
+          const uint32_t bgp[4] = {Elem16<T>::pack2(bg0.x, bg0.y), Elem16<T>::pack2(bg0.z, bg0.w), Elem16<T>::pack2(bg1.x, bg1.y),
+                                   Elem16<T>::pack2(bg1.z, bg1.w)};
+          const uint32_t bvp[4] = {Elem16<T>::pack2(bv0.x, bv0.y), Elem16<T>::pack2(bv0.z, bv0.w), Elem16<T>::pack2(bv1.x, bv1.y),
+                                   Elem16<T>::pack2(bv1.z, bv1.w)};
+          [[maybe_unused]] uint32_t rw[4];
+          if constexpr (Epi::kDrop) {
+            const uint4 r = epi.dv.bits(key, ((unsigned long long)m * (unsigned)H + (unsigned)nb) >> 3);
+            rw[0] = r.x; rw[1] = r.y; rw[2] = r.z; rw[3] = r.w;
+          }
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            float a[2], lo[2], hi[2];
+            const float2 bg2 = Elem16<T>::unpack2(bgp[j]), bv2 = Elem16<T>::unpack2(bvp[j]);
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+              const int c = q * 8 + 2 * j + e;
+              const float gg = Elem16<T>::round(fa[c] + (e ? bg2.y : bg2.x));
+              const float vv = Elem16<T>::round(fa[32 + c] + (e ? bv2.y : bv2.x));
+              float s, ds;
+              silu_and_grad(gg, s, ds);
+              const float sr = Elem16<T>::round(s);
+              a[e] = Elem16<T>::round(__fmul_rn(sr, vv));
+              lo[e] = __fmul_rn(vv, ds);
+              hi[e] = sr;
+              if constexpr (Epi::kDrop) {
+                const float f = ((e ? (rw[j] >> 16) : (rw[j] & 0xFFFFu)) < epi.dv.t) ? epi.dv.s : 0.f;
+                a[e] = __fmul_rn(a[e], f);
+                lo[e] = __fmul_rn(lo[e], f);
+                hi[e] = __fmul_rn(hi[e], f);
+              }
+            }
+            oa[j] = Elem16<T>::pack2(a[0], a[1]);
+            og[j] = Elem16<T>::pack2(lo[0], lo[1]);
+            ov[j] = Elem16<T>::pack2(hi[0], hi[1]);
+          }
+          const uint32_t off = (((uint32_t)(hf * 4 + q) ^ sw) << 4);
+          st_shared_v4(row_base + off, oa[0], oa[1], oa[2], oa[3]);
+          if (epi.with_aux) {
+            st_shared_v4(row_base + 4096u + off, og[0], og[1], og[2], og[3]);
+            st_shared_v4(row_base + 8192u + off, ov[0], ov[1], ov[2], ov[3]);
+          }
+        }
+      }
+      fence_proxy_async_smem();
+      __syncwarp();
+      if (lane == 0) {
+        if (n0 < H && m_warp0 < g.M) {
+          tma_store_2d(&tmap_c, my_stage, n0, m_warp0);
+          if (epi.with_aux) {
+            tma_store_2d(&tmap_c2, my_stage + 4096, n0, m_warp0);
+            tma_store_2d(&tmap_c3, my_stage + 8192, n0, m_warp0);
+          }
+        }
+        bulk_commit();
+      }
+      if (++acc == 2) { acc = 0; acc_phase ^= 1; }
+    }
+    if (lane == 0) bulk_wait<0>();
+  } else if constexpr (kSwi == 2) {
+    // ==================== SwiGLU backward epilogue (both CTAs): dh halves and fc1's bias gradient ===============
+    const int ew = warp - 2, quad = warp & 3, chalf = ew >> 2;
+    constexpr int kChunks = BN / 2 / 64;
+    uint8_t* my_stage = staging + ew * kStg;
+    const uint32_t stage_u32 = smem_u32(my_stage);
+    const uint32_t sw = (uint32_t)(lane & 7);
+    const uint32_t row_base = stage_u32 + (uint32_t)lane * 128u;
+    const int H = g.N;
+    int acc = 0;
+    uint32_t acc_phase = 0;
+    for (int unit = cluster_id; unit < total_units; unit += num_clusters) {
+      const int n_blk = unit % g.tiles_n, m_blk = unit / g.tiles_n;  // one k-split
+      const int m_warp0 = m_blk * (2 * kPM) + (int)rank * kPM + quad * 32;
+      mbar_wait_cluster(&bar_acc_full[acc], acc_phase);
+      tc_fence_after();
+      const uint32_t trow = tmem_base + ((uint32_t)(quad * 32) << 16) + acc * BN + chalf * (BN / 2);
+#pragma unroll 1
+      for (int c = 0; c < kChunks; ++c) {
+        const int n0 = n_blk * BN + chalf * (BN / 2) + c * 64;
+        // the warp's [32 rows][64] tiles of aux[:, n0..] and aux[:, H + n0..], loaded coalesced (as StoreEpi::mul)
+        // while the TMEM load is in flight
+        uint4 ml[8], mh[8];
+        const int nb = max(min(n0 + (lane & 7) * 8, H - 8), 0);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const int mr = min(m_warp0 + i * 4 + (lane >> 3), g.M - 1);
+          const T* p = epi.aux + (size_t)mr * 2 * H + nb;
+          ml[i] = __ldg(reinterpret_cast<const uint4*>(p));
+          mh[i] = __ldg(reinterpret_cast<const uint4*>(p + H));
+        }
+        // "lane = row" through the two staging buffers (the previous chunk's stores have been read) BEFORE the TMEM
+        // load: the multipliers and the 64 accumulators held together spilled registers
+        if (lane == 0) bulk_wait_read<0>();
+        __syncwarp();
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const uint32_t r = (uint32_t)(i * 4 + (lane >> 3));
+          const uint32_t off = r * 128u + ((((uint32_t)lane & 7u) ^ (r & 7u)) << 4);
+          st_shared_v4(stage_u32 + off, ml[i].x, ml[i].y, ml[i].z, ml[i].w);
+          st_shared_v4(stage_u32 + 4096u + off, mh[i].x, mh[i].y, mh[i].z, mh[i].w);
+        }
+        uint32_t v[64];
+        __syncwarp();
+        tmem_ld32(trow + c * 64, *reinterpret_cast<uint32_t(*)[32]>(&v[0]));
+        tmem_ld32(trow + c * 64 + 32, *reinterpret_cast<uint32_t(*)[32]>(&v[32]));
+        tmem_wait_ld();
+        if (c == kChunks - 1) {  // this warp has read everything it needs from the accumulator stage
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) mbar_arrive_cluster(mapa(smem_u32(&bar_acc_empty[acc]), 0));
+        }
+        const float* fa = reinterpret_cast<const float*>(v);
+#pragma unroll
+        for (int c8 = 0; c8 < 8; ++c8) {  // each lane reads and overwrites its own row's chunk: no other lane touches it
+          const uint32_t off = (((uint32_t)c8 ^ sw) << 4);
+          const uint4 ml4 = ld_shared_v4(row_base + off), mh4 = ld_shared_v4(row_base + 4096u + off);
+          const uint32_t wl[4] = {ml4.x, ml4.y, ml4.z, ml4.w}, wh[4] = {mh4.x, mh4.y, mh4.z, mh4.w};
+          uint32_t ol[4], oh[4];
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            const float2 a2 = make_float2(fa[c8 * 8 + 2 * j], fa[c8 * 8 + 2 * j + 1]);
+            const float2 l2 = Elem16<T>::unpack2(wl[j]), h2 = Elem16<T>::unpack2(wh[j]);
+            ol[j] = Elem16<T>::pack2(__fmul_rn(a2.x, l2.x), __fmul_rn(a2.y, l2.y));
+            oh[j] = Elem16<T>::pack2(__fmul_rn(a2.x, h2.x), __fmul_rn(a2.y, h2.y));
+          }
+          st_shared_v4(row_base + off, ol[0], ol[1], ol[2], ol[3]);
+          st_shared_v4(row_base + 4096u + off, oh[0], oh[1], oh[2], oh[3]);
+        }
+        fence_proxy_async_smem();
+        __syncwarp();
+        const bool store_ok = n0 < H && m_warp0 < g.M;
+        if (lane == 0) {
+          if (store_ok) {
+            tma_store_2d(&tmap_c, my_stage, n0, m_warp0);
+            tma_store_2d(&tmap_c2, my_stage + 4096, n0, m_warp0);
+          }
+          bulk_commit();
+        }
+        if (store_ok) {
+          // column sums of both tiles as stored (rows past M hold zeros: their dy rows were zero-filled)
+          float s0 = 0.f, s1 = 0.f, t0 = 0.f, t1 = 0.f;
+          const uint32_t cbase = stage_u32 + ((uint32_t)lane & 3u) * 4u;
+#pragma unroll 8
+          for (uint32_t r = 0; r < 32; ++r) {
+            const uint32_t off = r * 128u + ((((uint32_t)lane >> 2) ^ (r & 7u)) << 4);
+            const float2 l2 = Elem16<T>::unpack2(ld_shared_u32(cbase + off));
+            const float2 h2 = Elem16<T>::unpack2(ld_shared_u32(cbase + 4096u + off));
+            s0 += l2.x; s1 += l2.y; t0 += h2.x; t1 += h2.y;
+          }
+          const int col = n0 + 2 * lane;
+          if (col < H) {
+            atomicAdd(epi.colsum + col, s0);
+            atomicAdd(epi.colsum + col + 1, s1);
+            atomicAdd(epi.colsum + H + col, t0);
+            atomicAdd(epi.colsum + H + col + 1, t1);
+          }
+        }
+      }
+      if (++acc == 2) { acc = 0; acc_phase ^= 1; }
+    }
+    if (lane == 0) bulk_wait<0>();
   } else {
     // ====================================== epilogue (both CTAs) ==========================================
     const int ew = warp - 2;
@@ -685,11 +934,11 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
   if (warp == 1) tmem_dealloc_pair(tmem_base, kTmemCols);
 }
 
-template <int BN>
+template <int BN, int STG>
 constexpr size_t pair_smem_bytes() {
   constexpr int stage = kPM * kPK * 2 + (BN / 2) * kPK * 2;
-  constexpr int stages = (kSmemBudget - 1024 - kEpiWarps * kWarpStaging - 512) / stage;
-  return 1024 + (size_t)stages * stage + kEpiWarps * kWarpStaging + 512;
+  constexpr int stages = (kSmemBudget - 1024 - kEpiWarps * STG - 512) / stage;
+  return 1024 + (size_t)stages * stage + kEpiWarps * STG + 512;
 }
 
 // Pick the k-split count for accumulate/reduce GEMMs so that the work units fill whole waves of clusters.
@@ -708,21 +957,11 @@ int pick_splits(int tiles, int num_k, int clusters) {
   return best;
 }
 
+// Launch on prebuilt maps (tc3_: a third output map, read by the SwiGLU forward only).
 template <typename T, int BN, bool A_MN, bool B_MN, class Epi>
-int launch_pair(const void* a, const void* b, int M, int N, int K, int splits, const CUtensorMap& tc_, const CUtensorMap& tc2_,
-                const Epi& epi, cudaStream_t st) {
-  CUtensorMap ta, tb;
-  if (!A_MN) { if (int rc = make_tmap_2d(&ta, a, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)K, (uint64_t)K * 2, kPM, 64)) return rc; }
-  else       { if (int rc = make_tmap_2d(&ta, a, Elem16<T>::kTmap, (uint64_t)K, (uint64_t)M, (uint64_t)M * 2, 64, 64)) return rc; }
-  if (!B_MN) { if (int rc = make_tmap_2d(&tb, b, Elem16<T>::kTmap, (uint64_t)N, (uint64_t)K, (uint64_t)K * 2, BN / 2, 64)) return rc; }
-  else       { if (int rc = make_tmap_2d(&tb, b, Elem16<T>::kTmap, (uint64_t)K, (uint64_t)N, (uint64_t)N * 2, 64, 64)) return rc; }
-  PairShape g;
-  g.M = M; g.N = N; g.K = K;
-  g.tiles_m = ceil_div(M, 2 * kPM);
-  g.tiles_n = ceil_div(N, BN);
-  g.num_k = ceil_div(K, kPK);
-  g.splits = splits < 1 ? 1 : (splits > g.num_k ? g.num_k : splits);
-  constexpr size_t smem = pair_smem_bytes<BN>();
+int launch_pair_maps(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc_, const CUtensorMap& tc2_,
+                     const CUtensorMap& tc3_, const PairShape& g, const Epi& epi, cudaStream_t st) {
+  constexpr size_t smem = pair_smem_bytes<BN, Staging<Epi>::kBytes>();
   auto kern = gemm_pair_kernel<T, BN, A_MN, B_MN, Epi>;
   VRR_SMEM_ATTR_ONCE(kern, smem);
   const int clusters_max = sm_count() / 2;
@@ -740,9 +979,26 @@ int launch_pair(const void* a, const void* b, int M, int N, int K, int splits, c
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  VRR_CUDA(cudaLaunchKernelEx(&cfg, kern, ta, tb, tc_, tc2_, g, epi));
+  VRR_CUDA(cudaLaunchKernelEx(&cfg, kern, ta, tb, tc_, tc2_, tc3_, g, epi));
   VRR_LAUNCHED();
   return VRR_OK;
+}
+
+template <typename T, int BN, bool A_MN, bool B_MN, class Epi>
+int launch_pair(const void* a, const void* b, int M, int N, int K, int splits, const CUtensorMap& tc_, const CUtensorMap& tc2_,
+                const Epi& epi, cudaStream_t st) {
+  CUtensorMap ta, tb;
+  if (!A_MN) { if (int rc = make_tmap_2d(&ta, a, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)K, (uint64_t)K * 2, kPM, 64)) return rc; }
+  else       { if (int rc = make_tmap_2d(&ta, a, Elem16<T>::kTmap, (uint64_t)K, (uint64_t)M, (uint64_t)M * 2, 64, 64)) return rc; }
+  if (!B_MN) { if (int rc = make_tmap_2d(&tb, b, Elem16<T>::kTmap, (uint64_t)N, (uint64_t)K, (uint64_t)K * 2, BN / 2, 64)) return rc; }
+  else       { if (int rc = make_tmap_2d(&tb, b, Elem16<T>::kTmap, (uint64_t)K, (uint64_t)N, (uint64_t)N * 2, 64, 64)) return rc; }
+  PairShape g;
+  g.M = M; g.N = N; g.K = K;
+  g.tiles_m = ceil_div(M, 2 * kPM);
+  g.tiles_n = ceil_div(N, BN);
+  g.num_k = ceil_div(K, kPK);
+  g.splits = splits < 1 ? 1 : (splits > g.num_k ? g.num_k : splits);
+  return launch_pair_maps<T, BN, A_MN, B_MN, Epi>(ta, tb, tc_, tc2_, tc2_, g, epi, st);
 }
 
 template <typename T, bool A_MN, bool B_MN>
@@ -864,6 +1120,64 @@ int gemm_tc_drop(const void* a, const void* b, void* c, void* c2, const float* b
               "gemm (tcgen05, dropout): unsupported shape M=%d N=%d K=%d", M, N, K);
   if (dtype == VRR_F16) return launch_store_drop<__half>(a, b, c, c2, bias, M, N, K, epilogue, dv, st);
   return launch_store_drop<__nv_bfloat16>(a, b, c, c2, bias, M, N, K, epilogue, dv, st);
+}
+
+// ---- SwiGLU Mlp: fc1 with the gated activation, fc2's dX with its backward ----------------------------------
+template <typename T, bool DROP>
+static int swiglu_tc_t(const void* x, const void* w1, const float* b1, void* act, void* aux, int M, int H, int K,
+                       const DropView& dv, cudaStream_t st) {
+  SwiGluEpi<T, DROP> epi = {};
+  epi.bias = b1;
+  epi.with_aux = aux != nullptr;
+  epi.dv = dv;
+  CUtensorMap ta, tb, tc_, tc2_, tc3_;
+  if (int rc = make_tmap_2d(&ta, x, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)K, (uint64_t)K * 2, kPM, 64)) return rc;
+  // w1 [2][H][K]: box [1][128 rows][64]; plane 0 = gate rows, plane 1 = value rows
+  if (int rc = make_tmap_3d(&tb, w1, Elem16<T>::kTmap, (uint64_t)K, (uint64_t)H, 2, (uint64_t)K * 2, (uint64_t)H * K * 2, 64, 128))
+    return rc;
+  if (int rc = make_tmap_2d(&tc_, act, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)H, (uint64_t)H * 2, 32, 64)) return rc;
+  tc2_ = tc3_ = tc_;
+  if (aux) {
+    if (int rc = make_tmap_2d(&tc2_, aux, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)H, (uint64_t)H * 4, 32, 64)) return rc;
+    if (int rc = make_tmap_2d(&tc3_, (const T*)aux + H, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)H, (uint64_t)H * 4, 32, 64))
+      return rc;
+  }
+  PairShape g;
+  g.M = M; g.N = H; g.K = K;
+  g.tiles_m = ceil_div(M, 2 * kPM);
+  g.tiles_n = ceil_div(H, 128);
+  g.num_k = ceil_div(K, kPK);
+  g.splits = 1;
+  return launch_pair_maps<T, 256, false, false, SwiGluEpi<T, DROP>>(ta, tb, tc_, tc2_, tc3_, g, epi, st);
+}
+
+int gemm_tc_swiglu(const void* x, const void* w1, const float* b1, void* act, void* aux, int M, int H, int K, int dtype,
+                   const DropView* dv, cudaStream_t st) {
+  if (dtype == VRR_F16) {
+    if (dv) return swiglu_tc_t<__half, true>(x, w1, b1, act, aux, M, H, K, *dv, st);
+    return swiglu_tc_t<__half, false>(x, w1, b1, act, aux, M, H, K, DropView{}, st);
+  }
+  if (dv) return swiglu_tc_t<__nv_bfloat16, true>(x, w1, b1, act, aux, M, H, K, *dv, st);
+  return swiglu_tc_t<__nv_bfloat16, false>(x, w1, b1, act, aux, M, H, K, DropView{}, st);
+}
+
+template <typename T>
+static int swiglu_bwd_tc_t(const void* dy, const void* w2, const void* aux, void* dh, float* db1, int M, int H, int K,
+                           cudaStream_t st) {
+  SwiGluBwdEpi<T> epi{(const T*)aux, db1};
+  CUtensorMap tc_, tc2_;  // the halves of dh [M][2H]
+  if (int rc = make_tmap_2d(&tc_, dh, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)H, (uint64_t)H * 4, 32, 64)) return rc;
+  if (int rc = make_tmap_2d(&tc2_, (T*)dh + H, Elem16<T>::kTmap, (uint64_t)M, (uint64_t)H, (uint64_t)H * 4, 32, 64)) return rc;
+  VRR_CUDA(cudaMemsetAsync(db1, 0, (size_t)2 * H * sizeof(float), st));
+  // dA = dy [M][K] . w2 [K][H]: w2 is fc2.weight, stored [K][N] (B_MN)
+  if (H > 128) return launch_pair<T, 256, false, true, SwiGluBwdEpi<T>>(dy, w2, M, H, K, 1, tc_, tc2_, epi, st);
+  return launch_pair<T, 128, false, true, SwiGluBwdEpi<T>>(dy, w2, M, H, K, 1, tc_, tc2_, epi, st);
+}
+
+int gemm_tc_swiglu_bwd(const void* dy, const void* w2, const void* aux, void* dh, float* db1, int M, int H, int K, int dtype,
+                       cudaStream_t st) {
+  if (dtype == VRR_F16) return swiglu_bwd_tc_t<__half>(dy, w2, aux, dh, db1, M, H, K, st);
+  return swiglu_bwd_tc_t<__nv_bfloat16>(dy, w2, aux, dh, db1, M, H, K, st);
 }
 
 // ---- QKV projection + RoPE epilogue on the CTA-pair kernel -----------------------------------------------

@@ -59,6 +59,10 @@ int patch_embed_fwd_simt(const void* images, const void* weight, const void* bia
 int patch_embed_bwd_simt(const void* images, const void* d_tokens, float* d_weight, float* d_bias, float* d_prefix,
                          float* d_pos, int B, int C, int Hi, int Wi, int P, int E, int npre, int img_dtype, int dtype,
                          int tok_dtype, cudaStream_t st);
+// SwiGLU Mlp on the FFMA kernels (any H, K; dv NULL: no dropout; aux NULL: act only).  The backward writes dh only.
+int swiglu_simt(const void* x, const void* w1, const float* b1, void* act, void* aux, int M, int H, int K, int dtype,
+                const DropView* dv, cudaStream_t st);
+int swiglu_bwd_simt(const void* dy, const void* w2, const void* aux, void* dh, int M, int H, int K, int dtype, cudaStream_t st);
 int patch_prefix_rows(void* tokens, const void* prefix, int B, int Np, int E, int npre, int tok_dtype, cudaStream_t st);
 
 // gemm_tc2.cu (tcgen05 CTA pairs, cta_group::2: every operand layout, TMA-store epilogues)
@@ -68,6 +72,12 @@ int gemm_tc(const void* a, const void* b, void* c, void* c2, const float* bias, 
 // fc1 with element dropout on the GELU outputs (VRR_EPI_BIAS_GELU_GRAD / _ACT, trans_a 0, trans_b 1, C of dtype)
 int gemm_tc_drop(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int dtype,
                  int epilogue, const DropView& dv, cudaStream_t st);
+// SwiGLU Mlp (vrr.h: vrr_gemm_swiglu / vrr_gemm_swiglu_bwd): 16-bit, H % 8 == 0, K % 8 == 0, 16-byte aligned pointers.
+// dv NULL: no dropout; aux NULL: act only.  The backward writes db1 (it zeroes it first).
+int gemm_tc_swiglu(const void* x, const void* w1, const float* b1, void* act, void* aux, int M, int H, int K, int dtype,
+                   const DropView* dv, cudaStream_t st);
+int gemm_tc_swiglu_bwd(const void* dy, const void* w2, const void* aux, void* dh, float* db1, int M, int H, int K, int dtype,
+                       cudaStream_t st);
 // colsum (16-bit C, plain / bias / multiply epilogues): colsum[n] += sum_m C[m][n] of the values as stored; zeroed by the caller
 int rope_pack_tables(const float* cos_tab, const float* sin_tab, float* packed, int heads, int rows, int hd, cudaStream_t st);
 bool qkv_rope_fwd_tc_supported(int B, int N, int E, int H);

@@ -227,6 +227,14 @@ __device__ __forceinline__ void tma_load_2d_pair(void* smem_dst, const CUtensorM
       ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar_cluster_addr), "r"(c0), "r"(c1)
       : "memory");
 }
+// The same through a 3-D map (box [1][rows][cols]): the packed SwiGLU fc1 weight, plane c2 = gate (0) / value (1).
+__device__ __forceinline__ void tma_load_3d_pair(void* smem_dst, const CUtensorMap* map, uint32_t bar_cluster_addr, int c0,
+                                                 int c1, int c2) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
+      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2)
+      : "memory");
+}
 // TMA stores shared -> global (bulk async-group completion)
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void* smem_src, int c0, int c1) {
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"

@@ -476,6 +476,56 @@ int vrr_gemm_mul_colsum(const void* a, const void* b, void* c, const void* mul, 
   return colsum(c, col_sums, M, N, dtype, (cudaStream_t)stream);
 }
 
+// tcgen05 SwiGLU kernels: 16-bit, H and K multiples of 8 (TMA row strides, the 8-column bias / mask groups), pointers
+// 16-byte aligned (the value half of aux / dh starts H elements into each row)
+static bool swiglu_tc_ok(int dtype, int M, int H, int K, const void* p0, const void* p1, const void* p2, const void* p3,
+                         const void* p4) {
+  return is16(dtype) && H % 8 == 0 && K % 8 == 0 && (long long)M * 2 * H < (1ll << 40) &&
+         ((((uintptr_t)p0 | (uintptr_t)p1 | (uintptr_t)p2 | (uintptr_t)p3 | (uintptr_t)p4)) & 15) == 0;
+}
+
+int vrr_gemm_swiglu(const void* x, const void* w1, const float* b1, void* act, void* aux, int M, int H, int K, int dtype,
+                    const vrr_drop_desc* drop, void* stream) {
+  VRR_REQUIRE(x && w1 && b1 && act, VRR_ERR_INVALID_ARG, "gemm_swiglu: NULL pointer");
+  VRR_REQUIRE(M > 0 && H > 0 && K > 0, VRR_ERR_INVALID_ARG, "gemm_swiglu: bad sizes M=%d H=%d K=%d", M, H, K);
+  VRR_REQUIRE(dtype_ok(dtype), VRR_ERR_INVALID_ARG, "gemm_swiglu: bad dtype %d", dtype);
+  VRR_REQUIRE(!drop || drop->p_path == 0.f, VRR_ERR_INVALID_ARG, "gemm_swiglu: p_path must be 0");
+  DropView dv = {};
+  bool active = false;
+  if (int rc = drop_view(drop, M, H, &dv, &active)) return rc;
+  if (int rc = require_device()) return rc;
+  const int impl = g_impl.load();
+  if (impl != VRR_IMPL_SIMT && swiglu_tc_ok(dtype, M, H, K, x, w1, b1, act, aux)) {
+    VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
+    return gemm_tc_swiglu(x, w1, b1, act, aux, M, H, K, dtype, active ? &dv : nullptr, (cudaStream_t)stream);
+  }
+  VRR_REQUIRE(impl != VRR_IMPL_TCGEN05 || !is16(dtype), VRR_ERR_UNSUPPORTED,
+              "gemm_swiglu: tcgen05 kernel forced but M=%d H=%d K=%d needs H %% 8 == 0, K %% 8 == 0 and 16-byte aligned "
+              "pointers", M, H, K);
+  VRR_COUNT_FAMILY(VRR_IMPL_SIMT);
+  return swiglu_simt(x, w1, b1, act, aux, M, H, K, dtype, active ? &dv : nullptr, (cudaStream_t)stream);
+}
+
+int vrr_gemm_swiglu_bwd(const void* dy, const void* w2, const void* aux, void* dh, float* db1, int M, int H, int K, int dtype,
+                        void* stream) {
+  VRR_REQUIRE(dy && w2 && aux && dh && db1, VRR_ERR_INVALID_ARG, "gemm_swiglu_bwd: NULL pointer");
+  VRR_REQUIRE(M > 0 && H > 0 && K > 0 && H % 2 == 0, VRR_ERR_INVALID_ARG,
+              "gemm_swiglu_bwd: bad sizes M=%d H=%d K=%d (H %% 2 == 0)", M, H, K);
+  VRR_REQUIRE(dtype_ok(dtype), VRR_ERR_INVALID_ARG, "gemm_swiglu_bwd: bad dtype %d", dtype);
+  if (int rc = require_device()) return rc;
+  const int impl = g_impl.load();
+  if (impl != VRR_IMPL_SIMT && swiglu_tc_ok(dtype, M, H, K, dy, w2, aux, dh, db1)) {
+    VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
+    return gemm_tc_swiglu_bwd(dy, w2, aux, dh, db1, M, H, K, dtype, (cudaStream_t)stream);
+  }
+  VRR_REQUIRE(impl != VRR_IMPL_TCGEN05 || !is16(dtype), VRR_ERR_UNSUPPORTED,
+              "gemm_swiglu_bwd: tcgen05 kernel forced but M=%d H=%d K=%d needs H %% 8 == 0, K %% 8 == 0 and 16-byte "
+              "aligned pointers", M, H, K);
+  VRR_COUNT_FAMILY(VRR_IMPL_SIMT);
+  if (int rc = swiglu_bwd_simt(dy, w2, aux, dh, M, H, K, dtype, (cudaStream_t)stream)) return rc;
+  return colsum(dh, db1, M, 2 * H, dtype, (cudaStream_t)stream);
+}
+
 int vrr_attn_fwd(const void* planes, const vrr_bias_desc* bias, void* out, float* lse, int B, int H, int N,
                  int Dh, float scale, int dtype, void* stream) {
   VRR_REQUIRE(planes && out && lse, VRR_ERR_INVALID_ARG, "attn_fwd: NULL pointer");

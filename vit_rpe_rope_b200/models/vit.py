@@ -26,7 +26,14 @@ skips them (``num_prefix_tokens = 1 + R``).
 LayerScale (``VisionTransformer(init_values=)``, timm's name; DeiT III, DINOv2, DINOv3): a learnable per-channel
 ``gamma`` multiplies each residual branch before it is added.  Inside the fused block loop the add+LayerNorm kernels
 apply it in fp32 as they read the branch and reduce its gradient in the same backward pass.
+
+SwiGLU MLP (``VisionTransformer(mlp_layer=SwiGLUPacked)``, timm's ``GluMlp`` / ``SwiGLUPacked``; EVA-02, DINOv3):
+``fc2(silu(x W_g + b_g) * (x W_v + b_v))`` with the gate and value rows packed in ``fc1``.  fc1's GEMM pairs each gate
+column with its value column and applies SiLU, the product and drop1 in its epilogue; fc2's dX GEMM applies the
+backward.
 """
+import functools
+
 import torch
 import torch.nn as nn
 
@@ -113,6 +120,55 @@ class Mlp(nn.Module):
         return self.fc2(self.drop1(self.act(self.fc1(x))))
 
 
+class GluMlp(nn.Module):
+    """Gated MLP with timm's names and layout (timm.layers.GluMlp without ``use_conv``): fc1 is ``hidden_features``
+    wide (even), its output is split into halves ``x1, x2`` and ``act(x1) * x2`` (or ``x1 * act(x2)`` with
+    ``gate_last``) feeds fc2 (``hidden_features // 2`` -> out).  ``SwiGLUPacked`` (SiLU on the first half) runs fc1,
+    the gate and the product in one GEMM epilogue on CUDA, with drop1 there as in ``Mlp``; other configurations run
+    this module's torch forward."""
+
+    def __init__(self, in_features, hidden_features=None, out_features=None, act_layer=nn.Sigmoid, norm_layer=None,
+                 bias=True, drop=0., gate_last=True):
+        super().__init__()
+        out_features = out_features or in_features
+        hidden_features = hidden_features or in_features
+        assert hidden_features % 2 == 0
+        bias = bias if isinstance(bias, (tuple, list)) else (bias, bias)
+        drop_probs = drop if isinstance(drop, (tuple, list)) else (drop, drop)
+        self.chunk_dim = -1
+        self.gate_last = gate_last  # use second half of width for gate
+        self.fc1 = nn.Linear(in_features, hidden_features, bias=bias[0])
+        self.act = act_layer()
+        self.drop1 = nn.Dropout(drop_probs[0])
+        self.norm = norm_layer(hidden_features // 2) if norm_layer is not None else nn.Identity()
+        self.fc2 = nn.Linear(hidden_features // 2, out_features, bias=bias[1])
+        self.drop2 = nn.Dropout(drop_probs[1])
+
+    def forward(self, x):
+        drop1 = None
+        if self.training and _drop_p(self.drop1) > 0 and x.is_cuda:
+            drop1 = (_drop_p(self.drop1), 0., 1, 0, ops.new_seed(x.device))
+        return self.drop2(self._branch(x, drop1))
+
+    def _branch(self, x, drop1=None):
+        """fc2(norm(drop1(gate(fc1(x))))) without drop2; ``drop1``: the dropout site of fc1's epilogue, or None."""
+        if ops.can_fuse_swiglu(x, self):
+            dt = ops.compute_dtype(x)
+            return ops.swiglu_mlp(x, self.fc1, self.fc2, ops.lp_weight(self.fc1.weight, dt),
+                                  ops.lp_weight(self.fc2.weight, dt), drop1)
+        x1, x2 = self.fc1(x).chunk(2, dim=self.chunk_dim)
+        x = x1 * self.act(x2) if self.gate_last else self.act(x1) * x2
+        return self.fc2(self.norm(self.drop1(x)))
+
+
+SwiGLUPacked = functools.partial(GluMlp, act_layer=nn.SiLU, gate_last=False)
+
+
+def _is_glu_factory(layer):
+    return ((isinstance(layer, type) and issubclass(layer, GluMlp))
+            or (isinstance(layer, functools.partial) and isinstance(layer.func, type) and issubclass(layer.func, GluMlp)))
+
+
 class Attention(nn.Module):
     """Multi-head self-attention (reference vit.py:14-98) on the fused kernels."""
 
@@ -160,17 +216,23 @@ class Attention(nn.Module):
 
 class Block(nn.Module):
     """Pre-LN transformer block (reference vit.py:100-129); ``init_values`` adds timm's LayerScale ``ls1`` / ``ls2``
-    (None or 0: none, the reference's block)."""
+    (None or 0: none, the reference's block).  ``mlp_layer``: ``Mlp`` (default) or a ``GluMlp`` factory such as
+    ``SwiGLUPacked``, built with ``hidden_features = int(dim * mlp_ratio)`` (fc1's width) as timm does."""
 
     def __init__(self, dim, num_heads, mlp_ratio=4., qkv_bias=False, drop=0., attn_drop=0.,
-                 drop_path=0., act_layer=nn.GELU, norm_layer=nn.LayerNorm, init_values=None):
+                 drop_path=0., act_layer=nn.GELU, norm_layer=nn.LayerNorm, init_values=None, mlp_layer=Mlp):
         super().__init__()
+        if mlp_layer is not Mlp and not _is_glu_factory(mlp_layer):
+            raise ValueError(f"mlp_layer must be Mlp or a GluMlp factory (e.g. SwiGLUPacked), got {mlp_layer!r}")
         self.norm1 = norm_layer(dim)
         self.attn = Attention(dim, num_heads=num_heads, qkv_bias=qkv_bias, attn_drop=attn_drop, proj_drop=drop)
         self.ls1 = LayerScale(dim, init_values) if init_values else nn.Identity()
         self.drop_path = DropPath(drop_path) if drop_path > 0. else nn.Identity()
         self.norm2 = norm_layer(dim)
-        self.mlp = Mlp(in_features=dim, hidden_features=int(dim * mlp_ratio), act_layer=act_layer, drop=drop)
+        if mlp_layer is Mlp:
+            self.mlp = Mlp(in_features=dim, hidden_features=int(dim * mlp_ratio), act_layer=act_layer, drop=drop)
+        else:
+            self.mlp = mlp_layer(in_features=dim, hidden_features=int(dim * mlp_ratio), drop=drop)
         self.ls2 = LayerScale(dim, init_values) if init_values else nn.Identity()
 
     def forward(self, x, freqs_cis=None):
@@ -197,14 +259,19 @@ class VisionTransformer(nn.Module):
 
     ``init_values`` gives every block LayerScale (``blocks.{i}.ls1.gamma`` / ``ls2.gamma`` [E], filled with the value;
     no random numbers are drawn); None or 0, the default, means none.
+
+    ``mlp_layer`` is every block's MLP: ``Mlp`` (default) or a ``GluMlp`` factory; ``SwiGLUPacked`` with
+    ``mlp_ratio = 16 / 3`` matches the GELU MLP's parameters and FLOPs (fc1 ``E -> 2H``, fc2 ``H -> E``).
     """
 
     def __init__(self, img_size=32, patch_size=4, in_chans=3, num_classes=10,
                  embed_dim=192, depth=6, num_heads=6, mlp_ratio=4.,
                  pos_encoding='absolute', rope_theta=100.0,
                  poly_degree=3, poly_shared_heads=True, drop_rate=0., drop_path_rate=0., reg_tokens=0,
-                 init_values=None):
+                 init_values=None, mlp_layer=Mlp):
         super().__init__()
+        if mlp_layer is not Mlp and not _is_glu_factory(mlp_layer):
+            raise ValueError(f"mlp_layer must be Mlp or a GluMlp factory (e.g. SwiGLUPacked), got {mlp_layer!r}")
         if reg_tokens < 0:
             raise ValueError(f"reg_tokens must be >= 0, got {reg_tokens}")
         if reg_tokens > 0 and pos_encoding in ('relative', 'polynomial'):
@@ -244,7 +311,7 @@ class VisionTransformer(nn.Module):
 
         dpr = [r.item() for r in torch.linspace(0, drop_path_rate, depth)]  # draws no random numbers
         self.blocks = nn.ModuleList([Block(embed_dim, num_heads, mlp_ratio, drop=drop_rate, drop_path=dpr[i],
-                                           init_values=init_values) for i in range(depth)])
+                                           init_values=init_values, mlp_layer=mlp_layer) for i in range(depth)])
         if not self.use_pos_embed_in_forward:
             for blk in self.blocks:
                 blk.set_pos_encoding(self.pos_embed)  # one shared module, referenced by every block
@@ -338,13 +405,13 @@ class VisionTransformer(nn.Module):
         ws = [self.head.weight]
         for blk in self.blocks:
             ws += [blk.attn.qkv.weight, blk.attn.proj.weight]
-            if isinstance(blk.mlp, Mlp):
+            if isinstance(blk.mlp, (Mlp, GluMlp)):
                 ws += [blk.mlp.fc1.weight, blk.mlp.fc2.weight]
         return ws
 
     def _fusable(self, x):
         return len(self.blocks) > 0 and all(
-            type(blk) is Block and type(blk.drop_path) in (nn.Identity, DropPath) and type(blk.mlp) is Mlp
+            type(blk) is Block and type(blk.drop_path) in (nn.Identity, DropPath) and type(blk.mlp) in (Mlp, GluMlp)
             and type(blk.ls1) in (nn.Identity, LayerScale) and type(blk.ls2) in (nn.Identity, LayerScale)
             and type(blk.attn.proj_drop) is nn.Dropout and type(blk.mlp.drop2) is nn.Dropout
             and ops.can_fuse_add_layer_norm(x, blk.norm1) and ops.can_fuse_add_layer_norm(x, blk.norm2)

@@ -759,6 +759,79 @@ def can_fuse_mlp(x, m) -> bool:
             and isinstance(m.drop2, (torch.nn.Dropout, torch.nn.Identity)))
 
 
+class SwiGLUMlpFn(torch.autograd.Function):
+    """fc1 -> SwiGLU -> fc2 (timm ``SwiGLUPacked``: ``fc2(silu(x W_g^T + b_g) * (x W_v^T + b_v))``, fc1.weight holding
+    the gate rows then the value rows).  fc1's GEMM pairs each gate column with its value column and writes the
+    activation and both partial derivatives (``vrr_gemm_swiglu``); fc2 adds its bias.  Backward: fc2's dX GEMM applies
+    the SwiGLU backward and sums fc1's bias gradient (``vrr_gemm_swiglu_bwd``); dW2, dX and dW1 are plain GEMMs."""
+
+    @staticmethod
+    def forward(ctx, x, w1, b1, w2, b2, w1_lp=None, w2_lp=None, drop1=None):
+        """``drop1``: element dropout on the activation (a site with p_path 0), applied in fc1's epilogue to the
+        activation and to both derivatives - the backward is then Dropout's backward unchanged."""
+        _require_cuda(x, w1, b1, w2, b2)
+        lib = _lib.load()
+        dt = x.dtype
+        w1l = (w1_lp if w1_lp is not None else w1.detach().to(dt)).detach().contiguous()
+        w2l = (w2_lp if w2_lp is not None else w2.detach().to(dt)).detach().contiguous()
+        x2 = x.reshape(-1, x.shape[-1]).contiguous()
+        M, K, H = x2.shape[0], x2.shape[1], w1l.shape[0] // 2
+        b1_32 = _f32c(b1)
+        grad = any(ctx.needs_input_grad)
+        act = torch.empty(M, H, device=x.device, dtype=dt)
+        aux = torch.empty(M, 2 * H, device=x.device, dtype=dt) if grad else None  # inference: the activation alone
+        d = _drop_desc(drop1) if drop1 is not None else None
+        with torch.cuda.device(x.device), _timed("fc1_fwd"):
+            _lib.check(lib.vrr_gemm_swiglu(_ptr(x2), _ptr(w1l), _ptr(b1_32), _ptr(act), _ptr(aux), M, H, K, _DT[dt],
+                                           ctypes.byref(d) if d is not None else None, _stream()), "vrr_gemm_swiglu")
+        y = _gemm(act, w2l, False, True, dt, bias=b2, epilogue=_lib.EPI_BIAS, name="fc2_fwd")
+        if grad:
+            ctx.save_for_backward(x2, aux, act, w1l, w2l)
+            ctx.meta = (x.shape, w1.dtype, b1.dtype, w2.dtype, b2.dtype)
+        return y.view(*x.shape[:-1], w2l.shape[0])
+
+    @staticmethod
+    def backward(ctx, dy):
+        x2, aux, act, w1l, w2l = ctx.saved_tensors
+        x_shape, w1_dt, b1_dt, w2_dt, b2_dt = ctx.meta
+        lib = _lib.load()
+        dy2 = dy.contiguous().view(-1, dy.shape[-1])
+        if dy2.dtype != x2.dtype:
+            dy2 = dy2.to(x2.dtype)
+        M, K, H = dy2.shape[0], dy2.shape[1], act.shape[1]
+        with torch.cuda.device(dy.device):
+            dh = torch.empty(M, 2 * H, device=dy2.device, dtype=x2.dtype)
+            db1 = torch.empty(2 * H, device=dy2.device, dtype=torch.float32)
+            with _timed("fc2_dx"):
+                _lib.check(lib.vrr_gemm_swiglu_bwd(_ptr(dy2), _ptr(w2l), _ptr(aux), _ptr(dh), _ptr(db1), M, H, K,
+                                                   _DT[x2.dtype], _stream()), "vrr_gemm_swiglu_bwd")
+            dw2 = _gemm(dy2, act, True, False, w2_dt, name="fc2_dw")
+            with _timed("colsum"):
+                db2 = _colsum(dy2).to(b2_dt)
+            dx = _gemm(dh, w1l, False, False, x2.dtype, name="fc1_dx").view(x_shape)
+            dw1 = _gemm(dh, x2, True, False, w1_dt, name="fc1_dw")
+        return dx, dw1, db1.to(b1_dt), dw2, db2, None, None, None
+
+
+def swiglu_mlp(x, fc1: torch.nn.Linear, fc2: torch.nn.Linear, w1_lp=None, w2_lp=None, drop1=None):
+    dt = compute_dtype(x)
+    if w1_lp is not None and (w1_lp.dtype != dt or w2_lp is None or w2_lp.dtype != dt):
+        w1_lp = w2_lp = None
+    return SwiGLUMlpFn.apply(x.to(dt), fc1.weight, fc1.bias, fc2.weight, fc2.bias, w1_lp, w2_lp, drop1)
+
+
+def can_fuse_swiglu(x, m) -> bool:
+    """timm's SwiGLUPacked: SiLU on the first half of fc1's output (gate_last False), no norm inside, both biases; the
+    hidden width H is even and fc2's output width a multiple of 4 (the bias-gradient kernels), and H % 8 == 0 when
+    drop1 is on (the mask's groups).  The caller applies drop2."""
+    p1 = getattr(m.drop1, "p", 0.0) if isinstance(m.drop1, torch.nn.Dropout) else None
+    H = m.fc1.out_features // 2
+    return (x.is_cuda and x.dtype in _DT and type(m.act) is torch.nn.SiLU and not m.gate_last
+            and type(m.norm) is torch.nn.Identity and m.fc1.bias is not None and m.fc2.bias is not None
+            and m.fc1.out_features % 2 == 0 and H % 2 == 0 and m.fc2.in_features == H and m.fc2.out_features % 4 == 0
+            and p1 is not None and (p1 == 0.0 or H % 8 == 0) and isinstance(m.drop2, (torch.nn.Dropout, torch.nn.Identity)))
+
+
 # ------------------------------------------------------------------------------------------------
 class RopeApplyFn(torch.autograd.Function):
     """Stand-alone rotate-half of q and k (public ``apply_rotary_emb``, rope_utils.py:3-37)."""
