@@ -220,6 +220,33 @@ int vrr_qkv_rope_bwd_prefix(const void* d_planes, const void* planes, const floa
                             void* d_qkv, float* d_cos, float* d_sin, int B, int N, int E, int H, int n_prefix,
                             int rope_mode, int dtype, void* stream);
 
+/* QK-norm (timm's Attention(qk_norm=True); ViT-22B): a LayerNorm over the Dh channels of every q and k head row,
+ * including the prefix rows, before RoPE.  q_norm and k_norm are affine with weight / bias qn_w, qn_b / kn_w, kn_b
+ * (fp32 [Dh], shared by all heads, all required) and one `eps`.  For every token row and head, with T = `dtype`:
+ *   1. x = T(acc), the projection rounded to T (nn.Linear's output under autocast; x = acc for fp32);
+ *   2. mean = sum(x) / Dh, var = sum((x - mean)^2) / Dh (biased), rstd = rsqrtf(var + eps), all in fp32;
+ *      xhat = (x - mean) * rstd and y = xhat * g + b, each without FMA contraction of the subtraction and product;
+ *   3. rows t >= n_prefix: y rotated by RoPE in fp32 as in vrr_qkv_rope_fwd_prefix;
+ *   4. the result rounded to T once.  The v plane is the plain projection, as without the norm.
+ * (Without the norm the q / k rows are rotated from the unrounded accumulator: step 1 is what the backward saves.)
+ * Saved outputs (both or neither; NULL: inference): qk_pre [2][B][H][N][Dh] of T, the x of q (plane 0) and k
+ * (plane 1) in the layout of planes; qk_stats fp32 [2][B][H][N][2] = {mean, rstd}.  Arguments and kernel family
+ * choice are those of vrr_qkv_rope_fwd_prefix.  qk_pre / the norm tensors must be 16-byte aligned. */
+int vrr_qkv_rope_norm_fwd(const void* x, const void* w_qkv, const float* cos_tab, const float* sin_tab, const float* packed,
+                          void* planes, int B, int N, int E, int H, int n_prefix, int rope_mode, int dtype, const float* qn_w,
+                          const float* qn_b, const float* kn_w, const float* kn_b, float eps, void* qk_pre, float* qk_stats,
+                          void* stream);
+/* Backward of vrr_qkv_rope_norm_fwd from its saved outputs.  Per q / k row, dy = the un-rotated d_planes row in fp32
+ * (d_planes itself on prefix rows), xhat recomputed from qk_pre / qk_stats as in the forward:
+ *   d_qkv = T(rstd (g dy - mean(g dy) - xhat mean(g dy xhat)))   (v columns: d_planes[2] unchanged)
+ *   d_g = sum dy xhat, d_b = sum dy over images, tokens and heads (fp32 atomics: reproducible to ~1e-6, not bitwise)
+ *   d_cos / d_sin as in vrr_qkv_rope_bwd_prefix with the un-rotated value y = xhat g + b, recomputed bit for bit.
+ * d_qn_w, d_qn_b, d_kn_w, d_kn_b [Dh] are written (not accumulated): all four or none; d_cos / d_sin both or neither. */
+int vrr_qkv_rope_norm_bwd(const void* d_planes, const void* qk_pre, const float* qk_stats, const float* cos_tab,
+                          const float* sin_tab, const float* qn_w, const float* qn_b, const float* kn_w, const float* kn_b,
+                          void* d_qkv, float* d_cos, float* d_sin, float* d_qn_w, float* d_qn_b, float* d_kn_w,
+                          float* d_kn_b, int B, int N, int E, int H, int n_prefix, int rope_mode, int dtype, void* stream);
+
 /* Stand-alone rotate-half of rope_utils.py:3-37 (the public apply_rotary_emb): q,k [B][H][Nr][Dh]
  * dense, cos/sin fp32 [Nr][Dh/2] (AXIAL) or [H][Nr][Dh/2] (MIXED); every row is rotated.
  * inverse != 0 applies the transpose rotation (the gradient w.r.t. q,k). */

@@ -19,6 +19,7 @@ Additions (all off by default, so a reference command line behaves like the refe
   --reg_tokens R     R register tokens after the cls token (timm's reg_tokens; not with relative / polynomial)
   --init_values V    LayerScale in every block, gamma initialised to V (timm's init_values, e.g. 1e-5 as in DeiT III)
   --mlp_layer swiglu every block's MLP is timm's SwiGLUPacked (fc2(silu(x W_g + b_g) * (x W_v + b_v))) instead of Mlp
+  --qk_norm          QK-norm in every attention: LayerNorm of each q / k head row before RoPE (timm's qk_norm)
   --mlp_ratio R      fc1's width over embed_dim (default 4; 5.33334 gives a SwiGLU MLP the GELU MLP's parameters)
 There is no CPU path: a CUDA sm_100 device is required.
 """
@@ -73,6 +74,7 @@ def get_args(argv=None):
     p.add_argument("--reg_tokens", type=int, default=0, help="register tokens after the cls token")
     p.add_argument("--init_values", type=float, default=None, help="LayerScale initial value (default: no LayerScale)")
     p.add_argument("--mlp_layer", type=str, default="mlp", choices=["mlp", "swiglu"], help="Mlp (GELU) or SwiGLUPacked")
+    p.add_argument("--qk_norm", action="store_true", help="LayerNorm of each q / k head row before RoPE")
     p.add_argument("--mlp_ratio", type=float, default=4.0, help="fc1 width / embed_dim")
     return p.parse_args(argv)
 
@@ -168,7 +170,8 @@ def main(argv=None):
                               poly_shared_heads=args.poly_shared_heads, drop_rate=args.drop_rate,
                               drop_path_rate=args.drop_path_rate, reg_tokens=args.reg_tokens,
                               init_values=args.init_values, mlp_ratio=args.mlp_ratio,
-                              mlp_layer=SwiGLUPacked if args.mlp_layer == "swiglu" else Mlp).to(device)
+                              mlp_layer=SwiGLUPacked if args.mlp_layer == "swiglu" else Mlp,
+                              qk_norm=args.qk_norm).to(device)
     criterion = nn.CrossEntropyLoss()
     optimizer = torch.optim.AdamW(model.parameters(), lr=args.lr, weight_decay=args.weight_decay)
     scheduler = torch.optim.lr_scheduler.CosineAnnealingLR(optimizer, T_max=args.epochs)

@@ -60,6 +60,8 @@ SIGNATURES = {
     "vrr_qkv_rope_bwd": (c_int, [c_void_p] * 7 + [c_int] * 6 + [c_void_p]),
     "vrr_qkv_rope_fwd_prefix": (c_int, [c_void_p] * 6 + [c_int] * 7 + [c_void_p]),
     "vrr_qkv_rope_bwd_prefix": (c_int, [c_void_p] * 7 + [c_int] * 7 + [c_void_p]),
+    "vrr_qkv_rope_norm_fwd": (c_int, [c_void_p] * 6 + [c_int] * 7 + [c_void_p] * 4 + [c_float] + [c_void_p] * 3),
+    "vrr_qkv_rope_norm_bwd": (c_int, [c_void_p] * 16 + [c_int] * 7 + [c_void_p]),
     "vrr_rope_apply": (c_int, [c_void_p] * 6 + [c_int] * 7 + [c_void_p]),
     "vrr_rope_table_grad": (c_int, [c_void_p] * 6 + [c_int] * 6 + [c_void_p]),
     "vrr_gemm": (c_int, [c_void_p] * 3 + [c_int] * 7 + [c_void_p]),

@@ -186,6 +186,33 @@ __device__ __forceinline__ float4 mul4_rn(float4 a, float4 f) {
   return make_float4(__fmul_rn(a.x, f.x), __fmul_rn(a.y, f.y), __fmul_rn(a.z, f.z), __fmul_rn(a.w, f.w));
 }
 
+// QK-norm (vrr_qkv_rope_norm_fwd / _bwd): the LayerNorm of one q or k head row of n = Dh channels, in fp32.
+//   mean = (sum x) / n, var = (sum (x - mean)^2) / n (biased), rstd = rsqrtf(var + eps); each sum runs in four
+//   interleaved partials (channel 4i + e adds into partial e), combined as (p0 + p1) + (p2 + p3).
+// xhat and y are formed without contraction: the backward recomputes the y the forward rotated, bit for bit.
+__device__ __forceinline__ float qk_norm_xhat(float x, float mean, float rstd) { return __fmul_rn(__fsub_rn(x, mean), rstd); }
+__device__ __forceinline__ float qk_norm_y(float xhat, float g, float b) { return __fmaf_rn(xhat, g, b); }
+__device__ __forceinline__ float2 qk_norm_stats(const float* x, int n, float eps) {
+  const float inv = 1.f / (float)n;  // n is a power of two: exact
+  float p[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+  for (int i = 0; i < n; i += 4)
+#pragma unroll
+    for (int e = 0; e < 4; ++e) p[e] = __fadd_rn(p[e], x[i + e]);
+  const float mean = __fmul_rn(__fadd_rn(__fadd_rn(p[0], p[1]), __fadd_rn(p[2], p[3])), inv);
+#pragma unroll
+  for (int e = 0; e < 4; ++e) p[e] = 0.f;
+#pragma unroll
+  for (int i = 0; i < n; i += 4)
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const float d = __fsub_rn(x[i + e], mean);
+      p[e] = __fmaf_rn(d, d, p[e]);
+    }
+  const float var = __fmul_rn(__fadd_rn(__fadd_rn(p[0], p[1]), __fadd_rn(p[2], p[3])), inv);
+  return make_float2(mean, rsqrtf(__fadd_rn(var, eps)));
+}
+
 // vrr_drop_desc -> DropView (validated); `*active` = false when the desc draws nothing (NULL, or both
 // probabilities 0): the caller then runs the plain kernels.
 int drop_view(const vrr_drop_desc* d, int M, int E, DropView* v, bool* active);

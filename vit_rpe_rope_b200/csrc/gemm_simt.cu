@@ -12,6 +12,7 @@
 #include <type_traits>
 
 #include "common.cuh"
+#include "kernels.h"
 
 namespace vrr {
 
@@ -112,6 +113,7 @@ struct AtomicEpilogue {  // split-K accumulation into a zeroed fp32 C
 
 template <typename T>
 struct QkvRopeEpilogue {
+  static constexpr bool kRowPrep = false;
   T* planes;
   const float *cos_tab, *sin_tab;
   int B, N, E, H, Dh, rope_mode;
@@ -129,6 +131,48 @@ struct QkvRopeEpilogue {
     Elem<T>::st(planes + ((((size_t)which * B + b) * H + h) * N + t) * Dh + d, v);
   }
 };
+
+// QkvRopeEpilogue with QK-norm (vrr_qkv_rope_norm_fwd).  prep() runs once per (row, head) of the staged tile before
+// the per-element pass: for a q / k head it rounds the Dh accumulators to T (x), saves x and {mean, rstd}, and
+// overwrites the staged row with y = xhat g + b, which the per-element pass then rotates and stores.
+template <typename T>
+struct QkvNormRopeEpilogue : QkvRopeEpilogue<T> {
+  static constexpr bool kRowPrep = true;
+  QkNormArgs qn;
+  __device__ __forceinline__ void prep(int m, int n, float* seg) const {
+    const int Dh = this->Dh, which = n / this->E;
+    if (which == 2) return;
+    const int h = (n - which * this->E) / Dh, b = m / this->N, t = m - b * this->N;
+    for (int j = 0; j < Dh; ++j) seg[j] = Elem<T>::round(seg[j]);
+    const float2 st = qk_norm_stats(seg, Dh, qn.eps);
+    const size_t row = (((size_t)which * this->B + b) * this->H + h) * this->N + t;
+    if (qn.qk_pre != nullptr) {
+      T* pre = (T*)qn.qk_pre + row * Dh;
+      for (int j = 0; j < Dh; ++j) Elem<T>::st(pre + j, seg[j]);
+      reinterpret_cast<float2*>(qn.qk_stats)[row] = st;
+    }
+    const float *g = which ? qn.kn_w : qn.qn_w, *bb = which ? qn.kn_b : qn.qn_b;
+    for (int j = 0; j < Dh; ++j) seg[j] = qk_norm_y(qk_norm_xhat(seg[j], st.x, st.y), g[j], bb[j]);
+  }
+};
+
+// Epilogues with kRowPrep: prep(m, n, row segment) once per (row, head) of the staged tile (COLS columns, 64 rows),
+// after the tile is in shared memory and before the per-element pass.
+template <class Epi, class = void>
+struct HasRowPrep { static constexpr bool value = false; };
+template <class Epi>
+struct HasRowPrep<Epi, std::void_t<decltype(Epi::kRowPrep)>> { static constexpr bool value = Epi::kRowPrep; };
+template <class Epi, int COLS>
+__device__ __forceinline__ void row_prep(const Epi& epi, float* Cs, int m0, int n0, int M, int N) {
+  if constexpr (HasRowPrep<Epi>::value) {
+    const int segs = COLS / epi.Dh;
+    for (int s = threadIdx.x; s < 64 * segs; s += GT) {
+      const int r = s / segs, c0 = (s - r * segs) * epi.Dh;
+      if (m0 + r < M && n0 + c0 < N) epi.prep(m0 + r, n0 + c0, Cs + r * (COLS + 1) + c0);
+    }
+    __syncthreads();
+  }
+}
 
 // T: element type of images / weight / bias (the conv arithmetic); TT: element type of the token
 // stream (prefix tokens, pos_embed, tokens).  Under autocast T = bf16 and TT = fp32, which reproduces
@@ -201,6 +245,7 @@ __global__ void __launch_bounds__(GT) gemm_simt_kernel(AOp A, BOp Bop, Epi epi, 
 #pragma unroll
     for (int j = 0; j < 4; ++j) Cs[(ty * 4 + i) * (BN + 1) + tx * 4 + j] = acc[i][j];
   __syncthreads();
+  row_prep<Epi, BN>(epi, Cs, m0, n0, M, N);
   for (int e = tid; e < BM * BN; e += GT) {
     const int r = e / BN, c = e - r * BN;
     if (m0 + r < M && n0 + c < N) epi(m0 + r, n0 + c, Cs[r * (BN + 1) + c], Cs + r * (BN + 1), n0);
@@ -344,6 +389,7 @@ __global__ void __launch_bounds__(GT, 2) gemm_simt128_kernel(AOp A, BOp Bop, Epi
 #pragma unroll
         for (int j = 0; j < 4; ++j) Cs[(ty * 4 + i) * (TNN + 1) + b * 64 + tx * 4 + j] = acc[a][b][i][j];
     __syncthreads();
+    row_prep<Epi, TNN>(epi, Cs, m0 + a * 64, n0, M, N);
     for (int e = tid; e < 64 * TNN; e += GT) {
       const int r = e / TNN, c = e - r * TNN;
       const int m = m0 + a * 64 + r;
@@ -388,9 +434,22 @@ static int qkv_rope_fwd_t(const void* x, const void* w, const float* cos_tab, co
   return launch_gemm<StridedOperand<T>, StridedOperand<T>, QkvRopeEpilogue<T>, true, true>(
       A, W, epi, B * N, 3 * E, E, 1, st);
 }
+template <typename T>
+static int qkv_rope_norm_fwd_t(const void* x, const void* w, const float* cos_tab, const float* sin_tab, void* planes, int B,
+                               int N, int E, int H, int npre, int rope_mode, const QkNormArgs& qn, cudaStream_t st) {
+  StridedOperand<T> A{(const T*)x, E, 1}, W{(const T*)w, E, 1};
+  QkvNormRopeEpilogue<T> epi{{(T*)planes, cos_tab, sin_tab, B, N, E, H, E / H, rope_mode, npre, N - npre}, qn};
+  return launch_gemm<StridedOperand<T>, StridedOperand<T>, QkvNormRopeEpilogue<T>, true, true>(A, W, epi, B * N, 3 * E, E, 1, st);
+}
 int qkv_rope_fwd_simt(const void* x, const void* w, const float* cos_tab, const float* sin_tab,
                       void* planes, int B, int N, int E, int H, int npre, int rope_mode, int dtype,
-                      cudaStream_t st) {
+                      cudaStream_t st, const QkNormArgs* qn) {
+  if (qn != nullptr) {
+    if (dtype == VRR_F32) return qkv_rope_norm_fwd_t<float>(x, w, cos_tab, sin_tab, planes, B, N, E, H, npre, rope_mode, *qn, st);
+    if (dtype == VRR_BF16)
+      return qkv_rope_norm_fwd_t<__nv_bfloat16>(x, w, cos_tab, sin_tab, planes, B, N, E, H, npre, rope_mode, *qn, st);
+    return qkv_rope_norm_fwd_t<__half>(x, w, cos_tab, sin_tab, planes, B, N, E, H, npre, rope_mode, *qn, st);
+  }
   if (dtype == VRR_F32) return qkv_rope_fwd_t<float>(x, w, cos_tab, sin_tab, planes, B, N, E, H, npre, rope_mode, st);
   if (dtype == VRR_BF16) return qkv_rope_fwd_t<__nv_bfloat16>(x, w, cos_tab, sin_tab, planes, B, N, E, H, npre, rope_mode, st);
   return qkv_rope_fwd_t<__half>(x, w, cos_tab, sin_tab, planes, B, N, E, H, npre, rope_mode, st);

@@ -108,7 +108,61 @@ struct QkvRopeEpi2 {
     const int which = n0 / E, h = (n0 - which * E) >> 6;
     return (which * B + b) * H + h;
   }
+  static constexpr bool kNorm = false;
 };
+
+// QkvRopeEpi2 with QK-norm (vrr_qkv_rope_norm_fwd).  Per q / k head chunk the kernel rounds the 64 accumulators to T
+// (x), stores x to qk_pre (the map tmap_c2, same plane index as planes: its planes are planes' first 2 B H) through the
+// staging slot before the final tile's, then normalize() writes {mean, rstd} and replaces x by y = xhat g + b; rotate()
+// and the plane store follow as without the norm.  qk_pre / qk_stats null: inference, nothing saved.
+template <typename T>
+struct QkvNormRopeEpi2 : QkvRopeEpi2<T> {
+  static constexpr bool kNorm = true;
+  T* qk_pre;         // [2][B][H][N][64]
+  float2* qk_stats;  // [2][B][H][N]
+  const float4 *qn_w, *qn_b, *kn_w, *kn_b;  // [64] each
+  float eps;
+  __device__ __forceinline__ void normalize(int m, int n0, bool store, float (&f)[64]) const {
+    const float2 st = qk_norm_stats(f, 64, eps);
+    if (store && qk_stats != nullptr) {
+      const int b = m / this->N, t = m - b * this->N;
+      qk_stats[(size_t)this->plane_of(b, n0) * this->N + t] = st;  // lanes = consecutive rows: coalesced
+    }
+    const bool k = n0 >= this->E;
+    const float4 *gw = k ? kn_w : qn_w, *gb = k ? kn_b : qn_b;  // warp-uniform: broadcast loads
+#pragma unroll
+    for (int q = 0; q < 16; ++q) {
+      const float4 g = __ldg(gw + q), bb = __ldg(gb + q);
+      f[4 * q + 0] = qk_norm_y(qk_norm_xhat(f[4 * q + 0], st.x, st.y), g.x, bb.x);
+      f[4 * q + 1] = qk_norm_y(qk_norm_xhat(f[4 * q + 1], st.x, st.y), g.y, bb.y);
+      f[4 * q + 2] = qk_norm_y(qk_norm_xhat(f[4 * q + 2], st.x, st.y), g.z, bb.z);
+      f[4 * q + 3] = qk_norm_y(qk_norm_xhat(f[4 * q + 3], st.x, st.y), g.w, bb.w);
+    }
+  }
+};
+
+// One row of 64 values as T: into the swizzled [32 rows][128 B] staging buffer at row_base (lane = row), or straight to
+// global memory.
+template <typename T>
+__device__ __forceinline__ void stage_row64(uint32_t row_base, uint32_t sw, const float (&f)[64]) {
+#pragma unroll
+  for (int c8 = 0; c8 < 8; ++c8)
+    st_shared_v4(row_base + (((uint32_t)c8 ^ sw) << 4), Elem16<T>::pack2(f[c8 * 8 + 0], f[c8 * 8 + 1]),
+                 Elem16<T>::pack2(f[c8 * 8 + 2], f[c8 * 8 + 3]), Elem16<T>::pack2(f[c8 * 8 + 4], f[c8 * 8 + 5]),
+                 Elem16<T>::pack2(f[c8 * 8 + 6], f[c8 * 8 + 7]));
+}
+template <typename T>
+__device__ __forceinline__ void store_row64(T* dst, const float (&f)[64]) {
+#pragma unroll
+  for (int v8 = 0; v8 < 8; ++v8) {
+    uint4 wv;
+    wv.x = Elem16<T>::pack2(f[v8 * 8 + 0], f[v8 * 8 + 1]);
+    wv.y = Elem16<T>::pack2(f[v8 * 8 + 2], f[v8 * 8 + 3]);
+    wv.z = Elem16<T>::pack2(f[v8 * 8 + 4], f[v8 * 8 + 5]);
+    wv.w = Elem16<T>::pack2(f[v8 * 8 + 6], f[v8 * 8 + 7]);
+    *reinterpret_cast<uint4*>(dst + v8 * 8) = wv;
+  }
+}
 
 // tokens[b][npre+p][n] = round_T(acc + bias[n]) (+ pos[p][n]); TT = token-stream type
 template <typename T, typename TT>
@@ -642,6 +696,39 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         const int n0 = n_blk * BN + chalf * (BN / 2) + c * 64;
         float(&f)[64] = *reinterpret_cast<float(*)[64]>(v);
         if constexpr (Epi::kPlaneStore) {
+          if constexpr (Epi::kNorm) {
+            if (n0 < 2 * epi.E) {  // a q or k head (warp-uniform)
+#pragma unroll
+              for (int i = 0; i < 64; ++i) f[i] = Elem16<T>::round(f[i]);
+              const int pb0 = m_warp0 / epi.N, pt0 = m_warp0 - pb0 * epi.N;
+              const bool p_in_range = m_warp0 < g.M;
+              if (epi.qk_pre != nullptr) {
+                // staged in any case; the warp tile that runs into the next image copies each lane's own row out of the
+                // staging buffer (row stores straight from the registers spilled at BN = 256)
+                const bool whole = pt0 + 32 <= epi.N || !p_in_range;
+                const uint32_t sw = (uint32_t)(lane & 7);
+                const uint32_t buf = (chunk_counter & 1u) * 4096u, row_base = stage_u32 + buf + (uint32_t)lane * 128u;
+                if (lane == 0) bulk_wait_read<1>();
+                __syncwarp();
+                stage_row64<T>(row_base, sw, f);
+                if (whole) {
+                  fence_proxy_async_smem();
+                  __syncwarp();
+                } else if (m < g.M) {
+                  const int b = m / epi.N, t = m - b * epi.N;
+                  uint4* dst = reinterpret_cast<uint4*>(epi.qk_pre + ((size_t)epi.plane_of(b, n0) * epi.N + t) * 64);
+#pragma unroll
+                  for (int c8 = 0; c8 < 8; ++c8) dst[c8] = ld_shared_v4(row_base + (((uint32_t)c8 ^ sw) << 4));
+                }
+                if (lane == 0) {
+                  if (whole && p_in_range) tma_store_3d(&tmap_c2, my_stage + buf, 0, pt0, epi.plane_of(pb0, n0));
+                  bulk_commit();  // a group in either case: the ring's bulk_wait_read<1> counts one per slot use
+                }
+                ++chunk_counter;
+              }
+              epi.normalize(m, n0, m < g.M, f);
+            }
+          }
           epi.rotate(m, n0, f);
           const int b0 = m_warp0 / epi.N, t0 = m_warp0 - b0 * epi.N;
           const bool in_range = n0 < g.N && m_warp0 < g.M;
@@ -650,13 +737,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
             const uint32_t buf = (chunk_counter & 1u) * 4096u;
             if (lane == 0) bulk_wait_read<1>();
             __syncwarp();
-            const uint32_t sw = (uint32_t)(lane & 7);
-            const uint32_t row_base = stage_u32 + buf + (uint32_t)lane * 128u;
-#pragma unroll
-            for (int c8 = 0; c8 < 8; ++c8)
-              st_shared_v4(row_base + (((uint32_t)c8 ^ sw) << 4), Elem16<T>::pack2(f[c8 * 8 + 0], f[c8 * 8 + 1]),
-                           Elem16<T>::pack2(f[c8 * 8 + 2], f[c8 * 8 + 3]), Elem16<T>::pack2(f[c8 * 8 + 4], f[c8 * 8 + 5]),
-                           Elem16<T>::pack2(f[c8 * 8 + 6], f[c8 * 8 + 7]));
+            stage_row64<T>(stage_u32 + buf + (uint32_t)lane * 128u, (uint32_t)(lane & 7), f);
             fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) {
@@ -668,16 +749,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
             // the rows run into the next image (one warp tile in N / 32; TMA stores take no negative coordinates -
             // "illegal instruction" - and a box cannot be shortened): each thread stores its own row
             const int b = m / epi.N, t = m - b * epi.N;
-            T* dst = epi.planes + ((size_t)epi.plane_of(b, n0) * epi.N + t) * 64;
-#pragma unroll
-            for (int v8 = 0; v8 < 8; ++v8) {
-              uint4 wv;
-              wv.x = Elem16<T>::pack2(f[v8 * 8 + 0], f[v8 * 8 + 1]);
-              wv.y = Elem16<T>::pack2(f[v8 * 8 + 2], f[v8 * 8 + 3]);
-              wv.z = Elem16<T>::pack2(f[v8 * 8 + 4], f[v8 * 8 + 5]);
-              wv.w = Elem16<T>::pack2(f[v8 * 8 + 6], f[v8 * 8 + 7]);
-              *reinterpret_cast<uint4*>(dst + v8 * 8) = wv;
-            }
+            store_row64<T>(epi.planes + ((size_t)epi.plane_of(b, n0) * epi.N + t) * 64, f);
           }
         } else if constexpr (!Epi::kTma) {
           if (m < g.M && n0 < g.N) epi(m, n0, f);
@@ -1200,14 +1272,44 @@ static int qkv_rope_fwd_tc2_t(const void* x, const void* w, const float* cos_tab
   return launch_pair<T, 128, false, false, QkvRopeEpi2<T>>(x, w, B * N, 3 * E, E, 1, tplanes, tplanes, epi, st);
 }
 
+template <typename T>
+static int qkv_rope_norm_fwd_tc2_t(const void* x, const void* w, const float* cos_tab, const float* sin_tab,
+                                   const float* packed, void* planes, int B, int N, int E, int H, int npre, int rope_mode,
+                                   const QkNormArgs& qn, cudaStream_t st) {
+  QkvNormRopeEpi2<T> epi{{(T*)planes, cos_tab, sin_tab, reinterpret_cast<const float4*>(packed), B, N, E, H, rope_mode, npre},
+                         (T*)qn.qk_pre, reinterpret_cast<float2*>(qn.qk_stats), reinterpret_cast<const float4*>(qn.qn_w),
+                         reinterpret_cast<const float4*>(qn.qn_b), reinterpret_cast<const float4*>(qn.kn_w),
+                         reinterpret_cast<const float4*>(qn.kn_b), qn.eps};
+  CUtensorMap tplanes, tpre;  // planes[3 B H][N][64] and qk_pre[2 B H][N][64] of T, box = [1][32 rows][64]
+  if (int rc = make_tmap_3d(&tplanes, planes, Elem16<T>::kTmap, 64, (uint64_t)N, (uint64_t)3 * B * H, 128, (uint64_t)N * 128,
+                            64, 32))
+    return rc;
+  tpre = tplanes;
+  if (qn.qk_pre != nullptr)
+    if (int rc = make_tmap_3d(&tpre, qn.qk_pre, Elem16<T>::kTmap, 64, (uint64_t)N, (uint64_t)2 * B * H, 128, (uint64_t)N * 128,
+                              64, 32))
+      return rc;
+  if (3 * E > 128) return launch_pair<T, 256, false, false, QkvNormRopeEpi2<T>>(x, w, B * N, 3 * E, E, 1, tplanes, tpre, epi, st);
+  return launch_pair<T, 128, false, false, QkvNormRopeEpi2<T>>(x, w, B * N, 3 * E, E, 1, tplanes, tpre, epi, st);
+}
+
 int qkv_rope_fwd_tc2(const void* x, const void* w, const float* cos_tab, const float* sin_tab, const float* packed,
-                     void* planes, int B, int N, int E, int H, int npre, int rope_mode, int dtype, cudaStream_t st) {
+                     void* planes, int B, int N, int E, int H, int npre, int rope_mode, int dtype, cudaStream_t st,
+                     const QkNormArgs* qn) {
   VRR_REQUIRE(((uintptr_t)x & 15) == 0 && ((uintptr_t)w & 15) == 0 && ((uintptr_t)planes & 15) == 0,
               VRR_ERR_INVALID_ARG, "qkv_rope_fwd (tcgen05): x / w / planes must be 16-byte aligned");
   if (rope_mode != VRR_ROPE_NONE)
     VRR_REQUIRE(((uintptr_t)cos_tab & 15) == 0 && ((uintptr_t)sin_tab & 15) == 0, VRR_ERR_INVALID_ARG,
                 "qkv_rope_fwd (tcgen05): cos / sin must be 16-byte aligned");
   VRR_REQUIRE(((uintptr_t)packed & 15) == 0, VRR_ERR_INVALID_ARG, "qkv_rope_fwd (tcgen05): packed table must be 16-byte aligned");
+  if (qn != nullptr) {
+    VRR_REQUIRE((((uintptr_t)qn->qn_w | (uintptr_t)qn->qn_b | (uintptr_t)qn->kn_w | (uintptr_t)qn->kn_b | (uintptr_t)qn->qk_pre) & 15) == 0 &&
+                    ((uintptr_t)qn->qk_stats & 7) == 0,
+                VRR_ERR_INVALID_ARG, "qkv_rope_norm_fwd (tcgen05): norm tensors and qk_pre must be 16-byte aligned, qk_stats 8");
+    if (dtype == VRR_F16)
+      return qkv_rope_norm_fwd_tc2_t<__half>(x, w, cos_tab, sin_tab, packed, planes, B, N, E, H, npre, rope_mode, *qn, st);
+    return qkv_rope_norm_fwd_tc2_t<__nv_bfloat16>(x, w, cos_tab, sin_tab, packed, planes, B, N, E, H, npre, rope_mode, *qn, st);
+  }
   if (dtype == VRR_F16) return qkv_rope_fwd_tc2_t<__half>(x, w, cos_tab, sin_tab, packed, planes, B, N, E, H, npre, rope_mode, st);
   return qkv_rope_fwd_tc2_t<__nv_bfloat16>(x, w, cos_tab, sin_tab, packed, planes, B, N, E, H, npre, rope_mode, st);
 }

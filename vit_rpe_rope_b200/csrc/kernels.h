@@ -42,13 +42,23 @@ void attn_bwd_ws_set_debug(long long* buf);
 int attn_bwd_ws(const void* planes, const void* out, const void* d_out, const float* lse, void* d_planes, int B, int H,
                 int N, int Dh, float scale, int dtype, cudaStream_t st);
 
+// QK-norm of the QKV+RoPE forward (vrr_qkv_rope_norm_fwd): fp32 [Dh] affine parameters of q_norm / k_norm, eps, and
+// the saved outputs qk_pre [2][B][H][N][Dh] (the compute type) and qk_stats [2][B][H][N][2] {mean, rstd}, or both NULL
+struct QkNormArgs {
+  const float *qn_w, *qn_b, *kn_w, *kn_b;
+  float eps;
+  void* qk_pre;
+  float* qk_stats;
+};
+
 // gemm_simt.cu
 void layernorm_set_option(int which, int value);  // 0: ln_reg, 1: ln_bwd_minb
 void gemm_simt_set_tile(int v);  // 128 (default): 128 x 128 double-buffered kernel for problems with a full tile; 64: 64 x 64 always
 // npre: prefix tokens per image (token rows 0..npre-1: cls, then registers); they are never rotated, and the patch
 // rows t >= npre use table row t - npre
 int qkv_rope_fwd_simt(const void* x, const void* w, const float* cos_tab, const float* sin_tab, void* planes,
-                      int B, int N, int E, int H, int npre, int rope_mode, int dtype, cudaStream_t st);
+                      int B, int N, int E, int H, int npre, int rope_mode, int dtype, cudaStream_t st,
+                      const QkNormArgs* qn = nullptr);
 int gemm_simt(const void* a, const void* b, void* c, int M, int N, int K, int ta, int tb, int dtype,
               int c_dtype, cudaStream_t st);
 int gemm_simt_bias(const void* a, const void* b, void* c, void* c2, const float* bias, int M, int N, int K, int ta, int tb,
@@ -83,7 +93,7 @@ int rope_pack_tables(const float* cos_tab, const float* sin_tab, float* packed, 
 bool qkv_rope_fwd_tc_supported(int B, int N, int E, int H);
 // `packed`: optional output of rope_pack_tables for the same tables (NULL: the epilogue reads cos_tab / sin_tab)
 int qkv_rope_fwd_tc2(const void* x, const void* w, const float* cos_tab, const float* sin_tab, const float* packed, void* planes, int B, int N,
-                     int E, int H, int npre, int rope_mode, int dtype, cudaStream_t st);
+                     int E, int H, int npre, int rope_mode, int dtype, cudaStream_t st, const QkNormArgs* qn = nullptr);
 
 bool patch_embed_tc_supported(int B, int C, int Hi, int Wi, int P, int E);
 size_t patch_embed_tc_workspace_bytes(int B, int C, int Hi, int Wi, int P);
@@ -123,6 +133,14 @@ int dropout_mask(const DropView& dv, uint8_t* keep, uint8_t* keep_path, int M, i
 int qkv_rope_bwd(const void* d_planes, const void* planes, const float* cos_tab, const float* sin_tab,
                  void* d_qkv, float* d_cos, float* d_sin, int B, int N, int E, int H, int npre, int rope_mode, int dtype,
                  cudaStream_t st);
+// QK-norm backward (vrr_qkv_rope_norm_bwd): qn->qk_pre / qk_stats are the forward's saved outputs; d_w / d_b
+// [q, k] are written (zeroed here, atomically reduced), or all NULL
+struct QkNormGrads {
+  float *d_qn_w, *d_qn_b, *d_kn_w, *d_kn_b;
+};
+int qkv_rope_norm_bwd(const void* d_planes, const QkNormArgs& qn, const float* cos_tab, const float* sin_tab, void* d_qkv,
+                      float* d_cos, float* d_sin, const QkNormGrads& grads, int B, int N, int E, int H, int npre,
+                      int rope_mode, int dtype, cudaStream_t st);
 int rope_apply(const void* q_in, const void* k_in, const float* cos_tab, const float* sin_tab, void* q_out,
                void* k_out, int B, int H, int Nr, int Dh, int rope_mode, int inverse, int dtype, cudaStream_t st);
 

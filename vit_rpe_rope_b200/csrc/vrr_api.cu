@@ -341,6 +341,65 @@ int vrr_qkv_rope_bwd_prefix(const void* d_planes, const void* planes, const floa
                       (cudaStream_t)stream);
 }
 
+int vrr_qkv_rope_norm_fwd(const void* x, const void* w_qkv, const float* cos_tab, const float* sin_tab, const float* packed,
+                          void* planes, int B, int N, int E, int H, int n_prefix, int rope_mode, int dtype, const float* qn_w,
+                          const float* qn_b, const float* kn_w, const float* kn_b, float eps, void* qk_pre, float* qk_stats,
+                          void* stream) {
+  VRR_REQUIRE(x && w_qkv && planes, VRR_ERR_INVALID_ARG, "qkv_rope_norm_fwd: NULL pointer");
+  VRR_REQUIRE(qn_w && qn_b && kn_w && kn_b, VRR_ERR_INVALID_ARG, "qkv_rope_norm_fwd: q_norm / k_norm weight and bias are required");
+  VRR_REQUIRE((qk_pre == nullptr) == (qk_stats == nullptr), VRR_ERR_INVALID_ARG,
+              "qkv_rope_norm_fwd: qk_pre and qk_stats must both be given or both NULL");
+  VRR_REQUIRE(eps >= 0.f, VRR_ERR_INVALID_ARG, "qkv_rope_norm_fwd: eps must be >= 0");
+  VRR_REQUIRE(dtype_ok(dtype), VRR_ERR_INVALID_ARG, "qkv_rope_norm_fwd: bad dtype %d", dtype);
+  VRR_REQUIRE(rope_mode >= VRR_ROPE_NONE && rope_mode <= VRR_ROPE_MIXED, VRR_ERR_INVALID_ARG,
+              "qkv_rope_norm_fwd: bad rope_mode %d", rope_mode);
+  VRR_REQUIRE(rope_mode == VRR_ROPE_NONE || (cos_tab && sin_tab), VRR_ERR_INVALID_ARG,
+              "qkv_rope_norm_fwd: cos/sin required for rope_mode %d", rope_mode);
+  VRR_REQUIRE(B > 0 && N > 0 && H > 0 && E > 0 && E % H == 0, VRR_ERR_INVALID_ARG, "qkv_rope_norm_fwd: bad sizes");
+  VRR_REQUIRE(n_prefix >= 1 && n_prefix <= N, VRR_ERR_INVALID_ARG,
+              "qkv_rope_norm_fwd: n_prefix %d must lie in [1, N = %d]", n_prefix, N);
+  VRR_REQUIRE(dh_ok(E / H), VRR_ERR_UNSUPPORTED, "qkv_rope_norm_fwd: head dim %d unsupported (16, 32, 64)", E / H);
+  if (int rc = require_device()) return rc;
+  const QkNormArgs qn = {qn_w, qn_b, kn_w, kn_b, eps, qk_pre, qk_stats};
+  const int impl = g_impl.load();
+  if (is16(dtype) && impl != VRR_IMPL_SIMT && qkv_rope_fwd_tc_supported(B, N, E, H)) {
+    VRR_COUNT_FAMILY(VRR_IMPL_TCGEN05);
+    return qkv_rope_fwd_tc2(x, w_qkv, cos_tab, sin_tab, packed, planes, B, N, E, H, n_prefix, rope_mode, dtype,
+                            (cudaStream_t)stream, &qn);
+  }
+  VRR_REQUIRE(impl != VRR_IMPL_TCGEN05, VRR_ERR_UNSUPPORTED,
+              "qkv_rope_norm_fwd: tcgen05 kernel forced but shape/dtype unsupported (bf16 or fp16, Dh=64, E%%64==0)");
+  VRR_COUNT_FAMILY(VRR_IMPL_SIMT);
+  return qkv_rope_fwd_simt(x, w_qkv, cos_tab, sin_tab, planes, B, N, E, H, n_prefix, rope_mode, dtype, (cudaStream_t)stream,
+                           &qn);
+}
+
+int vrr_qkv_rope_norm_bwd(const void* d_planes, const void* qk_pre, const float* qk_stats, const float* cos_tab,
+                          const float* sin_tab, const float* qn_w, const float* qn_b, const float* kn_w, const float* kn_b,
+                          void* d_qkv, float* d_cos, float* d_sin, float* d_qn_w, float* d_qn_b, float* d_kn_w,
+                          float* d_kn_b, int B, int N, int E, int H, int n_prefix, int rope_mode, int dtype, void* stream) {
+  VRR_REQUIRE(d_planes && qk_pre && qk_stats && d_qkv, VRR_ERR_INVALID_ARG, "qkv_rope_norm_bwd: NULL pointer");
+  VRR_REQUIRE(qn_w && qn_b && kn_w && kn_b, VRR_ERR_INVALID_ARG, "qkv_rope_norm_bwd: q_norm / k_norm weight and bias are required");
+  VRR_REQUIRE((d_cos == nullptr) == (d_sin == nullptr), VRR_ERR_INVALID_ARG,
+              "qkv_rope_norm_bwd: d_cos and d_sin must both be given or both NULL");
+  const int n_grads = (d_qn_w != nullptr) + (d_qn_b != nullptr) + (d_kn_w != nullptr) + (d_kn_b != nullptr);
+  VRR_REQUIRE(n_grads == 0 || n_grads == 4, VRR_ERR_INVALID_ARG,
+              "qkv_rope_norm_bwd: d_qn_w, d_qn_b, d_kn_w and d_kn_b must all be given or all NULL");
+  VRR_REQUIRE(dtype_ok(dtype), VRR_ERR_INVALID_ARG, "qkv_rope_norm_bwd: bad dtype %d", dtype);
+  VRR_REQUIRE(rope_mode >= VRR_ROPE_NONE && rope_mode <= VRR_ROPE_MIXED, VRR_ERR_INVALID_ARG,
+              "qkv_rope_norm_bwd: bad rope_mode %d", rope_mode);
+  VRR_REQUIRE(rope_mode == VRR_ROPE_NONE || (cos_tab && sin_tab), VRR_ERR_INVALID_ARG, "qkv_rope_norm_bwd: cos/sin required");
+  VRR_REQUIRE(B > 0 && N > 0 && H > 0 && E > 0 && E % H == 0 && dh_ok(E / H), VRR_ERR_INVALID_ARG,
+              "qkv_rope_norm_bwd: bad sizes");
+  VRR_REQUIRE(n_prefix >= 1 && n_prefix <= N, VRR_ERR_INVALID_ARG,
+              "qkv_rope_norm_bwd: n_prefix %d must lie in [1, N = %d]", n_prefix, N);
+  if (int rc = require_device()) return rc;
+  const QkNormArgs qn = {qn_w, qn_b, kn_w, kn_b, 0.f, const_cast<void*>(qk_pre), const_cast<float*>(qk_stats)};
+  const QkNormGrads gr = {d_qn_w, d_qn_b, d_kn_w, d_kn_b};
+  return qkv_rope_norm_bwd(d_planes, qn, cos_tab, sin_tab, d_qkv, d_cos, d_sin, gr, B, N, E, H, n_prefix, rope_mode, dtype,
+                           (cudaStream_t)stream);
+}
+
 int vrr_rope_apply(const void* q_in, const void* k_in, const float* cos_tab, const float* sin_tab, void* q_out,
                    void* k_out, int B, int H, int Nr, int Dh, int rope_mode, int inverse, int dtype,
                    void* stream) {

@@ -31,6 +31,10 @@ SwiGLU MLP (``VisionTransformer(mlp_layer=SwiGLUPacked)``, timm's ``GluMlp`` / `
 ``fc2(silu(x W_g + b_g) * (x W_v + b_v))`` with the gate and value rows packed in ``fc1``.  fc1's GEMM pairs each gate
 column with its value column and applies SiLU, the product and drop1 in its epilogue; fc2's dX GEMM applies the
 backward.
+
+QK-norm (``VisionTransformer(qk_norm=True)``, timm's name; ViT-22B): a LayerNorm over each head's channels of q and
+of k before RoPE, against attention-logit growth in low-precision training.  The QKV GEMM's epilogue normalises and
+then rotates; the RoPE backward kernel takes the LayerNorm backward and the q_norm / k_norm gradients.
 """
 import functools
 
@@ -170,9 +174,13 @@ def _is_glu_factory(layer):
 
 
 class Attention(nn.Module):
-    """Multi-head self-attention (reference vit.py:14-98) on the fused kernels."""
+    """Multi-head self-attention (reference vit.py:14-98) on the fused kernels.  ``qk_norm`` (timm's name) adds
+    ``q_norm`` / ``k_norm = norm_layer(head_dim)``, applied to every q / k head row before RoPE inside the QKV GEMM's
+    epilogue; the kernel implements an affine ``nn.LayerNorm``, so any other ``norm_layer`` raises
+    NotImplementedError.  Without it both are ``nn.Identity``."""
 
-    def __init__(self, dim, num_heads=8, qkv_bias=False, attn_drop=0., proj_drop=0.):
+    def __init__(self, dim, num_heads=8, qkv_bias=False, attn_drop=0., proj_drop=0., qk_norm=False,
+                 norm_layer=nn.LayerNorm):
         super().__init__()
         if qkv_bias:
             raise NotImplementedError("qkv_bias=True is never used by the reference (vit.py:110,200) and the "
@@ -184,6 +192,10 @@ class Attention(nn.Module):
         self.head_dim = dim // num_heads
         self.scale = self.head_dim ** -0.5
         self.qkv = nn.Linear(dim, dim * 3, bias=qkv_bias)
+        self.q_norm = norm_layer(self.head_dim) if qk_norm else nn.Identity()
+        self.k_norm = norm_layer(self.head_dim) if qk_norm else nn.Identity()
+        if qk_norm:
+            ops.check_qk_norm(self.q_norm, self.k_norm, self.head_dim)
         self.attn_drop = nn.Dropout(attn_drop)
         self.proj = nn.Linear(dim, dim)
         self.proj_drop = nn.Dropout(proj_drop)
@@ -205,8 +217,10 @@ class Attention(nn.Module):
         elif isinstance(pe, PolynomialRPE):
             bias_mode, bias_param, bias_grid = _lib.BIAS_POLY, pe.coefficients, pe.grid_size
         dt = ops.compute_dtype(x)
+        qk = (None, None) if type(self.q_norm) is nn.Identity and type(self.k_norm) is nn.Identity else (self.q_norm,
+                                                                                                      self.k_norm)
         planes = ops.qkv_rope(x, self.qkv.weight, cos, sin, self.num_heads, ops.lp_weight(self.qkv.weight, dt),
-                              self.num_prefix_tokens)
+                              self.num_prefix_tokens, *qk)
         out = ops.fused_attention(planes, self.scale, bias_mode, bias_param, bias_grid)
         return ops.linear(out, self.proj, ops.lp_weight(self.proj.weight, dt))
 
@@ -217,15 +231,18 @@ class Attention(nn.Module):
 class Block(nn.Module):
     """Pre-LN transformer block (reference vit.py:100-129); ``init_values`` adds timm's LayerScale ``ls1`` / ``ls2``
     (None or 0: none, the reference's block).  ``mlp_layer``: ``Mlp`` (default) or a ``GluMlp`` factory such as
-    ``SwiGLUPacked``, built with ``hidden_features = int(dim * mlp_ratio)`` (fc1's width) as timm does."""
+    ``SwiGLUPacked``, built with ``hidden_features = int(dim * mlp_ratio)`` (fc1's width) as timm does.  ``qk_norm``:
+    QK-norm in the attention, with this block's ``norm_layer``."""
 
     def __init__(self, dim, num_heads, mlp_ratio=4., qkv_bias=False, drop=0., attn_drop=0.,
-                 drop_path=0., act_layer=nn.GELU, norm_layer=nn.LayerNorm, init_values=None, mlp_layer=Mlp):
+                 drop_path=0., act_layer=nn.GELU, norm_layer=nn.LayerNorm, init_values=None, mlp_layer=Mlp,
+                 qk_norm=False):
         super().__init__()
         if mlp_layer is not Mlp and not _is_glu_factory(mlp_layer):
             raise ValueError(f"mlp_layer must be Mlp or a GluMlp factory (e.g. SwiGLUPacked), got {mlp_layer!r}")
         self.norm1 = norm_layer(dim)
-        self.attn = Attention(dim, num_heads=num_heads, qkv_bias=qkv_bias, attn_drop=attn_drop, proj_drop=drop)
+        self.attn = Attention(dim, num_heads=num_heads, qkv_bias=qkv_bias, attn_drop=attn_drop, proj_drop=drop,
+                              qk_norm=qk_norm, norm_layer=norm_layer)
         self.ls1 = LayerScale(dim, init_values) if init_values else nn.Identity()
         self.drop_path = DropPath(drop_path) if drop_path > 0. else nn.Identity()
         self.norm2 = norm_layer(dim)
@@ -262,13 +279,16 @@ class VisionTransformer(nn.Module):
 
     ``mlp_layer`` is every block's MLP: ``Mlp`` (default) or a ``GluMlp`` factory; ``SwiGLUPacked`` with
     ``mlp_ratio = 16 / 3`` matches the GELU MLP's parameters and FLOPs (fc1 ``E -> 2H``, fc2 ``H -> E``).
+
+    ``qk_norm`` gives every attention QK-norm (``blocks.{i}.attn.q_norm`` / ``k_norm``, ``nn.LayerNorm(head_dim)``
+    initialised to ones / zeros; no random numbers are drawn).
     """
 
     def __init__(self, img_size=32, patch_size=4, in_chans=3, num_classes=10,
                  embed_dim=192, depth=6, num_heads=6, mlp_ratio=4.,
                  pos_encoding='absolute', rope_theta=100.0,
                  poly_degree=3, poly_shared_heads=True, drop_rate=0., drop_path_rate=0., reg_tokens=0,
-                 init_values=None, mlp_layer=Mlp):
+                 init_values=None, mlp_layer=Mlp, qk_norm=False):
         super().__init__()
         if mlp_layer is not Mlp and not _is_glu_factory(mlp_layer):
             raise ValueError(f"mlp_layer must be Mlp or a GluMlp factory (e.g. SwiGLUPacked), got {mlp_layer!r}")
@@ -311,7 +331,8 @@ class VisionTransformer(nn.Module):
 
         dpr = [r.item() for r in torch.linspace(0, drop_path_rate, depth)]  # draws no random numbers
         self.blocks = nn.ModuleList([Block(embed_dim, num_heads, mlp_ratio, drop=drop_rate, drop_path=dpr[i],
-                                           init_values=init_values, mlp_layer=mlp_layer) for i in range(depth)])
+                                           init_values=init_values, mlp_layer=mlp_layer, qk_norm=qk_norm)
+                                     for i in range(depth)])
         if not self.use_pos_embed_in_forward:
             for blk in self.blocks:
                 blk.set_pos_encoding(self.pos_embed)  # one shared module, referenced by every block

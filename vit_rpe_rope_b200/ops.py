@@ -260,14 +260,17 @@ def _packed_tables(cos32, sin32):
 
 
 class QkvRopeFn(torch.autograd.Function):
-    """planes[3, B, H, N, Dh] = split_heads(x @ w_qkv^T), q/k rows n_prefix.. rotated in the GEMM epilogue."""
+    """planes[3, B, H, N, Dh] = split_heads(x @ w_qkv^T), q/k rows n_prefix.. rotated in the GEMM epilogue; with QK-norm
+    (``qn_w`` .. ``kn_b`` given) every q / k head row is layer-normalised first (``vrr_qkv_rope_norm_fwd``)."""
 
     @staticmethod
-    def forward(ctx, x, w_qkv, cos, sin, num_heads, w_lp=None, n_prefix=1):
+    def forward(ctx, x, w_qkv, cos, sin, num_heads, w_lp=None, n_prefix=1, qn_w=None, qn_b=None, kn_w=None, kn_b=None,
+                eps=1e-5):
         """``w_qkv`` receives the gradient (fp32 master weight or a tensor already in x's dtype); ``w_lp`` is an
         optional ready-made copy of it in x's dtype (the model's 16-bit weight cache).  ``n_prefix``: the leading
-        token rows that are never rotated (cls and register tokens); row t >= n_prefix uses table row t - n_prefix."""
-        _require_cuda(x, w_qkv, cos, sin)
+        token rows that are never rotated (cls and register tokens); row t >= n_prefix uses table row t - n_prefix.
+        ``qn_w, qn_b, kn_w, kn_b``: the [Dh] weight and bias of q_norm / k_norm (all four or none), with ``eps``."""
+        _require_cuda(x, w_qkv, cos, sin, qn_w, qn_b, kn_w, kn_b)
         lib = _lib.load()
         B, N, E = x.shape
         H, Dh = num_heads, E // num_heads
@@ -277,22 +280,41 @@ class QkvRopeFn(torch.autograd.Function):
         ctx.w_grad_dtype = w_qkv.dtype
         cos32, sin32 = _f32c(cos), _f32c(sin)
         planes = torch.empty(3, B, H, N, Dh, device=x.device, dtype=x.dtype)
+        norm = qn_w is not None
         with torch.cuda.device(x.device):
             packed = None
             if mode != _lib.ROPE_NONE and x.dtype in _LP16 and Dh == 64:  # the tcgen05 epilogue's table layout
                 packed = _packed_tables(cos32, sin32)
+            if not norm:
+                with _timed("qkv_rope_fwd"):
+                    _lib.check(lib.vrr_qkv_rope_fwd_prefix(_ptr(x), _ptr(w), _ptr(cos32), _ptr(sin32), _ptr(packed),
+                                                           _ptr(planes), B, N, E, H, n_prefix, mode, _DT[x.dtype], _stream()),
+                               "vrr_qkv_rope_fwd_prefix")
+                ctx.save_for_backward(x, w, planes, cos32, sin32)
+                ctx.meta = (B, N, E, H, n_prefix, mode, None if cos is None else (cos.dtype, sin.dtype))
+                ctx.norm = None
+                return planes
+            nt = [_f32c(t) for t in (qn_w, qn_b, kn_w, kn_b)]
+            grad = any(ctx.needs_input_grad)
+            qk_pre = torch.empty(2, B, H, N, Dh, device=x.device, dtype=x.dtype) if grad else None  # inference: no saves
+            qk_stats = torch.empty(2, B, H, N, 2, device=x.device, dtype=torch.float32) if grad else None
             with _timed("qkv_rope_fwd"):
-                _lib.check(lib.vrr_qkv_rope_fwd_prefix(_ptr(x), _ptr(w), _ptr(cos32), _ptr(sin32), _ptr(packed), _ptr(planes),
-                                                       B, N, E, H, n_prefix, mode, _DT[x.dtype], _stream()),
-                           "vrr_qkv_rope_fwd_prefix")
-        ctx.save_for_backward(x, w, planes, cos32, sin32)
-        ctx.meta = (B, N, E, H, n_prefix, mode, None if cos is None else (cos.dtype, sin.dtype))
+                _lib.check(lib.vrr_qkv_rope_norm_fwd(_ptr(x), _ptr(w), _ptr(cos32), _ptr(sin32), _ptr(packed), _ptr(planes),
+                                                     B, N, E, H, n_prefix, mode, _DT[x.dtype], *map(_ptr, nt), float(eps),
+                                                     _ptr(qk_pre), _ptr(qk_stats), _stream()), "vrr_qkv_rope_norm_fwd")
+        if grad:
+            ctx.save_for_backward(x, w, qk_pre, qk_stats, cos32, sin32, *nt)
+            ctx.meta = (B, N, E, H, n_prefix, mode, None if cos is None else (cos.dtype, sin.dtype))
+            ctx.norm = tuple(t.dtype for t in (qn_w, qn_b, kn_w, kn_b))
         return planes
 
     @staticmethod
     def backward(ctx, d_planes):
         lib = _lib.load()
-        x, w, planes, cos32, sin32 = ctx.saved_tensors
+        if ctx.norm is None:
+            x, w, planes, cos32, sin32 = ctx.saved_tensors
+        else:
+            x, w, qk_pre, qk_stats, cos32, sin32, *nt = ctx.saved_tensors
         B, N, E, H, n_prefix, mode, cs_dtypes = ctx.meta
         d_planes = d_planes.contiguous()
         dev, dt = x.device, x.dtype
@@ -302,10 +324,22 @@ class QkvRopeFn(torch.autograd.Function):
             d_cs = torch.empty((2,) + tuple(cos32.shape), device=dev, dtype=torch.float32)
             d_cos, d_sin = d_cs[0], d_cs[1]
         d_qkv = torch.empty(B * N, 3 * E, device=dev, dtype=dt)
+        d_norm = [None] * 4
         with torch.cuda.device(dev):
-            _lib.check(lib.vrr_qkv_rope_bwd_prefix(_ptr(d_planes), _ptr(planes), _ptr(cos32), _ptr(sin32), _ptr(d_qkv),
-                                                   _ptr(d_cos), _ptr(d_sin), B, N, E, H, n_prefix, mode, _DT[dt], _stream()),
-                       "vrr_qkv_rope_bwd_prefix")
+            if ctx.norm is None:
+                with _timed("qkv_rope_bwd"):
+                    _lib.check(lib.vrr_qkv_rope_bwd_prefix(_ptr(d_planes), _ptr(planes), _ptr(cos32), _ptr(sin32),
+                                                           _ptr(d_qkv), _ptr(d_cos), _ptr(d_sin), B, N, E, H, n_prefix, mode,
+                                                           _DT[dt], _stream()), "vrr_qkv_rope_bwd_prefix")
+            else:
+                if any(ctx.needs_input_grad[7:11]):  # rows of one buffer: zeroed by one memset
+                    d_norm = list(torch.empty(4, E // H, device=dev, dtype=torch.float32))
+                with _timed("qkv_rope_bwd"):
+                    _lib.check(lib.vrr_qkv_rope_norm_bwd(_ptr(d_planes), _ptr(qk_pre), _ptr(qk_stats), _ptr(cos32),
+                                                         _ptr(sin32), *map(_ptr, nt), _ptr(d_qkv), _ptr(d_cos), _ptr(d_sin),
+                                                         *map(_ptr, d_norm), B, N, E, H, n_prefix, mode, _DT[dt],
+                                                         _stream()), "vrr_qkv_rope_norm_bwd")
+                d_norm = [None if g is None else g.to(t) for g, t in zip(d_norm, ctx.norm)]
             dx = dw = None
             if ctx.needs_input_grad[0]:
                 dx = _gemm(d_qkv, w, False, False, dt, name="qkv_dx").view(B, N, E)            # [BN,3E] . [3E,E]
@@ -313,7 +347,7 @@ class QkvRopeFn(torch.autograd.Function):
                 dw = _gemm(d_qkv, x.view(B * N, E), True, False, ctx.w_grad_dtype, name="qkv_dw")  # [3E,BN] . [BN,E]
         if need_cs:
             d_cos, d_sin = d_cos.to(cs_dtypes[0]), d_sin.to(cs_dtypes[1])
-        return dx, dw, d_cos, d_sin, None, None, None
+        return (dx, dw, d_cos, d_sin, None, None, None, *d_norm, None)
 
 
 def _gemm(a, b, trans_a, trans_b, out_dtype, bias=None, epilogue=_lib.EPI_NONE, out2=False, name="gemm", aux=None,
@@ -346,12 +380,29 @@ def _gemm(a, b, trans_a, trans_b, out_dtype, bias=None, epilogue=_lib.EPI_NONE, 
     return (c, c2) if out2 else c
 
 
-def qkv_rope(x, w_qkv, cos, sin, num_heads, w_lp=None, n_prefix=1):
-    """``n_prefix``: the leading token rows that RoPE leaves alone (the cls token and any register tokens)."""
+def qkv_rope(x, w_qkv, cos, sin, num_heads, w_lp=None, n_prefix=1, q_norm=None, k_norm=None):
+    """``n_prefix``: the leading token rows that RoPE leaves alone (the cls token and any register tokens).
+    ``q_norm`` / ``k_norm``: QK-norm, two affine ``nn.LayerNorm((Dh,))`` with one eps (:func:`check_qk_norm`), or None."""
     dt = compute_dtype(x)
     if w_lp is not None and w_lp.dtype != dt:
         w_lp = None
-    return QkvRopeFn.apply(x.to(dt), w_qkv, cos, sin, num_heads, w_lp, n_prefix)
+    if q_norm is None and k_norm is None:
+        return QkvRopeFn.apply(x.to(dt), w_qkv, cos, sin, num_heads, w_lp, n_prefix)
+    check_qk_norm(q_norm, k_norm, x.shape[-1] // num_heads)
+    return QkvRopeFn.apply(x.to(dt), w_qkv, cos, sin, num_heads, w_lp, n_prefix, q_norm.weight, q_norm.bias, k_norm.weight,
+                           k_norm.bias, q_norm.eps)
+
+
+def check_qk_norm(q_norm, k_norm, head_dim):
+    """The QK-norm the fused QKV kernels implement: q_norm and k_norm are affine ``nn.LayerNorm((head_dim,))`` with a
+    bias and the same eps.  Anything else (an RMSNorm, a LayerNorm without affine or bias) raises NotImplementedError."""
+    for name, m in (("q_norm", q_norm), ("k_norm", k_norm)):
+        if not (type(m) is torch.nn.LayerNorm and m.elementwise_affine and m.bias is not None
+                and tuple(m.normalized_shape) == (head_dim,)):
+            raise NotImplementedError(f"qk_norm: {name} is {m!r}; the fused QKV+RoPE kernel implements an affine "
+                                      f"nn.LayerNorm(({head_dim},)) with weight and bias only")
+    if q_norm.eps != k_norm.eps:
+        raise NotImplementedError(f"qk_norm: q_norm.eps {q_norm.eps} != k_norm.eps {k_norm.eps}; the fused kernel takes one eps")
 
 
 # ------------------------------------------------------------------------------------------------
